@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...     # the reference's own CPU implementation on the host cores
+    python bench.py ... --dump-outputs DIR   # also write the arrays of the last timed step as DIR/<name>.npy
 
 A "step" = one compute_and_apply_rhs over every element this job holds. Workload = BASELINE configs[3]:
 ne=120 cubed sphere (86400 elements), np=4, nlev=72, FP64 — per GPU (weak scaling: the element loop has no
@@ -32,6 +33,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree (which may be read-only)
 
 METRIC = "compute_and_apply_rhs_elem_lev_updates_per_s"
 UNIT = "elem*lev updates/s"
@@ -320,6 +322,34 @@ def max_pointwise_rel_err(got, want, names):
     return worst, where
 
 
+DUMP_BYTES = 64_000_000
+DUMP_SEED = 20261020
+
+
+def dump_elements(E, L):
+    """The elements --dump-outputs writes: all E when the seven mutated arrays of all of them fit DUMP_BYTES, else a
+    sample drawn with a fixed seed, in index order. Depends on (E, L) only, so two runs with the same arguments dump
+    the same elements."""
+    from tinman_sandbox_b200 import MUTATED_FIELDS, field_shape
+    per_elem = 8 * sum(int(np.prod(field_shape(n, 1, L))) for n in MUTATED_FIELDS)
+    n = (DUMP_BYTES - 4096) // per_elem                 # 4096: room for the .npy headers
+    if E <= n:
+        return np.arange(E)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(E, size=n, replace=False))
+
+
+def dump_outputs(h, E, L, out_dir):
+    """DIR/<name>.npy (float64) for each array the routine mutates, every time level, as a caller downloading from the
+    handle receives them, restricted to dump_elements(E, L)."""
+    from tinman_sandbox_b200 import MUTATED_FIELDS
+    elems = dump_elements(E, L)
+    runs = np.split(elems, np.flatnonzero(np.diff(elems) != 1) + 1)     # contiguous runs: one download each
+    parts = [h.download_range(int(r[0]), int(r[-1]) + 1, names=MUTATED_FIELDS) for r in runs]
+    os.makedirs(out_dir, exist_ok=True)
+    for n in MUTATED_FIELDS:
+        np.save(os.path.join(out_dir, n + ".npy"), np.concatenate([p[n] for p in parts]))
+
+
 def link_probe(dev, h2d_bytes, d2h_bytes, total=1 << 29, sync=None):
     """What this GPU's host link does right now, in this process (pinned buffers, two streams, best of 4): host->device
     alone, device->host alone, both at once with equal sizes (duplex), and both at once IN THE PROPORTION OF ONE e2e
@@ -383,7 +413,14 @@ def main():
     ap.add_argument("--no-clock-topup", action="store_true",
                     help="do not continue the kernel loop after a short timed region to collect 5 clock samples (keeps the "
                          "number of calls, hence the accumulators and their checksums, deterministic)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the arrays the routine mutates, as they stand after the last timed "
+                         "step, to DIR/<name>.npy (float64, rank 0's slice; a fixed sample of elements when the slice "
+                         f"would take more than {DUMP_BYTES // 10**6} MB). Inputs depend only on the arguments, so runs "
+                         "of two builds can be compared array by array")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = max(args.warmup, 1)
 
@@ -476,6 +513,8 @@ def main():
     barrier()
     launches = h.launch_count() - launches0
     calls_done = args.warmup + 2 + args.steps
+    if args.dump_outputs and rank == 0:       # before anything below runs more calls
+        dump_outputs(h, E, L, args.dump_outputs)
     # A timed region shorter than ~5 NVML samples (small or strong-scaled slices): keep the SAME load running, outside
     # the timed region, until the sampler has at least 5 — and say so; never print a clocks record with fewer.
     if sampler and sampler.count_since_mark() < 5 and not args.no_clock_topup:

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""tests/golden/make_golden.py — regenerates the committed golden fixtures. Runs only where
-/root/reference exists (the build container); the fixtures it writes travel with the repo.
+"""tests/golden/make_golden.py — regenerates the committed golden fixtures. All but the last need the
+reference's sources (REF below); the fixtures it writes travel with the repo.
 
   fortran_golden.npz        Ttest / v1test / v2test, the reference's own known-answer vectors
                             (compute_and_apply_rhs_test/fortran/test_mod.F90:8-296, 299-591, 594-886):
@@ -14,7 +14,13 @@
   ref_outputs_E3.npz        every array the reference routine mutates, for 3 elements of the closed-form
                             init after 1 and after 2 calls (oracle/_ref/libcaar_ref_L72.so), so the GPU
                             tests can check against the REAL reference even if oracle/_ref is absent.
+  full_size_digests.json    `make_golden.py --full-size`: sha256 of every mutated array of every window of
+                            test_parity_gpu.py::test_full_size_runs_against_the_compiled_reference after 2
+                            calls, computed by the CPU restatement (oracle/caar_oracle.c, bit-identical to the
+                            reference: tests/test_oracle.py), plus a digest of the inputs. Needs no reference
+                            checkout; the closed-form elements 0-2 are checked against ref_outputs_E3.npz first.
 """
+import json
 import os
 import re
 import subprocess
@@ -64,5 +70,31 @@ def main():
     print("wrote", os.listdir(HERE))
 
 
+def full_size_digests():
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import test_parity_gpu as T
+    from oracle import harness
+    orc = harness.PortOracle()
+    ref = np.load(os.path.join(HERE, "ref_outputs_E3.npz"))
+    out = {}
+    for E, L in ((86400, 72), (49152, 128)):
+        _, wins, states = T.full_size_inputs(E, L)
+        entry = {"inputs": T.inputs_digest(states), "windows": []}
+        for (a, b), s in zip(wins, states):
+            orc.run(s, 2, 1)
+            entry["windows"].append([[a, b], {n: T.digest(s.arrays[n]) for n in harness.MUTATED}])
+            if (E, L, a) == (86400, 72, 0):        # closed-form: its first elements are those of ref_outputs_E3
+                for n in harness.MUTATED:
+                    x = s.arrays[n][:3, int(s.ctl[3])] if n.startswith("elem_state") else s.arrays[n][:3]
+                    assert np.array_equal(x, ref[f"call2_{n}"]), n
+        out[f"{E}x{L}"] = entry
+    with open(os.path.join(HERE, "full_size_digests.json"), "w") as f:
+        json.dump(out, f, indent=1)
+        f.write("\n")
+
+
 if __name__ == "__main__":
-    main()
+    if "--full-size" in sys.argv:
+        full_size_digests()
+    else:
+        main()

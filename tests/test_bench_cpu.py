@@ -33,3 +33,25 @@ def test_reference_arm_json_line():
 def test_reference_arm_other_ranks_are_silent():
     p = _run({"RANK": "1", "WORLD_SIZE": "2", "LOCAL_RANK": "1"})
     assert p.returncode == 0 and p.stdout.strip() == ""
+
+
+def test_dump_sample_is_fixed_and_fits_the_budget():
+    """--dump-outputs writes every element of a small slice and a fixed, sorted sample of a large one, within 64 MB."""
+    import numpy as np
+    import bench
+    import tinman_sandbox_b200 as tb
+    for E, L in ((10, 72), (300, 72), (5400, 72), (86400, 72), (49152, 128), (393216, 128), (86400, 26)):
+        e = bench.dump_elements(E, L)
+        per_elem = 8 * sum(int(np.prod(tb.field_shape(n, 1, L))) for n in tb.MUTATED_FIELDS)
+        assert len(e) * per_elem <= 64_000_000 - 4096, (E, L)
+        assert e[0] >= 0 and e[-1] < E and np.all(np.diff(e) > 0), (E, L)
+        assert np.array_equal(e, bench.dump_elements(E, L))
+        if E * per_elem <= 60_000_000:
+            assert np.array_equal(e, np.arange(E))
+        else:
+            assert len(e) > 100
+
+
+def test_steps_must_be_positive():
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True)
+    assert p.returncode != 0 and "--steps" in p.stderr

@@ -66,6 +66,35 @@ def test_two_ranks_weak_scaling_fast_mode_parity():
     assert d["scaling"] == "weak" and d["gpu_launches"] > 0 and d["e2e"]["link"]["frac"] > 0
 
 
+def test_dumped_outputs_are_those_of_the_last_timed_step(tmp_path):
+    """--dump-outputs: the seven mutated arrays of the fixed element sample after warmup + 2 + steps calls (what the
+    timed loop leaves on the device), bit for bit those of the same number of strict calls made through the handle."""
+    import numpy as np
+    import bench
+    import tinman_sandbox_b200 as tb
+    from tinman_sandbox_b200.testdata import TestData
+    E, L = 3000, 72
+    d = _bench(1, ["--nelem", str(E), "--mode", "strict", "--steps", "4", "--no-e2e", "--no-parity",
+                   "--dump-outputs", str(tmp_path)])
+    assert d["steps"] == 4 and d["checksums"]["calls"] == 3 + 2 + 4
+    elems = bench.dump_elements(E, L)
+    assert 0 < len(elems) < E
+    td = TestData(E, L).init_data()
+    h = tb.Caar(E, L)
+    h.set_params(td.consts, td.dvv, td.ps0, td.hyai)
+    h.set_control(*[int(x) for x in td.ctl], dt2=td.dt2)
+    h.upload(td.arrays)
+    h.compute_and_apply_rhs(3 + 2 + 4, tb.MODE_STRICT)
+    h.download(td.arrays)
+    h.close()
+    total = 0
+    for n in tb.MUTATED_FIELDS:
+        a = np.load(tmp_path / f"{n}.npy")
+        total += (tmp_path / f"{n}.npy").stat().st_size
+        assert a.dtype == np.float64 and np.array_equal(a, td.arrays[n][elems]), n
+    assert total <= 64_000_000
+
+
 def test_single_rank_bench_line_is_self_validating():
     d = _bench(1, ["--nelem", "2000"])
     assert d["parity"]["ok"] and d["parity"]["oracle"] in ("reference", "port")
