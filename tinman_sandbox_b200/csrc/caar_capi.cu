@@ -78,6 +78,9 @@ struct caar_handle_s {
   double* hybi_dev;  // [nlev+1], Eulerian branch only
   double* extra[5];  // arrays beyond struct Arrays: vstar, qtens, tensorVisc, scalar in / out (allocated on first use)
   double* stage;  // device staging buffer of the Fortran-layout copies (allocated on first use)
+  // device [2]: the tile scheduler of the thread-per-level laplacians (next chunk, warps done), zero between launches.
+  // One pair per handle: all launches of a handle are ordered on its stream, so no two of them share it.
+  unsigned* lapflat_sched;
   caar::TmaMaps* tma_host;
   double* tma_host_key[CAAR_NUM_FIELDS];
 };
@@ -158,6 +161,7 @@ caar::KernelArgs make_args(const caar_handle_s* h, const caar_control* ctl, doub
   a.tma = h->tma;
   a.rsplit = h->rsplit;
   a.hybi = h->hybi_dev;
+  a.lapflat_sched = h->lapflat_sched;
   return a;
 }
 
@@ -218,6 +222,8 @@ int caar_create(caar_handle* out, const caar_dims* dims, int device) {
   if (e == cudaSuccess) e = cudaMalloc(&h->bits, (size_t)dims->nelem * 7 * sizeof(unsigned long long));
   if (e == cudaSuccess) e = cudaMalloc(&h->out3, 23 * sizeof(double));
   if (e == cudaSuccess) e = cudaMallocHost(&h->out3_host, 23 * sizeof(double));
+  if (e == cudaSuccess) e = cudaMalloc(&h->lapflat_sched, 2 * sizeof(unsigned));
+  if (e == cudaSuccess) e = cudaMemsetAsync(h->lapflat_sched, 0, 2 * sizeof(unsigned), h->own_stream);
   if (e == cudaSuccess) e = cudaStreamSynchronize(h->own_stream);
   if (e != cudaSuccess) {
     const int code = fail(e == cudaErrorMemoryAllocation ? CAAR_ERR_NOMEM : CAAR_ERR_CUDA, "caar_create: %s",
@@ -257,6 +263,7 @@ int caar_destroy(caar_handle h) {
     if (h->extra[x]) cudaFree(h->extra[x]);
   if (h->hybi_dev) cudaFree(h->hybi_dev);
   if (h->out3_host) cudaFreeHost(h->out3_host);
+  if (h->lapflat_sched) cudaFree(h->lapflat_sched);
   if (h->ev0) cudaEventDestroy(h->ev0);
   if (h->ev1) cudaEventDestroy(h->ev1);
   if (h->ev_fence) cudaEventDestroy(h->ev_fence);

@@ -50,6 +50,8 @@ struct KernelArgs {
   const double* hybi;
   // L2 prefetch distance in elements (0 = off): CTA e prefetches the early inputs of element e + pf_dist
   int pf_dist;
+  // the handle's tile scheduler pair of the thread-per-level laplacians (device [2], zero between launches)
+  unsigned* lapflat_sched;
 };
 
 // TMA tensor maps over the level-field arrays viewed as 3-D [slice][rows of 128 B][16 doubles] (slice = element x

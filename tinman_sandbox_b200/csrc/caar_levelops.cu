@@ -43,8 +43,6 @@
 // the tracer step's strict variant stays in caar_euler.cu.
 #include "caar_fused_kernel.cuh"
 
-#include <atomic>
-
 namespace caar {
 namespace {
 
@@ -779,17 +777,10 @@ cudaError_t launch_op(const LevelOpArgs& a, const LevelOpMaps& m, cudaStream_t s
   return cudaGetLastError();
 }
 
-// the scheduler's counters: a ring of pairs, one pair per launch (zero before and after each launch; launches that could
-// overlap on different streams draw different pairs)
-constexpr int SCHED_SLOTS = 256;
-__device__ unsigned g_lapflat_sched[SCHED_SLOTS][2];
-
 template <bool TENSOR>
 cudaError_t launch_lapflat(LapFlatArgs a, const LapFlatMaps& m, cudaStream_t s) {
   const size_t smem = (size_t)FW * FWARP_B + FW * FN * (sizeof(uint64_t) + sizeof(int)) + 1024;
   static int cached_per_sm[64] = {};
-  static unsigned* sched_base[64] = {};
-  static std::atomic<unsigned> seq{0};
   int dev = 0;
   cudaError_t e = cudaGetDevice(&dev);
   if (e != cudaSuccess) return e;
@@ -803,10 +794,6 @@ cudaError_t launch_lapflat(LapFlatArgs a, const LapFlatMaps& m, cudaStream_t s) 
     e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, laplace_flat_kernel<TENSOR>, 32 * FW, smem);
     if (e != cudaSuccess) return e;
     if (per_sm < 1) per_sm = 1;
-    void* p = nullptr;
-    e = cudaGetSymbolAddress(&p, g_lapflat_sched);
-    if (e != cudaSuccess) return e;
-    sched_base[dev] = static_cast<unsigned*>(p);
     cached_per_sm[dev] = per_sm;
   }
   // one wave of resident CTAs; chunks of 4 consecutive tiles (49152 x 128: 0.81 / 0.98 / 1.01 / 0.99 / 0.95 / 0.90 of the
@@ -814,7 +801,6 @@ cudaError_t launch_lapflat(LapFlatArgs a, const LapFlatMaps& m, cudaStream_t s) 
   static const int chunk_env = [] { const char* v = getenv("CAAR_LAPLACE_CHUNK"); return v ? atoi(v) : 0; }();
   const long long resident_warps = (long long)sm_count() * per_sm * FW;
   a.chunk = chunk_env > 0 ? chunk_env : (a.tiles < resident_warps * 16 ? 2 : 4);
-  a.sched = sched_base[dev] + 2 * (seq.fetch_add(1) % SCHED_SLOTS);
   long long blocks = (long long)sm_count() * per_sm;
   const long long need = (a.tiles + FW - 1) / FW;
   if (blocks > need) blocks = need;
@@ -847,6 +833,9 @@ cudaError_t launch_levelop(int op, const KernelArgs& k, const double* in, const 
     LapFlatArgs a;
     a.Dinv = k.Dinv; a.spheremp = k.spheremp; a.tensorvisc = tensorvisc;
     a.nlev = k.nlev; a.nets = nets; a.rows = flat_rows; a.tiles = (flat_rows + FT - 1) / FT; a.rrearth = k.rrearth;
+    // the calling handle's scheduler pair: launches of other handles, on other streams, never touch it
+    a.sched = k.lapflat_sched;
+    if (!a.sched) return cudaErrorInvalidValue;
     for (int i = 0; i < 16; ++i) a.dvv[i] = k.dvv[i];
     LapFlatMaps m;
     const size_t off = (size_t)nets * k.nlev * 16;
