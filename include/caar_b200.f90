@@ -65,7 +65,7 @@ module caar_b200
   end type caar_checksum
 
   public :: caar_create, caar_destroy, caar_set_params_f90, caar_set_vertical_coordinate, caar_upload_layout, &
-            caar_download_layout, caar_run, caar_run_stepping, caar_update_time_levels, caar_sync, caar_norms, &
+            caar_download_layout, caar_run, caar_run_stepping, caar_run_rk5, caar_update_time_levels, caar_sync, caar_norms, &
             caar_checksums, caar_euler_step, caar_sphere_wk, caar_extra_upload, caar_extra_download, caar_last_error, &
             caar_host_register, caar_host_unregister, caar_describe
 
@@ -126,6 +126,15 @@ module caar_b200
       import :: c_ptr, c_int, caar_control
       type(c_ptr), value :: handle
       type(caar_control), intent(inout) :: ctl
+      integer(c_int), value :: nsteps, mode
+      integer(c_int) :: rc
+    end function
+    ! int caar_run_rk5(caar_handle h, caar_control* ctl, double dt, int nsteps, int mode); tstep_type == 5
+    function caar_run_rk5(handle, ctl, dt, nsteps, mode) bind(C, name="caar_run_rk5") result(rc)
+      import :: c_ptr, c_int, c_double, caar_control
+      type(c_ptr), value :: handle
+      type(caar_control), intent(inout) :: ctl
+      real(c_double), value :: dt
       integer(c_int), value :: nsteps, mode
       integer(c_int) :: rc
     end function

@@ -232,8 +232,25 @@ int caar_describe(caar_handle h, int mode, char* buf, size_t len, int* is_fused)
    (nm1 = np1 = n0: forward Euler / RK stages, F/routine_extracted.F90:6-16) are legal in every entry point. */
 int caar_run_stepping(caar_handle h, caar_control* ctl, int nsteps, int mode);
 void caar_update_time_levels(caar_control* ctl);
+/* HOMME's default explicit dynamics step, tstep_type == 5 of prim_advance_exp (preqx prim_advance_mod.F90): nsteps
+   steps of five compute_and_apply_rhs calls on the resident state, asynchronously on the handle's stream, with the
+   rotation of caar_update_time_levels after each step. With (n0, np1, nm1) the levels on entry and w the eta_ave_w
+   of caar_set_params, one step is (ctl levels n0 / np1 / nm1, dt2, eta_ave_w; all scalars in double precision):
+     1  n0  / nm1 / n0    dt/5      w/4       u1 = u0 + dt/5 R(u0), stored in nm1
+     2  nm1 / np1 / n0    dt/5      0         u2 = u0 + dt/5 R(u1)
+     3  np1 / np1 / n0    dt/3      0         u3 = u0 + dt/3 R(u2)
+     4  np1 / np1 / n0    (2*dt)/3  0         u4 = u0 + 2dt/3 R(u3)
+     c  v, T, dp3d at nm1 = (5*X(nm1) - X(n0))/4 on [nets,nete), rounded as Fortran's expression
+     5  np1 / np1 / nm1   (3*dt)/4  (3*w)/4   u5 = (5u1 - u0)/4 + 3dt/4 R(u4)
+   After the step n0 holds u0, nm1 the combination and np1 u5; then the levels rotate. The per-stage dt2 and
+   eta_ave_w apply to that stage only: the handle's constants and ctl->dt2 are neither read nor written. Stages run
+   on the kernel caar_run would use in `mode`; each step issues 6 launches (none for an empty element range, which
+   still rotates). The levels must be pairwise distinct (stage 1 would overwrite u0), so ntl >= 3. Returns
+   CAAR_ERR_STATE before caar_set_params and CAAR_ERR_INVALID for a null control, nsteps < 0, a bad mode or
+   levels that are not pairwise distinct, leaving *ctl unchanged. No DSS runs between stages. */
+int caar_run_rk5(caar_handle h, caar_control* ctl, double dt, int nsteps, int mode);
 int caar_sync(caar_handle h);
-/* number of kernel launches issued by caar_run/caar_norms on this handle since creation */
+/* number of kernel launches issued through this handle since creation (caar_run, caar_run_rk5: 6 per step, caar_norms, ...) */
 long long caar_launch_count(caar_handle h);
 /* CUDA-event stopwatch on the stream the kernels are launched on: start records an event, stop records a
    second one, waits for it and returns the device time between the two in milliseconds. */

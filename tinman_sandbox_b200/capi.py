@@ -40,7 +40,7 @@ EXPORTED_SYMBOLS = (
     "caar_sync", "caar_launch_count", "caar_timer_start",
     "caar_timer_stop", "caar_norms", "caar_compute_and_apply_rhs_host", "caar_saxpby_device",
     "caar_saxpby_host", "caar_checksums", "caar_upload_range", "caar_download_range", "caar_describe",
-    "caar_sphere_wk",
+    "caar_sphere_wk", "caar_run_rk5",
 )
 CHECKSUM_FIELDS = ("elem_state_dp3d", "elem_state_v", "elem_state_T", "elem_derived_eta_dot_dpdn",
                    "elem_derived_omega_p", "elem_derived_phi", "elem_derived_vn0")
@@ -126,6 +126,7 @@ def load_library():
                                       C.POINTER(C.c_size_t)]
     lib.caar_set_vertical_coordinate.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_double)]
     lib.caar_run_stepping.argtypes = [C.c_void_p, C.POINTER(Control), C.c_int, C.c_int]
+    lib.caar_run_rk5.argtypes = [C.c_void_p, C.POINTER(Control), C.c_double, C.c_int, C.c_int]
     lib.caar_update_time_levels.argtypes = [C.POINTER(Control)]
     lib.caar_update_time_levels.restype = None
     lib.caar_extra_count.restype = C.c_size_t
@@ -335,6 +336,14 @@ class Caar:
         """nsteps evaluations with TestData::update_time_levels (PO/data_structures.cpp:174-180) after each;
         self.control holds the rotated time levels afterwards."""
         _check(self.lib, self.lib.caar_run_stepping(self.h, C.byref(self.control), nsteps, mode), "caar_run_stepping")
+        if sync:
+            self.sync()
+
+    def run_rk5(self, nsteps, dt, mode=MODE_FAST, sync=True):
+        """nsteps steps of HOMME's five-stage Runge-Kutta dynamics step (tstep_type 5, caar_run_rk5) of length dt;
+        self.control holds the rotated time levels afterwards and its dt2 is not used."""
+        _check(self.lib, self.lib.caar_run_rk5(self.h, C.byref(self.control), float(dt), int(nsteps), mode),
+               "caar_run_rk5")
         if sync:
             self.sync()
 

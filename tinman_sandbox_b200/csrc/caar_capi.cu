@@ -469,21 +469,68 @@ int caar_describe(caar_handle h, int mode, char* buf, size_t len, int* is_fused)
   return CAAR_OK;
 }
 
-int caar_run(caar_handle h, const caar_control* ctl, int nsteps, int mode) {
+namespace {
+
+// The checks of caar_run and caar_run_rk5; *fast = the kernel `mode` selects on this handle (fused or strict)
+int check_run(caar_handle h, const caar_control* ctl, int nsteps, int mode, const char* who, bool* fast) {
   if (!h) return fail(CAAR_ERR_INVALID, "null handle");
-  if (!h->params_set) return fail(CAAR_ERR_STATE, "caar_set_params must be called before caar_run");
+  if (!h->params_set) return fail(CAAR_ERR_STATE, "caar_set_params must be called before %s", who);
   if (int rc = validate_control(h, ctl)) return rc;
   if (nsteps < 0) return fail(CAAR_ERR_INVALID, "nsteps=%d", nsteps);
   if (mode != CAAR_MODE_FAST && mode != CAAR_MODE_STRICT) return fail(CAAR_ERR_INVALID, "mode=%d", mode);
-  DeviceGuard guard(h->device);
-  const caar::KernelArgs a = make_args(h, ctl);
-  const bool fast = uses_fused(h, mode);
-  if (!fast && caar::strict_smem_bytes(h->dims.nlev) > 200 * 1024)
+  *fast = uses_fused(h, mode);
+  if (!*fast && caar::strict_smem_bytes(h->dims.nlev) > 200 * 1024)
     return fail(CAAR_ERR_UNSUPPORTED, "nlev=%d too large for the strict kernel", h->dims.nlev);
-  if (ctl->nete == ctl->nets) return CAAR_OK;
-  for (int s = 0; s < nsteps; ++s) {
+  return CAAR_OK;
+}
+
+// ncalls evaluations of compute_and_apply_rhs with the arguments `a` on the handle's stream (caller holds the device)
+int launch_rhs(caar_handle h, const caar::KernelArgs& a, int ncalls, bool fast) {
+  if (a.nete == a.nets) return CAAR_OK;
+  for (int s = 0; s < ncalls; ++s) {
     CU_TRY(fast ? caar::launch_fused(a, h->stream) : caar::launch_strict(a, h->stream));
     ++h->launches;
+  }
+  return CAAR_OK;
+}
+
+}  // namespace
+
+int caar_run(caar_handle h, const caar_control* ctl, int nsteps, int mode) {
+  bool fast = false;
+  if (int rc = check_run(h, ctl, nsteps, mode, "caar_run", &fast)) return rc;
+  DeviceGuard guard(h->device);
+  return launch_rhs(h, make_args(h, ctl), nsteps, fast);
+}
+
+int caar_run_rk5(caar_handle h, caar_control* ctl, double dt, int nsteps, int mode) {
+  bool fast = false;
+  if (int rc = check_run(h, ctl, nsteps, mode, "caar_run_rk5", &fast)) return rc;
+  if (ctl->n0 == ctl->np1 || ctl->n0 == ctl->nm1 || ctl->np1 == ctl->nm1)  // stage 1 would overwrite u0
+    return fail(CAAR_ERR_INVALID, "caar_run_rk5 needs pairwise distinct time levels (n0=%d np1=%d nm1=%d)", ctl->n0,
+                ctl->np1, ctl->nm1);
+  DeviceGuard guard(h->device);
+  const double w = h->c.eta_ave_w;
+  for (int s = 0; s < nsteps; ++s) {
+    const int n0 = ctl->n0, np1 = ctl->np1, nm1 = ctl->nm1;
+    // prim_advance_exp, tstep_type == 5: {n0, np1, nm1, dt2, eta_ave_w} of the five compute_and_apply_rhs calls
+    const struct { int n0, np1, nm1; double dt2, eta_ave_w; } stage[5] = {
+        {n0, nm1, n0, dt / 5, w / 4},          {nm1, np1, n0, dt / 5, 0.0},          {np1, np1, n0, dt / 3, 0.0},
+        {np1, np1, n0, (2 * dt) / 3, 0.0},     {np1, np1, nm1, (3 * dt) / 4, (3 * w) / 4}};
+    for (int k = 0; k < 5 && ctl->nete > ctl->nets; ++k) {
+      if (k == 4) {  // u(nm1) = (5 u1 - u0)/4
+        CU_TRY(caar::launch_rk5_combine(make_args(h, ctl), ctl->nets, ctl->nete, nm1, n0, h->stream));
+        ++h->launches;
+      }
+      caar::KernelArgs a = make_args(h, ctl);
+      a.n0 = stage[k].n0;
+      a.np1 = stage[k].np1;
+      a.nm1 = stage[k].nm1;
+      a.dt2 = stage[k].dt2;
+      a.eta_ave_w = stage[k].eta_ave_w;
+      if (int rc = launch_rhs(h, a, 1, fast)) return rc;
+    }
+    caar_update_time_levels(ctl);
   }
   return CAAR_OK;
 }

@@ -88,6 +88,8 @@ cudaError_t launch_levelop(int op, const KernelArgs& k, const double* in, const 
                            const double* tensorvisc, int nets, int nete, int qn0, int qsize, double dt, bool strict,
                            cudaStream_t s);
 cudaError_t launch_saxpby(double a, double b, double* x, const double* y, size_t n, cudaStream_t s);
+// RK5 step (caar_aux.cu): v, T, dp3d at nm1 = (5*X(nm1) - X(n0))/4 on [nets,nete), one launch; nm1 != n0
+cudaError_t launch_rk5_combine(const KernelArgs& a, int nets, int nete, int nm1, int n0, cudaStream_t s);
 // checksums of the seven mutated arrays + energy norms (caar_aux.cu); partial [nelem][8][2], bits [nelem][7]
 cudaError_t launch_checksums(const KernelArgs& a, int tl, int nets, int nete, double cp, double* partial,
                              unsigned long long* bits, double* out16, unsigned long long* out7, cudaStream_t s);
