@@ -66,7 +66,7 @@ module caar_b200
 
   public :: caar_create, caar_destroy, caar_set_params_f90, caar_set_vertical_coordinate, caar_upload_layout, &
             caar_download_layout, caar_run, caar_run_stepping, caar_run_rk5, caar_update_time_levels, caar_sync, caar_norms, &
-            caar_checksums, caar_euler_step, caar_sphere_wk, caar_extra_upload, caar_extra_download, caar_last_error, &
+            caar_checksums, caar_euler_step, caar_advect_tracers, caar_sphere_wk, caar_extra_upload, caar_extra_download, caar_last_error, &
             caar_host_register, caar_host_unregister, caar_describe
 
   interface
@@ -168,6 +168,19 @@ module caar_b200
       integer(c_int), value :: nets, nete, qn0, qsize
       real(c_double), value :: dt
       integer(c_int), value :: mode
+      integer(c_int) :: rc
+    end function
+    ! int caar_advect_tracers(caar_handle h, int nets, int nete, int* qn0, int qsize, double dt, int nsteps, int mode);
+    ! HOMME's three-stage tracer step (rkstage = 3); qn0 (zero-based n0_qdp) comes back toggled once per step
+    function caar_advect_tracers(handle, nets, nete, qn0, qsize, dt, nsteps, mode) bind(C, name="caar_advect_tracers") &
+        result(rc)
+      import :: c_ptr, c_int, c_double
+      type(c_ptr), value :: handle
+      integer(c_int), value :: nets, nete
+      integer(c_int), intent(inout) :: qn0
+      integer(c_int), value :: qsize
+      real(c_double), value :: dt
+      integer(c_int), value :: nsteps, mode
       integer(c_int) :: rc
     end function
     function caar_sphere_wk(handle, op, nets, nete, mode) bind(C, name="caar_sphere_wk") result(rc)

@@ -250,7 +250,8 @@ void caar_update_time_levels(caar_control* ctl);
    levels that are not pairwise distinct, leaving *ctl unchanged. No DSS runs between stages. */
 int caar_run_rk5(caar_handle h, caar_control* ctl, double dt, int nsteps, int mode);
 int caar_sync(caar_handle h);
-/* number of kernel launches issued through this handle since creation (caar_run, caar_run_rk5: 6 per step, caar_norms, ...) */
+/* number of kernel launches issued through this handle since creation (caar_run, caar_run_rk5: 6 per step,
+   caar_advect_tracers: 4 per step, caar_euler_step, caar_norms, ...) */
 long long caar_launch_count(caar_handle h);
 /* CUDA-event stopwatch on the stream the kernels are launched on: start records an event, stop records a
    second one, waits for it and returns the device time between the two in milliseconds. */
@@ -273,6 +274,26 @@ size_t caar_extra_count(const caar_dims* dims, int which);
 int caar_extra_upload(caar_handle h, int which, const double* host);
 int caar_extra_download(caar_handle h, int which, double* host);
 int caar_euler_step(caar_handle h, int nets, int nete, int qn0, int qsize, double dt, int mode);
+/* HOMME's Eulerian tracer advection step with rkstage = 3 (prim_advection_mod: three euler_step calls and
+   qdp_time_avg): nsteps steps of length dt on the resident Qdp, asynchronously on the handle's stream. With n0 = *qn0
+   on entry and np1 = 1 - n0, one step is, for tracers iq < qsize of elements [nets,nete):
+     1  Qdp(np1) = Qdp(n0)  - dt/2 div(vstar Qdp(n0))
+     2  Qdp(np1) = Qdp(np1) - dt/2 div(vstar Qdp(np1))      (in place)
+     3  Qdp(np1) = Qdp(np1) - dt/2 div(vstar Qdp(np1))      (in place)
+     a  Qdp(np1) = (Qdp(n0) + 2*Qdp(np1))/3, rounded as Fortran's expression (one add, one division; 2*b is exact)
+   then *qn0 = np1 (TimeLevel_Qdp swaps n0_qdp and np1_qdp). Each stage is exactly caar_euler_step with dt/2 (exact in
+   double) on the kernel caar_euler_step uses in `mode` (CAAR_EULER_V1 included), storing into Qdp(np1) instead of
+   CAAR_X_QTENS, so a stage is bit-identical to caar_euler_step's qtens. The stability polynomial is
+   1 + z + z^2/2 + z^3/12: second order. Only Qdp[nets:nete][0:qsize][np1] changes: Qdp(n0), the tracers iq >= qsize,
+   the elements outside the range, CAAR_X_VSTAR and CAAR_X_QTENS (which this call does not allocate) keep their values.
+   Element-local, like caar_run_rk5: no DSS, no limiter and no tracer hyperviscosity run between stages. HOMME stores
+   spheremp*Qtens, runs the DSS and multiplies by rspheremp; without the DSS the two products cancel up to rounding,
+   so a stage stores Qtens itself. vstar is CAAR_X_VSTAR, fixed for all three stages; HOMME recomputes it each stage
+   from vn0 and a dp that moves with rhs_multiplier, so the two agree only when that term vanishes (coupling vstar to
+   vn0 is not part of this call). Each step issues 4 launches (none for an empty range or qsize == 0, which still
+   toggle *qn0). Returns CAAR_ERR_STATE before caar_set_params and CAAR_ERR_INVALID for a null handle or qn0,
+   *qn0 not 0 or 1, a bad element range, qsize outside [0, qsize_d], nsteps < 0 or a bad mode, leaving *qn0 unchanged. */
+int caar_advect_tracers(caar_handle h, int nets, int nete, int* qn0, int qsize, double dt, int nsteps, int mode);
 
 /* ---- the weak-form operators behind hyperviscosity (SURVEY §8f rank 4) ----
    Level-local like the tracer step, on the same kernel skeleton, in the pointers_only index conventions

@@ -40,7 +40,7 @@ EXPORTED_SYMBOLS = (
     "caar_sync", "caar_launch_count", "caar_timer_start",
     "caar_timer_stop", "caar_norms", "caar_compute_and_apply_rhs_host", "caar_saxpby_device",
     "caar_saxpby_host", "caar_checksums", "caar_upload_range", "caar_download_range", "caar_describe",
-    "caar_sphere_wk", "caar_run_rk5",
+    "caar_sphere_wk", "caar_run_rk5", "caar_advect_tracers",
 )
 CHECKSUM_FIELDS = ("elem_state_dp3d", "elem_state_v", "elem_state_T", "elem_derived_eta_dot_dpdn",
                    "elem_derived_omega_p", "elem_derived_phi", "elem_derived_vn0")
@@ -135,6 +135,8 @@ def load_library():
     lib.caar_extra_download.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_double)]
     lib.caar_sphere_wk.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int]
     lib.caar_euler_step.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, C.c_int]
+    lib.caar_advect_tracers.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_int), C.c_int, C.c_double, C.c_int,
+                                        C.c_int]
     lib.caar_upload_layout.argtypes = [C.c_void_p, C.POINTER(Arrays), C.c_uint, C.c_int]
     lib.caar_download_layout.argtypes = [C.c_void_p, C.POINTER(Arrays), C.c_uint, C.c_int]
     lib.caar_set_params_f90.argtypes = [C.c_void_p, C.POINTER(Constants), C.POINTER(C.c_double), C.c_double,
@@ -361,6 +363,18 @@ class Caar:
                "caar_euler_step")
         if sync:
             self.sync()
+
+    def advect_tracers(self, qn0, qsize, dt, nsteps=1, mode=MODE_FAST, nets=None, nete=None, sync=True):
+        """nsteps steps of HOMME's three-stage tracer step (rkstage = 3, caar_advect_tracers) of length dt on the
+        resident Qdp, starting from time level qn0 (0 or 1) -> the qn0 of the new state."""
+        nets = self.control.nets if nets is None else nets
+        nete = self.control.nete if nete is None else nete
+        q = C.c_int(int(qn0))
+        _check(self.lib, self.lib.caar_advect_tracers(self.h, nets, nete, C.byref(q), int(qsize), float(dt),
+                                                      int(nsteps), mode), "caar_advect_tracers")
+        if sync:
+            self.sync()
+        return q.value
 
     def download_qtens(self, qtens=None):
         E, L, Q, _ = self.shape_args

@@ -2,7 +2,8 @@
 //   * norms: sum of squares of v, T, dp3d at one time level per element, then over elements
 //     (what print_results_2norm reduces, PO/compute_and_apply_rhs.cpp:372-399);
 //   * saxpby: x = a*x + b*y, the reference's bandwidth yardstick (saxpby_test/cxx/common.cpp:3-15);
-//   * the RK5 step's combination of two time levels (caar_run_rk5).
+//   * the RK5 step's combination of two time levels (caar_run_rk5) and the tracer SSP step's time average of Qdp
+//     (caar_advect_tracers), on one grid-stride skeleton.
 #include "caar_device.cuh"
 
 namespace caar {
@@ -213,50 +214,86 @@ struct Rk5Combine {
   double *v, *T, *dp;
   unsigned per, lf2;  // double2 rows per element (32L) and per time-level slice of T / dp3d (8L)
   int ntl, nets, nm1, n0;
+  static constexpr int ROWS = 4;  // rows of 16 B per thread and trip in flight
+
+  // row i of the combination at time level nm1; *dn0 = distance in double2 to the same row at n0
+  __device__ __forceinline__ double2* row(size_t i, ptrdiff_t* dn0) const {
+    const size_t e = (size_t)nets + i / per;
+    unsigned r = (unsigned)(i % per);
+    double* f = v;
+    unsigned slice = 2 * lf2;
+    if (r >= slice) {
+      r -= slice;
+      slice = lf2;
+      f = r < slice ? T : dp;
+      if (r >= slice) r -= slice;
+    }
+    *dn0 = (ptrdiff_t)(n0 - nm1) * slice;
+    return reinterpret_cast<double2*>(f) + (e * ntl + nm1) * slice + r;
+  }
+  // a = the row at nm1, b = the same row at n0
+  static __device__ __forceinline__ double mix(double a, double b) { return __dmul_rn(__dsub_rn(__dmul_rn(5.0, a), b), 0.25); }
 };
 
-// row i of the combination at time level nm1; *dn0 = distance in double2 to the same row at n0
-__device__ __forceinline__ double2* rk5_row(const Rk5Combine& c, size_t i, ptrdiff_t* dn0) {
-  const size_t e = (size_t)c.nets + i / c.per;
-  unsigned r = (unsigned)(i % c.per);
-  double* f = c.v;
-  unsigned slice = 2 * c.lf2;
-  if (r >= slice) {
-    r -= slice;
-    slice = c.lf2;
-    f = r < slice ? c.T : c.dp;
-    if (r >= slice) r -= slice;
+// Tracer SSP step (caar_advect_tracers), after its third stage: Qdp(np1) = (Qdp(n0) + 2*Qdp(np1))/3 for tracers
+// iq < qsize of elements [nets, nete). Per element the rows are qsize blocks of 8L double2, one per tracer, each the
+// tracer's np1 slice of Qdp [E][qsize_d][2][L][16] (128 B aligned). Rounded as Fortran's (a + 2*b)/3: 2*b is exact, then
+// one rounded add and one rounded division, never contracted and never a multiplication by 1/3, in both modes.
+// np1 != n0, so the n0 slices are read-only here.
+struct QdpAverage {
+  double* Qdp;
+  unsigned per, lf2;  // double2 rows per element (qsize * 8L) and per tracer slice (8L)
+  int qsize_d, nets, np1, n0;
+  // rows per thread and trip: with 4, the registers live across the division's slow-path call exceed the 64 of two
+  // resident CTAs of 512 and spill
+  static constexpr int ROWS = 2;
+
+  // row i of the average at np1; *dn0 = distance in double2 to the same row at n0
+  __device__ __forceinline__ double2* row(size_t i, ptrdiff_t* dn0) const {
+    const size_t e = (size_t)nets + i / per;
+    const unsigned r = (unsigned)(i % per), iq = r / lf2;
+    *dn0 = (ptrdiff_t)(n0 - np1) * lf2;
+    return reinterpret_cast<double2*>(Qdp) + ((e * qsize_d + iq) * 2 + np1) * lf2 + (r - iq * lf2);
   }
-  *dn0 = (ptrdiff_t)(c.n0 - c.nm1) * slice;
-  return reinterpret_cast<double2*>(f) + (e * c.ntl + c.nm1) * slice + r;
-}
+  // a = the row at np1 (stage 3's result), b = the same row at n0
+  static __device__ __forceinline__ double mix(double a, double b) { return __ddiv_rn(__dadd_rn(b, __dmul_rn(2.0, a)), 3.0); }
+};
 
-__device__ __forceinline__ double rk5_mix(double a, double b) { return __dmul_rn(__dsub_rn(__dmul_rn(5.0, a), b), 0.25); }
+template <class C>
+__device__ __forceinline__ double2 mix2(double2 a, double2 b) { return make_double2(C::mix(a.x, b.x), C::mix(a.y, b.y)); }
 
-__device__ __forceinline__ double2 rk5_mix2(double2 a, double2 b) { return make_double2(rk5_mix(a.x, b.x), rk5_mix(a.y, b.y)); }
-
-// grid-stride, 4 rows of 16 B per thread per trip in flight
-__global__ void __launch_bounds__(512, 2) rk5_combine_kernel(const Rk5Combine c, size_t n) {
+// x = C::mix(x, y) over the rows C::row maps out, y the row *dn0 away (read-only in the launch); grid-stride,
+// C::ROWS rows of 16 B per thread per trip in flight
+template <class C>
+__global__ void __launch_bounds__(512, 2) combine_kernel(const C c, size_t n) {
+  constexpr int R = C::ROWS;
   const size_t stride = (size_t)gridDim.x * blockDim.x;
   size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  for (; i + 3 * stride < n; i += 4 * stride) {
-    double2* p[4];
-    double2 a[4], b[4];
+  for (; i + (R - 1) * stride < n; i += R * stride) {
+    double2* p[R];
+    double2 a[R], b[R];
 #pragma unroll
-    for (int u = 0; u < 4; ++u) {
+    for (int u = 0; u < R; ++u) {
       ptrdiff_t d;
-      p[u] = rk5_row(c, i + u * stride, &d);
+      p[u] = c.row(i + u * stride, &d);
       a[u] = *p[u];
       b[u] = __ldg(p[u] + d);
     }
 #pragma unroll
-    for (int u = 0; u < 4; ++u) *p[u] = rk5_mix2(a[u], b[u]);
+    for (int u = 0; u < R; ++u) *p[u] = mix2<C>(a[u], b[u]);
   }
   for (; i < n; i += stride) {
     ptrdiff_t d;
-    double2* p = rk5_row(c, i, &d);
-    *p = rk5_mix2(*p, __ldg(p + d));
+    double2* p = c.row(i, &d);
+    *p = mix2<C>(*p, __ldg(p + d));
   }
+}
+
+// blocks of the combination kernels: 4 rows per thread, at most two resident CTAs of 512 per SM
+unsigned combine_blocks(size_t n) {
+  size_t blocks = (n + 512 * 4 - 1) / (512 * 4);
+  if (blocks > (size_t)sm_count() * 2) blocks = (size_t)sm_count() * 2;
+  return (unsigned)blocks;
 }
 
 // ---- host-layout conversion for the Fortran (F90 flat pointer) boundary --------------------------------------
@@ -344,9 +381,16 @@ cudaError_t launch_saxpby(double a, double b, double* x, const double* y, size_t
 cudaError_t launch_rk5_combine(const KernelArgs& a, int nets, int nete, int nm1, int n0, cudaStream_t s) {
   if (nete <= nets) return cudaSuccess;
   const size_t n = (size_t)(nete - nets) * a.nlev * 32;  // double2 rows
-  size_t blocks = (n + 512 * 4 - 1) / (512 * 4);
-  if (blocks > (size_t)sm_count() * 2) blocks = (size_t)sm_count() * 2;  // two resident CTAs of 512 per SM
-  rk5_combine_kernel<<<(unsigned)blocks, 512, 0, s>>>(Rk5Combine{a.v, a.T, a.dp3d, 32u * a.nlev, 8u * a.nlev, a.ntl, nets, nm1, n0}, n);
+  combine_kernel<<<combine_blocks(n), 512, 0, s>>>(Rk5Combine{a.v, a.T, a.dp3d, 32u * a.nlev, 8u * a.nlev, a.ntl, nets, nm1, n0}, n);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_qdp_avg(const KernelArgs& a, int nets, int nete, int qsize, int n0, int np1, cudaStream_t s) {
+  if (nete <= nets || qsize <= 0) return cudaSuccess;
+  const size_t n = (size_t)(nete - nets) * qsize * a.nlev * 8;  // double2 rows
+  // the kernel writes Qdp; the mirror is const only for the operators that read it
+  const QdpAverage c{const_cast<double*>(a.Qdp), (unsigned)qsize * 8u * a.nlev, 8u * a.nlev, a.qsize_d, nets, np1, n0};
+  combine_kernel<<<combine_blocks(n), 512, 0, s>>>(c, n);
   return cudaGetLastError();
 }
 

@@ -820,26 +820,69 @@ int caar_extra_download(caar_handle h, int which, double* host) {
   return CAAR_OK;
 }
 
-int caar_euler_step(caar_handle h, int nets, int nete, int qn0, int qsize, double dt, int mode) {
+namespace {
+
+// The checks of caar_euler_step and caar_advect_tracers
+int check_euler(caar_handle h, int nets, int nete, int qn0, int qsize, int mode, const char* who) {
   if (!h) return fail(CAAR_ERR_INVALID, "null handle");
-  if (!h->params_set) return fail(CAAR_ERR_STATE, "caar_set_params must be called before caar_euler_step");
+  if (!h->params_set) return fail(CAAR_ERR_STATE, "caar_set_params must be called before %s", who);
   if (nets < 0 || nete > h->dims.nelem || nets > nete) return fail(CAAR_ERR_INVALID, "element range [%d,%d)", nets, nete);
   if (qn0 < 0 || qn0 > 1) return fail(CAAR_ERR_INVALID, "qn0=%d must be 0 or 1", qn0);
   if (qsize < 0 || qsize > h->dims.qsize_d) return fail(CAAR_ERR_INVALID, "qsize=%d outside [0,%d]", qsize, h->dims.qsize_d);
   if (mode != CAAR_MODE_FAST && mode != CAAR_MODE_STRICT) return fail(CAAR_ERR_INVALID, "mode=%d", mode);
+  return CAAR_OK;
+}
+
+// One tracer step Qdp(qn0) - dt div(vstar Qdp(qn0)) on the handle's stream (caller holds the device); tracer iq of
+// element e goes to the level slice (e * qsize_d + iq) * out_stride + out_off of `out`: (qtens, 1, 0) or (Qdp, 2, np1).
+// Fast mode: the TMA-pipelined level-local skeleton (caar_levelops.cu); CAAR_EULER_V1=1 keeps the first-generation
+// LDG/STG kernel for A/B runs. Strict mode: the reference-order kernel of caar_euler.cu.
+int launch_tracer_step(caar_handle h, const caar::KernelArgs& a, const double* vstar, double* out, int out_stride,
+                       int out_off, int nets, int nete, int qn0, int qsize, double dt, int mode) {
+  static const bool v1 = [] { const char* e = getenv("CAAR_EULER_V1"); return e && atoi(e) != 0; }();
+  if (mode == CAAR_MODE_STRICT || v1)
+    CU_TRY(caar::launch_euler_step(a, vstar, out, out_stride, out_off, nets, nete, qn0, qsize, dt,
+                                   mode == CAAR_MODE_STRICT, h->stream));
+  else
+    CU_TRY(caar::launch_levelop(0, a, a.Qdp, vstar, out, nullptr, nets, nete, qn0, qsize, dt, out_stride, out_off,
+                                false, h->stream));
+  if (nete > nets && qsize > 0) ++h->launches;
+  return CAAR_OK;
+}
+
+}  // namespace
+
+int caar_euler_step(caar_handle h, int nets, int nete, int qn0, int qsize, double dt, int mode) {
+  if (int rc = check_euler(h, nets, nete, qn0, qsize, mode, "caar_euler_step")) return rc;
   DeviceGuard guard(h->device);
   double *vstar = nullptr, *qtens = nullptr;
   if (int rc = extra_buffer(h, CAAR_X_VSTAR, &vstar)) return rc;
   if (int rc = extra_buffer(h, CAAR_X_QTENS, &qtens)) return rc;
+  return launch_tracer_step(h, make_args(h, nullptr), vstar, qtens, 1, 0, nets, nete, qn0, qsize, dt, mode);
+}
+
+int caar_advect_tracers(caar_handle h, int nets, int nete, int* qn0, int qsize, double dt, int nsteps, int mode) {
+  if (!qn0) return fail(CAAR_ERR_INVALID, "qn0 is null");
+  if (int rc = check_euler(h, nets, nete, *qn0, qsize, mode, "caar_advect_tracers")) return rc;
+  if (nsteps < 0) return fail(CAAR_ERR_INVALID, "nsteps=%d", nsteps);
+  DeviceGuard guard(h->device);
+  double* vstar = nullptr;
+  if (int rc = extra_buffer(h, CAAR_X_VSTAR, &vstar)) return rc;
   const caar::KernelArgs a = make_args(h, nullptr);
-  // fast mode: the TMA-pipelined level-local skeleton (caar_levelops.cu); CAAR_EULER_V1=1 keeps the first-generation
-  // LDG/STG kernel for A/B runs. Strict mode: the reference-order kernel of caar_euler.cu.
-  static const bool v1 = [] { const char* e = getenv("CAAR_EULER_V1"); return e && atoi(e) != 0; }();
-  if (mode == CAAR_MODE_STRICT || v1)
-    CU_TRY(caar::launch_euler_step(a, vstar, qtens, nets, nete, qn0, qsize, dt, mode == CAAR_MODE_STRICT, h->stream));
-  else
-    CU_TRY(caar::launch_levelop(0, a, a.Qdp, vstar, qtens, nullptr, nets, nete, qn0, qsize, dt, false, h->stream));
-  if (nete > nets && qsize > 0) ++h->launches;
+  double* Qdp = const_cast<double*>(a.Qdp);  // the handle's own mirror; const in KernelArgs for the kernels that read it
+  const double half = dt / 2;
+  for (int s = 0; s < nsteps; ++s) {
+    const int n0 = *qn0, np1 = 1 - n0;
+    if (nete > nets && qsize > 0) {
+      // three euler_step stages of dt/2 into Qdp(np1), stages 2 and 3 in place, then the time average
+      for (int k = 0; k < 3; ++k)
+        if (int rc = launch_tracer_step(h, a, vstar, Qdp, 2, np1, nets, nete, k == 0 ? n0 : np1, qsize, half, mode))
+          return rc;
+      CU_TRY(caar::launch_qdp_avg(a, nets, nete, qsize, n0, np1, h->stream));
+      ++h->launches;
+    }
+    *qn0 = np1;  // TimeLevel_Qdp: n0_qdp <-> np1_qdp
+  }
   return CAAR_OK;
 }
 
@@ -863,7 +906,7 @@ int caar_sphere_wk(caar_handle h, int op, int nets, int nete, int mode) {
     if (int rc = extra_buffer(h, CAAR_X_TENSORVISC, &tv)) return rc;
   const caar::KernelArgs a = make_args(h, nullptr);
   const int kop = op == CAAR_OP_DIVERGENCE_WK ? 1 : op == CAAR_OP_LAPLACE_SIMPLE ? 2 : 3;
-  CU_TRY(caar::launch_levelop(kop, a, kop == 1 ? vin : sin, nullptr, out, tv, nets, nete, 0, 1, 0.0,
+  CU_TRY(caar::launch_levelop(kop, a, kop == 1 ? vin : sin, nullptr, out, tv, nets, nete, 0, 1, 0.0, 1, 0,
                               mode == CAAR_MODE_STRICT, h->stream));
   if (nete > nets) ++h->launches;
   return CAAR_OK;

@@ -79,17 +79,20 @@ cudaError_t launch_norms(const KernelArgs& a, int tl, int nets, int nete, double
 cudaError_t launch_relayout(double* cxx, double* f90, size_t nblocks, int kind, bool to_cxx, int q_dim, int nlev,
                             size_t blk0, cudaStream_t s);
 cudaError_t launch_reciprocal(double* out, const double* in, size_t n, cudaStream_t s);
-// tracer step after CAAR (caar_euler.cu): qtens = Qdp(qn0) - dt*divergence_sphere(vstar*Qdp(qn0))
-cudaError_t launch_euler_step(const KernelArgs& a, const double* vstar, double* qtens, int nets, int nete, int qn0,
-                              int qsize, double dt, bool strict, cudaStream_t s);
-// level-local operators on the TMA-pipelined skeleton (caar_levelops.cu): op 0 tracer step, 1 divergence_sphere_wk,
-// 2 laplace_simple, 3 laplace_tensor
+// tracer step after CAAR (caar_euler.cu): Qdp(qn0) - dt*divergence_sphere(vstar*Qdp(qn0)) into the level slice
+// (e * qsize_d + iq) * out_stride + out_off of out [slice][L][16]: (qtens, 1, 0), or (Qdp, 2, np1) in place
+cudaError_t launch_euler_step(const KernelArgs& a, const double* vstar, double* out, int out_stride, int out_off,
+                              int nets, int nete, int qn0, int qsize, double dt, bool strict, cudaStream_t s);
+// level-local operators on the TMA-pipelined skeleton (caar_levelops.cu): op 0 tracer step (output slices as in
+// launch_euler_step), 1 divergence_sphere_wk, 2 laplace_simple, 3 laplace_tensor
 cudaError_t launch_levelop(int op, const KernelArgs& k, const double* in, const double* item, double* out,
-                           const double* tensorvisc, int nets, int nete, int qn0, int qsize, double dt, bool strict,
-                           cudaStream_t s);
+                           const double* tensorvisc, int nets, int nete, int qn0, int qsize, double dt, int out_stride,
+                           int out_off, bool strict, cudaStream_t s);
 cudaError_t launch_saxpby(double a, double b, double* x, const double* y, size_t n, cudaStream_t s);
 // RK5 step (caar_aux.cu): v, T, dp3d at nm1 = (5*X(nm1) - X(n0))/4 on [nets,nete), one launch; nm1 != n0
 cudaError_t launch_rk5_combine(const KernelArgs& a, int nets, int nete, int nm1, int n0, cudaStream_t s);
+// tracer SSP step (caar_aux.cu): Qdp(np1) = (Qdp(n0) + 2*Qdp(np1))/3 for tracers < qsize on [nets,nete), one launch
+cudaError_t launch_qdp_avg(const KernelArgs& a, int nets, int nete, int qsize, int n0, int np1, cudaStream_t s);
 // checksums of the seven mutated arrays + energy norms (caar_aux.cu); partial [nelem][8][2], bits [nelem][7]
 cudaError_t launch_checksums(const KernelArgs& a, int tl, int nets, int nete, double cp, double* partial,
                              unsigned long long* bits, double* out16, unsigned long long* out7, cudaStream_t s);

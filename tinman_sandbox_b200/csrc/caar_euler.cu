@@ -18,6 +18,14 @@
 // (element, level) index space in groups of 64 rows with a grid-stride loop; 3 CTAs per SM. The flux weights w = metdet * Dinv * vstar are
 // formed once per level and kept in registers over the tracer loop, which is unrolled by two so that two Qdp rows
 // are in flight per thread.
+//
+// The output of tracer iq of element e is the level slice (e * qsize_d + iq) * out_stride + out_off of `out`
+// ([slice][L][16]): (qtens, 1, 0) for caar_euler_step, (Qdp, 2, np1) for a stage of caar_advect_tracers, which may
+// read and write the same Qdp level (qn0 == np1). That in-place form is safe as the kernel stands: a thread loads only
+// its own GLL row of each tracer (ld4 of qbase below), takes its neighbours' values through shuffles of registers the
+// neighbours already loaded, and stores that same row afterwards; no thread reads a row another thread stores (the
+// clamped tail rows only feed dead lanes). Qdp is read with plain loads, never __ldg / ld.global.nc, because the
+// launch may write it.
 #include <cstdlib>
 
 #include "caar_device.cuh"
@@ -33,7 +41,8 @@ struct EulerArgs {
   const double* rmetdet;
   const double* Qdp;    // [E][qsize_d][2][L][16]
   const double* vstar;  // [E][L][16][2]
-  double* qtens;        // [E][qsize_d][L][16]
+  double* out;          // tracer 0 of element 0 of the output: qtens, or Qdp + np1 * lf
+  size_t out_stride;    // doubles from one tracer to the next in `out`: lf (qtens) or 2 lf (Qdp)
   int nlev, qsize_d, nets, nelem_run, qn0, qsize;
   double dt, rrearth;
   double dvv[16];
@@ -143,35 +152,39 @@ __global__ void __launch_bounds__(256, STRICT ? 2 : 3) euler_step_kernel(const _
       }
     }
     const double* qbase = A.Qdp + (e * A.qsize_d * 2 + A.qn0) * lf + off;  // + iq * 2 * lf
-    double* obase = A.qtens + e * A.qsize_d * lf + off;                    // + iq * lf
+    double* obase = A.out + e * A.qsize_d * A.out_stride + off;            // + iq * out_stride
     int iq = 0;
-    for (; iq + 1 < A.qsize; iq += 2) {
+    // two tracers per trip in fast mode; one in strict mode, whose reference-order evaluation keeps more values live
+    // (two per trip spilled at the 128 registers of two resident CTAs per SM)
+    for (; !STRICT && iq + 1 < A.qsize; iq += 2) {
       double qa[4], qb[4], oa[4], ob[4];
       ld4(qbase + (size_t)iq * 2 * lf, qa);
       ld4(qbase + (size_t)(iq + 1) * 2 * lf, qb);
       tracer_row<STRICT>(A, qa, u, v, di, met, rmet, w1, w2, cx, lane, r, oa);
       tracer_row<STRICT>(A, qb, u, v, di, met, rmet, w1, w2, cx, lane, r, ob);
       if (live) {
-        st4(obase + (size_t)iq * lf, oa);
-        st4(obase + (size_t)(iq + 1) * lf, ob);
+        st4(obase + (size_t)iq * A.out_stride, oa);
+        st4(obase + (size_t)(iq + 1) * A.out_stride, ob);
       }
     }
-    if (iq < A.qsize) {
+    for (; iq < A.qsize; ++iq) {
       double qa[4], oa[4];
       ld4(qbase + (size_t)iq * 2 * lf, qa);
       tracer_row<STRICT>(A, qa, u, v, di, met, rmet, w1, w2, cx, lane, r, oa);
-      if (live) st4(obase + (size_t)iq * lf, oa);
+      if (live) st4(obase + (size_t)iq * A.out_stride, oa);
     }
   }
 }
 
 }  // namespace
 
-cudaError_t launch_euler_step(const KernelArgs& a, const double* vstar, double* qtens, int nets, int nete, int qn0,
-                              int qsize, double dt, bool strict, cudaStream_t s) {
+cudaError_t launch_euler_step(const KernelArgs& a, const double* vstar, double* out, int out_stride, int out_off,
+                              int nets, int nete, int qn0, int qsize, double dt, bool strict, cudaStream_t s) {
   if (nete <= nets || qsize <= 0) return cudaSuccess;
+  const size_t lf = (size_t)a.nlev * PTS;
   EulerArgs e;
-  e.Dinv = a.Dinv; e.metdet = a.metdet; e.rmetdet = a.rmetdet; e.Qdp = a.Qdp; e.vstar = vstar; e.qtens = qtens;
+  e.Dinv = a.Dinv; e.metdet = a.metdet; e.rmetdet = a.rmetdet; e.Qdp = a.Qdp; e.vstar = vstar;
+  e.out = out + (size_t)out_off * lf; e.out_stride = (size_t)out_stride * lf;
   e.nlev = a.nlev; e.qsize_d = a.qsize_d; e.nets = nets; e.nelem_run = nete - nets; e.qn0 = qn0; e.qsize = qsize;
   e.dt = dt; e.rrearth = a.rrearth;
   for (int i = 0; i < 16; ++i) e.dvv[i] = a.dvv[i];

@@ -70,6 +70,7 @@ struct LevelOpArgs {
   const double* spheremp;
   const double* tensorvisc;
   int nlev, nets, ngroups, Q, qn0, qsize_d;
+  int out_stride, out_off;  // OP_EULER: unit (e, iq) stores slice (e * qsize_d + iq) * out_stride + out_off of M.out
   long long units;  // elements * ngroups * Q
   double dt, rrearth;
   double dvv[16];
@@ -105,6 +106,13 @@ enum { OP_EULER = 0, OP_DIVWK = 1, OP_LAP_SIMPLE = 2, OP_LAP_TENSOR = 3 };
 // Every WARP is an independent pipeline over a contiguous range of units (element, group of 8 levels, tracer), tracer
 // fastest: its lane 0 issues the TMA loads NS tiles ahead and the TMA stores, the warp waits on its own mbarriers and
 // synchronises with __syncwarp only.
+//
+// OP_EULER in place (a stage of caar_advect_tracers with qn0 == np1: M.out is the Qdp map, out_stride 2, out_off np1,
+// so every unit loads and stores the same tile). Safe because each unit owns exactly one tile, which no other unit of
+// any warp loads or stores; a unit's input tile is in shared memory (its mbarrier has completed and every lane has
+// read it) before its store is issued; and the ring only prefetches tiles of this warp's later units, never one an
+// earlier unit of any warp stores. The next stage reads the stored tiles back with TMA: the bulk stores are complete
+// when the grid is, and the exit below only waits for their shared-memory reads, as the in-place laplacian does.
 template <int OP>
 __global__ void __launch_bounds__(32 * WPC, LEVELOP_MINB) levelop_kernel(const __grid_constant__ LevelOpArgs A,
                                                               const __grid_constant__ LevelOpMaps M) {
@@ -355,7 +363,7 @@ __global__ void __launch_bounds__(32 * WPC, LEVELOP_MINB) levelop_kernel(const _
     fence_proxy_async();
     __syncwarp();  // the output tile is complete and visible to the TMA engine
     if (lane == 0) {
-      tma_store(&M.out, lev0, OP == OP_EULER ? e * A.qsize_d + iq : e, otile);
+      tma_store(&M.out, lev0, OP == OP_EULER ? (e * A.qsize_d + iq) * A.out_stride + A.out_off : e, otile);
       bulk_commit();
     }
   }
@@ -810,12 +818,14 @@ cudaError_t launch_lapflat(LapFlatArgs a, const LapFlatMaps& m, cudaStream_t s) 
 
 }  // namespace
 
-// Level-local operator on elements [nets,nete). op: 0 tracer step (in = Qdp mirror, item = vstar, out = qtens),
-// 1 divergence_sphere_wk (in = vector [E][L][16][2]), 2 laplace_simple, 3 laplace_tensor (in = scalar [E][L][16]);
-// out [E][L][16] (tracer step: [E][qsize_d][L][16]). in == out is allowed for 2 and 3 (the reference's *_replace).
+// Level-local operator on elements [nets,nete). op: 0 tracer step (in = Qdp mirror, item = vstar, out = qtens or
+// Qdp), 1 divergence_sphere_wk (in = vector [E][L][16][2]), 2 laplace_simple, 3 laplace_tensor (in = scalar
+// [E][L][16]); out [E][L][16] (tracer step: [slice][L][16], tracer iq of element e at slice (e * qsize_d + iq) *
+// out_stride + out_off; other ops ignore the two). in == out is allowed for 2 and 3 (the reference's *_replace) and
+// for 0 with (2, qn0) (a stage of caar_advect_tracers).
 cudaError_t launch_levelop(int op, const KernelArgs& k, const double* in, const double* item, double* out,
-                           const double* tensorvisc, int nets, int nete, int qn0, int qsize, double dt, bool strict,
-                           cudaStream_t s) {
+                           const double* tensorvisc, int nets, int nete, int qn0, int qsize, double dt, int out_stride,
+                           int out_off, bool strict, cudaStream_t s) {
   if (nete <= nets || (op == 0 && qsize <= 0)) return cudaSuccess;
   if (strict) {
     if (op == 0) return cudaErrorInvalidValue;  // the strict tracer step lives in caar_euler.cu
@@ -846,6 +856,7 @@ cudaError_t launch_levelop(int op, const KernelArgs& k, const double* in, const 
   LevelOpArgs a;
   a.Dinv = k.Dinv; a.metdet = k.metdet; a.rmetdet = k.rmetdet; a.spheremp = k.spheremp; a.tensorvisc = tensorvisc;
   a.nlev = k.nlev; a.nets = nets; a.qn0 = qn0; a.qsize_d = k.qsize_d; a.dt = dt; a.rrearth = k.rrearth;
+  a.out_stride = out_stride; a.out_off = out_off;
   for (int i = 0; i < 16; ++i) a.dvv[i] = k.dvv[i];
   a.ngroups = (k.nlev + GL - 1) / GL;  // groups of 8 levels; the last one may stick out of the column (zero-filled / clipped)
   a.Q = op == 0 ? qsize : 1;
@@ -856,7 +867,7 @@ cudaError_t launch_levelop(int op, const KernelArgs& k, const double* in, const 
   if (op == 0) {
     bad |= encode3(&m.in, in, E * (cuuint64_t)k.qsize_d * 2, L, GL);
     bad |= encode3(&m.item, item, E, 2 * L, 2 * GL);
-    bad |= encode3(&m.out, out, E * (cuuint64_t)k.qsize_d, L, GL);
+    bad |= encode3(&m.out, out, E * (cuuint64_t)k.qsize_d * (cuuint64_t)out_stride, L, GL);
   } else {
     bad |= encode3(&m.in, in, E, op == 1 ? 2 * L : L, op == 1 ? 2 * GL : GL);
     bad |= encode3(&m.out, out, E, L, GL);

@@ -126,7 +126,7 @@ def profiled_kernel_ms(h, mode, steps):
         h.run_rk5(steps, DT, mode)
         torch.cuda.synchronize()
     ev = sorted((e for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA
-                 and ("caar_" in e.name or "rk5_combine" in e.name)), key=lambda e: e.time_range.start)
+                 and ("caar_" in e.name or "combine_kernel" in e.name)), key=lambda e: e.time_range.start)
     if len(ev) != 6 * steps:
         return None, [e.name for e in ev[:8]]
     per = [sum(ev[6 * s + k].time_range.elapsed_us() for s in range(steps)) / steps / 1e3 for k in range(6)]
