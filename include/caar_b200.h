@@ -282,7 +282,7 @@ int caar_euler_step(caar_handle h, int nets, int nete, int qn0, int qsize, doubl
      3  Qdp(np1) = Qdp(np1) - dt/2 div(vstar Qdp(np1))      (in place)
      a  Qdp(np1) = (Qdp(n0) + 2*Qdp(np1))/3, rounded as Fortran's expression (one add, one division; 2*b is exact)
    then *qn0 = np1 (TimeLevel_Qdp swaps n0_qdp and np1_qdp). Each stage is exactly caar_euler_step with dt/2 (exact in
-   double) on the kernel caar_euler_step uses in `mode` (CAAR_EULER_V1 included), storing into Qdp(np1) instead of
+   double) on the kernel caar_euler_step uses in `mode`, storing into Qdp(np1) instead of
    CAAR_X_QTENS, so a stage is bit-identical to caar_euler_step's qtens. The stability polynomial is
    1 + z + z^2/2 + z^3/12: second order. Only Qdp[nets:nete][0:qsize][np1] changes: Qdp(n0), the tracers iq >= qsize,
    the elements outside the range, CAAR_X_VSTAR and CAAR_X_QTENS (which this call does not allocate) keep their values.

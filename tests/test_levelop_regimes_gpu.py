@@ -9,8 +9,7 @@ reference (oracle/hp_reference.py) with the pointwise gate |g - v| <= K u M, and
 2. Knob legs. Every knob is read once per process into a `static`, so each setting runs in a child process
    (`python tests/test_levelop_regimes_gpu.py --knob-worker SPEC`) that loads the library fresh, runs its jobs and
    writes .npz files; the parent computes the same jobs in process at default knobs and gates the child's results.
-   Knobs that only change the schedule must leave the results bit-identical; the two that select other arithmetic
-   (CAAR_LAPLACE_V1, CAAR_EULER_V1) are gated pointwise.
+   Every knob only changes the schedule and must leave the results bit-identical.
 
 The report (test_zz_report_regimes) prints, per kernel, case and knob, the regime, the worst ratio against K and
 where the worst point sits in the work distribution: (warp, unit) for levelop_kernel, (tile, chunk) for the flat
@@ -33,13 +32,12 @@ import tinman_sandbox_b200 as tb  # noqa: E402
 from oracle import harness  # noqa: E402
 from oracle import hp_reference as hp  # noqa: E402
 from test_levelop_regimes_cpu import (CASES, FT, GL, case_regime, hp_slice, lean_inputs, levelop_unit_warp,  # noqa: E402
-                                      missed, regime, sub_state)
+                                      missed, sub_state)
 from test_pointwise_cpu import TLS, rhs_case_state  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 DT = 150.0
-KNOBS = ("CAAR_LEVELOP_WAVES", "CAAR_LAPLACE_CHUNK", "CAAR_LAPLACE_V1", "CAAR_EULER_V1", "CAAR_EULER_WAVES",
-         "CAAR_CLUSTER_POLICY", "CAAR_PF_DIST")
+KNOBS = ("CAAR_LEVELOP_WAVES", "CAAR_LAPLACE_CHUNK", "CAAR_EULER_WAVES", "CAAR_CLUSTER_POLICY", "CAAR_PF_DIST")
 REPORT = []          # lines of the final report
 LAP_OPS = (("laplace_simple", tb.OP_LAPLACE_SIMPLE, hp.K_LAPLACE_SIMPLE),
            ("laplace_tensor", tb.OP_LAPLACE_TENSOR, hp.K_LAPLACE_TENSOR))
@@ -126,8 +124,6 @@ def run_job(j, inputs=None):
 def locate(c, idx, sms):
     """Where a point of a case's output sits in the work distribution (at the ptxas occupancy)."""
     lo, L = c["range"][0], c["nlev"]
-    if c.get("v1"):                                     # euler_step_kernel: groups of 64 rows, grid-stride
-        return f"row group {((idx[0] - lo) * L + idx[2]) // 64}"
     r = case_regime(c, sms)
     if c["op"] == "lap_flat":
         tile = ((idx[0] - lo) * L + idx[1]) // FT
@@ -210,13 +206,13 @@ def port_reference(c, s, vin, sin, tv):
             for name, _, _ in LAP_OPS}
 
 
-def gate_fast(c, got, inputs, knob, sms, tag=""):
+def gate_fast(c, got, inputs, knob, sms):
     """Every fast-mode output of a case against the reference; laplace_tensor_replace bit-equal to laplace_tensor."""
     s, vin, sin, tv = inputs
     q = c["qsize"]
     kind = {"euler": "euler_step", "divwk": "divergence_sphere_wk", "lap_rows": "levelop", "lap_flat": "flat"}[c["op"]]
     if c["op"] == "euler":
-        gate_sliced(f"euler_step_fast{tag}", c, got["qtens"][:, :q], "euler_step", (s, vin, None), hp.K_EULER, knob,
+        gate_sliced("euler_step_fast", c, got["qtens"][:, :q], "euler_step", (s, vin, None), hp.K_EULER, knob,
                     sms, qn0=c["qn0"], qsize=q)
     elif c["op"] == "divwk":
         gate_sliced("divergence_sphere_wk_fast", c, got[kind], kind, (s, vin, None), hp.K_DIVWK, knob, sms)
@@ -291,13 +287,6 @@ LAP_CHUNK_JOBS = [dict(_shrunk("F2", 4096, range=(1, 4096)), ranges=50), dict(_s
 SCHEDULE_JOBS = ([dict(T2, mode=tb.MODE_FAST, id="T2_fast"), dict(T2, mode=tb.MODE_STRICT, id="T2_strict"),
                   dict(D1, mode=tb.MODE_FAST, id="D1_fast")]
                  + [dict(j, mode=tb.MODE_FAST, id=j["id"] + "_fast") for j in LAP_CHUNK_JOBS] + _rhs_jobs())
-# the row decomposition for every nlev: about 24000 units, 10 per warp
-LAP_V1_JOBS = [dict(_shrunk("F1", E, nlev=L), mode=tb.MODE_FAST) for L, E in ((16, 12000), (30, 6000), (72, 2700),
-                                                                             (128, 1500))]
-EULER_V1_JOB = dict(_by_id("T2"), id="V1", E=1200, range=(0, 1200), Q=5, qsize=5, qn0=0, gen="stratified",
-                    mode=tb.MODE_FAST, v1=True)
-for _j in LAP_V1_JOBS:
-    _j["id"] = f"V1_L{_j['nlev']}"
 
 # Schedule-only knob values are combined into three children: each knob is read by one kernel only.
 SCHEDULE_LEGS = [
@@ -306,11 +295,6 @@ SCHEDULE_LEGS = [
     {"CAAR_LEVELOP_WAVES": "16", "CAAR_LAPLACE_CHUNK": "3", "CAAR_EULER_WAVES": "0", "CAAR_CLUSTER_POLICY": "2",
      "CAAR_PF_DIST": "1"},
     {"CAAR_LEVELOP_WAVES": "200", "CAAR_LAPLACE_CHUNK": "64", "CAAR_PF_DIST": str(600 + 5)},
-]
-ARITHMETIC_LEGS = [
-    ({"CAAR_LAPLACE_V1": "1", "CAAR_EULER_V1": "1", "CAAR_EULER_WAVES": "1"}, LAP_V1_JOBS + [EULER_V1_JOB]),
-    ({"CAAR_EULER_V1": "1", "CAAR_EULER_WAVES": "2"}, [EULER_V1_JOB]),
-    ({"CAAR_EULER_V1": "1", "CAAR_EULER_WAVES": "0"}, [EULER_V1_JOB]),
 ]
 
 
@@ -365,32 +349,6 @@ def test_schedule_knobs_are_bit_identical(tmp_path, default_knobs):
                 bad.append((j["id"], env_knobs))
         assert np.array_equal(got["T2_strict"]["qtens"][:, :T2["qsize"]], port[:, :T2["qsize"]]), env_knobs
     assert not bad, bad
-
-
-def test_arithmetic_knobs_pass_the_pointwise_gate(tmp_path, default_knobs):
-    """CAAR_LAPLACE_V1=1 runs the row-decomposed laplacians at nlev 16, 30, 72 and 128 (about 10 units per warp);
-    CAAR_EULER_V1=1 the first-generation tracer step at nlev 72, qsize_d = qsize = 5 (odd: the remainder of its
-    unroll by two), with CAAR_EULER_WAVES 1, 2 and 0. Each is gated pointwise; the three V1 tracer runs, which differ
-    in their grid only, must also agree bit for bit."""
-    sms = device_sms()
-    v1_runs = []
-    for n, (env_knobs, jobs) in enumerate(ARITHMETIC_LEGS):
-        got = run_worker(env_knobs, jobs, tmp_path, f"arith{n}")
-        for j in jobs:
-            g = got[j["id"]]
-            if j["op"] == "euler":
-                check_sentinel(j, g["qtens"])
-                v1_runs.append(g["qtens"])
-                knob = knob_str(env_knobs, ("CAAR_EULER_V1", "CAAR_EULER_WAVES"))
-                gate_fast(j, g, job_inputs(j), knob, sms, tag="_v1")
-            else:
-                inputs = job_inputs(j)
-                for name, v in g.items():
-                    check_sentinel(j, v, name, inputs[2])
-                c = dict(j, op="lap_rows")
-                gate_fast(c, g, inputs, knob_str(env_knobs, ("CAAR_LAPLACE_V1",)), sms)
-                assert regime("lap_rows", j["E"], j["nlev"], sms=sms)["per_warp"] >= 4
-    assert all(np.array_equal(v, v1_runs[0]) for v in v1_runs[1:])
 
 
 def test_zz_report_regimes(capsys):

@@ -2,28 +2,21 @@
 tests/tracer_ssp_oracle.py and against the public calls it replaces: the strict kernel bit for bit with the FP64
 composition; fast mode bit for bit with three public caar_euler_step(dt/2) calls composed on the host, within 1e-12
 per field and within k_ssp u M of the long-double composition. Also the in-place stages at the sizes where the
-per-warp pipelines wrap, CAAR_EULER_V1=1, the average kernel where its grid-stride loop wraps, launch counts, qn0
-toggling, error paths, run-to-run bits, and a dynamics step followed by a tracer step followed by CAAR."""
+per-warp pipelines wrap, the average kernel where its grid-stride loop wraps, launch counts, qn0 toggling, error
+paths, run-to-run bits, and a dynamics step followed by a tracer step followed by CAAR."""
 import ctypes as C
-import os
-import subprocess
-import sys
 import time
 
 import numpy as np
 import pytest
 
-if __name__ == "__main__":                          # CAAR_EULER_V1 worker: the repository and tests/ on the path
-    _HERE = os.path.dirname(os.path.abspath(__file__))
-    sys.path[:0] = [os.path.dirname(_HERE), _HERE]
-
-import tinman_sandbox_b200 as tb  # noqa: E402
-from oracle import harness  # noqa: E402
-from oracle import hp_reference as hp  # noqa: E402
-import rk5_oracle as ro  # noqa: E402
-import tracer_ssp_oracle as so  # noqa: E402
-from test_levelop_regimes_cpu import CASES as REGIME_CASES, lean_inputs  # noqa: E402
-from test_pointwise_cpu import level_local_inputs  # noqa: E402
+import tinman_sandbox_b200 as tb
+from oracle import harness
+from oracle import hp_reference as hp
+import rk5_oracle as ro
+import tracer_ssp_oracle as so
+from test_levelop_regimes_cpu import CASES as REGIME_CASES, lean_inputs
+from test_pointwise_cpu import level_local_inputs
 
 pytestmark = pytest.mark.gpu
 T0 = time.time()
@@ -215,29 +208,6 @@ def test_in_place_at_regime_sizes(c, mode):
     assert np.isfinite(got[lo:hi, :c["qsize"]]).all()
 
 
-# ---- CAAR_EULER_V1=1 ------------------------------------------------------------------------------------------------
-
-V1_CASES = [dict(nlev=72, qsize=5, qn0=1, nsteps=2, gen="stratified", E=9, range=(1, 8), seed=5101),
-            dict(nlev=30, qsize=34, qn0=0, nsteps=1, gen="randomize", E=7, range=(0, 7), seed=5102)]
-
-
-def v1_check(c):
-    s, vstar = case_inputs(c)
-    lo, hi = c["range"]
-    got, _ = gpu_advect(s, vstar, c["qn0"], c["qsize"], DT, c["nsteps"], tb.MODE_FAST, lo, hi)
-    pub, _ = public_ssp(s, vstar, c["qn0"], c["qsize"], DT, c["nsteps"], tb.MODE_FAST, lo, hi)
-    assert np.array_equal(bits(got), bits(pub)), c
-
-
-def test_euler_v1_equals_its_public_calls():
-    """CAAR_EULER_V1 is read once per process: a child runs fast mode on the first-generation kernel."""
-    env = dict(os.environ, CAAR_EULER_V1="1")
-    p = subprocess.run([sys.executable, os.path.abspath(__file__), "--v1-worker"], env=env, capture_output=True,
-                       text=True, timeout=900)
-    assert p.returncode == 0, f"{p.stdout[-3000:]}\n{p.stderr[-3000:]}"
-    assert "v1 ok" in p.stdout
-
-
 # ---- the average kernel where its grid-stride loop wraps -----------------------------------------------------------
 
 def test_average_kernel_at_scale():
@@ -346,9 +316,3 @@ def test_zz_report(capsys):
         worst = ", ".join(f"{k} {v:.2e}" for k, v in sorted(WORST.items()))
         print(f"\n[tracer ssp] worst pointwise ratio / k_ssp (fast): {worst or 'n/a'}; "
               f"tests/test_tracer_ssp_gpu.py wall time {time.time() - T0:.1f} s")
-
-
-if __name__ == "__main__" and sys.argv[1:] == ["--v1-worker"]:
-    for _c in V1_CASES:
-        v1_check(_c)
-    print("v1 ok")

@@ -835,14 +835,12 @@ int check_euler(caar_handle h, int nets, int nete, int qn0, int qsize, int mode,
 
 // One tracer step Qdp(qn0) - dt div(vstar Qdp(qn0)) on the handle's stream (caller holds the device); tracer iq of
 // element e goes to the level slice (e * qsize_d + iq) * out_stride + out_off of `out`: (qtens, 1, 0) or (Qdp, 2, np1).
-// Fast mode: the TMA-pipelined level-local skeleton (caar_levelops.cu); CAAR_EULER_V1=1 keeps the first-generation
-// LDG/STG kernel for A/B runs. Strict mode: the reference-order kernel of caar_euler.cu.
+// Fast mode: the TMA-pipelined level-local skeleton (caar_levelops.cu). Strict mode: the reference-order kernel of
+// caar_euler.cu.
 int launch_tracer_step(caar_handle h, const caar::KernelArgs& a, const double* vstar, double* out, int out_stride,
                        int out_off, int nets, int nete, int qn0, int qsize, double dt, int mode) {
-  static const bool v1 = [] { const char* e = getenv("CAAR_EULER_V1"); return e && atoi(e) != 0; }();
-  if (mode == CAAR_MODE_STRICT || v1)
-    CU_TRY(caar::launch_euler_step(a, vstar, out, out_stride, out_off, nets, nete, qn0, qsize, dt,
-                                   mode == CAAR_MODE_STRICT, h->stream));
+  if (mode == CAAR_MODE_STRICT)
+    CU_TRY(caar::launch_euler_step(a, vstar, out, out_stride, out_off, nets, nete, qn0, qsize, dt, h->stream));
   else
     CU_TRY(caar::launch_levelop(0, a, a.Qdp, vstar, out, nullptr, nets, nete, qn0, qsize, dt, out_stride, out_off,
                                 false, h->stream));

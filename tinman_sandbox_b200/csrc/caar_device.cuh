@@ -79,10 +79,10 @@ cudaError_t launch_norms(const KernelArgs& a, int tl, int nets, int nete, double
 cudaError_t launch_relayout(double* cxx, double* f90, size_t nblocks, int kind, bool to_cxx, int q_dim, int nlev,
                             size_t blk0, cudaStream_t s);
 cudaError_t launch_reciprocal(double* out, const double* in, size_t n, cudaStream_t s);
-// tracer step after CAAR (caar_euler.cu): Qdp(qn0) - dt*divergence_sphere(vstar*Qdp(qn0)) into the level slice
+// strict tracer step after CAAR (caar_euler.cu): Qdp(qn0) - dt*divergence_sphere(vstar*Qdp(qn0)) into the level slice
 // (e * qsize_d + iq) * out_stride + out_off of out [slice][L][16]: (qtens, 1, 0), or (Qdp, 2, np1) in place
 cudaError_t launch_euler_step(const KernelArgs& a, const double* vstar, double* out, int out_stride, int out_off,
-                              int nets, int nete, int qn0, int qsize, double dt, bool strict, cudaStream_t s);
+                              int nets, int nete, int qn0, int qsize, double dt, cudaStream_t s);
 // level-local operators on the TMA-pipelined skeleton (caar_levelops.cu): op 0 tracer step (output slices as in
 // launch_euler_step), 1 divergence_sphere_wk, 2 laplace_simple, 3 laplace_tensor
 cudaError_t launch_levelop(int op, const KernelArgs& k, const double* in, const double* item, double* out,

@@ -25,8 +25,7 @@
 // Math:
 //   * sphere operators (PO/sphere_operators.cpp:9-129): derivative along jgp is thread-local (Dvv from the
 //     constant bank); derivative along igp: one DMMA.8x8x4 per jgp column differentiates all 8 levels of the warp at
-//     once and one 64-bit shuffle per value brings the (transposed) result home — see deriv_i(const Row&, const
-//     DerivMma&). (-DCAAR_DERIV_MMA=0: the other three rows of the level from lanes lane^1,2,3 and 16 DFMA.)
+//     once and one 64-bit shuffle per value brings the (transposed) result home — see deriv_i.
 //   * vertical integrals (PO:76-97, 280-312, 314-352) in scan form: warp-shuffle scans over the 8 levels of
 //     a warp (lane stride 4); the per-warp totals are combined over the nlev/8 warps of the column — inside a CTA
 //     through shared memory, between the CTAs of the cluster through distributed shared memory: a warp sends its
@@ -37,7 +36,7 @@
 // (~1e-15 relative); tests/test_parity_gpu.py holds it to 1e-12 per field.
 //
 // EUL instances: the Eulerian vertical coordinate (rsplit == 0), see the comment at the kernel.
-// CL = 1 (one CTA per element; -DCAAR_CL72=1) is the previous generation of this kernel, kept compilable.
+// Level counts up to 64 run with one CTA per element (CL = 1, at most 256 threads); see cluster_for().
 #pragma once
 #include <cstdio>
 #include <cstdlib>
@@ -190,26 +189,18 @@ __device__ __forceinline__ double2 lds2(const double* p) {
   return v;
 }
 
-// out[j] = sum_m Dvv[m][r] * s_m[j]; rows m of this level live in lanes lane^x; cx[x] = Dvv[r^x][r]
-__device__ __forceinline__ Row deriv_i(const Row& s, const double (&cx)[4]) {
-  Row o;
-#pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    double acc = cx[0] * s.x[j];
-#pragma unroll
-    for (int x = 1; x < 4; ++x) acc = fma(cx[x], __shfl_xor_sync(FULL, s.x[j], x), acc);
-    o.x[j] = acc;
-  }
-  return o;
-}
-// The same derivative on the FP64 tensor core (CAAR_DERIV_MMA): for a fixed jgp j the eight levels of a warp form ONE
-// 8x8x4 product D_j = A B_j with A[i'][m] = Dvv[m][i' & 3] (rows 4-7 repeat rows 0-3) and B_j[m][n] = s of level n at
-// (igp m, jgp j). In the mma.m8n8k4 fragment layout the thread lane = 4*level + igp holds exactly B_j[lane & 3][lane >> 2]
-// = its own x[j], and one constant element of A. The result lands transposed: thread (q = lane >> 2, c = lane & 3) holds
-// D_j[q][2c], D_j[q][2c+1] = the derivative at igp q & 3 of the levels 2c and 2c+1. Since the rows q and q + 4 are
-// copies, the lanes with q < 4 hand out their even level and the lanes with q >= 4 their odd one, and every thread
-// fetches its value with ONE 64-bit shuffle: 4 DMMA + 8 SHFL per call instead of 16 DFMA + 24 SHFL — a third of the
-// shared-memory-pipe wavefronts of the derivative (the L1 data pipe is this kernel's co-limiter, DESIGN.md 5.1).
+// The igp derivative out[j] = sum_m Dvv[m][r] * s_m[j] (s_m: row m of this level) on the FP64 tensor core: for a
+// fixed jgp j the eight levels of a warp form ONE 8x8x4 product D_j = A B_j with A[i'][m] = Dvv[m][i' & 3] (rows 4-7
+// repeat rows 0-3) and B_j[m][n] = s of level n at (igp m, jgp j). In the mma.m8n8k4 fragment layout the thread
+// lane = 4*level + igp holds exactly B_j[lane & 3][lane >> 2] = its own x[j], and one constant element of A. The
+// result lands transposed: thread (q = lane >> 2, c = lane & 3) holds D_j[q][2c], D_j[q][2c+1] = the derivative at
+// igp q & 3 of the levels 2c and 2c+1. Since the rows q and q + 4 are copies, the lanes with q < 4 hand out their even
+// level and the lanes with q >= 4 their odd one, and every thread fetches its value with ONE 64-bit shuffle: 4 DMMA +
+// 8 SHFL per call instead of 16 DFMA + 24 SHFL — a third of the shared-memory-pipe wavefronts of the derivative (the
+// L1 data pipe is this kernel's co-limiter, DESIGN.md 5.1). A/B against the shuffle form on one box
+// (profiles/r2u_mma_ab.jsonl): nlev 72 1.055 -> 1.065 of the measured peak at full clocks and 0.935 -> 1.014 on a
+// power-capped GPU (~1.6 GHz), aliased time levels 0.88 -> 0.91-0.98, Eulerian nlev 72 / 128 0.931 -> 0.984 /
+// 0.904 -> 0.952.
 struct DerivMma {
   double a;   // A[lane >> 2][lane & 3] = Dvv[lane & 3][(lane >> 2) & 3]
   int src;    // lane that holds this thread's result
@@ -251,8 +242,7 @@ __device__ __forceinline__ Row deriv_j(const Row& s, const double* __restrict__ 
 
 // gradient_sphere (PO/sphere_operators.cpp:9-48) for this thread's row; di = this row's Dinv*rrearth in smem,
 // [jgp][2*a+b]
-template <class CX>
-__device__ __forceinline__ void gradient(const Row& s, const double* di, const CX& cx,
+__device__ __forceinline__ void gradient(const Row& s, const double* di, const DerivMma& cx,
                                          const double* __restrict__ dvv, Row& g0, Row& g1) {
   const Row a = deriv_i(s, cx);   // v1[igp][jgp]
   const Row b = deriv_j(s, dvv);  // v2[igp][jgp]
@@ -282,35 +272,13 @@ __device__ __forceinline__ double scan_up(double v, int lane) {  // towards smal
   return v;
 }
 
-#ifndef CAAR_DERIV_MMA
-// 1 = igp derivatives of the fused kernel as DMMA.8x8x4 + one shuffle per value, 0 = 16 DFMA + 24 SHFL per call. A/B on one
-// box (profiles/r2u_mma_ab.jsonl): nlev 72 1.055 -> 1.065 of the measured peak at full clocks and 0.935 -> 1.014 on a
-// power-capped GPU (~1.6 GHz), aliased time levels 0.88 -> 0.91-0.98, Eulerian nlev 72 / 128 0.931 -> 0.984 / 0.904 -> 0.952
-#define CAAR_DERIV_MMA 1
-#endif
-#ifndef CAAR_EUL_REGS
-// register cap of the single-CTA (CL = 1) Eulerian nlev=72 instance. Its live set (dsave, dp, vtens, ttens through the scans) does not
-// fit 96 registers: measured 0.46 of the HBM peak at 96 (2 CTAs/SM, 480 B of spills), 0.55 at 128, 0.61 at 168
-// (1 CTA/SM, no spills) — profiles/README.md.
-#define CAAR_EUL_REGS 168
-#endif
 // Sum over the warps ww in [lo, hi) of the per-warp scan totals tot[ww][r*4 + j], j = 0..3, delivered to every lane
-// for its own GLL row r. Lane (q = lane/4, r) loads rows q, q+8, ... and the eight partial sums of a row meet in a
-// butterfly over the lane bits 2..4: 2*NWT/8 LDS.128 + 24 SHFL per call instead of up to 2*NWT LDS.128 per thread.
-// Used by every cluster instance (the carry chain of dependent DADDs becomes a 3-step butterfly).
-#ifndef CAAR_WARP_TOTALS_V2
-#define CAAR_WARP_TOTALS_V2 1
-#endif
-#ifndef CAAR_WT_BOTH
-#define CAAR_WT_BOTH CAAR_WARP_TOTALS_V2  // Eulerian, columns of at most 96 levels: carry and column total of div(v dp) from one pass
-                                          // (nlev 72 / 96: 0.919 -> 0.932 / 0.930; nlev 128: 0.904 -> 0.899, so not there)
-#endif
+// for its own GLL row r. Lane c (+16) sums column c of the rows lo, lo+2, ... (lo+1, lo+3, ...): one 256-byte LDS.64
+// per pair of rows, the two halves meet in one xor-shuffle and every lane picks the four columns of its GLL row: about
+// NWT + 10 shared-memory wavefronts per call against 40 for a butterfly over the lane bits 2..4 (which is what the
+// LSU-bound Eulerian instances feel).
 template <int NWT>
 __device__ __forceinline__ void warp_totals(const double (*tot)[16], int lo, int hi, int lane, double (&out)[4]) {
-#if CAAR_WARP_TOTALS_V2
-  // Lane c (+16) sums column c of the rows lo, lo+2, ... (lo+1, lo+3, ...): one 256-byte LDS.64 per pair of rows, the two
-  // halves meet in one xor-shuffle and every lane picks the four columns of its GLL row: about NWT + 10 shared-memory
-  // wavefronts per call against 40 for the butterfly below (which is what the LSU-bound Eulerian instances feel).
   const int c = lane & 15, h = lane >> 4, r = lane & 3;
   double acc = 0.0, acc2 = 0.0;
 #pragma unroll
@@ -326,28 +294,10 @@ __device__ __forceinline__ void warp_totals(const double (*tot)[16], int lo, int
   acc += __shfl_xor_sync(FULL, acc, 16);
 #pragma unroll
   for (int j = 0; j < 4; ++j) out[j] = __shfl_sync(FULL, acc, r * 4 + j);
-#else
-  const int q = lane >> 2, r = lane & 3;
-  double acc[4] = {0, 0, 0, 0};
-#pragma unroll
-  for (int base = 0; base < NWT; base += 8) {
-    const int ww = base + q;
-    if (ww < NWT && ww >= lo && ww < hi) {
-      const Row c = ld_row(&tot[ww][r * 4]);
-#pragma unroll
-      for (int j = 0; j < 4; ++j) acc[j] += c.x[j];
-    }
-  }
-#pragma unroll
-  for (int d = 4; d < 32; d <<= 1)
-#pragma unroll
-    for (int j = 0; j < 4; ++j) acc[j] += __shfl_xor_sync(FULL, acc[j], d);
-#pragma unroll
-  for (int j = 0; j < 4; ++j) out[j] = acc[j];
-#endif
 }
 // The same pass delivering two sums: rows [0, hi) (the carry of this warp) and all NWT rows (the column total that the
-// Eulerian branch needs next): one set of loads instead of two calls.
+// Eulerian branch needs next): one set of loads instead of two calls. Used for columns of at most 96
+// levels (NWT <= 12): A/B nlev 72 / 96 0.919 -> 0.932 / 0.930 of the measured peak, nlev 128 0.904 -> 0.899.
 template <int NWT>
 __device__ __forceinline__ void warp_totals_both(const double (*tot)[16], int hi, int lane, double (&pre)[4],
                                                  double (&all)[4]) {
@@ -377,28 +327,16 @@ __device__ __forceinline__ void warp_totals_both(const double (*tot)[16], int hi
   }
 }
 
-#ifndef CAAR_PARK
-#define CAAR_PARK 1
-#endif
-#ifndef CAAR_EUL_HOIST
-#define CAAR_EUL_HOIST 56  // Eulerian instances with at least this many levels per CTA issue the block's two global loads
-                           // (dp3d re-read, eta_dot_dpdn) at its start: A/B nlev=128 (64 levels per CTA) 0.847 -> 0.861 of
-                           // the measured peak, nlev=72 (24 per CTA) 0.878 -> 0.849 (the 16 live registers cost more there)
-#endif
-#ifndef CAAR_CL72
-#define CAAR_CL72 3   // nlev = 72: the column is split over a cluster of three 96-thread CTAs (24 levels each)
-#endif
-#ifndef CAAR_CL128
-#define CAAR_CL128 2  // nlev = 128: the column is split over a cluster of two 256-thread CTAs
-#endif
-#ifndef CAAR_REGS_SMALL
-#define CAAR_REGS_SMALL 96  // CL = 1, nlev = 72: 2 CTAs of 9 warps per SM = 5 warps on the fullest SMSP: 16384/(5*32) = 102 -> 96
-#endif
+// Eulerian instances with at least this many levels per CTA issue the block's two global loads (dp3d re-read,
+// eta_dot_dpdn) at its start: A/B nlev=128 (64 levels per CTA) 0.847 -> 0.861 of the measured peak, nlev=72 (24 per
+// CTA) 0.878 -> 0.849 (the 16 live registers cost more there)
+constexpr int EUL_HOIST_LEVELS = 56;
 
 // CTAs per element (cluster size) for every level count with a compiled instance; 0 = none.
 // Levels per CTA = nlev / cluster_for(nlev), a multiple of 8 (a warp scans 8 levels).
+// nlev = 72: a cluster of three 96-thread CTAs (24 levels each); nlev = 128: a cluster of two 256-thread CTAs.
 __host__ __device__ constexpr int cluster_for(int nlev) {
-  return nlev == 72 ? CAAR_CL72 : nlev == 128 ? CAAR_CL128
+  return nlev == 72 ? 3 : nlev == 128 ? 2
          : (nlev >= 8 && nlev <= 64 && nlev % 8 == 0) ? 1
          : nlev == 80 ? 2 : nlev == 96 ? 3 : nlev == 112 ? 2 : nlev == 120 ? 3 : 0;
 }
@@ -410,21 +348,13 @@ __host__ __device__ constexpr int instance_for(int nlev) {
          : nlev <= 112 ? 112 : nlev <= 120 ? 120 : nlev <= 128 ? 128 : 0;
 }
 
-// register budget per thread for a CTA of `threads` threads
-constexpr int regs_for(int threads, bool eul = false) {
-  return (eul && threads > 256 && threads <= 320 && CAAR_EUL_REGS > 0) ? CAAR_EUL_REGS  // CL = 1 Eulerian nlev = 72: one 288-thread CTA per SM
-         : threads <= 256 ? 128              // cluster CTAs: 5 x 96 or 2 x 256 threads x 128 registers per SM
-         : threads <= 320 ? CAAR_REGS_SMALL  // CL = 1: 2 x 288 threads (nlev = 72)
-                          : 128;             // CL = 1: one 512-thread CTA per SM (nlev = 128)
-}
-
-// Park the two velocity-tendency rows in shared memory through the scan phase (instead of letting the compiler spill
-// them to local memory)? Each thread reuses its OWN 32 bytes of the T(n0) and Qdp input tiles, which it alone reads
-// and which are dead by then — no extra shared memory. Only where registers are short: nlev=72 Lagrangian.
-__host__ __device__ constexpr bool park_for(int L, int CL, bool eul) { return CAAR_PARK && L == 72 && CL == 1 && !eul; }
+// register budget per thread of every instance (CTAs of at most 256 threads: 5 x 96 or 2 x 256 threads per SM).
+// A function of the block size because nvcc (12.9) rejects a literal __maxnreg__ next to __launch_bounds__ and takes
+// both only when the cap depends on a template parameter.
+constexpr int regs_for(int /*threads*/) { return 128; }
 
 // L = levels held by this CTA, NWT = warps per element (scan totals of the whole column), EUL = Eulerian variant
-template <int L, int NWT, bool EUL, bool PARK = false>
+template <int L, int NWT, bool EUL>
 struct Smem {
   static constexpr int LF = L * PTS;  // doubles per scalar level-field (this CTA's slab)
   // late inputs, overwritten in place by the outputs of the same shape
@@ -458,7 +388,7 @@ struct Smem {
 // global memory (L1/L2 hits: neighbouring threads loaded them), derived_eta_dot_dpdn is updated in place, and the
 // dp3d update moves behind the scan. +259 B per element*level of algorithmic traffic (the eta_dot_dpdn RMW).
 template <int L, int CL, bool EUL>
-__global__ void __launch_bounds__(4 * L / CL) __maxnreg__(regs_for(4 * L / CL, EUL))
+__global__ void __launch_bounds__(4 * L / CL) __maxnreg__(regs_for(4 * L / CL))
 caar_fused_kernel(const __grid_constant__ KernelArgs A, const __grid_constant__ TmaMaps M) {
   constexpr int LC = L / CL;        // levels per CTA
   constexpr int NW = LC / 8;        // warps per CTA
@@ -469,8 +399,7 @@ caar_fused_kernel(const __grid_constant__ KernelArgs A, const __grid_constant__ 
   static_assert(L % (8 * CL) == 0, "a warp holds 8 levels");
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   // swizzled TMA tiles need 1024-byte alignment; the launch adds 1 KB of slack for this round-up
-  constexpr bool PARK = park_for(L, CL, EUL);
-  Smem<LC, NWT, EUL, PARK>& S = *reinterpret_cast<Smem<LC, NWT, EUL, PARK>*>(smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u));
+  Smem<LC, NWT, EUL>& S = *reinterpret_cast<Smem<LC, NWT, EUL>*>(smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u));
 
   const int t = threadIdx.x;
   const int lane = t & 31, w = t >> 5;
@@ -582,19 +511,7 @@ caar_fused_kernel(const __grid_constant__ KernelArgs A, const __grid_constant__ 
     }
   }
 
-#if CAAR_DERIV_MMA
   const DerivMma cx = deriv_mma_setup(A.dvv, lane);  // igp derivatives on the FP64 tensor core (see deriv_i)
-#else
-  double cx[4];  // cx[x] = Dvv[r^x][r]; static indices + selects keep Dvv in the constant bank
-#pragma unroll
-  for (int x = 0; x < 4; ++x) {
-    double c = A.dvv[(0 ^ x) * 4 + 0];
-    if (r == 1) c = A.dvv[(1 ^ x) * 4 + 1];
-    if (r == 2) c = A.dvv[(2 ^ x) * 4 + 2];
-    if (r == 3) c = A.dvv[(3 ^ x) * 4 + 3];
-    cx[x] = c;
-  }
-#endif
 
   // ---- A: p = hyai0*ps0 + sum_{l<k} dp_l + dp_k/2   (PO:76-97)
   Row rp;
@@ -610,10 +527,10 @@ caar_fused_kernel(const __grid_constant__ KernelArgs A, const __grid_constant__ 
     }
     __syncthreads();  // (1) tot[0], geometry, mbarrier init visible
     if (CL > 1 && rank > 0) mbar_wait(&S.xbar[0], 0);  // the lower ranks' totals have landed
-    // see warp_totals(). A/B: nlev=128 0.831 -> 0.844 (Eulerian 0.575 -> 0.674); nlev=72 on CTA triples 0.965 -> 0.993
-    // (and no spills left); only the single-CTA nlev=72 instance at 96 registers is better off with the plain loop
-    // (0.902 vs 0.899)
-    constexpr bool LANE_CARRY = (CL > 1) || (NWT >= 16) || EUL;
+    // The cluster and Eulerian instances combine the warp totals with warp_totals(). A/B: nlev=128 0.831 -> 0.844
+    // (Eulerian 0.575 -> 0.674); nlev=72 on CTA triples 0.965 -> 0.993 (and no spills left). The single-CTA Lagrangian
+    // instances (at most 8 warps) keep the plain loop; warp_totals() has not been measured there.
+    constexpr bool LANE_CARRY = (CL > 1) || EUL;
     double carry[4] = {0, 0, 0, 0};
     if constexpr (LANE_CARRY) {
       warp_totals<NWT>(S.tot[0], 0, gw, lane, carry);
@@ -655,9 +572,9 @@ caar_fused_kernel(const __grid_constant__ KernelArgs A, const __grid_constant__ 
     Row gp0, gp1;
     // w = Dinv.v: v.grad(s) = a_s*w1 + b_s*w2 with (a_s,b_s) the raw igp/jgp derivatives of s
     // (PO/sphere_operators.cpp:21-47), and the divergence flux is metdet*dp*w (PO/sphere_operators.cpp:62-72): one
-    // pass over Dinv serves -v.grad T (PO:200-209) and divergence_sphere(v*dp) (PO:122). Where registers allow
-    // (the 128-register instances) the same pass also produces grad p; at 96 registers that costs more in spill
-    // reloads than the 8 LDS.128 it saves (measured 0.845 vs 0.891), so w is formed later there.
+    // pass over Dinv serves -v.grad T (PO:200-209) and divergence_sphere(v*dp) (PO:122). In the cluster instances
+    // the same pass also produces grad p, which saves 8 LDS.128; the single-CTA instances form w after grad p.
+    // Whether they would gain from the fused pass has not been measured.
     constexpr bool FUSE_W = (CL > 1);
     Row w1, w2;
     if constexpr (FUSE_W) {
@@ -710,10 +627,6 @@ caar_fused_kernel(const __grid_constant__ KernelArgs A, const __grid_constant__ 
       const Row a = deriv_i(T, cx), b = deriv_j(T, A.dvv);
 #pragma unroll
       for (int j = 0; j < 4; ++j) ttp.x[j] = -fma(a.x[j], w1.x[j], b.x[j] * w2.x[j]);
-    }
-    if (PARK) {  // vtens (without grad Ephi) is not needed before the end of the kernel
-      st_tile(S.Tn0, sw1, vt1);
-      st_tile(S.Qd, sw1, vt2);
     }
     if (EUL) st_tile(S.Qd, sw1, vt2);  // Eulerian: T(n0) stays in use (vertical neighbours), the Qdp slot is free
 
@@ -823,7 +736,7 @@ caar_fused_kernel(const __grid_constant__ KernelArgs A, const __grid_constant__ 
     double S4[4] = {0, 0, 0, 0};  // Eulerian: column total of div(v dp)
     if constexpr (LANE_CARRY) {
       warp_totals<NWT>(S.tot[1], gw + 1, NWT, lane, cq);
-      if constexpr (EUL && CAAR_WT_BOTH && NWT <= 12) warp_totals_both<NWT>(S.tot[2], gw, lane, cd, S4);
+      if constexpr (EUL && NWT <= 12) warp_totals_both<NWT>(S.tot[2], gw, lane, cd, S4);
       else warp_totals<NWT>(S.tot[2], 0, gw, lane, cd);
     } else {
 #pragma unroll
@@ -845,7 +758,7 @@ caar_fused_kernel(const __grid_constant__ KernelArgs A, const __grid_constant__ 
     mbar_wait(&S.bar[1], 0);
     const Row mp = ld_row(S.mp + r * 4);
     Row eta_old, dpk_early;  // Eulerian: the two global loads of this block, issued before the math that hides their latency
-    constexpr bool HOIST = EUL && (CAAR_EUL_HOIST > 0) && (LC >= CAAR_EUL_HOIST);
+    constexpr bool HOIST = EUL && LC >= EUL_HOIST_LEVELS;
     if (EUL) {
       if (HOIST && live) {
         dpk_early = ld_row(A.dp3d + on0);
@@ -871,16 +784,7 @@ caar_fused_kernel(const __grid_constant__ KernelArgs A, const __grid_constant__ 
       st_tile(S.pec, sw1, ph);
       // column total S of div(v dp) and the vertical mass flux at this level's two interfaces
       // (F/routine_extracted.F90:233-254): eta(k+1) = hybi(k+1)*S - sum_{l<=k} divdp_l, 0 at the top and bottom
-      if constexpr (LANE_CARRY) {
-        if constexpr (!(CAAR_WT_BOTH && NWT <= 12)) warp_totals<NWT>(S.tot[2], 0, NWT, lane, S4);
-      } else {
-#pragma unroll
-        for (int ww = 0; ww < NWT; ++ww) {
-          const Row c = ld_row(&S.tot[2][ww][r * 4]);
-#pragma unroll
-          for (int j = 0; j < 4; ++j) S4[j] += c.x[j];
-        }
-      }
+      if constexpr (NWT > 12) warp_totals<NWT>(S.tot[2], 0, NWT, lane, S4);  // else warp_totals_both delivered it
       const int kg = lev0 + (t >> 2);
       const double hb_lo = A.hybi[kg < nl ? kg : nl], hb_hi = A.hybi[kg < nl ? kg + 1 : nl];
       Row ehi, elo;
@@ -986,10 +890,6 @@ caar_fused_kernel(const __grid_constant__ KernelArgs A, const __grid_constant__ 
       gradient(kep, S.dinv + r * GS, cx, A.dvv, g0, g1);
       Row a0, a1;
       ld_tile2(S.vm1, sw2, a0, a1);
-      if (PARK) {
-        vt1 = ld_tile(S.Tn0, sw1);
-        vt2 = ld_tile(S.Qd, sw1);
-      }
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
         a0.x[j] = mp.x[j] * fma(A.dt2, vt1.x[j] - g0.x[j], a0.x[j]);
@@ -1020,10 +920,9 @@ caar_fused_kernel(const __grid_constant__ KernelArgs A, const __grid_constant__ 
 
 template <int L, int CL, bool EUL>
 cudaError_t launch_L(const KernelArgs& a, cudaStream_t s) {
-  static_assert((4 * L / CL) * regs_for(4 * L / CL, EUL) <= 65536, "one CTA must fit the 64K-register file of an SM");
   const int n = a.nete - a.nets;
   if (n <= 0) return cudaSuccess;
-  constexpr int SMEM = (int)sizeof(Smem<L / CL, L / 8, EUL, park_for(L, CL, EUL)>) + 1024;
+  constexpr int SMEM = (int)sizeof(Smem<L / CL, L / 8, EUL>) + 1024;
   // function attributes are per device: set once per (instance, device), not on every launch
   static bool configured[64] = {};
   int dev = 0;

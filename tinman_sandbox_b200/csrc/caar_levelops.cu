@@ -100,6 +100,18 @@ __device__ __forceinline__ void dvv_row(const double* __restrict__ dvv, int r, d
     c[m] = x;
   }
 }
+// out[j] = sum_m Dvv[m][r] * s_m[j]; rows m of this level live in lanes lane^x; cx[x] = Dvv[r^x][r]
+__device__ __forceinline__ Row deriv_i_shfl(const Row& s, const double (&cx)[4]) {
+  Row o;
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    double acc = cx[0] * s.x[j];
+#pragma unroll
+    for (int x = 1; x < 4; ++x) acc = fma(cx[x], __shfl_xor_sync(FULL, s.x[j], x), acc);
+    o.x[j] = acc;
+  }
+  return o;
+}
 
 enum { OP_EULER = 0, OP_DIVWK = 1, OP_LAP_SIMPLE = 2, OP_LAP_TENSOR = 3 };
 
@@ -335,8 +347,8 @@ __global__ void __launch_bounds__(32 * WPC, LEVELOP_MINB) levelop_kernel(const _
         ld_tile2(reinterpret_cast<const double*>(tile), sw2, g0, g1);
       } else {
         const Row sc = ld_tile(reinterpret_cast<const double*>(tile), sw1);
-        g0 = deriv_i(sc, cx);     // sum_m Dvv[m][r] s(m,j)   (PO/sphere_operators.cpp:21-35)
-        g1 = deriv_j(sc, A.dvv);  // sum_m Dvv[m][j] s(r,m)
+        g0 = deriv_i_shfl(sc, cx);  // sum_m Dvv[m][r] s(m,j)   (PO/sphere_operators.cpp:21-35)
+        g1 = deriv_j(sc, A.dvv);    // sum_m Dvv[m][j] s(r,m)
       }
       if (lane == 0) asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(NO - 1) : "memory");
       __syncwarp();
@@ -590,11 +602,6 @@ __global__ void __launch_bounds__(32 * FW, LAPFLAT_MINB) laplace_flat_kernel(con
       }
     }
     unsigned char* otile = out_tiles + (i % FO) * FT_B;
-#if defined(LAPFLAT_DIAG_COPY)  // development: the pipeline without the math
-#pragma unroll
-    for (int c = 0; c < 8; ++c)
-      *reinterpret_cast<double2*>(otile + swz + (((uint32_t)c ^ x7) << 4)) = make_double2(sv[2 * c], sv[2 * c + 1] + (double)e_t);
-#else
     // raw derivatives: g0(i,j) = sum_m Dvv[m][i] s(m,j), g1(i,j) = sum_m Dvv[m][j] s(i,m); then s = N g in place
     double g0[16], g1[16];
 #pragma unroll
@@ -635,7 +642,6 @@ __global__ void __launch_bounds__(32 * FW, LAPFLAT_MINB) laplace_flat_kernel(con
       }
       *reinterpret_cast<double2*>(otile + swz + (((uint32_t)c ^ x7) << 4)) = make_double2(o[0], o[1]);
     }
-#endif
     __syncwarp();  // after a jump the staged elements may take the cache slots this tile was reading
     if (gb_ok) store_n(gb_e, gb);
     if (filled < gb_hi) filled = gb_hi;
@@ -837,9 +843,8 @@ cudaError_t launch_levelop(int op, const KernelArgs& k, const double* in, const 
     sphere_wk_strict_kernel<<<(unsigned)((rows + 15) / 16), 256, 0, s>>>(a);
     return cudaGetLastError();
   }
-  static const bool lap_v1 = [] { const char* v = getenv("CAAR_LAPLACE_V1"); return v && atoi(v) != 0; }();
   const long long flat_rows = (long long)(nete - nets) * k.nlev;
-  if (op >= 2 && !lap_v1 && k.nlev >= 16 && flat_rows + FT < (1ll << 31)) {  // thread-per-level laplacians
+  if (op >= 2 && k.nlev >= 16 && flat_rows + FT < (1ll << 31)) {  // thread-per-level laplacians
     LapFlatArgs a;
     a.Dinv = k.Dinv; a.spheremp = k.spheremp; a.tensorvisc = tensorvisc;
     a.nlev = k.nlev; a.nets = nets; a.rows = flat_rows; a.tiles = (flat_rows + FT - 1) / FT; a.rrearth = k.rrearth;

@@ -5,7 +5,7 @@ kinds alone.
 Prints one JSON line per configuration and mode:
   ms_per_step         CUDA events around --steps back-to-back steps, best of 3 windows, after a warm-up step
   kind_ms             kernel time of each launch kind from a torch.profiler capture of --steps steps: the stage
-                      (levelop_kernel<OP_EULER> in fast mode, euler_step_kernel<true> in strict mode; the mean of the
+                      (levelop_kernel<OP_EULER> in fast mode, euler_step_kernel in strict mode; the mean of the
                       three stages) and the average (combine_kernel<QdpAverage>)
   euler_step_ms       caar_euler_step (into CAAR_X_QTENS) at the same size and dt/2, event-timed in windows that
                       alternate with the step windows: the fast stage runs its body, so the two rates should match

@@ -8,7 +8,6 @@ echo "pytest rc=$?" >> $OUT/r2e_pytest.log
 for q in 1 4 8; do timeout 300 python tools/levelop_bench.py --nelem 21600 --nlev 72 --qsize $q --ops euler --modes fast; done
 timeout 300 python tools/levelop_bench.py --nelem 2700 --nlev 72 --qsize 35 --ops euler --modes fast
 timeout 300 python tools/levelop_bench.py --nelem 10800 --nlev 128 --qsize 8 --ops euler --modes fast
-CAAR_EULER_V1=1 timeout 300 python tools/levelop_bench.py --nelem 21600 --nlev 72 --qsize 4 --ops euler --modes fast
 timeout 300 python tools/levelop_bench.py --nelem 43200 --nlev 72 --qsize 1 --ops divwk,lap,lapt
 timeout 300 python tools/levelop_bench.py --nelem 43200 --nlev 30 --qsize 1 --ops lap --modes fast
 CAAR_LEVELOP_WAVES=1 timeout 300 python tools/levelop_bench.py --nelem 21600 --nlev 72 --qsize 4 --ops euler,lap --modes fast

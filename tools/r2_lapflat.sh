@@ -12,8 +12,6 @@ for W in 2 4; do
   CAAR_LEVELOP_WAVES=$W run python tools/levelop_bench.py --ops lap,lapt --modes fast --nlev 72
   echo "# ^ waves=$W" >> $OUT/lf_bench.jsonl
 done
-CAAR_LAPLACE_V1=1 run python tools/levelop_bench.py --ops lap,lapt --modes fast --nlev 72
-echo "# ^ first generation" >> $OUT/lf_bench.jsonl
 for v in a b c d; do
   for L in 72 128; do
     run python tools/levelop_bench.py --ops lap,lapt --modes fast --nlev $L --lib tools/_variants/libcaar_b200_lf_$v.so
