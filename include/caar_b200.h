@@ -354,7 +354,8 @@ int caar_run_host(caar_handle h, const caar_arrays* host, const caar_control* ct
    Needs every array page-locked AND device-mapped (caar_host_register, cudaHostAlloc, torch pinned memory);
    fails with CAAR_ERR_INVALID otherwise. The device mirrors are NOT updated on this path. */
 #define CAAR_HOST_ZERO_COPY (-1)
-/* bytes one caar_run_host call with this control moves in each direction */
+/* bytes one caar_run_host call with this control moves in each direction; CAAR_ERR_INVALID for a null argument, a
+   bad control or a bad mode */
 int caar_host_traffic(caar_handle h, const caar_control* ctl, int mode, size_t* h2d_bytes, size_t* d2h_bytes);
 
 /* Reference-facing one-shot: create -> set_params -> caar_run_host -> destroy on `device`, i.e. exactly what

@@ -3,16 +3,11 @@
 #include <cstdarg>
 #include <cstddef>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <initializer_list>
 #include <new>
 
 #include "caar_device.cuh"
-
-#ifndef CAAR_HOST_DEFAULT_ZERO_COPY
-#define CAAR_HOST_DEFAULT_ZERO_COPY 0  // chunk_elems == 0 uses the staged pipeline unless CAAR_HOST_PATH=zerocopy
-#endif
 
 namespace {
 
@@ -69,7 +64,7 @@ struct caar_handle_s {
   long long launches;
   caar::TmaMaps* tma;  // TMA descriptors of the device mirrors (nlev with a TMA-pipelined kernel only)
   // caar_run_host pipeline: copy-in and copy-out streams, two events per element chunk (grown on demand)
-  cudaStream_t s_in, s_in2, s_out;  // s_in2: second copy-in stream (CAAR_HOST_IN_STREAMS=2)
+  cudaStream_t s_in, s_out;
   cudaEvent_t* chunk_ev;
   int n_chunk_ev;
   cudaEvent_t ev_fence;
@@ -111,36 +106,51 @@ struct DeviceGuard {
   }
 };
 
+// the argument checks every entry point shares; each returns CAAR_OK or the error code (and sets the message)
+int check_handle(const caar_handle_s* h, const char* who) {
+  if (!h) return fail(CAAR_ERR_INVALID, "%s: null handle", who);
+  if (!h->params_set) return fail(CAAR_ERR_STATE, "caar_set_params must be called before %s", who);
+  return CAAR_OK;
+}
+int check_range(const caar_handle_s* h, int nets, int nete) {
+  if (nets < 0 || nete > h->dims.nelem || nets > nete)
+    return fail(CAAR_ERR_INVALID, "element range [%d,%d) outside [0,%d)", nets, nete, h->dims.nelem);
+  return CAAR_OK;
+}
+int check_mode(int mode) {
+  if (mode != CAAR_MODE_FAST && mode != CAAR_MODE_STRICT) return fail(CAAR_ERR_INVALID, "mode=%d", mode);
+  return CAAR_OK;
+}
+int check_time_level(const caar_handle_s* h, int tl) {
+  if (tl < 0 || tl >= h->dims.ntl) return fail(CAAR_ERR_INVALID, "time level %d outside [0,%d)", tl, h->dims.ntl);
+  return CAAR_OK;
+}
+
 int validate_control(const caar_handle_s* h, const caar_control* ctl) {
-  const caar_dims& d = h->dims;
   if (!ctl) return fail(CAAR_ERR_INVALID, "control is null");
-  if (ctl->nets < 0 || ctl->nete > d.nelem || ctl->nets > ctl->nete)
-    return fail(CAAR_ERR_INVALID, "element range [%d,%d) outside [0,%d)", ctl->nets, ctl->nete, d.nelem);
-  const int tl[3] = {ctl->n0, ctl->np1, ctl->nm1};
-  for (int i = 0; i < 3; ++i)
-    if (tl[i] < 0 || tl[i] >= d.ntl) return fail(CAAR_ERR_INVALID, "time level %d outside [0,%d)", tl[i], d.ntl);
+  if (int rc = check_range(h, ctl->nets, ctl->nete)) return rc;
+  for (int tl : {ctl->n0, ctl->np1, ctl->nm1})
+    if (int rc = check_time_level(h, tl)) return rc;
   if (ctl->qn0 < -1 || ctl->qn0 >= 2) return fail(CAAR_ERR_INVALID, "qn0=%d must be -1, 0 or 1", ctl->qn0);
   return CAAR_OK;
 }
 
-// the fused kernels cover the vertically Lagrangian branch, and the Eulerian one where launch_fused says so;
-// everything else runs on the generic reference-order kernel (still on the GPU)
-bool uses_fused(const caar_handle_s* h, int mode) {
-  const bool fused = mode == CAAR_MODE_FAST && caar::fused_supports(h->dims.nlev) &&
-                     (h->rsplit > 0 || caar::fused_supports_eulerian(h->dims.nlev));
-  if (mode == CAAR_MODE_FAST && !fused) {  // never silent: the reference-order kernel is ~6x slower
-    static bool told = false;
-    if (!told) {
-      told = true;
-      fprintf(stderr, "[caar] CAAR_MODE_FAST: no fused kernel instance for nlev=%d (instances cover nlev <= 128); "
-                      "running the reference-order kernel instead (see caar_describe)\n", h->dims.nlev);
-    }
-  }
-  return fused;
+// the fused kernels cover both vertical coordinates at every nlev they support; everything else runs on the generic
+// reference-order kernel (still on the GPU)
+bool selects_fused(const caar_handle_s* h, int mode) {
+  return mode == CAAR_MODE_FAST && caar::fused_supports(h->dims.nlev);
 }
 // eta_dot_dpdn travels when the kernel really updates it: the reference-order kernel always does (+= 0 included),
 // the fused kernels only on the Eulerian branch
-bool moves_eta(const caar_handle_s* h, int mode) { return !uses_fused(h, mode) || h->rsplit == 0; }
+bool moves_eta(const caar_handle_s* h, int mode) { return !selects_fused(h, mode) || h->rsplit == 0; }
+
+// caar_destroy that leaves caar_last_error() with the error that made the caller give up on the handle
+void destroy_keeping_error(caar_handle_s* h) {
+  char keep[sizeof g_err];
+  std::memcpy(keep, g_err, sizeof keep);
+  caar_destroy(h);
+  std::memcpy(g_err, keep, sizeof keep);
+}
 
 caar::KernelArgs make_args(const caar_handle_s* h, const caar_control* ctl, double* const* ptr = nullptr) {
   caar::KernelArgs a;
@@ -194,7 +204,7 @@ int caar_create(caar_handle* out, const caar_dims* dims, int device) {
   if (dims->nelem < 1 || dims->nlev < 2 || dims->qsize_d < 1 || dims->ntl < 1)
     return fail(CAAR_ERR_INVALID, "bad dims nelem=%d nlev=%d qsize_d=%d ntl=%d", dims->nelem, dims->nlev,
                 dims->qsize_d, dims->ntl);
-  if (caar::strict_smem_bytes(dims->nlev) > 200 * 1024 && !caar::fused_supports(dims->nlev))
+  if (!caar::strict_supports(dims->nlev) && !caar::fused_supports(dims->nlev))
     return fail(CAAR_ERR_UNSUPPORTED, "nlev=%d not covered by the compiled kernels", dims->nlev);
   int ndev = 0;
   CU_TRY(cudaGetDeviceCount(&ndev));
@@ -211,7 +221,6 @@ int caar_create(caar_handle* out, const caar_dims* dims, int device) {
   if (e == cudaSuccess) e = cudaEventCreate(&h->ev1);
   if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->ev_fence, cudaEventDisableTiming);
   if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&h->s_in, cudaStreamNonBlocking);
-  if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&h->s_in2, cudaStreamNonBlocking);
   if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&h->s_out, cudaStreamNonBlocking);
   for (int f = 0; f < CAAR_NUM_FIELDS && e == cudaSuccess; ++f) {
     const size_t bytes = field_count(*dims, f) * sizeof(double);
@@ -228,10 +237,7 @@ int caar_create(caar_handle* out, const caar_dims* dims, int device) {
   if (e != cudaSuccess) {
     const int code = fail(e == cudaErrorMemoryAllocation ? CAAR_ERR_NOMEM : CAAR_ERR_CUDA, "caar_create: %s",
                           cudaGetErrorString(e));
-    char keep[sizeof g_err];
-    std::memcpy(keep, g_err, sizeof keep);
-    caar_destroy(h);
-    std::memcpy(g_err, keep, sizeof keep);
+    destroy_keeping_error(h);
     cudaGetLastError();
     return code;
   }
@@ -270,7 +276,6 @@ int caar_destroy(caar_handle h) {
   for (int i = 0; i < h->n_chunk_ev; ++i) cudaEventDestroy(h->chunk_ev[i]);
   delete[] h->chunk_ev;
   if (h->s_in) cudaStreamSynchronize(h->s_in), cudaStreamDestroy(h->s_in);
-  if (h->s_in2) cudaStreamSynchronize(h->s_in2), cudaStreamDestroy(h->s_in2);
   if (h->s_out) cudaStreamSynchronize(h->s_out), cudaStreamDestroy(h->s_out);
   if (h->own_stream) cudaStreamDestroy(h->own_stream);
   delete h->tma;
@@ -316,27 +321,10 @@ int caar_set_stream(caar_handle h, void* cuda_stream) {
   return CAAR_OK;
 }
 
-static int copy_fields(caar_handle h, const caar_arrays* host, unsigned mask, bool to_device) {
-  if (!h || !host) return fail(CAAR_ERR_INVALID, "null argument");
-  DeviceGuard guard(h->device);
-  double* const* tab = as_table(host);
-  for (int f = 0; f < CAAR_NUM_FIELDS; ++f) {
-    if (!(mask & (1u << f))) continue;
-    if (!tab[f]) return fail(CAAR_ERR_INVALID, "host pointer of field %d is null", f);
-    const size_t bytes = field_count(h->dims, f) * sizeof(double);
-    if (to_device)
-      CU_TRY(cudaMemcpyAsync(h->dev[f], tab[f], bytes, cudaMemcpyHostToDevice, h->stream));
-    else
-      CU_TRY(cudaMemcpyAsync(tab[f], h->dev[f], bytes, cudaMemcpyDeviceToHost, h->stream));
-  }
-  CU_TRY(cudaStreamSynchronize(h->stream));
-  return CAAR_OK;
-}
-
 // element range [e0,e1) of the selected fields <-> host arrays that hold ONLY that range
 static int copy_range(caar_handle h, const caar_arrays* host, unsigned mask, int e0, int e1, bool to_device) {
   if (!h || !host) return fail(CAAR_ERR_INVALID, "null argument");
-  if (e0 < 0 || e1 > h->dims.nelem || e0 > e1) return fail(CAAR_ERR_INVALID, "element range [%d,%d) outside [0,%d)", e0, e1, h->dims.nelem);
+  if (int rc = check_range(h, e0, e1)) return rc;
   DeviceGuard guard(h->device);
   double* const* tab = as_table(host);
   for (int f = 0; f < CAAR_NUM_FIELDS; ++f) {
@@ -359,8 +347,12 @@ int caar_download_range(caar_handle h, const caar_arrays* host, unsigned mask, i
   return copy_range(h, host, mask, e0, e1, false);
 }
 
-int caar_upload(caar_handle h, const caar_arrays* host, unsigned mask) { return copy_fields(h, host, mask, true); }
-int caar_download(caar_handle h, const caar_arrays* host, unsigned mask) { return copy_fields(h, host, mask, false); }
+// every element of the selected fields (copy_range rejects a null handle before it uses the range)
+static int copy_all(caar_handle h, const caar_arrays* host, unsigned mask, bool to_device) {
+  return copy_range(h, host, mask, 0, h ? h->dims.nelem : 0, to_device);
+}
+int caar_upload(caar_handle h, const caar_arrays* host, unsigned mask) { return copy_all(h, host, mask, true); }
+int caar_download(caar_handle h, const caar_arrays* host, unsigned mask) { return copy_all(h, host, mask, false); }
 
 // ---- Fortran (F90 flat pointer) host layout: copies go through a device staging buffer and a relayout kernel
 static const size_t kStageBytes = (size_t)256 << 20;
@@ -414,13 +406,13 @@ static int copy_fields_f90(caar_handle h, const caar_arrays* host, unsigned mask
 }
 
 int caar_upload_layout(caar_handle h, const caar_arrays* host, unsigned mask, int layout) {
-  if (layout == CAAR_LAYOUT_CXX) return copy_fields(h, host, mask, true);
+  if (layout == CAAR_LAYOUT_CXX) return copy_all(h, host, mask, true);
   if (layout == CAAR_LAYOUT_F90) return copy_fields_f90(h, host, mask, true);
   return fail(CAAR_ERR_INVALID, "layout=%d", layout);
 }
 
 int caar_download_layout(caar_handle h, const caar_arrays* host, unsigned mask, int layout) {
-  if (layout == CAAR_LAYOUT_CXX) return copy_fields(h, host, mask, false);
+  if (layout == CAAR_LAYOUT_CXX) return copy_all(h, host, mask, false);
   if (layout == CAAR_LAYOUT_F90) return copy_fields_f90(h, host, mask, false);
   return fail(CAAR_ERR_INVALID, "layout=%d", layout);
 }
@@ -454,9 +446,9 @@ int caar_device_arrays(caar_handle h, caar_arrays* out) {
 
 int caar_describe(caar_handle h, int mode, char* buf, size_t len, int* is_fused) {
   if (!h || !buf || !len) return fail(CAAR_ERR_INVALID, "null argument");
-  if (mode != CAAR_MODE_FAST && mode != CAAR_MODE_STRICT) return fail(CAAR_ERR_INVALID, "mode=%d", mode);
+  if (int rc = check_mode(mode)) return rc;
   const int nlev = h->dims.nlev;
-  const bool fused = mode == CAAR_MODE_FAST && caar::fused_supports(nlev);
+  const bool fused = selects_fused(h, mode);
   if (fused)
     snprintf(buf, len, "caar_fused_kernel<%d,%d,%d>: nlev=%d%s, %d CTA(s) of %d threads per element",
              caar::fused_instance_levels(nlev), caar::fused_instance_cluster(nlev), h->rsplit == 0 ? 1 : 0, nlev,
@@ -471,15 +463,23 @@ int caar_describe(caar_handle h, int mode, char* buf, size_t len, int* is_fused)
 
 namespace {
 
-// The checks of caar_run and caar_run_rk5; *fast = the kernel `mode` selects on this handle (fused or strict)
+// The checks of caar_run, caar_run_rk5 and caar_run_host; *fast = the kernel `mode` selects on this handle (fused or
+// strict)
 int check_run(caar_handle h, const caar_control* ctl, int nsteps, int mode, const char* who, bool* fast) {
-  if (!h) return fail(CAAR_ERR_INVALID, "null handle");
-  if (!h->params_set) return fail(CAAR_ERR_STATE, "caar_set_params must be called before %s", who);
+  if (int rc = check_handle(h, who)) return rc;
   if (int rc = validate_control(h, ctl)) return rc;
   if (nsteps < 0) return fail(CAAR_ERR_INVALID, "nsteps=%d", nsteps);
-  if (mode != CAAR_MODE_FAST && mode != CAAR_MODE_STRICT) return fail(CAAR_ERR_INVALID, "mode=%d", mode);
-  *fast = uses_fused(h, mode);
-  if (!*fast && caar::strict_smem_bytes(h->dims.nlev) > 200 * 1024)
+  if (int rc = check_mode(mode)) return rc;
+  *fast = selects_fused(h, mode);
+  if (mode == CAAR_MODE_FAST && !*fast) {  // never silent: the reference-order kernel is ~6x slower
+    static bool told = false;
+    if (!told) {
+      told = true;
+      fprintf(stderr, "[caar] CAAR_MODE_FAST: no fused kernel instance for nlev=%d (instances cover nlev <= 128); "
+                      "running the reference-order kernel instead (see caar_describe)\n", h->dims.nlev);
+    }
+  }
+  if (!*fast && !caar::strict_supports(h->dims.nlev))
     return fail(CAAR_ERR_UNSUPPORTED, "nlev=%d too large for the strict kernel", h->dims.nlev);
   return CAAR_OK;
 }
@@ -561,16 +561,6 @@ bool host_arrays_mapped(double* const* tab, double** dev) {
   return true;
 }
 
-bool zero_copy_default() {
-  static const int v = [] {
-    const char* e = getenv("CAAR_HOST_PATH");  // "staged" | "zerocopy"
-    if (e && std::strcmp(e, "staged") == 0) return 0;
-    if (e && std::strcmp(e, "zerocopy") == 0) return 1;
-    return CAAR_HOST_DEFAULT_ZERO_COPY;
-  }();
-  return v != 0;
-}
-
 int add_levels(Slice* out, int n, int f, size_t lf, int ntl, int tl_a, int tl_b) {
   out[n++] = Slice{f, lf * ntl, lf * tl_a, lf};
   if (tl_b != tl_a) out[n++] = Slice{f, lf * ntl, lf * tl_b, lf};
@@ -588,9 +578,9 @@ cudaError_t copy_slice(const Slice& s, double* dev, double* host, int e0, int e1
   const size_t pitch = s.per_elem * sizeof(double), width = s.len * sizeof(double);
   // Pitched DMA over PCIe runs markedly slower with 18 KB rows than with 9 KB rows while the other direction
   // is busy (measured: tools/pcie_probe.cu, profiles/README.md), so wide rows are cut into pieces of <= row_max B
-  static const size_t row_max = [] { const char* e = getenv("CAAR_HOST_ROW"); return e ? (size_t)atol(e) : (size_t)9216; }();
-  static const int split_dirs = [] { const char* e = getenv("CAAR_HOST_SPLIT"); return e ? atoi(e) : 3; }();  // 1 = in, 2 = out
-  if (row_max > 0 && width > row_max && (split_dirs & (to_device ? 1 : 2))) {
+  // in both directions
+  const size_t row_max = 9216;
+  if (width > row_max) {
     for (size_t o = 0; o < width; o += row_max) {
       const size_t wd = (width - o < row_max) ? width - o : row_max;
       const cudaError_t e = to_device ? cudaMemcpy2DAsync((char*)d + o, pitch, (char*)h + o, pitch, wd, n, kind, st)
@@ -606,15 +596,11 @@ cudaError_t copy_slice(const Slice& s, double* dev, double* host, int e0, int e1
 }  // namespace
 
 int caar_run_host(caar_handle h, const caar_arrays* host, const caar_control* ctl, int mode, int chunk_elems) {
-  if (!h || !host) return fail(CAAR_ERR_INVALID, "null argument");
-  if (!h->params_set) return fail(CAAR_ERR_STATE, "caar_set_params must be called before caar_run_host");
-  if (int rc = validate_control(h, ctl)) return rc;
-  if (mode != CAAR_MODE_FAST && mode != CAAR_MODE_STRICT) return fail(CAAR_ERR_INVALID, "mode=%d", mode);
+  if (!host) return fail(CAAR_ERR_INVALID, "null argument");
+  bool fast = false;
+  if (int rc = check_run(h, ctl, 1, mode, "caar_run_host", &fast)) return rc;
   if (chunk_elems < 0 && chunk_elems != CAAR_HOST_ZERO_COPY) return fail(CAAR_ERR_INVALID, "chunk_elems=%d", chunk_elems);
   const caar_dims& d = h->dims;
-  const bool fast = uses_fused(h, mode);
-  if (!fast && caar::strict_smem_bytes(d.nlev) > 200 * 1024)
-    return fail(CAAR_ERR_UNSUPPORTED, "nlev=%d too large for the strict kernel", d.nlev);
   const int n = ctl->nete - ctl->nets;
   if (n == 0) return CAAR_OK;
 
@@ -650,12 +636,11 @@ int caar_run_host(caar_handle h, const caar_arrays* host, const caar_control* ct
   DeviceGuard guard(h->device);
   // ---- zero-copy path: the kernel itself reads the caller's arrays over PCIe (TMA / LDG on mapped host memory)
   // and writes the results straight back: one launch, both link directions busy, no staging copies
-  double* mapped[CAAR_NUM_FIELDS];
-  const bool can_map = host_arrays_mapped(tab, mapped);
-  if (chunk_elems == CAAR_HOST_ZERO_COPY && !can_map)
-    return fail(CAAR_ERR_INVALID, "CAAR_HOST_ZERO_COPY needs page-locked, device-mapped host arrays "
-                                  "(caar_host_register / cudaHostAlloc)");
-  if (can_map && (chunk_elems == CAAR_HOST_ZERO_COPY || (chunk_elems == 0 && zero_copy_default()))) {
+  if (chunk_elems == CAAR_HOST_ZERO_COPY) {
+    double* mapped[CAAR_NUM_FIELDS];
+    if (!host_arrays_mapped(tab, mapped))
+      return fail(CAAR_ERR_INVALID, "CAAR_HOST_ZERO_COPY needs page-locked, device-mapped host arrays "
+                                    "(caar_host_register / cudaHostAlloc)");
     caar::KernelArgs za = make_args(h, ctl, mapped);
     za.tma = nullptr;
     za.pf_dist = -1;  // no L2 prefetch of host memory
@@ -697,13 +682,13 @@ int caar_run_host(caar_handle h, const caar_arrays* host, const caar_control* ct
     tail[++ntail] = a1;
   }
   const int nchunks = full - 1 + ntail;
-  if (h->n_chunk_ev < 3 * nchunks) {
-    cudaEvent_t* ev = new (std::nothrow) cudaEvent_t[3 * nchunks];
+  if (h->n_chunk_ev < 2 * nchunks) {
+    cudaEvent_t* ev = new (std::nothrow) cudaEvent_t[2 * nchunks];
     if (!ev) return fail(CAAR_ERR_NOMEM, "host allocation failed");
     for (int i = 0; i < h->n_chunk_ev; ++i) ev[i] = h->chunk_ev[i];
     delete[] h->chunk_ev;
     h->chunk_ev = ev;
-    while (h->n_chunk_ev < 3 * nchunks) {
+    while (h->n_chunk_ev < 2 * nchunks) {
       CU_TRY(cudaEventCreateWithFlags(&h->chunk_ev[h->n_chunk_ev], cudaEventDisableTiming));
       ++h->n_chunk_ev;
     }
@@ -711,9 +696,6 @@ int caar_run_host(caar_handle h, const caar_arrays* host, const caar_control* ct
   // the copy-in stream must not overtake work already queued on the compute stream (it rewrites the mirrors)
   CU_TRY(cudaEventRecord(h->ev_fence, h->stream));
   CU_TRY(cudaStreamWaitEvent(h->s_in, h->ev_fence, 0));
-  // the copy-in of a chunk may be dealt over two streams (two copy engines reading the host at once)
-  static const int in_streams = [] { const char* e = getenv("CAAR_HOST_IN_STREAMS"); return e ? atoi(e) : 1; }();
-  if (in_streams > 1) CU_TRY(cudaStreamWaitEvent(h->s_in2, h->ev_fence, 0));
   caar::KernelArgs a = make_args(h, ctl);
   // On any failure inside the pipeline the three streams are drained before returning, so that no DMA is still
   // reading or writing the caller's arrays when the caller sees the error (the host arrays may then hold the results
@@ -729,13 +711,9 @@ int caar_run_host(caar_handle h, const caar_arrays* host, const caar_control* ct
     const int e0 = c < full - 1 ? ctl->nets + c * chunk : tail[c - (full - 1)];
     const int e1 = c < full - 1 ? e0 + chunk : tail[c - (full - 1) + 1];
     for (int i = 0; i < ni; ++i)
-      PIPE_TRY(copy_slice(in[i], h->dev[in[i].f], tab[in[i].f], e0, e1, true, (in_streams > 1 && (i & 1)) ? h->s_in2 : h->s_in));
+      PIPE_TRY(copy_slice(in[i], h->dev[in[i].f], tab[in[i].f], e0, e1, true, h->s_in));
     PIPE_TRY(cudaEventRecord(h->chunk_ev[2 * c], h->s_in));
     PIPE_TRY(cudaStreamWaitEvent(h->stream, h->chunk_ev[2 * c], 0));
-    if (in_streams > 1) {
-      PIPE_TRY(cudaEventRecord(h->chunk_ev[2 * nchunks + c], h->s_in2));
-      PIPE_TRY(cudaStreamWaitEvent(h->stream, h->chunk_ev[2 * nchunks + c], 0));
-    }
     a.nets = e0;
     a.nete = e1;
     PIPE_TRY(fast ? caar::launch_fused(a, h->stream) : caar::launch_strict(a, h->stream));
@@ -747,7 +725,6 @@ int caar_run_host(caar_handle h, const caar_arrays* host, const caar_control* ct
 #undef PIPE_TRY
   if (ce != cudaSuccess) {
     cudaStreamSynchronize(h->s_in);
-    cudaStreamSynchronize(h->s_in2);
     cudaStreamSynchronize(h->stream);
     cudaStreamSynchronize(h->s_out);
     cudaGetLastError();
@@ -762,11 +739,10 @@ int caar_run_host(caar_handle h, const caar_arrays* host, const caar_control* ct
 int caar_host_traffic(caar_handle h, const caar_control* ctl, int mode, size_t* h2d_bytes, size_t* d2h_bytes) {
   if (!h || !ctl || !h2d_bytes || !d2h_bytes) return fail(CAAR_ERR_INVALID, "null argument");
   if (int rc = validate_control(h, ctl)) return rc;
+  if (int rc = check_mode(mode)) return rc;
   const caar_dims& d = h->dims;
-  const bool fast = uses_fused(h, mode);
   const size_t lf = (size_t)d.nlev * 16, le = (size_t)(d.nlev + 1) * 16;
   const size_t lv = (ctl->n0 == ctl->nm1) ? 1 : 2;
-  (void)fast;
   const size_t eta = moves_eta(h, mode) ? le : 0;
   size_t in = 2 * 64 + 5 * 16 + lv * 4 * lf + (ctl->qn0 != -1 ? lf : 0) + 4 * lf + eta;
   size_t out = 8 * lf + eta;
@@ -798,39 +774,32 @@ static int extra_buffer(caar_handle h, int which, double** out) {
   return CAAR_OK;
 }
 
-int caar_extra_upload(caar_handle h, int which, const double* host) {
-  if (!host) return fail(CAAR_ERR_INVALID, "null argument");
-  double* dev = nullptr;
-  if (!h) return fail(CAAR_ERR_INVALID, "null handle");
+static int copy_extra(caar_handle h, int which, double* host, bool to_device) {
+  if (!h || !host) return fail(CAAR_ERR_INVALID, "null argument");
   DeviceGuard guard(h->device);
+  double* dev = nullptr;
   if (int rc = extra_buffer(h, which, &dev)) return rc;
-  CU_TRY(cudaMemcpyAsync(dev, host, caar_extra_count(&h->dims, which) * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+  const size_t bytes = caar_extra_count(&h->dims, which) * sizeof(double);
+  CU_TRY(to_device ? cudaMemcpyAsync(dev, host, bytes, cudaMemcpyHostToDevice, h->stream)
+                   : cudaMemcpyAsync(host, dev, bytes, cudaMemcpyDeviceToHost, h->stream));
   CU_TRY(cudaStreamSynchronize(h->stream));
   return CAAR_OK;
 }
 
-int caar_extra_download(caar_handle h, int which, double* host) {
-  if (!host) return fail(CAAR_ERR_INVALID, "null argument");
-  double* dev = nullptr;
-  if (!h) return fail(CAAR_ERR_INVALID, "null handle");
-  DeviceGuard guard(h->device);
-  if (int rc = extra_buffer(h, which, &dev)) return rc;
-  CU_TRY(cudaMemcpyAsync(host, dev, caar_extra_count(&h->dims, which) * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-  CU_TRY(cudaStreamSynchronize(h->stream));
-  return CAAR_OK;
+int caar_extra_upload(caar_handle h, int which, const double* host) {
+  return copy_extra(h, which, const_cast<double*>(host), true);
 }
+int caar_extra_download(caar_handle h, int which, double* host) { return copy_extra(h, which, host, false); }
 
 namespace {
 
 // The checks of caar_euler_step and caar_advect_tracers
 int check_euler(caar_handle h, int nets, int nete, int qn0, int qsize, int mode, const char* who) {
-  if (!h) return fail(CAAR_ERR_INVALID, "null handle");
-  if (!h->params_set) return fail(CAAR_ERR_STATE, "caar_set_params must be called before %s", who);
-  if (nets < 0 || nete > h->dims.nelem || nets > nete) return fail(CAAR_ERR_INVALID, "element range [%d,%d)", nets, nete);
+  if (int rc = check_handle(h, who)) return rc;
+  if (int rc = check_range(h, nets, nete)) return rc;
   if (qn0 < 0 || qn0 > 1) return fail(CAAR_ERR_INVALID, "qn0=%d must be 0 or 1", qn0);
   if (qsize < 0 || qsize > h->dims.qsize_d) return fail(CAAR_ERR_INVALID, "qsize=%d outside [0,%d]", qsize, h->dims.qsize_d);
-  if (mode != CAAR_MODE_FAST && mode != CAAR_MODE_STRICT) return fail(CAAR_ERR_INVALID, "mode=%d", mode);
-  return CAAR_OK;
+  return check_mode(mode);
 }
 
 // One tracer step Qdp(qn0) - dt div(vstar Qdp(qn0)) on the handle's stream (caller holds the device); tracer iq of
@@ -885,11 +854,10 @@ int caar_advect_tracers(caar_handle h, int nets, int nete, int* qn0, int qsize, 
 }
 
 int caar_sphere_wk(caar_handle h, int op, int nets, int nete, int mode) {
-  if (!h) return fail(CAAR_ERR_INVALID, "null handle");
-  if (!h->params_set) return fail(CAAR_ERR_STATE, "caar_set_params must be called before caar_sphere_wk");
-  if (nets < 0 || nete > h->dims.nelem || nets > nete) return fail(CAAR_ERR_INVALID, "element range [%d,%d)", nets, nete);
+  if (int rc = check_handle(h, "caar_sphere_wk")) return rc;
+  if (int rc = check_range(h, nets, nete)) return rc;
   if (op < CAAR_OP_DIVERGENCE_WK || op > CAAR_OP_LAPLACE_TENSOR_REPLACE) return fail(CAAR_ERR_INVALID, "op=%d", op);
-  if (mode != CAAR_MODE_FAST && mode != CAAR_MODE_STRICT) return fail(CAAR_ERR_INVALID, "mode=%d", mode);
+  if (int rc = check_mode(mode)) return rc;
   DeviceGuard guard(h->device);
   double *vin = nullptr, *sin = nullptr, *out = nullptr, *tv = nullptr;
   if (int rc = extra_buffer(h, CAAR_X_SCALAR_OUT, &out)) return rc;
@@ -955,8 +923,8 @@ int caar_timer_stop(caar_handle h, float* ms) {
 
 int caar_norms(caar_handle h, int tl, int nets, int nete, double sumsq[3]) {
   if (!h || !sumsq) return fail(CAAR_ERR_INVALID, "null argument");
-  if (tl < 0 || tl >= h->dims.ntl) return fail(CAAR_ERR_INVALID, "time level %d", tl);
-  if (nets < 0 || nete > h->dims.nelem || nets > nete) return fail(CAAR_ERR_INVALID, "element range [%d,%d)", nets, nete);
+  if (int rc = check_time_level(h, tl)) return rc;
+  if (int rc = check_range(h, nets, nete)) return rc;
   DeviceGuard guard(h->device);
   const caar::KernelArgs a = make_args(h, nullptr);
   CU_TRY(caar::launch_norms(a, tl, nets, nete, h->partial, h->out3, h->stream));
@@ -969,8 +937,8 @@ int caar_norms(caar_handle h, int tl, int nets, int nete, double sumsq[3]) {
 
 int caar_checksums(caar_handle h, int tl, int nets, int nete, caar_checksum* out) {
   if (!h || !out) return fail(CAAR_ERR_INVALID, "null argument");
-  if (tl < 0 || tl >= h->dims.ntl) return fail(CAAR_ERR_INVALID, "time level %d", tl);
-  if (nets < 0 || nete > h->dims.nelem || nets > nete) return fail(CAAR_ERR_INVALID, "element range [%d,%d)", nets, nete);
+  if (int rc = check_time_level(h, tl)) return rc;
+  if (int rc = check_range(h, nets, nete)) return rc;
   DeviceGuard guard(h->device);
   const caar::KernelArgs a = make_args(h, nullptr);
   unsigned long long* out7 = reinterpret_cast<unsigned long long*>(h->out3 + 16);
@@ -996,10 +964,7 @@ int caar_compute_and_apply_rhs_host(const caar_dims* dims, const caar_arrays* ho
   if (rc) return rc;
   rc = caar_set_params(h, c, dvv, ps0, hyai);
   if (!rc) rc = caar_run_host(h, host, ctl, mode, 0);
-  char keep[sizeof g_err];
-  std::memcpy(keep, g_err, sizeof keep);
-  caar_destroy(h);
-  std::memcpy(g_err, keep, sizeof keep);
+  destroy_keeping_error(h);
   return rc;
 }
 

@@ -62,16 +62,55 @@ struct alignas(64) TmaMaps {
 };
 // returns 0 on success; on failure writes a message
 int build_tma_maps(TmaMaps* out, const KernelArgs& a, char* err, size_t errlen);
+// The one tensor-map format of the fused kernel and the level operators: *m over the doubles at `base` as
+// [slices][rows of 128 B][16 doubles], box = box_rows rows of one slice, SWIZZLE_128B, 256 B L2 promotion. A box that
+// sticks out of its slice is zero-filled on load and clipped on store. Returns 0 on success; on failure writes a
+// message naming the map `name` into err (errlen may be 0).
+int encode_tma_map(CUtensorMap* m, const void* base, cuuint64_t slices, cuuint64_t rows, cuuint32_t box_rows,
+                   const char* name, char* err, size_t errlen);
+
+// Launch set-up of one kernel on the current device: its dynamic shared-memory limit becomes `smem`, it asks for the
+// largest shared-memory carveout (so that several CTAs can be resident per SM), and *per_sm (>= 1) is how many CTAs of
+// `threads` threads and `smem` bytes an SM holds. Function attributes are per (kernel, device), so this is done once per
+// device and `smem`, remembered in `cache`: one static per kernel, owned by its launcher (a static inside this template
+// would be shared by all kernels of one signature). Device ordinals >= 64 are set up again on every call.
+struct LaunchCache {
+  size_t smem[64];
+  int per_sm[64];
+};
+template <typename Kernel>
+cudaError_t setup_launch(Kernel* kernel, int threads, size_t smem, LaunchCache& cache, int* per_sm) {
+  int dev = 0;
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e != cudaSuccess) return e;
+  const bool cached = dev >= 0 && dev < 64;
+  if (cached && cache.per_sm[dev] > 0 && cache.smem[dev] == smem) {
+    *per_sm = cache.per_sm[dev];
+    return cudaSuccess;
+  }
+  int n = 0;
+  e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
+  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kernel, threads, smem);
+  if (e != cudaSuccess) return e;
+  *per_sm = n < 1 ? 1 : n;
+  if (cached) {
+    cache.smem[dev] = smem;
+    cache.per_sm[dev] = *per_sm;
+  }
+  return cudaSuccess;
+}
 
 // launchers (defined in the .cu files); return cudaError_t of the launch
 cudaError_t launch_strict(const KernelArgs& a, cudaStream_t s);
 cudaError_t launch_fused(const KernelArgs& a, cudaStream_t s);
-bool fused_supports(int nlev);
-bool fused_supports_eulerian(int nlev);  // rsplit == 0 on the fused path
+bool fused_supports(int nlev);           // both vertical coordinates
 int fused_instance_levels(int nlev);     // compiled level count that serves nlev (>= nlev), 0 = none
 int fused_instance_cluster(int nlev);    // CTAs per element of that instance
 cudaError_t launch_fused_more(const KernelArgs& a, cudaStream_t s);  // level counts other than 72 / 128
 size_t strict_smem_bytes(int nlev);
+bool strict_supports(int nlev);  // the strict kernel's shared memory fits
 
 cudaError_t launch_norms(const KernelArgs& a, int tl, int nets, int nete, double* partial /*[nelem][3]*/,
                          double* out3, cudaStream_t s);

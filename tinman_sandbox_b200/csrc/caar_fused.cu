@@ -5,24 +5,47 @@
 #include "caar_fused_kernel.cuh"
 
 namespace caar {
-int build_tma_maps(TmaMaps* out, const KernelArgs& a, char* err, size_t errlen) {
+int encode_tma_map(CUtensorMap* m, const void* base, cuuint64_t slices, cuuint64_t rows, cuuint32_t box_rows,
+                   const char* name, char* err, size_t errlen) {
   typedef CUresult (*encode_t)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-  void* fn = nullptr;
-  cudaDriverEntryPointQueryResult qres;
-  cudaError_t ce = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres);
-  if (ce != cudaSuccess || !fn || qres != cudaDriverEntryPointSuccess) {
-    snprintf(err, errlen, "cuTensorMapEncodeTiled entry point unavailable (%s)", cudaGetErrorString(ce));
+  static cudaError_t lookup = cudaSuccess;
+  static const encode_t encode = [] {
+    void* fn = nullptr;
+    cudaDriverEntryPointQueryResult qres;
+    lookup = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres);
+    return lookup == cudaSuccess && fn && qres == cudaDriverEntryPointSuccess ? reinterpret_cast<encode_t>(fn) : nullptr;
+  }();
+  if (!encode) {
+    snprintf(err, errlen, "cuTensorMapEncodeTiled entry point unavailable (%s)", cudaGetErrorString(lookup));
     return 1;
   }
-  const encode_t encode = reinterpret_cast<encode_t>(fn);
+  if (box_rows > 256 || slices >= (1ull << 31)) {
+    snprintf(err, errlen, "tensor map %s: box of %u rows / %llu slices out of range", name, box_rows,
+             (unsigned long long)slices);
+    return 1;
+  }
+  const cuuint64_t gdim[3] = {16, rows, slices};
+  const cuuint64_t gstride[2] = {128, rows * 128};
+  const cuuint32_t box[3] = {16, box_rows, 1};
+  const cuuint32_t estride[3] = {1, 1, 1};
+  const CUresult r = encode(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 3, const_cast<void*>(base), gdim, gstride, box, estride,
+                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) {
+    snprintf(err, errlen, "cuTensorMapEncodeTiled(%s) failed with CUresult %d", name, (int)r);
+    return 1;
+  }
+  return 0;
+}
+
+int build_tma_maps(TmaMaps* out, const KernelArgs& a, char* err, size_t errlen) {
   const cuuint64_t E = (cuuint64_t)a.nelem, L = (cuuint64_t)a.nlev, ntl = (cuuint64_t)a.ntl;
   const int inst = instance_for(a.nlev);  // compiled level count serving this nlev (>= nlev)
   const cuuint32_t LB = (cuuint32_t)(inst / (cluster_for(inst) > 0 ? cluster_for(inst) : 1));  // levels per CTA = box rows
   // every array as [slices][rows][16 doubles]: rows = the levels of one element (x time level, tracer ...) slice, x2 for
-  // the interleaved (u,v) fields. A box that sticks out of its slice (padding levels) is zero-filled on load and
-  // clipped on store, and its missing rows cost no HBM traffic.
+  // the interleaved (u,v) fields. A box that sticks out of its slice (padding levels) costs no HBM traffic.
   struct Spec { CUtensorMap* m; const void* base; cuuint64_t slices; cuuint64_t rows; cuuint32_t box; const char* name; };
   const Spec specs[8] = {
       {&out->Qdp, a.Qdp, E * (cuuint64_t)a.qsize_d * 2, L, LB, "Qdp"},
@@ -34,28 +57,10 @@ int build_tma_maps(TmaMaps* out, const KernelArgs& a, char* err, size_t errlen) 
       {&out->omega_p, a.omega_p, E, L, LB, "omega_p"},
       {&out->phi, a.phi, E, L, LB, "phi"},
   };
-  for (const Spec& sp : specs) {
-    const cuuint64_t gdim[3] = {16, sp.rows, sp.slices};
-    const cuuint64_t gstride[2] = {128, sp.rows * 128};
-    const cuuint32_t box[3] = {16, sp.box, 1};
-    const cuuint32_t estride[3] = {1, 1, 1};
-    if (sp.box > 256 || sp.slices >= (1ull << 31)) {
-      snprintf(err, errlen, "tensor map %s: box of %u rows / %llu slices out of range", sp.name, sp.box,
-               (unsigned long long)sp.slices);
-      return 1;
-    }
-    const CUresult r = encode(sp.m, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 3, const_cast<void*>(sp.base), gdim, gstride, box,
-                              estride, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                              CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      snprintf(err, errlen, "cuTensorMapEncodeTiled(%s) failed with CUresult %d", sp.name, (int)r);
-      return 1;
-    }
-  }
+  for (const Spec& sp : specs)
+    if (encode_tma_map(sp.m, sp.base, sp.slices, sp.rows, sp.box, sp.name, err, errlen)) return 1;
   return 0;
 }
-
-bool fused_supports_eulerian(int nlev) { return instance_for(nlev) > 0; }
 
 bool fused_supports(int nlev) { return instance_for(nlev) > 0; }
 

@@ -923,28 +923,10 @@ cudaError_t launch_L(const KernelArgs& a, cudaStream_t s) {
   const int n = a.nete - a.nets;
   if (n <= 0) return cudaSuccess;
   constexpr int SMEM = (int)sizeof(Smem<L / CL, L / 8, EUL>) + 1024;
-  // function attributes are per device: set once per (instance, device), not on every launch
-  static bool configured[64] = {};
-  int dev = 0;
-  cudaError_t e = cudaGetDevice(&dev);
-  if (e != cudaSuccess) return e;
-  if (dev < 0 || dev >= 64 || !configured[dev]) {
-    e = cudaFuncSetAttribute(caar_fused_kernel<L, CL, EUL>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM);
-    if (e != cudaSuccess) return e;
-    // ask for the largest shared-memory carveout so that several ~30-80 KB CTAs are resident per SM
-    e = cudaFuncSetAttribute(caar_fused_kernel<L, CL, EUL>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                             (int)cudaSharedmemCarveoutMaxShared);
-    if (e != cudaSuccess) return e;
-    if (dev >= 0 && dev < 64) configured[dev] = true;
-  }
+  static LaunchCache cache;
+  int per_sm = 0;
+  if (cudaError_t e = setup_launch(caar_fused_kernel<L, CL, EUL>, 4 * L / CL, SMEM, cache, &per_sm)) return e;
   if (!a.tma) return cudaErrorInvalidValue;
-  static const bool debug_occ = getenv("CAAR_DEBUG_OCC") != nullptr;
-  if (debug_occ) {
-    int nb = -1;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, caar_fused_kernel<L, CL, EUL>, 4 * L / CL, SMEM);
-    fprintf(stderr, "[caar] caar_fused_kernel<%d,%d,%d>: %d threads, %d B dynamic smem -> %d CTAs/SM\n", L, CL, (int)EUL,
-            4 * L / CL, SMEM, nb);
-  }
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)n * CL, 1, 1);
   cfg.blockDim = dim3(4 * L / CL, 1, 1);

@@ -734,47 +734,14 @@ __global__ void __launch_bounds__(256) sphere_wk_strict_kernel(const StrictWkArg
   if (live) A.out[n + q] = dd;
 }
 
-int encode3(CUtensorMap* m, const void* base, cuuint64_t slices, cuuint64_t rows, cuuint32_t box_rows) {
-  typedef CUresult (*encode_t)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                               const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                               CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-  static encode_t encode = nullptr;
-  if (!encode) {
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess || !fn) return 1;
-    encode = reinterpret_cast<encode_t>(fn);
-  }
-  const cuuint64_t gdim[3] = {16, rows, slices};
-  const cuuint64_t gstride[2] = {128, rows * 128};
-  const cuuint32_t box[3] = {16, box_rows, 1};
-  const cuuint32_t estride[3] = {1, 1, 1};
-  return encode(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 3, const_cast<void*>(base), gdim, gstride, box, estride,
-                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS ? 0 : 1;
-}
-
 template <int OP>
 cudaError_t launch_op(const LevelOpArgs& a, const LevelOpMaps& m, cudaStream_t s) {
   const unsigned in_b = (OP == OP_DIVWK) ? 2048u : 1024u, item_b = (OP == OP_EULER) ? 2048u : 0u;
   const size_t smem = (size_t)WPC * (NS * in_b + NO * 1024u + 2 * item_b) + WPC * (NS + 2) * sizeof(uint64_t) +
                       WPC * 80 * sizeof(double) + 1024;
-  // function attributes and occupancy are per (instance, device): set / queried once
-  static int cached_per_sm[64] = {};
-  int dev = 0;
-  cudaError_t e = cudaGetDevice(&dev);
-  if (e != cudaSuccess) return e;
-  int per_sm = (dev >= 0 && dev < 64) ? cached_per_sm[dev] : 0;
-  if (per_sm == 0) {
-    e = cudaFuncSetAttribute(levelop_kernel<OP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(levelop_kernel<OP>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
-    if (e != cudaSuccess) return e;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, levelop_kernel<OP>, 32 * WPC, smem);
-    if (e != cudaSuccess) return e;
-    if (per_sm < 1) per_sm = 1;
-    if (dev >= 0 && dev < 64) cached_per_sm[dev] = per_sm;
-  }
+  static LaunchCache cache;
+  int per_sm = 0;
+  if (cudaError_t e = setup_launch(levelop_kernel<OP>, 32 * WPC, smem, cache, &per_sm)) return e;
   // grid = waves x the resident CTAs. A static cut into one range per resident warp (1 wave) leaves the early finishers
   // idle, many short CTAs pay their pipeline fill more often; the best number of waves grows with the size (tracer step,
   // qsize 4: 1-2 at 5400 elements, 6-8 at 21600, 16 at 86400; divergence_sphere_wk: 1 / 8 / 16 — profiles/README.md):
@@ -794,22 +761,9 @@ cudaError_t launch_op(const LevelOpArgs& a, const LevelOpMaps& m, cudaStream_t s
 template <bool TENSOR>
 cudaError_t launch_lapflat(LapFlatArgs a, const LapFlatMaps& m, cudaStream_t s) {
   const size_t smem = (size_t)FW * FWARP_B + FW * FN * (sizeof(uint64_t) + sizeof(int)) + 1024;
-  static int cached_per_sm[64] = {};
-  int dev = 0;
-  cudaError_t e = cudaGetDevice(&dev);
-  if (e != cudaSuccess) return e;
-  if (dev < 0 || dev >= 64) return cudaErrorInvalidDevice;
-  int per_sm = cached_per_sm[dev];
-  if (per_sm == 0) {
-    e = cudaFuncSetAttribute(laplace_flat_kernel<TENSOR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(laplace_flat_kernel<TENSOR>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
-    if (e != cudaSuccess) return e;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, laplace_flat_kernel<TENSOR>, 32 * FW, smem);
-    if (e != cudaSuccess) return e;
-    if (per_sm < 1) per_sm = 1;
-    cached_per_sm[dev] = per_sm;
-  }
+  static LaunchCache cache;
+  int per_sm = 0;
+  if (cudaError_t e = setup_launch(laplace_flat_kernel<TENSOR>, 32 * FW, smem, cache, &per_sm)) return e;
   // one wave of resident CTAs; chunks of 4 consecutive tiles (49152 x 128: 0.81 / 0.98 / 1.01 / 0.99 / 0.95 / 0.90 of the
   // measured peak with 1 / 2 / 4 / 8 / 16 / 32; one tile per chunk exposes the draw), 2 when a warp sees few tiles
   static const int chunk_env = [] { const char* v = getenv("CAAR_LAPLACE_CHUNK"); return v ? atoi(v) : 0; }();
@@ -854,7 +808,8 @@ cudaError_t launch_levelop(int op, const KernelArgs& k, const double* in, const 
     for (int i = 0; i < 16; ++i) a.dvv[i] = k.dvv[i];
     LapFlatMaps m;
     const size_t off = (size_t)nets * k.nlev * 16;
-    if (encode3(&m.in, in + off, 1, (cuuint64_t)flat_rows, FT) | encode3(&m.out, out + off, 1, (cuuint64_t)flat_rows, FT))
+    if (encode_tma_map(&m.in, in + off, 1, (cuuint64_t)flat_rows, FT, "in", nullptr, 0) |
+        encode_tma_map(&m.out, out + off, 1, (cuuint64_t)flat_rows, FT, "out", nullptr, 0))
       return cudaErrorInvalidValue;
     return op == 2 ? launch_lapflat<false>(a, m, s) : launch_lapflat<true>(a, m, s);
   }
@@ -870,12 +825,12 @@ cudaError_t launch_levelop(int op, const KernelArgs& k, const double* in, const 
   const cuuint64_t E = (cuuint64_t)k.nelem, L = (cuuint64_t)k.nlev;
   int bad = 0;
   if (op == 0) {
-    bad |= encode3(&m.in, in, E * (cuuint64_t)k.qsize_d * 2, L, GL);
-    bad |= encode3(&m.item, item, E, 2 * L, 2 * GL);
-    bad |= encode3(&m.out, out, E * (cuuint64_t)k.qsize_d * (cuuint64_t)out_stride, L, GL);
+    bad |= encode_tma_map(&m.in, in, E * (cuuint64_t)k.qsize_d * 2, L, GL, "in", nullptr, 0);
+    bad |= encode_tma_map(&m.item, item, E, 2 * L, 2 * GL, "item", nullptr, 0);
+    bad |= encode_tma_map(&m.out, out, E * (cuuint64_t)k.qsize_d * (cuuint64_t)out_stride, L, GL, "out", nullptr, 0);
   } else {
-    bad |= encode3(&m.in, in, E, op == 1 ? 2 * L : L, op == 1 ? 2 * GL : GL);
-    bad |= encode3(&m.out, out, E, L, GL);
+    bad |= encode_tma_map(&m.in, in, E, op == 1 ? 2 * L : L, op == 1 ? 2 * GL : GL, "in", nullptr, 0);
+    bad |= encode_tma_map(&m.out, out, E, L, GL, "out", nullptr, 0);
     m.item = m.in;
   }
   if (bad) return cudaErrorInvalidValue;

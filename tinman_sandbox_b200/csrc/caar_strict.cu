@@ -281,11 +281,13 @@ __global__ void __launch_bounds__(512) caar_strict_kernel(const KernelArgs A) {
 }  // namespace
 
 size_t strict_smem_bytes(int nlev) { return ((size_t)12 * nlev + 1) * PTS * sizeof(double); }
+bool strict_supports(int nlev) { return strict_smem_bytes(nlev) <= 200 * 1024; }
 
 cudaError_t launch_strict(const KernelArgs& a, cudaStream_t s) {
   const size_t smem = strict_smem_bytes(a.nlev);
-  cudaError_t err = cudaFuncSetAttribute(caar_strict_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (err != cudaSuccess) return err;
+  static LaunchCache cache;
+  int per_sm = 0;
+  if (cudaError_t e = setup_launch(caar_strict_kernel, 512, smem, cache, &per_sm)) return e;
   const int n = a.nete - a.nets;
   if (n <= 0) return cudaSuccess;
   caar_strict_kernel<<<n, 512, smem, s>>>(a);
