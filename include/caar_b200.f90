@@ -66,7 +66,8 @@ module caar_b200
 
   public :: caar_create, caar_destroy, caar_set_params_f90, caar_set_vertical_coordinate, caar_upload_layout, &
             caar_download_layout, caar_run, caar_run_stepping, caar_run_rk5, caar_update_time_levels, caar_sync, caar_norms, &
-            caar_checksums, caar_euler_step, caar_advect_tracers, caar_sphere_wk, caar_extra_upload, caar_extra_download, caar_last_error, &
+            caar_checksums, caar_euler_step, caar_advect_tracers, caar_tracer_bounds, caar_limit_tracers, &
+            caar_bounds_upload, caar_bounds_download, caar_sphere_wk, caar_extra_upload, caar_extra_download, caar_last_error, &
             caar_host_register, caar_host_unregister, caar_describe
 
   interface
@@ -181,6 +182,32 @@ module caar_b200
       integer(c_int), value :: qsize
       real(c_double), value :: dt
       integer(c_int), value :: nsteps, mode
+      integer(c_int) :: rc
+    end function
+    ! HOMME's quasi-monotone limiter (limiter_option 8) on the resident Qdp; qtl and dp_tl are zero-based.
+    ! bounds(2, nlev, qsize_d, nelemd) = (qmin, qmax): the handle's array, copied whole by caar_bounds_upload / _download
+    function caar_tracer_bounds(handle, nets, nete, qtl, qsize, dp_tl) bind(C, name="caar_tracer_bounds") result(rc)
+      import :: c_ptr, c_int
+      type(c_ptr), value :: handle
+      integer(c_int), value :: nets, nete, qtl, qsize, dp_tl
+      integer(c_int) :: rc
+    end function
+    function caar_limit_tracers(handle, nets, nete, qtl, qsize, dp_tl) bind(C, name="caar_limit_tracers") result(rc)
+      import :: c_ptr, c_int
+      type(c_ptr), value :: handle
+      integer(c_int), value :: nets, nete, qtl, qsize, dp_tl
+      integer(c_int) :: rc
+    end function
+    function caar_bounds_upload(handle, host) bind(C, name="caar_bounds_upload") result(rc)
+      import :: c_ptr, c_int, c_double
+      type(c_ptr), value :: handle
+      real(c_double), intent(in) :: host(*)
+      integer(c_int) :: rc
+    end function
+    function caar_bounds_download(handle, host) bind(C, name="caar_bounds_download") result(rc)
+      import :: c_ptr, c_int, c_double
+      type(c_ptr), value :: handle
+      real(c_double), intent(out) :: host(*)
       integer(c_int) :: rc
     end function
     function caar_sphere_wk(handle, op, nets, nete, mode) bind(C, name="caar_sphere_wk") result(rc)

@@ -251,7 +251,8 @@ void caar_update_time_levels(caar_control* ctl);
 int caar_run_rk5(caar_handle h, caar_control* ctl, double dt, int nsteps, int mode);
 int caar_sync(caar_handle h);
 /* number of kernel launches issued through this handle since creation (caar_run, caar_run_rk5: 6 per step,
-   caar_advect_tracers: 4 per step, caar_euler_step, caar_norms, ...) */
+   caar_advect_tracers: 4 per step, caar_tracer_bounds and caar_limit_tracers: 1 per call (none for an empty range or
+   qsize == 0), caar_euler_step, caar_norms, ...) */
 long long caar_launch_count(caar_handle h);
 /* CUDA-event stopwatch on the stream the kernels are launched on: start records an event, stop records a
    second one, waits for it and returns the device time between the two in milliseconds. */
@@ -294,6 +295,62 @@ int caar_euler_step(caar_handle h, int nets, int nete, int qn0, int qsize, doubl
    toggle *qn0). Returns CAAR_ERR_STATE before caar_set_params and CAAR_ERR_INVALID for a null handle or qn0,
    *qn0 not 0 or 1, a bad element range, qsize outside [0, qsize_d], nsteps < 0 or a bad mode, leaving *qn0 unchanged. */
 int caar_advect_tracers(caar_handle h, int nets, int nete, int* qn0, int qsize, double dt, int nsteps, int mode);
+
+/* ---- the tracer limiter: HOMME's quasi-monotone limiter, euler_step with limiter_option == 8 ----
+   The element-local bounds at the start of a tracer step, and limiter_optim_iter_full, which euler_step applies to
+   Qtens with the weights spheremp and dp_star. Both work on the handle's Qdp, dp3d and spheremp mirrors and on one more
+   handle-owned array (it is not a CAAR_X_* extra array):
+     bounds [E][qsize_d][L][2] = (qmin, qmax) per element, tracer and level; zero on first use.
+   caar_bounds_upload / caar_bounds_download copy the whole array and return when the copy is complete.
+
+   One problem is one (e, iq, k) with e in [nets, nete), iq < qsize, k < L; p[n] are the 16 values of
+   Qdp[e][iq][qtl][k], d[n] those of dp3d[e][dp_tl][k], w[n] those of spheremp[e]. The index n visits the points in
+   Fortran sequence-association order, i fastest: Fortran (i,j) is [igp][jgp] here, so n runs over the offsets
+   4*igp + jgp in the order 0, 4, 8, 12, 1, 5, ... . Every sum is sequential in that order, and every operation is
+   rounded separately (no FMA contraction).
+
+   caar_tracer_bounds: per problem qmin = min_n p[n]/d[n], qmax = max_n p[n]/d[n], then if (qmin < 0) qmin = 0, written
+   to bounds[e][iq][k]. This is HOMME's Qtens_biharmonic = Qdp(n0)/dp; qmin = max(minval, 0); qmax = maxval. HOMME
+   then widens the bounds over neighbouring elements (neighbor_minmax); that is the caller's job, between the two calls,
+   through caar_bounds_download and caar_bounds_upload.
+
+   caar_limit_tracers: per problem, in place on Qdp(qtl) and on the problem's bounds (minp, maxp), with TOL = 5e-14 and
+   MAXITER = 15 (np*np - 1):
+     c[n] = w[n]*d[n];  x[n] = p[n]/d[n]
+     sumc = sum c[n]
+     if (sumc <= 0) leave the problem (p and its bounds) untouched
+     mass = sum (c[n]*x[n])
+     if (mass < minp*sumc) minp = mass/sumc            relax the bounds so that a solution exists
+     if (mass > maxp*sumc) maxp = mass/sumc
+     repeat MAXITER times:
+       addmass = 0
+       for n: if (x[n] > maxp) { addmass = addmass + (x[n]-maxp)*c[n]; x[n] = maxp }
+              if (x[n] < minp) { addmass = addmass - (minp-x[n])*c[n]; x[n] = minp }
+       if (|addmass| <= TOL*|mass|) exit
+       if (addmass > 0) { ws = sum over x[n] < maxp of c[n]; if (ws == 0) exit; for x[n] < maxp: x[n] = x[n] + addmass/ws }
+       else             { ws = sum over x[n] > minp of c[n]; if (ws == 0) exit; for x[n] > minp: x[n] = x[n] + addmass/ws }
+     p[n] = x[n]*d[n];  bounds[e][iq][k] = (minp, maxp)    the relaxed bounds persist (Fortran's intent(inout))
+   A problem that leaves the loop after MAXITER keeps the state after its last redistribution, as HOMME does. The one
+   departure from the literal Fortran is the ws == 0 exit: there the Fortran divides by zero. After the relaxation
+   that point can only be reached through rounding.
+
+   Both calls are asynchronous on the handle's stream, always run in this order (there is no mode: the results are
+   bit-reproducible) and read no parameter, so they work before caar_set_params. They leave dp3d, spheremp, the other
+   Qdp time level, the tracers iq >= qsize, the elements outside [nets, nete) and the bounds outside the problems
+   untouched; caar_tracer_bounds leaves Qdp untouched too. Each call adds one launch, none for an empty range or
+   qsize == 0. CAAR_ERR_INVALID for a null handle or host pointer, a bad element range, qtl not 0 or 1, dp_tl outside
+   [0, ntl) or qsize outside [0, qsize_d]; a rejected call launches nothing and changes nothing.
+
+   One limited tracer step on the resident state (the bounds of the step's input, the limiter once on its output; this
+   is not HOMME's per-stage limiting inside the step, whose dp_star this library does not hold):
+     1  caar_tracer_bounds(h, nets, nete, qn0, qsize, dp_tl)
+     2  optionally widen the bounds over neighbours: caar_bounds_download, the caller's neighbor_minmax, caar_bounds_upload
+     3  caar_advect_tracers(h, nets, nete, &qn0, qsize, dt, 1, mode)
+     4  caar_limit_tracers(h, nets, nete, qn0, qsize, dp_tl)          with the new qn0 */
+int caar_bounds_upload(caar_handle h, const double* host);
+int caar_bounds_download(caar_handle h, double* host);
+int caar_tracer_bounds(caar_handle h, int nets, int nete, int qtl, int qsize, int dp_tl);
+int caar_limit_tracers(caar_handle h, int nets, int nete, int qtl, int qsize, int dp_tl);
 
 /* ---- the weak-form operators behind hyperviscosity (SURVEY §8f rank 4) ----
    Level-local like the tracer step, on the same kernel skeleton, in the pointers_only index conventions

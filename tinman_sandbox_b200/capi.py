@@ -40,7 +40,8 @@ EXPORTED_SYMBOLS = (
     "caar_sync", "caar_launch_count", "caar_timer_start",
     "caar_timer_stop", "caar_norms", "caar_compute_and_apply_rhs_host", "caar_saxpby_device",
     "caar_saxpby_host", "caar_checksums", "caar_upload_range", "caar_download_range", "caar_describe",
-    "caar_sphere_wk", "caar_run_rk5", "caar_advect_tracers",
+    "caar_sphere_wk", "caar_run_rk5", "caar_advect_tracers", "caar_bounds_upload", "caar_bounds_download",
+    "caar_tracer_bounds", "caar_limit_tracers",
 )
 CHECKSUM_FIELDS = ("elem_state_dp3d", "elem_state_v", "elem_state_T", "elem_derived_eta_dot_dpdn",
                    "elem_derived_omega_p", "elem_derived_phi", "elem_derived_vn0")
@@ -137,6 +138,10 @@ def load_library():
     lib.caar_euler_step.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, C.c_int]
     lib.caar_advect_tracers.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_int), C.c_int, C.c_double, C.c_int,
                                         C.c_int]
+    lib.caar_bounds_upload.argtypes = [C.c_void_p, C.POINTER(C.c_double)]
+    lib.caar_bounds_download.argtypes = [C.c_void_p, C.POINTER(C.c_double)]
+    lib.caar_tracer_bounds.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]
+    lib.caar_limit_tracers.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]
     lib.caar_upload_layout.argtypes = [C.c_void_p, C.POINTER(Arrays), C.c_uint, C.c_int]
     lib.caar_download_layout.argtypes = [C.c_void_p, C.POINTER(Arrays), C.c_uint, C.c_int]
     lib.caar_set_params_f90.argtypes = [C.c_void_p, C.POINTER(Constants), C.POINTER(C.c_double), C.c_double,
@@ -375,6 +380,42 @@ class Caar:
         if sync:
             self.sync()
         return q.value
+
+    # -- the tracer limiter (limiter_option 8): element-local bounds and limiter_optim_iter_full --------------------
+    def upload_bounds(self, bounds):
+        """bounds [E][qsize_d][L][2] = (qmin, qmax): the whole handle-owned array (caar_bounds_upload)."""
+        E, L, Q, _ = self.shape_args
+        if bounds.dtype != np.float64 or not bounds.flags["C_CONTIGUOUS"] or bounds.size != E * Q * L * 2:
+            raise CaarError("bounds: need a C-contiguous float64 array [E][qsize_d][L][2]")
+        _check(self.lib, self.lib.caar_bounds_upload(self.h, _dp(bounds)), "caar_bounds_upload")
+
+    def download_bounds(self, bounds=None):
+        E, L, Q, _ = self.shape_args
+        if bounds is None:
+            bounds = np.zeros((E, Q, L, 2))
+        if bounds.dtype != np.float64 or not bounds.flags["C_CONTIGUOUS"] or bounds.size != E * Q * L * 2:
+            raise CaarError("bounds: need a C-contiguous float64 array [E][qsize_d][L][2]")
+        _check(self.lib, self.lib.caar_bounds_download(self.h, _dp(bounds)), "caar_bounds_download")
+        return bounds
+
+    def tracer_bounds(self, qtl, qsize, dp_tl, nets=None, nete=None, sync=True):
+        """caar_tracer_bounds: bounds of Qdp(qtl)/dp3d(dp_tl) per element, tracer iq < qsize and level, qmin >= 0."""
+        nets = self.control.nets if nets is None else nets
+        nete = self.control.nete if nete is None else nete
+        _check(self.lib, self.lib.caar_tracer_bounds(self.h, nets, nete, int(qtl), int(qsize), int(dp_tl)),
+               "caar_tracer_bounds")
+        if sync:
+            self.sync()
+
+    def limit_tracers(self, qtl, qsize, dp_tl, nets=None, nete=None, sync=True):
+        """caar_limit_tracers: HOMME's limiter_optim_iter_full on Qdp(qtl) with weights spheremp * dp3d(dp_tl), within
+        the handle's bounds (relaxed bounds are written back)."""
+        nets = self.control.nets if nets is None else nets
+        nete = self.control.nete if nete is None else nete
+        _check(self.lib, self.lib.caar_limit_tracers(self.h, nets, nete, int(qtl), int(qsize), int(dp_tl)),
+               "caar_limit_tracers")
+        if sync:
+            self.sync()
 
     def download_qtens(self, qtens=None):
         E, L, Q, _ = self.shape_args

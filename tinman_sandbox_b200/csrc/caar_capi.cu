@@ -72,6 +72,7 @@ struct caar_handle_s {
   int rsplit;        // > 0 vertically Lagrangian (default 1), 0 Eulerian
   double* hybi_dev;  // [nlev+1], Eulerian branch only
   double* extra[5];  // arrays beyond struct Arrays: vstar, qtens, tensorVisc, scalar in / out (allocated on first use)
+  double* bounds;  // [nelem][qsize_d][nlev][2] tracer limiter bounds (allocated and zeroed on first use)
   double* stage;  // device staging buffer of the Fortran-layout copies (allocated on first use)
   // device [2]: the tile scheduler of the thread-per-level laplacians (next chunk, warps done), zero between launches.
   // One pair per handle: all launches of a handle are ordered on its stream, so no two of them share it.
@@ -265,6 +266,7 @@ int caar_destroy(caar_handle h) {
   if (h->bits) cudaFree(h->bits);
   if (h->out3) cudaFree(h->out3);
   if (h->stage) cudaFree(h->stage);
+  if (h->bounds) cudaFree(h->bounds);
   for (int x = 0; x < CAAR_NUM_EXTRA; ++x)
     if (h->extra[x]) cudaFree(h->extra[x]);
   if (h->hybi_dev) cudaFree(h->hybi_dev);
@@ -851,6 +853,66 @@ int caar_advect_tracers(caar_handle h, int nets, int nete, int* qn0, int qsize, 
     *qn0 = np1;  // TimeLevel_Qdp: n0_qdp <-> np1_qdp
   }
   return CAAR_OK;
+}
+
+// ---- tracer limiter (limiter_option 8) ---------------------------------------------------------------------------
+namespace {
+
+size_t bounds_count(const caar_dims& d) { return (size_t)d.nelem * d.qsize_d * d.nlev * 2; }
+
+// the handle's bounds array, allocated and zeroed on first use (caller holds the device)
+int bounds_buffer(caar_handle h, double** out) {
+  if (!h->bounds) {
+    const size_t bytes = bounds_count(h->dims) * sizeof(double);
+    CU_TRY(cudaMalloc(&h->bounds, bytes));
+    CU_TRY(cudaMemsetAsync(h->bounds, 0, bytes, h->stream));
+  }
+  *out = h->bounds;
+  return CAAR_OK;
+}
+
+int copy_bounds(caar_handle h, double* host, bool to_device) {
+  if (!h || !host) return fail(CAAR_ERR_INVALID, "null argument");
+  DeviceGuard guard(h->device);
+  double* dev = nullptr;
+  if (int rc = bounds_buffer(h, &dev)) return rc;
+  const size_t bytes = bounds_count(h->dims) * sizeof(double);
+  CU_TRY(to_device ? cudaMemcpyAsync(dev, host, bytes, cudaMemcpyHostToDevice, h->stream)
+                   : cudaMemcpyAsync(host, dev, bytes, cudaMemcpyDeviceToHost, h->stream));
+  CU_TRY(cudaStreamSynchronize(h->stream));
+  return CAAR_OK;
+}
+
+// the checks and the launch of caar_tracer_bounds and caar_limit_tracers; they read no parameter, so they do not need
+// caar_set_params
+int run_limiter(caar_handle h, int nets, int nete, int qtl, int qsize, int dp_tl, bool limit) {
+  if (!h) return fail(CAAR_ERR_INVALID, "null handle");
+  if (int rc = check_range(h, nets, nete)) return rc;
+  if (qtl < 0 || qtl > 1) return fail(CAAR_ERR_INVALID, "qtl=%d must be 0 or 1", qtl);
+  if (qsize < 0 || qsize > h->dims.qsize_d) return fail(CAAR_ERR_INVALID, "qsize=%d outside [0,%d]", qsize, h->dims.qsize_d);
+  if (int rc = check_time_level(h, dp_tl)) return rc;
+  if (nete == nets || qsize == 0) return CAAR_OK;
+  DeviceGuard guard(h->device);
+  double* bounds = nullptr;
+  if (int rc = bounds_buffer(h, &bounds)) return rc;
+  const caar::KernelArgs a = make_args(h, nullptr);
+  CU_TRY(limit ? caar::launch_limit_tracers(a, nets, nete, qtl, qsize, dp_tl, bounds, h->stream)
+               : caar::launch_tracer_bounds(a, nets, nete, qtl, qsize, dp_tl, bounds, h->stream));
+  ++h->launches;
+  return CAAR_OK;
+}
+
+}  // namespace
+
+int caar_bounds_upload(caar_handle h, const double* host) { return copy_bounds(h, const_cast<double*>(host), true); }
+int caar_bounds_download(caar_handle h, double* host) { return copy_bounds(h, host, false); }
+
+int caar_tracer_bounds(caar_handle h, int nets, int nete, int qtl, int qsize, int dp_tl) {
+  return run_limiter(h, nets, nete, qtl, qsize, dp_tl, false);
+}
+
+int caar_limit_tracers(caar_handle h, int nets, int nete, int qtl, int qsize, int dp_tl) {
+  return run_limiter(h, nets, nete, qtl, qsize, dp_tl, true);
 }
 
 int caar_sphere_wk(caar_handle h, int op, int nets, int nete, int mode) {

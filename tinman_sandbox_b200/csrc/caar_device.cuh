@@ -132,6 +132,14 @@ cudaError_t launch_saxpby(double a, double b, double* x, const double* y, size_t
 cudaError_t launch_rk5_combine(const KernelArgs& a, int nets, int nete, int nm1, int n0, cudaStream_t s);
 // tracer SSP step (caar_aux.cu): Qdp(np1) = (Qdp(n0) + 2*Qdp(np1))/3 for tracers < qsize on [nets,nete), one launch
 cudaError_t launch_qdp_avg(const KernelArgs& a, int nets, int nete, int qsize, int n0, int np1, cudaStream_t s);
+// tracer limiter (caar_limiter.cu), one launch each, on problems (e, iq, k) of [nets,nete) x [0,qsize) x [0,L):
+// bounds[e][iq][k] = (max(min Qdp(qtl)/dp3d(dp_tl), 0), max Qdp(qtl)/dp3d(dp_tl)), and limiter_optim_iter_full on
+// Qdp(qtl) with weights spheremp * dp3d(dp_tl) within bounds[e][iq][k] (relaxed bounds written back);
+// bounds [E][qsize_d][L][2]
+cudaError_t launch_tracer_bounds(const KernelArgs& a, int nets, int nete, int qtl, int qsize, int dp_tl, double* bounds,
+                                 cudaStream_t s);
+cudaError_t launch_limit_tracers(const KernelArgs& a, int nets, int nete, int qtl, int qsize, int dp_tl, double* bounds,
+                                 cudaStream_t s);
 // checksums of the seven mutated arrays + energy norms (caar_aux.cu); partial [nelem][8][2], bits [nelem][7]
 cudaError_t launch_checksums(const KernelArgs& a, int tl, int nets, int nete, double cp, double* partial,
                              unsigned long long* bits, double* out16, unsigned long long* out7, cudaStream_t s);
