@@ -31,6 +31,7 @@ module caar_b200
                                        CAAR_X_SCALAR_OUT = 4
   integer(c_int), parameter, public :: CAAR_OP_DIVERGENCE_WK = 0, CAAR_OP_LAPLACE_SIMPLE = 1, CAAR_OP_LAPLACE_TENSOR = 2, &
                                        CAAR_OP_LAPLACE_TENSOR_REPLACE = 3
+  integer(c_int), parameter, public :: CAAR_DSS_ASSEMBLE = 0, CAAR_DSS_PROJECT = 1
 
   ! ---- struct caar_dims (5 x int = 20 bytes)
   type, bind(C), public :: caar_dims
@@ -68,7 +69,8 @@ module caar_b200
             caar_download_layout, caar_run, caar_run_stepping, caar_run_rk5, caar_update_time_levels, caar_sync, caar_norms, &
             caar_checksums, caar_euler_step, caar_advect_tracers, caar_tracer_bounds, caar_limit_tracers, &
             caar_bounds_upload, caar_bounds_download, caar_sphere_wk, caar_extra_upload, caar_extra_download, caar_last_error, &
-            caar_host_register, caar_host_unregister, caar_describe
+            caar_host_register, caar_host_unregister, caar_describe, caar_set_connectivity, caar_dss, caar_neighbor_minmax, &
+            caar_run_rk5_dss
 
   interface
     ! int caar_create(caar_handle* out, const caar_dims* dims, int device);
@@ -208,6 +210,35 @@ module caar_b200
       import :: c_ptr, c_int, c_double
       type(c_ptr), value :: handle
       real(c_double), intent(out) :: host(*)
+      integer(c_int) :: rc
+    end function
+    ! the DSS over shared GLL points. gid(np, np, nelemd) is elem(ie)%gdofP with CAAR_LAYOUT_F90
+    function caar_set_connectivity(handle, gid, layout) bind(C, name="caar_set_connectivity") result(rc)
+      import :: c_ptr, c_int, c_long_long
+      type(c_ptr), value :: handle
+      integer(c_long_long), intent(in) :: gid(*)
+      integer(c_int), value :: layout
+      integer(c_int) :: rc
+    end function
+    ! field_mask within CAAR_F_DP3D + CAAR_F_V + CAAR_F_T + CAAR_F_QDP; tl and qtl are zero-based
+    function caar_dss(handle, field_mask, tl, qtl, qsize, weighting) bind(C, name="caar_dss") result(rc)
+      import :: c_ptr, c_int
+      type(c_ptr), value :: handle
+      integer(c_int), value :: field_mask, tl, qtl, qsize, weighting
+      integer(c_int) :: rc
+    end function
+    function caar_neighbor_minmax(handle, qsize) bind(C, name="caar_neighbor_minmax") result(rc)
+      import :: c_ptr, c_int
+      type(c_ptr), value :: handle
+      integer(c_int), value :: qsize
+      integer(c_int) :: rc
+    end function
+    function caar_run_rk5_dss(handle, ctl, dt, nsteps, mode) bind(C, name="caar_run_rk5_dss") result(rc)
+      import :: c_ptr, c_int, c_double, caar_control
+      type(c_ptr), value :: handle
+      type(caar_control), intent(inout) :: ctl
+      real(c_double), value :: dt
+      integer(c_int), value :: nsteps, mode
       integer(c_int) :: rc
     end function
     function caar_sphere_wk(handle, op, nets, nete, mode) bind(C, name="caar_sphere_wk") result(rc)

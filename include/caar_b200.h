@@ -247,12 +247,13 @@ void caar_update_time_levels(caar_control* ctl);
    on the kernel caar_run would use in `mode`; each step issues 6 launches (none for an empty element range, which
    still rotates). The levels must be pairwise distinct (stage 1 would overwrite u0), so ntl >= 3. Returns
    CAAR_ERR_STATE before caar_set_params and CAAR_ERR_INVALID for a null control, nsteps < 0, a bad mode or
-   levels that are not pairwise distinct, leaving *ctl unchanged. No DSS runs between stages. */
+   levels that are not pairwise distinct, leaving *ctl unchanged. No DSS runs between stages; caar_run_rk5_dss runs one. */
 int caar_run_rk5(caar_handle h, caar_control* ctl, double dt, int nsteps, int mode);
 int caar_sync(caar_handle h);
 /* number of kernel launches issued through this handle since creation (caar_run, caar_run_rk5: 6 per step,
-   caar_advect_tracers: 4 per step, caar_tracer_bounds and caar_limit_tracers: 1 per call (none for an empty range or
-   qsize == 0), caar_euler_step, caar_norms, ...) */
+   caar_run_rk5_dss: 11 per step, caar_advect_tracers: 4 per step, caar_tracer_bounds and caar_limit_tracers: 1 per call
+   (none for an empty range or qsize == 0), caar_dss and caar_neighbor_minmax: 1 per call (none when nothing is
+   selected), caar_euler_step, caar_norms, ...) */
 long long caar_launch_count(caar_handle h);
 /* CUDA-event stopwatch on the stream the kernels are launched on: start records an event, stop records a
    second one, waits for it and returns the device time between the two in milliseconds. */
@@ -344,13 +345,72 @@ int caar_advect_tracers(caar_handle h, int nets, int nete, int* qn0, int qsize, 
    One limited tracer step on the resident state (the bounds of the step's input, the limiter once on its output; this
    is not HOMME's per-stage limiting inside the step, whose dp_star this library does not hold):
      1  caar_tracer_bounds(h, nets, nete, qn0, qsize, dp_tl)
-     2  optionally widen the bounds over neighbours: caar_bounds_download, the caller's neighbor_minmax, caar_bounds_upload
+     2  caar_neighbor_minmax(h, qsize)                                 widen the bounds over neighbouring elements
      3  caar_advect_tracers(h, nets, nete, &qn0, qsize, dt, 1, mode)
-     4  caar_limit_tracers(h, nets, nete, qn0, qsize, dp_tl)          with the new qn0 */
+     4  caar_limit_tracers(h, nets, nete, qn0, qsize, dp_tl)          with the new qn0
+     5  caar_dss(h, CAAR_F_QDP, 0, qn0, qsize, CAAR_DSS_PROJECT)      with the new qn0
+   Steps 2 and 5 need caar_set_connectivity and act on every element of the handle. HOMME also runs a DSS
+   after each of the three stages inside the step; caar_advect_tracers does not, so this step equals HOMME's only up to
+   that difference. */
 int caar_bounds_upload(caar_handle h, const double* host);
 int caar_bounds_download(caar_handle h, double* host);
 int caar_tracer_bounds(caar_handle h, int nets, int nete, int qtl, int qsize, int dp_tl);
 int caar_limit_tracers(caar_handle h, int nets, int nete, int qtl, int qsize, int dp_tl);
+
+/* ---- the direct stiffness summation (DSS) over shared element-boundary points ----
+   HOMME's compute_and_apply_rhs stores spheremp*(state + dt*rhs) and then assembles the values at the GLL points that two
+   to four elements share: edgeVpack, bndry_exchangeV, edgeVunpack, then a multiply by rspheremp
+   (F/routine_extracted.F90:519+); euler_step does the same to spheremp*Qtens. These calls do that on the device, over
+   every element of the handle, from a map of the points' global ids.
+
+   caar_set_connectivity: gid[E][4][4] is the global id of every GLL point, in the [igp][jgp] order of the C++ layout with
+   CAAR_LAYOUT_CXX; with CAAR_LAYOUT_F90 it is the memory order of HOMME's elem%gdofP(np,np,nelemd) = [ie][j][i]. Points
+   with equal ids are one point; any 64-bit values are accepted, and two points of one element may share an id.
+   Synchronous; replaces an earlier map; works before caar_set_params. The tables are built once on the host
+   (a sort of the 16 E copies) and kept on the device until caar_destroy. CAAR_ERR_INVALID for a null handle or gid or a
+   bad layout, CAAR_ERR_UNSUPPORTED for nelem >= 2^27 (a copy is packed as e*16 + p in 32 bits).
+
+   caar_dss, exactly. The copies of a point are the pairs (e, p) with equal gid, p = 4*igp + jgp, ordered by ascending
+   (e, p); the first is the point's owner. With f_c the field value at copy c and s_c = spheremp[e][p] at call time
+   (a re-uploaded spheremp is used; nothing is cached):
+     m = s_c0 + s_c1 + ...                   sequential in copy order
+     r = 1.0 / m                             IEEE division: HOMME's rspheremp, the reciprocal of the assembled mass
+     CAAR_DSS_ASSEMBLE: S = f_c0 + f_c1 + ...               for inputs that carry spheremp already (the output of
+                                                            compute_and_apply_rhs, weak-form operators)
+     CAAR_DSS_PROJECT:  S = s_c0*f_c0 + s_c1*f_c1 + ...     each product rounded; for fields without the factor (Qtens
+                                                            as caar_advect_tracers stores it, Qdp)
+     every copy = S * r
+   Every operation is rounded separately (no FMA contraction; there is no mode), so the result is bit-reproducible; a
+   point with one copy gets f*r or (s*f)*r, with no add. Each component of v is a scalar field of its own (HOMME's v is
+   in lat-lon components, continuous across panels). m == 0 gives what IEEE gives. The fields are those of field_mask
+   within {CAAR_F_DP3D, CAAR_F_V, CAAR_F_T} at time level tl, and Qdp(qtl) of tracers iq < qsize when CAAR_F_QDP is set;
+   nothing else changes. tl, qtl and qsize are checked whatever the mask.
+   Departure from HOMME: edgeVunpack adds an element's neighbours to that element's own value, so HOMME's copies of one
+   point may differ in the last bit; here every copy receives the identical value.
+   Partitioned handles: only the copies this handle holds are summed. Exchanging the sums of shared points with other
+   handles (HOMME's bndry_exchangeV between ranks) is not provided.
+
+   caar_neighbor_minmax: HOMME's neighbor_minmax on the handle's limiter bounds (caar_tracer_bounds). N(e) is the set of
+   elements other than e that share at least one gid with e (on a cubed sphere the edge and vertex neighbours). For every
+   e, tracer iq < qsize and level k: qmin starts from e's own value, then for each n in N(e) in ascending order
+   if (qmin_n < qmin) qmin = qmin_n; qmax the same with >. Every neighbour's bounds are read before any is changed (a
+   second handle-owned array), so the result does not depend on launch order. Tracers iq >= qsize are unchanged.
+
+   Both are asynchronous on the handle's stream and add one launch; caar_dss none when nothing is selected (mask 0, or
+   only CAAR_F_QDP with qsize == 0), caar_neighbor_minmax none for qsize == 0. They need no caar_set_params.
+   CAAR_ERR_STATE before caar_set_connectivity; CAAR_ERR_INVALID for a null handle, mask bits outside the four fields,
+   tl outside [0, ntl), qtl not 0 or 1, qsize outside [0, qsize_d] or a weighting other than the two below. A rejected
+   call launches nothing and changes nothing. */
+enum { CAAR_DSS_ASSEMBLE = 0, CAAR_DSS_PROJECT = 1 };
+int caar_set_connectivity(caar_handle h, const long long* gid, int layout);
+int caar_dss(caar_handle h, unsigned field_mask, int tl, int qtl, int qsize, int weighting);
+int caar_neighbor_minmax(caar_handle h, int qsize);
+/* caar_run_rk5's step with caar_dss(h, CAAR_F_V | CAAR_F_T | CAAR_F_DP3D, np1 of the stage, 0, 0, CAAR_DSS_ASSEMBLE)
+   after each of its five stages: HOMME's tstep_type 5 with the DSS of compute_and_apply_rhs. The combination reads the
+   assembled u1. Each step issues 11 launches (5 stages, the combination, 5 DSS); the levels rotate as in caar_run_rk5.
+   Returns CAAR_ERR_STATE before caar_set_params or caar_set_connectivity, CAAR_ERR_INVALID for an element range other than
+   [0, nelem) (the DSS spans the handle), and every error of caar_run_rk5, leaving *ctl unchanged. */
+int caar_run_rk5_dss(caar_handle h, caar_control* ctl, double dt, int nsteps, int mode);
 
 /* ---- the weak-form operators behind hyperviscosity (SURVEY §8f rank 4) ----
    Level-local like the tracer step, on the same kernel skeleton, in the pointers_only index conventions

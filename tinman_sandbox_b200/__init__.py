@@ -16,7 +16,7 @@ from .capi import (  # noqa: F401
     Caar, CaarError, FIELD_NAMES, MUTATED_FIELDS, MODE_FAST, MODE_STRICT, lib_path, load_library,
     field_shape, compute_and_apply_rhs, saxpby_host, EXPORTED_SYMBOLS, HOST_ZERO_COPY, host_register,
     host_unregister, CHECKSUM_FIELDS, X_VSTAR, X_QTENS, X_TENSORVISC, X_SCALAR_IN, X_SCALAR_OUT, OP_DIVERGENCE_WK,
-    OP_LAPLACE_SIMPLE, OP_LAPLACE_TENSOR, OP_LAPLACE_TENSOR_REPLACE,
+    OP_LAPLACE_SIMPLE, OP_LAPLACE_TENSOR, OP_LAPLACE_TENSOR_REPLACE, DSS_ASSEMBLE, DSS_PROJECT, DSS_FIELDS,
 )
 
 __all__ = [

@@ -29,6 +29,8 @@ MODE_FAST, MODE_STRICT = 0, 1
 LAYOUT_CXX, LAYOUT_F90 = 0, 1
 X_VSTAR, X_QTENS, X_TENSORVISC, X_SCALAR_IN, X_SCALAR_OUT = 0, 1, 2, 3, 4
 OP_DIVERGENCE_WK, OP_LAPLACE_SIMPLE, OP_LAPLACE_TENSOR, OP_LAPLACE_TENSOR_REPLACE = 0, 1, 2, 3
+DSS_ASSEMBLE, DSS_PROJECT = 0, 1
+DSS_FIELDS = ("elem_state_dp3d", "elem_state_v", "elem_state_T", "elem_state_Qdp")   # what caar_dss can select
 
 # every symbol include/caar_b200.h declares (tests check the library exports all of them)
 EXPORTED_SYMBOLS = (
@@ -41,7 +43,8 @@ EXPORTED_SYMBOLS = (
     "caar_timer_stop", "caar_norms", "caar_compute_and_apply_rhs_host", "caar_saxpby_device",
     "caar_saxpby_host", "caar_checksums", "caar_upload_range", "caar_download_range", "caar_describe",
     "caar_sphere_wk", "caar_run_rk5", "caar_advect_tracers", "caar_bounds_upload", "caar_bounds_download",
-    "caar_tracer_bounds", "caar_limit_tracers",
+    "caar_tracer_bounds", "caar_limit_tracers", "caar_set_connectivity", "caar_dss", "caar_neighbor_minmax",
+    "caar_run_rk5_dss",
 )
 CHECKSUM_FIELDS = ("elem_state_dp3d", "elem_state_v", "elem_state_T", "elem_derived_eta_dot_dpdn",
                    "elem_derived_omega_p", "elem_derived_phi", "elem_derived_vn0")
@@ -142,6 +145,10 @@ def load_library():
     lib.caar_bounds_download.argtypes = [C.c_void_p, C.POINTER(C.c_double)]
     lib.caar_tracer_bounds.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]
     lib.caar_limit_tracers.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]
+    lib.caar_set_connectivity.argtypes = [C.c_void_p, C.POINTER(C.c_longlong), C.c_int]
+    lib.caar_dss.argtypes = [C.c_void_p, C.c_uint, C.c_int, C.c_int, C.c_int, C.c_int]
+    lib.caar_neighbor_minmax.argtypes = [C.c_void_p, C.c_int]
+    lib.caar_run_rk5_dss.argtypes = [C.c_void_p, C.POINTER(Control), C.c_double, C.c_int, C.c_int]
     lib.caar_upload_layout.argtypes = [C.c_void_p, C.POINTER(Arrays), C.c_uint, C.c_int]
     lib.caar_download_layout.argtypes = [C.c_void_p, C.POINTER(Arrays), C.c_uint, C.c_int]
     lib.caar_set_params_f90.argtypes = [C.c_void_p, C.POINTER(Constants), C.POINTER(C.c_double), C.c_double,
@@ -414,6 +421,43 @@ class Caar:
         nete = self.control.nete if nete is None else nete
         _check(self.lib, self.lib.caar_limit_tracers(self.h, nets, nete, int(qtl), int(qsize), int(dp_tl)),
                "caar_limit_tracers")
+        if sync:
+            self.sync()
+
+    # -- the direct stiffness summation over shared element-boundary points -------------------------------------------
+    def set_connectivity(self, gid, layout=LAYOUT_CXX):
+        """caar_set_connectivity: gid [E][4][4] int64, the global id of every GLL point ([igp][jgp] with LAYOUT_CXX, the
+        memory order of HOMME's gdofP(np,np,nelemd) with LAYOUT_F90)."""
+        E = self.shape_args[0]
+        gid = np.ascontiguousarray(gid, dtype=np.int64)
+        if gid.size != E * 16:
+            raise CaarError(f"gid: need {E * 16} ids, got {gid.size}")
+        _check(self.lib, self.lib.caar_set_connectivity(self.h, gid.ctypes.data_as(C.POINTER(C.c_longlong)), int(layout)),
+               "caar_set_connectivity")
+
+    def dss(self, names, tl=None, qtl=0, qsize=0, weighting=DSS_ASSEMBLE, sync=True):
+        """caar_dss in place on the named fields of DSS_FIELDS: dp3d, v, T at time level tl (default control.np1) and
+        Qdp(qtl) of tracers < qsize."""
+        tl = self.control.np1 if tl is None else tl
+        for n in names:
+            if n not in DSS_FIELDS:
+                raise CaarError(f"{n}: caar_dss assembles only {DSS_FIELDS}")
+        _check(self.lib, self.lib.caar_dss(self.h, _mask(names) if names else 0, int(tl), int(qtl), int(qsize),
+                                           int(weighting)), "caar_dss")
+        if sync:
+            self.sync()
+
+    def neighbor_minmax(self, qsize, sync=True):
+        """caar_neighbor_minmax: widen the handle's limiter bounds of tracers < qsize over neighbouring elements."""
+        _check(self.lib, self.lib.caar_neighbor_minmax(self.h, int(qsize)), "caar_neighbor_minmax")
+        if sync:
+            self.sync()
+
+    def run_rk5_dss(self, nsteps, dt, mode=MODE_FAST, sync=True):
+        """run_rk5 with caar_dss of v, T and dp3d after every stage (caar_run_rk5_dss); needs set_connectivity and the
+        control's range [0, nelem)."""
+        _check(self.lib, self.lib.caar_run_rk5_dss(self.h, C.byref(self.control), float(dt), int(nsteps), mode),
+               "caar_run_rk5_dss")
         if sync:
             self.sync()
 

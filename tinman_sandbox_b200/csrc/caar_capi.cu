@@ -6,6 +6,7 @@
 #include <cstring>
 #include <initializer_list>
 #include <new>
+#include <vector>
 
 #include "caar_device.cuh"
 
@@ -73,6 +74,8 @@ struct caar_handle_s {
   double* hybi_dev;  // [nlev+1], Eulerian branch only
   double* extra[5];  // arrays beyond struct Arrays: vstar, qtens, tensorVisc, scalar in / out (allocated on first use)
   double* bounds;  // [nelem][qsize_d][nlev][2] tracer limiter bounds (allocated and zeroed on first use)
+  double* bounds_next;  // the same shape: caar_neighbor_minmax writes it, then it and `bounds` swap
+  caar::DssTables dss;  // connectivity of caar_set_connectivity (dss.start == nullptr before it)
   double* stage;  // device staging buffer of the Fortran-layout copies (allocated on first use)
   // device [2]: the tile scheduler of the thread-per-level laplacians (next chunk, warps done), zero between launches.
   // One pair per handle: all launches of a handle are ordered on its stream, so no two of them share it.
@@ -125,6 +128,26 @@ int check_mode(int mode) {
 int check_time_level(const caar_handle_s* h, int tl) {
   if (tl < 0 || tl >= h->dims.ntl) return fail(CAAR_ERR_INVALID, "time level %d outside [0,%d)", tl, h->dims.ntl);
   return CAAR_OK;
+}
+
+int check_qsize(const caar_handle_s* h, int qsize) {
+  if (qsize < 0 || qsize > h->dims.qsize_d) return fail(CAAR_ERR_INVALID, "qsize=%d outside [0,%d]", qsize, h->dims.qsize_d);
+  return CAAR_OK;
+}
+int check_qtl(int qtl) {
+  if (qtl < 0 || qtl > 1) return fail(CAAR_ERR_INVALID, "qtl=%d must be 0 or 1", qtl);
+  return CAAR_OK;
+}
+// the handle is set and caar_set_connectivity was called
+int check_connected(const caar_handle_s* h, const char* who) {
+  if (!h) return fail(CAAR_ERR_INVALID, "%s: null handle", who);
+  if (!h->dss.start) return fail(CAAR_ERR_STATE, "caar_set_connectivity must be called before %s", who);
+  return CAAR_OK;
+}
+
+void free_dss_tables(const caar::DssTables& t) {
+  for (int* p : {t.start, t.copy, t.nb_start, t.nb})
+    if (p) cudaFree(p);
 }
 
 int validate_control(const caar_handle_s* h, const caar_control* ctl) {
@@ -267,6 +290,8 @@ int caar_destroy(caar_handle h) {
   if (h->out3) cudaFree(h->out3);
   if (h->stage) cudaFree(h->stage);
   if (h->bounds) cudaFree(h->bounds);
+  if (h->bounds_next) cudaFree(h->bounds_next);
+  free_dss_tables(h->dss);
   for (int x = 0; x < CAAR_NUM_EXTRA; ++x)
     if (h->extra[x]) cudaFree(h->extra[x]);
   if (h->hybi_dev) cudaFree(h->hybi_dev);
@@ -505,12 +530,22 @@ int caar_run(caar_handle h, const caar_control* ctl, int nsteps, int mode) {
   return launch_rhs(h, make_args(h, ctl), nsteps, fast);
 }
 
-int caar_run_rk5(caar_handle h, caar_control* ctl, double dt, int nsteps, int mode) {
+namespace {
+
+// The checks and the step loop of caar_run_rk5 and caar_run_rk5_dss; with `dss`, caar_dss of v, T and dp3d at the
+// stage's np1 follows every stage
+int run_rk5(caar_handle h, caar_control* ctl, double dt, int nsteps, int mode, bool dss, const char* who) {
   bool fast = false;
-  if (int rc = check_run(h, ctl, nsteps, mode, "caar_run_rk5", &fast)) return rc;
+  if (int rc = check_run(h, ctl, nsteps, mode, who, &fast)) return rc;
   if (ctl->n0 == ctl->np1 || ctl->n0 == ctl->nm1 || ctl->np1 == ctl->nm1)  // stage 1 would overwrite u0
-    return fail(CAAR_ERR_INVALID, "caar_run_rk5 needs pairwise distinct time levels (n0=%d np1=%d nm1=%d)", ctl->n0,
+    return fail(CAAR_ERR_INVALID, "%s needs pairwise distinct time levels (n0=%d np1=%d nm1=%d)", who, ctl->n0,
                 ctl->np1, ctl->nm1);
+  if (dss) {
+    if (int rc = check_connected(h, who)) return rc;
+    if (ctl->nets != 0 || ctl->nete != h->dims.nelem)
+      return fail(CAAR_ERR_INVALID, "%s: element range [%d,%d) is not [0,%d): the DSS spans the handle", who, ctl->nets,
+                  ctl->nete, h->dims.nelem);
+  }
   DeviceGuard guard(h->device);
   const double w = h->c.eta_ave_w;
   for (int s = 0; s < nsteps; ++s) {
@@ -531,10 +566,25 @@ int caar_run_rk5(caar_handle h, caar_control* ctl, double dt, int nsteps, int mo
       a.dt2 = stage[k].dt2;
       a.eta_ave_w = stage[k].eta_ave_w;
       if (int rc = launch_rhs(h, a, 1, fast)) return rc;
+      if (dss) {
+        CU_TRY(caar::launch_dss(a, h->dss, CAAR_F_V | CAAR_F_T | CAAR_F_DP3D, stage[k].np1, 0, 0, CAAR_DSS_ASSEMBLE,
+                                h->stream));
+        ++h->launches;
+      }
     }
     caar_update_time_levels(ctl);
   }
   return CAAR_OK;
+}
+
+}  // namespace
+
+int caar_run_rk5(caar_handle h, caar_control* ctl, double dt, int nsteps, int mode) {
+  return run_rk5(h, ctl, dt, nsteps, mode, false, "caar_run_rk5");
+}
+
+int caar_run_rk5_dss(caar_handle h, caar_control* ctl, double dt, int nsteps, int mode) {
+  return run_rk5(h, ctl, dt, nsteps, mode, true, "caar_run_rk5_dss");
 }
 
 // ---- caar_run_host: one RHS evaluation on HOST arrays, pipelined over element chunks --------------------
@@ -800,7 +850,7 @@ int check_euler(caar_handle h, int nets, int nete, int qn0, int qsize, int mode,
   if (int rc = check_handle(h, who)) return rc;
   if (int rc = check_range(h, nets, nete)) return rc;
   if (qn0 < 0 || qn0 > 1) return fail(CAAR_ERR_INVALID, "qn0=%d must be 0 or 1", qn0);
-  if (qsize < 0 || qsize > h->dims.qsize_d) return fail(CAAR_ERR_INVALID, "qsize=%d outside [0,%d]", qsize, h->dims.qsize_d);
+  if (int rc = check_qsize(h, qsize)) return rc;
   return check_mode(mode);
 }
 
@@ -888,8 +938,8 @@ int copy_bounds(caar_handle h, double* host, bool to_device) {
 int run_limiter(caar_handle h, int nets, int nete, int qtl, int qsize, int dp_tl, bool limit) {
   if (!h) return fail(CAAR_ERR_INVALID, "null handle");
   if (int rc = check_range(h, nets, nete)) return rc;
-  if (qtl < 0 || qtl > 1) return fail(CAAR_ERR_INVALID, "qtl=%d must be 0 or 1", qtl);
-  if (qsize < 0 || qsize > h->dims.qsize_d) return fail(CAAR_ERR_INVALID, "qsize=%d outside [0,%d]", qsize, h->dims.qsize_d);
+  if (int rc = check_qtl(qtl)) return rc;
+  if (int rc = check_qsize(h, qsize)) return rc;
   if (int rc = check_time_level(h, dp_tl)) return rc;
   if (nete == nets || qsize == 0) return CAAR_OK;
   DeviceGuard guard(h->device);
@@ -913,6 +963,73 @@ int caar_tracer_bounds(caar_handle h, int nets, int nete, int qtl, int qsize, in
 
 int caar_limit_tracers(caar_handle h, int nets, int nete, int qtl, int qsize, int dp_tl) {
   return run_limiter(h, nets, nete, qtl, qsize, dp_tl, true);
+}
+
+// ---- direct stiffness summation and neighbour bounds -------------------------------------------------------------
+int caar_set_connectivity(caar_handle h, const long long* gid, int layout) {
+  if (!h || !gid) return fail(CAAR_ERR_INVALID, "null argument");
+  if (layout != CAAR_LAYOUT_CXX && layout != CAAR_LAYOUT_F90) return fail(CAAR_ERR_INVALID, "layout=%d", layout);
+  const int E = h->dims.nelem;
+  if (E >= (1 << 27)) return fail(CAAR_ERR_UNSUPPORTED, "nelem=%d: copies are packed as e*16 + p in 32 bits", E);
+  std::vector<long long> cxx(gid, gid + (size_t)E * 16);
+  if (layout == CAAR_LAYOUT_F90)  // gdofP(i,j,ie) at [ie][j][i]; Fortran (i,j) is [igp][jgp]
+    for (size_t e = 0; e < (size_t)E; ++e)
+      for (int i = 0; i < 4; ++i)
+        for (int j = 0; j < 4; ++j) cxx[e * 16 + 4 * i + j] = gid[e * 16 + 4 * j + i];
+  caar::DssHostTables t;
+  caar::DssTables d;
+  std::memset(&d, 0, sizeof d);
+  d.ngroups = caar::build_dss_tables(cxx.data(), E, &t);
+  DeviceGuard guard(h->device);
+  cudaError_t e = cudaSuccess;
+  int** dst[4] = {&d.start, &d.copy, &d.nb_start, &d.nb};
+  const std::vector<int>* src[4] = {&t.start, &t.copy, &t.nb_start, &t.nb};
+  for (int i = 0; i < 4 && e == cudaSuccess; ++i) {
+    const size_t bytes = (src[i]->empty() ? 1 : src[i]->size()) * sizeof(int);
+    e = cudaMalloc(dst[i], bytes);
+    if (e == cudaSuccess && !src[i]->empty())
+      e = cudaMemcpyAsync(*dst[i], src[i]->data(), src[i]->size() * sizeof(int), cudaMemcpyHostToDevice, h->stream);
+  }
+  if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+  if (e != cudaSuccess) {  // the earlier map stays
+    free_dss_tables(d);
+    return fail(e == cudaErrorMemoryAllocation ? CAAR_ERR_NOMEM : CAAR_ERR_CUDA, "caar_set_connectivity: %s",
+                cudaGetErrorString(e));
+  }
+  free_dss_tables(h->dss);  // the stream is idle: no launch still reads the earlier map
+  h->dss = d;
+  return CAAR_OK;
+}
+
+int caar_dss(caar_handle h, unsigned field_mask, int tl, int qtl, int qsize, int weighting) {
+  if (int rc = check_connected(h, "caar_dss")) return rc;
+  const unsigned fields = CAAR_F_DP3D | CAAR_F_V | CAAR_F_T | CAAR_F_QDP;
+  if (field_mask & ~fields) return fail(CAAR_ERR_INVALID, "field_mask=0x%x: only dp3d, v, T and Qdp", field_mask);
+  if (int rc = check_time_level(h, tl)) return rc;
+  if (int rc = check_qtl(qtl)) return rc;
+  if (int rc = check_qsize(h, qsize)) return rc;
+  if (weighting != CAAR_DSS_ASSEMBLE && weighting != CAAR_DSS_PROJECT) return fail(CAAR_ERR_INVALID, "weighting=%d", weighting);
+  if (!(field_mask & (CAAR_F_DP3D | CAAR_F_V | CAAR_F_T)) && !((field_mask & CAAR_F_QDP) && qsize > 0)) return CAAR_OK;
+  DeviceGuard guard(h->device);
+  CU_TRY(caar::launch_dss(make_args(h, nullptr), h->dss, field_mask, tl, qtl, qsize, weighting, h->stream));
+  ++h->launches;
+  return CAAR_OK;
+}
+
+int caar_neighbor_minmax(caar_handle h, int qsize) {
+  if (int rc = check_connected(h, "caar_neighbor_minmax")) return rc;
+  if (int rc = check_qsize(h, qsize)) return rc;
+  if (qsize == 0) return CAAR_OK;
+  DeviceGuard guard(h->device);
+  double* bounds = nullptr;
+  if (int rc = bounds_buffer(h, &bounds)) return rc;
+  if (!h->bounds_next) CU_TRY(cudaMalloc(&h->bounds_next, bounds_count(h->dims) * sizeof(double)));
+  CU_TRY(caar::launch_neighbor_minmax(h->dss, h->dims.nelem, h->dims.qsize_d, h->dims.nlev, qsize, bounds,
+                                      h->bounds_next, h->stream));
+  ++h->launches;
+  h->bounds = h->bounds_next;
+  h->bounds_next = bounds;
+  return CAAR_OK;
 }
 
 int caar_sphere_wk(caar_handle h, int op, int nets, int nete, int mode) {

@@ -2,6 +2,7 @@
 #pragma once
 #include <cstddef>
 #include <cstdint>
+#include <vector>
 #include <cuda.h>
 #include <cuda_runtime.h>
 
@@ -140,6 +141,27 @@ cudaError_t launch_tracer_bounds(const KernelArgs& a, int nets, int nete, int qt
                                  cudaStream_t s);
 cudaError_t launch_limit_tracers(const KernelArgs& a, int nets, int nete, int qtl, int qsize, int dp_tl, double* bounds,
                                  cudaStream_t s);
+// DSS and neighbour bounds (caar_dss.cu) over the connectivity of caar_set_connectivity. The groups of copies of one
+// global id, in the order of their owners (first copies in (e, p) order): group g is copy[start[g] .. start[g+1]), each
+// copy e*16 + p in (e, p) order. nb[nb_start[e] .. nb_start[e+1]) are the other elements that share a point with e,
+// ascending.
+struct DssHostTables {
+  std::vector<int> start, copy, nb_start, nb;
+};
+struct DssTables {  // the same on the device
+  int ngroups;
+  int *start, *copy, *nb_start, *nb;
+};
+// gid [nelem][16] in the C order; returns the number of groups
+int build_dss_tables(const long long* gid, int nelem, DssHostTables* t);
+// in place on the selected slices (CAAR_F_DP3D / V / T at time level tl, Qdp(qtl) of tracers < qsize); one launch,
+// none when nothing is selected
+cudaError_t launch_dss(const KernelArgs& a, const DssTables& t, unsigned mask, int tl, int qtl, int qsize,
+                       int weighting, cudaStream_t s);
+// out = neighbor_minmax(in) for tracers < qsize, out = in for the others; bounds [nelem][qsize_d][L][2]; one launch,
+// none for qsize == 0
+cudaError_t launch_neighbor_minmax(const DssTables& t, int nelem, int qsize_d, int L, int qsize, const double* in,
+                                   double* out, cudaStream_t s);
 // checksums of the seven mutated arrays + energy norms (caar_aux.cu); partial [nelem][8][2], bits [nelem][7]
 cudaError_t launch_checksums(const KernelArgs& a, int tl, int nets, int nete, double cp, double* partial,
                              unsigned long long* bits, double* out16, unsigned long long* out7, cudaStream_t s);

@@ -1,0 +1,136 @@
+#!/usr/bin/env python
+"""Times caar_dss, caar_neighbor_minmax and caar_run_rk5_dss on resident data over cubed-sphere connectivity.
+    python tools/dss_bench.py [--reps 10]
+Prints one JSON line per case:
+  state DSS (v, T, dp3d; ASSEMBLE) at 86400 x 72 (ne = 120) and 48600 x 128 (ne = 90)
+  Qdp DSS (PROJECT) at 86400 x 72 with qsize 4 and 21600 x 72 (ne = 60) with qsize 35
+  caar_neighbor_minmax at the two Qdp sizes
+each in two element orders: "panel" (face by face, row by row: close to HOMME's space-filling order, neighbours a face
+row apart) and "shuffled" (a random permutation with rotated element blocks: the neighbours of a group are anywhere, the
+adversarial case for L2); and caar_run_rk5 against caar_run_rk5_dss at 86400 x 72 in fast mode, alternating call by call.
+spheremp is 1, so ASSEMBLE and PROJECT both average the copies and the data stays bounded over repeated in-place calls.
+Reported: min and median ms of --reps calls between CUDA events on the handle's stream, the compulsory bytes (every
+selected value read and written once), GB/s over them, the fraction of the device-to-device copy rate measured in the
+same process, the byte-bound time at that rate, and the card's name, power limit and SM clocks from a read-only
+nvidia-smi query. A second pass under torch.profiler gives each case's kernel time (it writes no trace)."""
+import argparse
+import json
+import os
+import sys
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path[:0] = [ROOT, os.path.join(ROOT, "tests"), os.path.join(ROOT, "tools")]
+import tinman_sandbox_b200 as tb  # noqa: E402
+from rk5_bench import copy_peak_gbps, gpu_info  # noqa: E402
+
+import dss_oracle as do  # noqa: E402
+from oracle import harness  # noqa: E402
+
+STATE = ("elem_state_dp3d", "elem_state_v", "elem_state_T")
+
+
+def mesh(ne, order):
+    return do.cubed_sphere_gid(ne, np.random.default_rng(ne) if order == "shuffled" else None)
+
+
+def timed(h, fn, reps):
+    fn()
+    h.sync()
+    ms = []
+    for _ in range(reps):
+        h.timer_start()
+        fn()
+        ms.append(h.timer_stop())
+    return min(ms), float(np.median(ms))
+
+
+def kernel_ms(fn, h, reps, name):
+    """mean device time of the kernels whose name contains `name`, over reps calls under torch.profiler"""
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    h.sync()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for _ in range(reps):
+            fn()
+        h.sync()
+    ev = [e for e in prof.key_averages() if name in e.key]
+    total = sum(getattr(e, "device_time_total", getattr(e, "cuda_time_total", 0.0)) for e in ev)
+    count = sum(e.count for e in ev)
+    torch.cuda.synchronize()
+    return total / 1e3 / count if count else None
+
+
+def report(case, order, E, L, nbytes, best, med, kms, peak, info):
+    print(json.dumps(dict(case=case, order=order, E=E, L=L, bytes_gb=round(nbytes / 1e9, 3), min_ms=round(best, 4),
+                          median_ms=round(med, 4), kernel_ms=None if kms is None else round(kms, 4),
+                          gbps=round(nbytes / best / 1e6, 1), of_copy_rate=round(nbytes / best / 1e6 / peak, 3),
+                          bound_ms=round(nbytes / peak / 1e6, 3), copy_gbps=round(peak, 1), **info)), flush=True)
+
+
+def dss_cases(reps, peak, info):
+    for case, ne, L, Qd, qs in (("state", 120, 72, 1, 0), ("state", 90, 128, 1, 0), ("qdp", 120, 72, 4, 4),
+                                ("qdp", 60, 72, 35, 35)):
+        E = 6 * ne * ne
+        h = tb.Caar(E, L, Qd, 3 if case == "state" else 1)
+        h.upload({"elem_spheremp": np.ones((E, 4, 4))}, names=("elem_spheremp",))
+        for order in ("panel", "shuffled"):
+            h.set_connectivity(mesh(ne, order))
+            if case == "state":
+                fn = lambda: h.dss(STATE, tl=1, sync=False)
+                nbytes = 2 * 4 * E * L * 16 * 8
+            else:
+                fn = lambda: h.dss(("elem_state_Qdp",), tl=0, qtl=1, qsize=qs, weighting=tb.DSS_PROJECT, sync=False)
+                nbytes = 2 * qs * E * L * 16 * 8
+            best, med = timed(h, fn, reps)
+            report(f"dss_{case}" + (f"_q{qs}" if qs else ""), order, E, L, nbytes, best, med,
+                   kernel_ms(fn, h, reps, "dss_kernel"), peak, info)
+            if case == "qdp":
+                fn = lambda: h.neighbor_minmax(qs, sync=False)
+                nbytes = 2 * qs * E * L * 16
+                best, med = timed(h, fn, reps)
+                report(f"neighbor_minmax_q{qs}", order, E, L, nbytes, best, med,
+                       kernel_ms(fn, h, reps, "neighbor_minmax"), peak, info)
+        h.close()
+
+
+def rk5_case(reps, peak, info):
+    E, L, P = 86400, 72, 257
+    pool = harness.PortOracle().init(P, L)
+    pool.arrays["elem_spheremp"][...] = 1.0
+    h = tb.Caar(E, L)
+    h.set_params(pool.consts, pool.dvv, pool.ps0, pool.hyai)
+    h.set_control(0, E, 0, 1, 2, int(pool.ctl[5]), dt2=pool.dt2)
+    for e0 in range(0, E, P):
+        e1 = min(E, e0 + P)
+        h.upload_range({n: np.ascontiguousarray(a[:e1 - e0]) for n, a in pool.arrays.items()}, e0, e1)
+    h.set_connectivity(mesh(120, "panel"))
+    runs = {"rk5": lambda: h.run_rk5(1, 1.0, tb.MODE_FAST, sync=False),
+            "rk5_dss": lambda: h.run_rk5_dss(1, 1.0, tb.MODE_FAST, sync=False)}
+    ms = {k: [] for k in runs}
+    for k, fn in runs.items():
+        fn()
+    h.sync()
+    for _ in range(reps):
+        for k, fn in runs.items():
+            h.timer_start()
+            fn()
+            ms[k].append(h.timer_stop())
+    h.close()
+    for k, nbytes in (("rk5", 90.7e9), ("rk5_dss", 122.5e9)):
+        report(f"step_{k}", "panel", E, L, nbytes, min(ms[k]), float(np.median(ms[k])), None, peak, info)
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--reps", type=int, default=10)
+    args = ap.parse_args()
+    info = gpu_info()
+    peak = copy_peak_gbps()
+    dss_cases(args.reps, peak, info)
+    rk5_case(max(3, args.reps // 2), peak, info)
+
+
+if __name__ == "__main__":
+    main()
