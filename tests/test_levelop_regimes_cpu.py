@@ -27,29 +27,26 @@ SMS_B200 = 148
 # shared memory of launch_op / launch_lapflat:
 LEVELOP_PER_SM = 4   # levelop_kernel<OP>: 128 registers x 128 threads, 4 stages of 1-2 KB per warp
 LAPFLAT_PER_SM = 2   # laplace_flat_kernel<TENSOR>: 194 (simple) / 212 (tensor) registers x 128 threads, ~100 KB smem
-WPC = 4              # warps per CTA of both kernels (LEVELOP_WPC, LAPFLAT_WPC)
+WPC = 4              # warps per CTA of both kernels (WPC and FW in caar_levelops.cu)
 GL = 8               # levels per unit of levelop_kernel
 FT = 32              # rows (element x level) per tile of laplace_flat_kernel
-EULER_STRICT_CAP = 3 * 2   # euler_step_kernel: CTAs per SM times CAAR_EULER_WAVES (default 2)
 
 
-def regime(op, E, L, Q=1, sms=SMS_B200, per_sm=None, waves=0, chunk=0):
+def regime(op, E, L, Q=1, sms=SMS_B200, per_sm=None):
     """The work distribution a launch on E elements gets: mirrors launch_op, launch_lapflat (csrc/caar_levelops.cu)
     and launch_euler_step (csrc/caar_euler.cu) and must follow them when they change. op: "euler" (fast tracer step),
-    "divwk", "lap_rows" (the row-decomposed laplacians, nlev < 16), "lap_flat", "euler_strict". waves / chunk: the
-    CAAR_LEVELOP_WAVES / CAAR_LAPLACE_CHUNK (CAAR_EULER_WAVES for euler_strict) override, 0 = default."""
+    "divwk", "lap_rows" (the row-decomposed laplacians, nlev < 16), "lap_flat", "euler_strict"."""
     if op == "lap_flat":
         per_sm = LAPFLAT_PER_SM if per_sm is None else per_sm
         tiles = -(-E * L // FT)
         resident = sms * per_sm * WPC
-        c = chunk if chunk > 0 else (2 if tiles < resident * 16 else 4)
+        c = 2 if tiles < resident * 16 else 4
         warps = min(sms * per_sm, -(-tiles // WPC)) * WPC
         return dict(tiles=tiles, chunk=c, warps=warps, per_warp=tiles / warps, chunks=-(-tiles // c),
                     elems_per_tile=max((FT * t % L + FT - 1) // L + 1 for t in range(L)))
     if op == "euler_strict":
         groups = -(-E * L // 64)
-        w = waves if waves != 0 else 2
-        blocks = min(groups, sms * 3 * w) if w > 0 else groups
+        blocks = min(groups, sms * 3 * 2)
         return dict(groups=groups, blocks=blocks, iters=groups / blocks)
     per_sm = LEVELOP_PER_SM if per_sm is None else per_sm
     ng = -(-L // GL)
@@ -57,7 +54,6 @@ def regime(op, E, L, Q=1, sms=SMS_B200, per_sm=None, waves=0, chunk=0):
     per_wave = sms * per_sm * WPC * (48 if op == "euler" else 12)
     wv = (units + per_wave // 2) // per_wave
     wv = 1 if (wv < 1 or op == "lap_rows") else min(wv, 16)
-    wv = waves if waves > 0 else wv
     warps = min(sms * per_sm * wv, -(-units // WPC)) * WPC
     upw = units / warps
     return dict(units=units, waves=wv, warps=warps, per_warp=upw, items_per_warp=upw / Q,

@@ -1,49 +1,37 @@
 """The level-local kernels in the regimes their persistent warps reach in production, against the extended-precision
-reference (oracle/hp_reference.py) with the pointwise gate |g - v| <= K u M, and under every launch knob of DESIGN §7b.
+reference (oracle/hp_reference.py) with the pointwise gate |g - v| <= K u M.
 
-1. The steady-state matrix (CASES of tests/test_levelop_regimes_cpu.py) at default knobs: tracer step (T), fast and
-   strict; divergence_sphere_wk (D); the row-decomposed laplacians (R, nlev < 16); the flat laplacians (F, chunk 4).
-   Each case must reach its regime on this device (the test fails, not skips, when it does not). Fast mode is gated
-   pointwise; strict mode must equal the FP64 restatement (PortOracle) bit for bit. Rows outside the element range and
-   tracers past qsize must keep their -7 sentinel.
-2. Knob legs. Every knob is read once per process into a `static`, so each setting runs in a child process
-   (`python tests/test_levelop_regimes_gpu.py --knob-worker SPEC`) that loads the library fresh, runs its jobs and
-   writes .npz files; the parent computes the same jobs in process at default knobs and gates the child's results.
-   Every knob only changes the schedule and must leave the results bit-identical.
+The steady-state matrix (CASES of tests/test_levelop_regimes_cpu.py): tracer step (T), fast and strict;
+divergence_sphere_wk (D); the row-decomposed laplacians (R, nlev < 16); the flat laplacians (F, chunk 4). Each case must
+reach its regime on this device (the test fails, not skips, when it does not). Fast mode is checked pointwise; strict mode
+must equal the FP64 restatement (PortOracle) bit for bit. Rows outside the element range and tracers past qsize must
+keep their -7 sentinel. F2 and F3 then queue 50 flat-laplacian launches over random element ranges into one buffer,
+which must equal, bit for bit, the element-wise composition of whole-handle launches.
 
-The report (test_zz_report_regimes) prints, per kernel, case and knob, the regime, the worst ratio against K and
-where the worst point sits in the work distribution: (warp, unit) for levelop_kernel, (tile, chunk) for the flat
-laplacians."""
-import json
+The report (test_zz_report_regimes) prints, per kernel and case, the regime, the worst ratio against K and where the
+worst point sits in the work distribution: (warp, unit) for levelop_kernel, (tile, chunk) for the flat laplacians."""
 import multiprocessing
 import os
-import subprocess
-import sys
 from concurrent.futures import ProcessPoolExecutor
 
 import numpy as np
 import pytest
 
-if __name__ == "__main__":                          # knob worker: the repository and tests/ on the path
-    _HERE = os.path.dirname(os.path.abspath(__file__))
-    sys.path[:0] = [os.path.dirname(_HERE), _HERE]
-
-import tinman_sandbox_b200 as tb  # noqa: E402
-from oracle import harness  # noqa: E402
-from oracle import hp_reference as hp  # noqa: E402
-from test_levelop_regimes_cpu import (CASES, FT, GL, case_regime, hp_slice, lean_inputs, levelop_unit_warp,  # noqa: E402
-                                      missed, sub_state)
-from test_pointwise_cpu import TLS, rhs_case_state  # noqa: E402
+import tinman_sandbox_b200 as tb
+from oracle import harness
+from oracle import hp_reference as hp
+from test_levelop_regimes_cpu import (CASES, FT, GL, case_regime, hp_slice, lean_inputs, levelop_unit_warp, missed,
+                                      sub_state)
 
 pytestmark = pytest.mark.gpu
 DT = 150.0
-KNOBS = ("CAAR_LEVELOP_WAVES", "CAAR_LAPLACE_CHUNK", "CAAR_EULER_WAVES", "CAAR_CLUSTER_POLICY", "CAAR_PF_DIST")
 REPORT = []          # lines of the final report
 LAP_OPS = (("laplace_simple", tb.OP_LAPLACE_SIMPLE, hp.K_LAPLACE_SIMPLE),
            ("laplace_tensor", tb.OP_LAPLACE_TENSOR, hp.K_LAPLACE_TENSOR))
+RANDOM_RANGES = ("F2", "F3")  # flat laplacian cases at chunk 4 that also run the random-range composition check
 
 
-# ---- running a job on the device (in process, or in a knob worker) -------------------------------------------------
+# ---- running a job on the device -------------------------------------------------------------------------------------
 
 def _handle(s, E, L, Q, names):
     h = tb.Caar(E, L, Q)
@@ -60,21 +48,7 @@ def job_inputs(j):
 
 
 def run_job(j, inputs=None):
-    """-> dict of output arrays. j: a case of CASES (plus "mode"), or a "rhs" job (fused kernel on an RHS_CASES-style
-    state). "ranges": after the first run, that many more launches of the laplacians over random element ranges,
-    queued without synchronisation; the output is the buffer after the last."""
-    if j["op"] == "rhs":
-        s, hybi = rhs_case_state(j)
-        h = tb.Caar(s.nelem, s.nlev, s.qsize_d, s.ntl)
-        h.set_params(s.consts, s.dvv, s.ps0, s.hyai)
-        if hybi is not None:
-            h.set_vertical_coordinate(0, hybi)
-        h.set_control(*[int(x) for x in s.ctl], dt2=s.dt2)
-        h.upload(s.arrays)
-        h.compute_and_apply_rhs(2, j["mode"])
-        h.download(s.arrays, names=harness.MUTATED)
-        h.close()
-        return {n: s.arrays[n] for n in harness.MUTATED}
+    """-> dict of output arrays. j: a case of CASES plus "mode"."""
     s, vin, sin, tv = inputs or job_inputs(j)
     E, L, (lo, hi), mode = j["E"], j["nlev"], j["range"], j["mode"]
     if j["op"] == "euler":
@@ -106,17 +80,52 @@ def run_job(j, inputs=None):
     h.upload_extra(tb.X_SCALAR_OUT, sin)
     h.sphere_wk(tb.OP_LAPLACE_TENSOR_REPLACE, mode, nets=lo, nete=hi)
     out["laplace_tensor_replace"] = h.download_extra(tb.X_SCALAR_OUT, shape)
-    if j.get("ranges"):
-        rng = np.random.default_rng(j["seed"] + 1)
-        h.upload_extra(tb.X_SCALAR_OUT, sentinel)
-        for n in range(j["ranges"]):
-            a = int(rng.integers(0, E - 1))
-            b = int(rng.integers(a + 1, E + 1))
-            h.sphere_wk(LAP_OPS[n % 2][1], mode, nets=a, nete=b, sync=False)
-        h.sync()
-        out["random_ranges"] = h.download_extra(tb.X_SCALAR_OUT, shape)
     h.close()
     return out
+
+
+def lap_buffers(c, inputs, runs):
+    """One handle on a case's inputs; per run, a sentinel-filled output buffer and the run's fast-mode (op, nets, nete)
+    launches queued without synchronisation -> the buffers after each run."""
+    s, _, sin, tv = inputs
+    E, L = c["E"], c["nlev"]
+    h = _handle(s, E, L, 1, ("elem_Dinv", "elem_spheremp"))
+    h.upload_extra(tb.X_SCALAR_IN, sin)
+    h.upload_extra(tb.X_TENSORVISC, tv)
+    out = []
+    for launches in runs:
+        h.upload_extra(tb.X_SCALAR_OUT, np.full((E, L, 4, 4), -7.0))
+        for op, a, b in launches:
+            h.sphere_wk(op, tb.MODE_FAST, nets=a, nete=b, sync=False)
+        h.sync()
+        out.append(h.download_extra(tb.X_SCALAR_OUT, (E, L, 4, 4)))
+    h.close()
+    return out
+
+
+def check_random_ranges(c, inputs, fast):
+    """50 launches over seeded random element ranges, alternating laplace_simple and laplace_tensor, queued into one
+    sentinel-filled buffer: a tile-scheduler counter left non-zero by one launch would make the next skip tiles. A row
+    of the flat laplacians depends only on its own element's data and geometry, so every element must hold, bit for
+    bit, the whole-handle [0, E) output of the op of the last launch that covered it, and the sentinel if none did."""
+    E = c["E"]
+    rng = np.random.default_rng(c["seed"] + 1)
+    launches = []
+    for n in range(50):
+        a = int(rng.integers(0, E - 1))
+        launches.append((LAP_OPS[n % 2], a, int(rng.integers(a + 1, E + 1))))
+    whole = fast
+    if c["range"] != (0, E):  # the tested range (F2: from element 1) is not the whole handle
+        whole = dict(zip([name for name, _, _ in LAP_OPS],
+                         lap_buffers(c, inputs, [[(op, 0, E)] for _, op, _ in LAP_OPS])))
+    got, = lap_buffers(c, inputs, [[(op, a, b) for (_, op, _), a, b in launches]])
+    want = np.full(got.shape, -7.0)
+    for (name, _, _), a, b in launches:
+        want[a:b] = whole[name][a:b]
+    same = np.array_equal(got, want)
+    REPORT.append(f"{'laplace_flat random ranges':30s} {c['id']:4s} 50 launches "
+                  f"{'bit-identical to' if same else 'DIFFER from'} the composition of whole-handle launches")
+    assert same, (c["id"], "elements that differ", np.flatnonzero(np.any(got != want, axis=(1, 2, 3)))[:20])
 
 
 # ---- gating and reporting -------------------------------------------------------------------------------------------
@@ -163,7 +172,7 @@ def _shutdown_pool():
         _POOL.pop().shutdown()
 
 
-def gate_sliced(kernel, c, got, name, inputs, K, knob, sms, qn0=0, qsize=0):
+def gate_sliced(kernel, c, got, name, inputs, K, sms, qn0=0, qsize=0):
     """The pointwise gate over [nets,nete) of `got` (elements first); the extended-precision reference of `name` is
     computed in slices of elements, in parallel."""
     lo, hi = c["range"]
@@ -177,9 +186,9 @@ def gate_sliced(kernel, c, got, name, inputs, K, knob, sms, qn0=0, qsize=0):
         if r > worst[0]:
             worst = (r, (at[0] + a,) + at[1:], vm)
     r, at, vm = worst
-    REPORT.append(f"{kernel:30s} {c['id']:4s} {knob:34s} worst ratio {r:7.3f} (K {K}) at {at}, |v|/M {vm:.1e}, "
+    REPORT.append(f"{kernel:30s} {c['id']:4s} worst ratio {r:7.3f} (K {K}) at {at}, |v|/M {vm:.1e}, "
                   f"{locate(c, at, sms)}")
-    assert r <= K, (kernel, c["id"], knob, r, at, vm, locate(c, at, sms))
+    assert r <= K, (kernel, c["id"], r, at, vm, locate(c, at, sms))
 
 
 def check_sentinel(c, got, name="", sin=None):
@@ -206,21 +215,21 @@ def port_reference(c, s, vin, sin, tv):
             for name, _, _ in LAP_OPS}
 
 
-def gate_fast(c, got, inputs, knob, sms):
+def gate_fast(c, got, inputs, sms):
     """Every fast-mode output of a case against the reference; laplace_tensor_replace bit-equal to laplace_tensor."""
     s, vin, sin, tv = inputs
     q = c["qsize"]
     kind = {"euler": "euler_step", "divwk": "divergence_sphere_wk", "lap_rows": "levelop", "lap_flat": "flat"}[c["op"]]
     if c["op"] == "euler":
-        gate_sliced("euler_step_fast", c, got["qtens"][:, :q], "euler_step", (s, vin, None), hp.K_EULER, knob,
-                    sms, qn0=c["qn0"], qsize=q)
+        gate_sliced("euler_step_fast", c, got["qtens"][:, :q], "euler_step", (s, vin, None), hp.K_EULER, sms,
+                    qn0=c["qn0"], qsize=q)
     elif c["op"] == "divwk":
-        gate_sliced("divergence_sphere_wk_fast", c, got[kind], kind, (s, vin, None), hp.K_DIVWK, knob, sms)
+        gate_sliced("divergence_sphere_wk_fast", c, got[kind], kind, (s, vin, None), hp.K_DIVWK, sms)
     else:
         for name, _, K in LAP_OPS:
-            gate_sliced(f"{name}_{kind}", c, got[name], name, (s, sin, tv), K, knob, sms)
+            gate_sliced(f"{name}_{kind}", c, got[name], name, (s, sin, tv), K, sms)
         lo, hi = c["range"]
-        assert np.array_equal(got["laplace_tensor_replace"][lo:hi], got["laplace_tensor"][lo:hi]), (c["id"], knob)
+        assert np.array_equal(got["laplace_tensor_replace"][lo:hi], got["laplace_tensor"][lo:hi]), c["id"]
 
 
 def device_sms():
@@ -228,17 +237,10 @@ def device_sms():
     return torch.cuda.get_device_properties(0).multi_processor_count
 
 
-@pytest.fixture(scope="module")
-def default_knobs():
-    """The in-process runs are the default-knob runs: none of the knobs may be set for this process."""
-    set_ = [k for k in KNOBS if k in os.environ]
-    assert not set_, f"run without {set_}: the in-process results stand for the default knobs"
-
-
-# ---- 1. the steady-state matrix at default knobs --------------------------------------------------------------------
+# ---- the steady-state matrix -----------------------------------------------------------------------------------------
 
 @pytest.mark.parametrize("c", CASES, ids=lambda c: c["id"])
-def test_steady_state_matrix(c, default_knobs):
+def test_steady_state_matrix(c):
     sms = device_sms()
     r = case_regime(c, sms)
     assert not missed(c, r), f"{c['id']} misses its regime on {sms} SMs: {missed(c, r)} ({r})"
@@ -251,122 +253,20 @@ def test_steady_state_matrix(c, default_knobs):
         lo, hi = c["range"]
         assert np.array_equal(g[lo:hi, :c["qsize"]] if c["op"] == "euler" else g[lo:hi],
                               w[lo:hi, :c["qsize"]] if c["op"] == "euler" else w[lo:hi]), (c["id"], name, "strict")
-    REPORT.append(f"{c['op'] + '_strict':30s} {c['id']:4s} {'default':34s} bit-identical to the FP64 restatement "
+    REPORT.append(f"{c['op'] + '_strict':30s} {c['id']:4s} bit-identical to the FP64 restatement "
                   f"({', '.join(f'{k} {v:.3g}' for k, v in r.items())})")
     fast = run_job(dict(c, mode=tb.MODE_FAST), inputs)
     for name, g in fast.items():
         check_sentinel(c, g, name, inputs[2])
-    gate_fast(c, fast, inputs, "default", sms)
-
-
-# ---- 2. knob legs in child processes --------------------------------------------------------------------------------
-
-def _by_id(cid):
-    return next(c for c in CASES if c["id"] == cid)
-
-
-def _shrunk(cid, E, **kw):
-    c = dict(_by_id(cid), E=E, range=(0, E))
-    c.update(kw, id=f"{cid}@{E}")
-    return c
-
-
-def _rhs_jobs():
-    jobs = []
-    for i, (L, eul) in enumerate(((30, False), (72, False), (96, False), (128, False), (72, True))):
-        for mode in (tb.MODE_STRICT, tb.MODE_FAST):
-            E = 600
-            jobs.append(dict(id=f"rhs{'_eul' if eul else ''}{L}_{'strict' if mode else 'fast'}", op="rhs", nlev=L,
-                             eulerian=eul, gen=("stratified", "randomize")[i % 2], tls=TLS[i % 3], qn0=(i % 3) - 1,
-                             E=E, range=(2, E - 1) if i % 2 else (0, E), seed=9000 + i, mode=mode))
-    return jobs
-
-
-T2, D1 = _by_id("T2"), _by_id("D1")
-LAP_CHUNK_JOBS = [dict(_shrunk("F2", 4096, range=(1, 4096)), ranges=50), dict(_shrunk("F3", 4096), ranges=50)]
-SCHEDULE_JOBS = ([dict(T2, mode=tb.MODE_FAST, id="T2_fast"), dict(T2, mode=tb.MODE_STRICT, id="T2_strict"),
-                  dict(D1, mode=tb.MODE_FAST, id="D1_fast")]
-                 + [dict(j, mode=tb.MODE_FAST, id=j["id"] + "_fast") for j in LAP_CHUNK_JOBS] + _rhs_jobs())
-
-# Schedule-only knob values are combined into three children: each knob is read by one kernel only.
-SCHEDULE_LEGS = [
-    {"CAAR_LEVELOP_WAVES": "1", "CAAR_LAPLACE_CHUNK": "1", "CAAR_EULER_WAVES": "1", "CAAR_CLUSTER_POLICY": "1",
-     "CAAR_PF_DIST": "0"},
-    {"CAAR_LEVELOP_WAVES": "16", "CAAR_LAPLACE_CHUNK": "3", "CAAR_EULER_WAVES": "0", "CAAR_CLUSTER_POLICY": "2",
-     "CAAR_PF_DIST": "1"},
-    {"CAAR_LEVELOP_WAVES": "200", "CAAR_LAPLACE_CHUNK": "64", "CAAR_PF_DIST": str(600 + 5)},
-]
-
-
-def run_worker(env_knobs, jobs, tmp_path, tag):
-    """One child process with the knobs set: -> {job id: {name: array}}."""
-    out = tmp_path / tag
-    out.mkdir()
-    spec = tmp_path / f"{tag}.json"
-    spec.write_text(json.dumps({"out": str(out), "jobs": jobs}))
-    env = {k: v for k, v in os.environ.items() if k not in KNOBS}
-    env.update(env_knobs)
-    p = subprocess.run([sys.executable, os.path.abspath(__file__), "--knob-worker", str(spec)], env=env,
-                       capture_output=True, text=True, timeout=900)
-    assert p.returncode == 0, f"knob worker {env_knobs} failed:\n{p.stdout[-3000:]}\n{p.stderr[-3000:]}"
-    res = {}
-    for j in jobs:
-        with np.load(out / f"{j['id']}.npz") as z:
-            res[j["id"]] = {k: z[k] for k in z.files}
-    return res
-
-
-def knob_str(env_knobs, kernel_knobs):
-    return ",".join(f"{k[5:]}={v}" for k, v in env_knobs.items() if k in kernel_knobs) or "default"
-
-
-KNOBS_OF = {"euler_fast": ("CAAR_LEVELOP_WAVES",), "euler_strict": ("CAAR_EULER_WAVES",),
-            "divwk": ("CAAR_LEVELOP_WAVES",), "lap_flat": ("CAAR_LAPLACE_CHUNK",),
-            "rhs": ("CAAR_CLUSTER_POLICY", "CAAR_PF_DIST")}
-
-
-def test_schedule_knobs_are_bit_identical(tmp_path, default_knobs):
-    """CAAR_LEVELOP_WAVES 1 / 16 / 200 (tracer step T2, divergence_sphere_wk D1: about 124 units per warp down to
-    one), CAAR_LAPLACE_CHUNK 1 / 3 / 64 (F2 and F3 shapes at 4096 elements, then 50 launches over random ranges
-    queued without synchronisation: a scheduler counter left non-zero skips tiles of the next launch),
-    CAAR_EULER_WAVES 1 / 0 (strict tracer step T2, which must also still equal the FP64 restatement),
-    CAAR_CLUSTER_POLICY 1 / 2 and CAAR_PF_DIST 0 / 1 / E + 5 (the fused kernel, both modes, nlev 30, 72, 96, 128 and
-    Eulerian 72 at 600 elements) change who computes what, never a result."""
-    want = {j["id"]: run_job(j) for j in SCHEDULE_JOBS}
-    s, vin, _, _ = job_inputs(T2)
-    port = port_reference(T2, s, vin, None, None)["qtens"]
-    assert np.array_equal(want["T2_strict"]["qtens"][:, :T2["qsize"]], port[:, :T2["qsize"]])
-    bad = []
-    for n, env_knobs in enumerate(SCHEDULE_LEGS):
-        got = run_worker(env_knobs, SCHEDULE_JOBS, tmp_path, f"schedule{n}")
-        for j in SCHEDULE_JOBS:
-            key = "rhs" if j["op"] == "rhs" else ("euler_strict" if j["id"] == "T2_strict" else
-                                                 "euler_fast" if j["op"] == "euler" else j["op"])
-            same = all(np.array_equal(got[j["id"]][k], v) for k, v in want[j["id"]].items())
-            REPORT.append(f"{j['id']:30s} {'':4s} {knob_str(env_knobs, KNOBS_OF[key]):34s} "
-                          f"{'bit-identical to the default knobs' if same else 'DIFFERS from the default knobs'}")
-            if not same:
-                bad.append((j["id"], env_knobs))
-        assert np.array_equal(got["T2_strict"]["qtens"][:, :T2["qsize"]], port[:, :T2["qsize"]]), env_knobs
-    assert not bad, bad
+    gate_fast(c, fast, inputs, sms)
+    if c["id"] in RANDOM_RANGES:
+        check_random_ranges(c, inputs, fast)
 
 
 def test_zz_report_regimes(capsys):
-    """Not a gate: what the tests above measured, per kernel, case and knob."""
+    """Not a gate: what the tests above measured, per kernel and case."""
     with capsys.disabled():
         for line in REPORT:
             print(f"\n[regimes] {line}", end="")
         print()
 
-
-def _knob_worker(spec_path):
-    spec = json.loads(open(spec_path).read())
-    for j in spec["jobs"]:
-        j["range"] = tuple(j["range"])
-        if "tls" in j:
-            j["tls"] = tuple(j["tls"])
-        np.savez(os.path.join(spec["out"], f"{j['id']}.npz"), **run_job(j))
-
-
-if __name__ == "__main__" and len(sys.argv) == 3 and sys.argv[1] == "--knob-worker":
-    _knob_worker(sys.argv[2])

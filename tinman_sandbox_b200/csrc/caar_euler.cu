@@ -140,10 +140,9 @@ cudaError_t launch_euler_step(const KernelArgs& a, const double* vstar, double* 
   e.dt = dt; e.rrearth = a.rrearth;
   for (int i = 0; i < 16; ++i) e.dvv[i] = a.dvv[i];
   const long long rows = (long long)(nete - nets) * a.nlev;
-  long long groups = (rows + 63) / 64;
-  static const int waves = [] { const char* v = getenv("CAAR_EULER_WAVES"); return v ? atoi(v) : 2; }();
-  const long long cap = (long long)sm_count() * 3 * (waves > 0 ? waves : 1);  // persistent CTAs: `waves` times 3 per SM
-  const unsigned blocks = (unsigned)(waves > 0 && groups > cap ? cap : groups);
+  const long long groups = (rows + 63) / 64;
+  const long long cap = (long long)sm_count() * 3 * 2;  // persistent CTAs: 2 waves of 3 per SM
+  const unsigned blocks = (unsigned)(groups > cap ? cap : groups);
   euler_step_kernel<<<blocks, 256, 0, s>>>(e);
   return cudaGetLastError();
 }

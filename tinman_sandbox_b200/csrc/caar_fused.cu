@@ -69,14 +69,10 @@ int fused_instance_cluster(int nlev) { return instance_for(nlev) ? cluster_for(i
 
 cudaError_t launch_fused(const KernelArgs& a0, cudaStream_t s) {
   KernelArgs a = a0;
-  static const int pf_env = [] {
-    const char* v = getenv("CAAR_PF_DIST");
-    return v ? atoi(v) : -1;
-  }();
-  // default distance: nlev=72 (CTA triples) -> 74 elements (16: 0.921, 32: 0.937, 74: 0.946, 148: 0.944 of the
-  // measured peak); nlev=128 (CTA pairs) -> 32 (flat optimum 4...48, 0.74 at 148).
-  // Sweeps: profiles/README.md.
-  a.pf_dist = a0.pf_dist < 0 ? 0 : (pf_env >= 0 ? pf_env : (a.nlev == 72 ? sm_count() / 2 : 32));  // 74 on a 148-SM B200
+  // distance: nlev=72 (CTA triples) -> 74 elements (16: 0.921, 32: 0.937, 74: 0.946, 148: 0.944 of the measured peak);
+  // nlev=128 (CTA pairs) -> 32 (flat optimum 4...48, 0.74 at 148). Sweeps: profiles/README.md.
+  // A caller's pf_dist < 0 turns the prefetch off (the zero-copy host path).
+  a.pf_dist = a0.pf_dist < 0 ? 0 : (a.nlev == 72 ? sm_count() / 2 : 32);  // 74 on a 148-SM B200
   switch (instance_for(a.nlev)) {
     case 72: return launch_nlev<72>(a, s);
     case 128: return launch_nlev<128>(a, s);

@@ -938,10 +938,8 @@ cudaError_t launch_L(const KernelArgs& a, cudaStream_t s) {
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
   // cluster scheduling policy: load balancing for the CTA triples (A/B at nlev=72: 1.037-1.040 of the measured peak vs
-  // 0.995-1.014 with the default spread policy), spread for pairs (nlev=128: no difference). CAAR_CLUSTER_POLICY=1|2
-  // forces spread | load balancing.
-  static const int policy_env = [] { const char* v = getenv("CAAR_CLUSTER_POLICY"); return v ? atoi(v) : 0; }();
-  const bool balance = policy_env ? (policy_env == 2) : (CL >= 3);
+  // 0.995-1.014 with the default spread policy), spread for pairs (nlev=128: no difference)
+  const bool balance = CL >= 3;
   attr[1].id = cudaLaunchAttributeClusterSchedulingPolicyPreference;
   attr[1].val.clusterSchedulingPolicyPreference =
       balance ? cudaClusterSchedulingPolicyLoadBalancing : cudaClusterSchedulingPolicySpread;

@@ -46,22 +46,11 @@
 namespace caar {
 namespace {
 
-#ifndef LEVELOP_NS
-#define LEVELOP_NS 4
-#endif
-#ifndef LEVELOP_NO
-#define LEVELOP_NO 2
-#endif
-#ifndef LEVELOP_WPC
-#define LEVELOP_WPC 4
-#endif
-#ifndef LEVELOP_MINB
-#define LEVELOP_MINB 4
-#endif
-constexpr int NS = LEVELOP_NS;    // input tiles in flight per warp
-constexpr int NO = LEVELOP_NO;    // output tiles in flight per warp
-constexpr int WPC = LEVELOP_WPC;  // warps per CTA (independent pipelines: no CTA-wide barrier after the prologue)
-constexpr int GL = 8;   // levels per tile = levels per warp (8 levels x 4 GLL rows = 32 lanes)
+constexpr int NS = 4;    // input tiles in flight per warp
+constexpr int NO = 2;    // output tiles in flight per warp
+constexpr int WPC = 4;   // warps per CTA (independent pipelines: no CTA-wide barrier after the prologue)
+constexpr int MINB = 4;  // resident CTAs per SM the register budget is set for
+constexpr int GL = 8;    // levels per tile = levels per warp (8 levels x 4 GLL rows = 32 lanes)
 
 struct LevelOpArgs {
   const double* Dinv;
@@ -126,8 +115,8 @@ enum { OP_EULER = 0, OP_DIVWK = 1, OP_LAP_SIMPLE = 2, OP_LAP_TENSOR = 3 };
 // earlier unit of any warp stores. The next stage reads the stored tiles back with TMA: the bulk stores are complete
 // when the grid is, and the exit below only waits for their shared-memory reads, as the in-place laplacian does.
 template <int OP>
-__global__ void __launch_bounds__(32 * WPC, LEVELOP_MINB) levelop_kernel(const __grid_constant__ LevelOpArgs A,
-                                                              const __grid_constant__ LevelOpMaps M) {
+__global__ void __launch_bounds__(32 * WPC, MINB) levelop_kernel(const __grid_constant__ LevelOpArgs A,
+                                                                 const __grid_constant__ LevelOpMaps M) {
   constexpr unsigned IN_B = (OP == OP_DIVWK) ? 2048u : 1024u;  // bytes of a streamed input tile (8 levels)
   constexpr unsigned OUT_B = 1024u, ITEM_B = (OP == OP_EULER) ? 2048u : 0u;
   constexpr unsigned WARP_B = NS * IN_B + NO * OUT_B + 2 * ITEM_B;
@@ -394,20 +383,11 @@ __global__ void __launch_bounds__(32 * WPC, LEVELOP_MINB) levelop_kernel(const _
 // the math (loaded on demand, a quarter of all warp stall samples sat on those loads; one tile ahead, still 7 %: under
 // load a line takes longer than a tile's math). Same per-warp TMA pipeline as above (FN input tiles ahead, FO output
 // tiles draining); the tiles themselves are drawn in chunks from a global counter (see the kernel).
-#ifndef LAPFLAT_NS
-#define LAPFLAT_NS 3
-#endif
-#ifndef LAPFLAT_NO
-#define LAPFLAT_NO 2
-#endif
-#ifndef LAPFLAT_WPC
-#define LAPFLAT_WPC 4
-#endif
-#ifndef LAPFLAT_MINB
-#define LAPFLAT_MINB 2
-#endif
-static_assert(LAPFLAT_NS >= 3, "the geometry stages look two tiles ahead in the ring of tile numbers");
-constexpr int FN = LAPFLAT_NS, FO = LAPFLAT_NO, FW = LAPFLAT_WPC;
+constexpr int FN = 3;             // input tiles in flight per warp
+constexpr int FO = 2;             // output tiles in flight per warp
+constexpr int FW = 4;             // warps per CTA
+constexpr int FMINB = 2;          // resident CTAs per SM the register budget is set for
+static_assert(FN >= 3, "the geometry stages look two tiles ahead in the ring of tile numbers");
 constexpr int FT = 32;            // rows (element x level) per tile
 constexpr unsigned FT_B = 4096u;  // bytes of a tile
 constexpr int FSLOT = 8;          // cached elements per warp (slot = element & 7): <= 3 of this tile + <= 3 of the next
@@ -430,8 +410,8 @@ struct alignas(64) LapFlatMaps {
 };
 
 template <bool TENSOR>
-__global__ void __launch_bounds__(32 * FW, LAPFLAT_MINB) laplace_flat_kernel(const __grid_constant__ LapFlatArgs A,
-                                                                             const __grid_constant__ LapFlatMaps M) {
+__global__ void __launch_bounds__(32 * FW, FMINB) laplace_flat_kernel(const __grid_constant__ LapFlatArgs A,
+                                                                      const __grid_constant__ LapFlatMaps M) {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   unsigned char* base = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -746,11 +726,10 @@ cudaError_t launch_op(const LevelOpArgs& a, const LevelOpMaps& m, cudaStream_t s
   // idle, many short CTAs pay their pipeline fill more often; the best number of waves grows with the size (tracer step,
   // qsize 4: 1-2 at 5400 elements, 6-8 at 21600, 16 at 86400; divergence_sphere_wk: 1 / 8 / 16 — profiles/README.md):
   // about 48 (tracer step) / 12 (weak-form operators) units per warp and CTA, at most 16 waves
-  static const int waves_env = [] { const char* v = getenv("CAAR_LEVELOP_WAVES"); return v ? atoi(v) : 0; }();
   const long long per_wave = (long long)sm_count() * per_sm * WPC * (OP == OP_EULER ? 48 : 12);
-  long long wv = (a.units + per_wave / 2) / per_wave;
-  wv = (wv < 1 || OP == OP_LAP_SIMPLE || OP == OP_LAP_TENSOR) ? 1 : wv > 16 ? 16 : wv;  // row-decomposed laplacians (nlev < 16): 1
-  const int waves = waves_env > 0 ? waves_env : (int)wv;
+  long long waves = (a.units + per_wave / 2) / per_wave;
+  // row-decomposed laplacians (nlev < 16): 1
+  waves = (waves < 1 || OP == OP_LAP_SIMPLE || OP == OP_LAP_TENSOR) ? 1 : waves > 16 ? 16 : waves;
   long long blocks = (long long)sm_count() * per_sm * waves;
   const long long need = (a.units + WPC - 1) / WPC;
   if (blocks > need) blocks = need;
@@ -766,9 +745,8 @@ cudaError_t launch_lapflat(LapFlatArgs a, const LapFlatMaps& m, cudaStream_t s) 
   if (cudaError_t e = setup_launch(laplace_flat_kernel<TENSOR>, 32 * FW, smem, cache, &per_sm)) return e;
   // one wave of resident CTAs; chunks of 4 consecutive tiles (49152 x 128: 0.81 / 0.98 / 1.01 / 0.99 / 0.95 / 0.90 of the
   // measured peak with 1 / 2 / 4 / 8 / 16 / 32; one tile per chunk exposes the draw), 2 when a warp sees few tiles
-  static const int chunk_env = [] { const char* v = getenv("CAAR_LAPLACE_CHUNK"); return v ? atoi(v) : 0; }();
   const long long resident_warps = (long long)sm_count() * per_sm * FW;
-  a.chunk = chunk_env > 0 ? chunk_env : (a.tiles < resident_warps * 16 ? 2 : 4);
+  a.chunk = a.tiles < resident_warps * 16 ? 2 : 4;
   long long blocks = (long long)sm_count() * per_sm;
   const long long need = (a.tiles + FW - 1) / FW;
   if (blocks > need) blocks = need;

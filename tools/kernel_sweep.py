@@ -1,12 +1,11 @@
 #!/usr/bin/env python
-"""Times caar_run (resident state, CUDA events on the launching stream) for one library build.
+"""Times caar_run (resident state, CUDA events on the launching stream).
 
-    python tools/kernel_sweep.py [--lib path/to/libcaar_b200_variant.so] [--nelem 86400] [--nlev 72]
-                                 [--steps 20] [--warmup 3] [--tag name] [--host-steps 0] [--chunk 0]
+    python tools/kernel_sweep.py [--nelem 86400] [--nlev 72] [--steps 20] [--warmup 3] [--tag name]
+                                 [--host-steps 0] [--chunk 0]
 
 Prints one JSON line per run: updates/s, ms/step, algorithmic GB/s, fraction of the measured copy peak.
-A development tool (variant A/B runs on the GPU box); bench.py is the judged measurement.
-Variants are built with tools/build_variant.sh NAME "-DFLAG ...".
+A development tool; bench.py is the judged measurement.
 """
 import argparse
 import json
@@ -22,7 +21,6 @@ sys.path.insert(0, ROOT)
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--lib", default=None)
     ap.add_argument("--nelem", type=int, default=86400)
     ap.add_argument("--nlev", type=int, default=72)
     ap.add_argument("--steps", type=int, default=20)
@@ -41,10 +39,6 @@ def main():
                          "read, 20). spheremp = 1 and dt2 = 1e-9 keep the state finite over the repeated in-place calls")
     args = ap.parse_args()
 
-    from tinman_sandbox_b200 import capi
-    if args.lib:
-        path = os.path.abspath(args.lib)
-        capi.lib_path = lambda: path
     import tinman_sandbox_b200 as tb
     from tinman_sandbox_b200.testdata import TestData
     import torch
@@ -103,11 +97,11 @@ def main():
         fields = 21 - (4 if aliased else 0) - (1 if dry else 0)
         balg = fields * 128.0 + 1664.0 / L + (256.0 * (L + 1) / L if args.eulerian else 0.0)
         rate = E * L / (best * 1e-3)
-        out = {"tag": args.tag, "lib": args.lib or "default", "nelem": E, "nlev": L, "mode": args.mode,
+        out = {"tag": args.tag, "nelem": E, "nlev": L, "mode": args.mode,
                "variant": variant, "eulerian": bool(args.eulerian), "B_alg": round(balg, 1),
                "ms_per_step": round(best, 4), "Mupdates_per_s": round(rate / 1e6, 1),
                "GBps": round(rate * balg / 1e9, 1), "frac_measured": round(rate * balg / 1e9 / peak, 4),
-               "clock_after": clk, "env": {k: v for k, v in os.environ.items() if k.startswith("CAAR_")}}
+               "clock_after": clk}
         print(json.dumps(out), flush=True)
     if args.host_steps > 0:
         h2d, d2h = h.host_traffic(mode)

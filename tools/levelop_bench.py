@@ -23,12 +23,7 @@ def main():
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--ops", default="euler,divwk,lap,lapt")
     ap.add_argument("--modes", default="fast,strict")
-    ap.add_argument("--lib", default=None, help="a variant library built with tools/build_variant.sh")
     args = ap.parse_args()
-    if args.lib:
-        from tinman_sandbox_b200 import capi
-        path = os.path.abspath(args.lib)
-        capi.lib_path = lambda: path
     E, L, Q = args.nelem, args.nlev, args.qsize
     peak = 6545.6
     try:
@@ -64,9 +59,7 @@ def main():
             print(json.dumps({"op": name, "mode": mode_name, "nelem": E, "nlev": L, "qsize": Q if key == "euler" else None,
                               "ms": round(best, 4), "Mupdates_per_s": round(rate / 1e6, 1),
                               "B_alg": round(balg, 1), "GBps": round(rate * balg / 1e9, 1),
-                              "frac_measured": round(rate * balg / 1e9 / peak, 4),
-                              "lib": os.path.basename(args.lib) if args.lib else "default",
-                              "env": {k: v for k, v in os.environ.items() if k.startswith("CAAR_")}}), flush=True)
+                              "frac_measured": round(rate * balg / 1e9 / peak, 4)}), flush=True)
     h.close()
 
 

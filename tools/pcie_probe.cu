@@ -1,6 +1,6 @@
 // tools/pcie_probe.cu — what the host link of this box can do: 1-D and pitched (one time level out of three)
 // copies, each direction alone and both at once. Development probe for caar_run_host's pipeline.
-//   nvcc -O2 -o tools/_variants/pcie_probe tools/pcie_probe.cu && tools/_variants/pcie_probe
+//   mkdir -p build && nvcc -O2 -o build/pcie_probe tools/pcie_probe.cu && build/pcie_probe
 #include <cuda_runtime.h>
 #include <chrono>
 #include <cstdio>

@@ -1,7 +1,7 @@
 // tools/pcie_probe_multi.cu — what the host links of this box do when 1, 2, 4, 8 GPUs copy AT THE SAME TIME: the
 // ceiling the end-to-end (host arrays in / host arrays out) leg of bench.py runs against at N > 1.
-//   nvcc -O2 -std=c++17 -o tools/_variants/pcie_probe_multi tools/pcie_probe_multi.cu -lpthread
-//   tools/_variants/pcie_probe_multi [--gb 1.0] [--wc] [--bind] [--max-gpus 8]
+//   mkdir -p build && nvcc -O2 -std=c++17 -o build/pcie_probe_multi tools/pcie_probe_multi.cu -lpthread
+//   build/pcie_probe_multi [--gb 1.0] [--wc] [--bind] [--max-gpus 8]
 // One host thread per GPU; every thread allocates its own pinned buffers AFTER cudaSetDevice (and, with --bind, after
 // pinning itself to the CPUs of the GPU's NUMA node, so first touch places the pages there); --wc allocates the
 // host->device source write-combined. Each configuration is timed between two barriers (wall clock, max over
