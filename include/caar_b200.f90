@@ -32,6 +32,7 @@ module caar_b200
   integer(c_int), parameter, public :: CAAR_OP_DIVERGENCE_WK = 0, CAAR_OP_LAPLACE_SIMPLE = 1, CAAR_OP_LAPLACE_TENSOR = 2, &
                                        CAAR_OP_LAPLACE_TENSOR_REPLACE = 3
   integer(c_int), parameter, public :: CAAR_DSS_ASSEMBLE = 0, CAAR_DSS_PROJECT = 1
+  integer(c_int), parameter, public :: CAAR_HALO_DSS = 0, CAAR_HALO_MINMAX = 1
 
   ! ---- struct caar_dims (5 x int = 20 bytes)
   type, bind(C), public :: caar_dims
@@ -70,7 +71,8 @@ module caar_b200
             caar_checksums, caar_euler_step, caar_advect_tracers, caar_tracer_bounds, caar_limit_tracers, &
             caar_bounds_upload, caar_bounds_download, caar_sphere_wk, caar_extra_upload, caar_extra_download, caar_last_error, &
             caar_host_register, caar_host_unregister, caar_describe, caar_set_connectivity, caar_dss, caar_neighbor_minmax, &
-            caar_run_rk5_dss
+            caar_run_rk5_dss, caar_set_partition, caar_dss_pack, caar_dss_unpack, caar_neighbor_minmax_pack, &
+            caar_neighbor_minmax_unpack, caar_halo_segments
 
   interface
     ! int caar_create(caar_handle* out, const caar_dims* dims, int device);
@@ -239,6 +241,53 @@ module caar_b200
       type(caar_control), intent(inout) :: ctl
       real(c_double), value :: dt
       integer(c_int), value :: nsteps, mode
+      integer(c_int) :: rc
+    end function
+    ! the DSS across ranks: edgeVpack -> caar_dss_pack, bndry_exchangeV -> MPI_Isend / MPI_Irecv of the segments of
+    ! caar_halo_segments, edgeVunpack + rspheremp -> caar_dss_unpack. gid is the whole mesh's gdofP in the ranks'
+    ! element order; part_start(0:nparts) the first global element of every rank's block (zero-based), part this rank
+    function caar_set_partition(handle, gid, nelem_global, part_start, nparts, part, layout) &
+        bind(C, name="caar_set_partition") result(rc)
+      import :: c_ptr, c_int, c_long_long
+      type(c_ptr), value :: handle
+      integer(c_long_long), intent(in) :: gid(*)
+      integer(c_int), value :: nelem_global, nparts, part, layout
+      integer(c_int), intent(in) :: part_start(*)
+      integer(c_int) :: rc
+    end function
+    function caar_dss_pack(handle, field_mask, tl, qtl, qsize, weighting) bind(C, name="caar_dss_pack") result(rc)
+      import :: c_ptr, c_int
+      type(c_ptr), value :: handle
+      integer(c_int), value :: field_mask, tl, qtl, qsize, weighting
+      integer(c_int) :: rc
+    end function
+    function caar_dss_unpack(handle, field_mask, tl, qtl, qsize, weighting) bind(C, name="caar_dss_unpack") result(rc)
+      import :: c_ptr, c_int
+      type(c_ptr), value :: handle
+      integer(c_int), value :: field_mask, tl, qtl, qsize, weighting
+      integer(c_int) :: rc
+    end function
+    function caar_neighbor_minmax_pack(handle, qsize) bind(C, name="caar_neighbor_minmax_pack") result(rc)
+      import :: c_ptr, c_int
+      type(c_ptr), value :: handle
+      integer(c_int), value :: qsize
+      integer(c_int) :: rc
+    end function
+    function caar_neighbor_minmax_unpack(handle, qsize) bind(C, name="caar_neighbor_minmax_unpack") result(rc)
+      import :: c_ptr, c_int
+      type(c_ptr), value :: handle
+      integer(c_int), value :: qsize
+      integer(c_int) :: rc
+    end function
+    ! send and recv are device addresses (CUDA-aware MPI takes them directly); send_off(0:nparts) and recv_off(0:nparts)
+    ! are offsets in doubles: segment q is send(send_off(q)+1 : send_off(q+1))
+    function caar_halo_segments(handle, op, field_mask, qsize, send, recv, send_off, recv_off) &
+        bind(C, name="caar_halo_segments") result(rc)
+      import :: c_ptr, c_int, c_size_t
+      type(c_ptr), value :: handle
+      integer(c_int), value :: op, field_mask, qsize
+      type(c_ptr), intent(out) :: send, recv
+      integer(c_size_t), intent(out) :: send_off(*), recv_off(*)
       integer(c_int) :: rc
     end function
     function caar_sphere_wk(handle, op, nets, nete, mode) bind(C, name="caar_sphere_wk") result(rc)

@@ -253,7 +253,9 @@ int caar_sync(caar_handle h);
 /* number of kernel launches issued through this handle since creation (caar_run, caar_run_rk5: 6 per step,
    caar_run_rk5_dss: 11 per step, caar_advect_tracers: 4 per step, caar_tracer_bounds and caar_limit_tracers: 1 per call
    (none for an empty range or qsize == 0), caar_dss and caar_neighbor_minmax: 1 per call (none when nothing is
-   selected), caar_euler_step, caar_norms, ...) */
+   selected), caar_dss_pack / caar_dss_unpack and caar_neighbor_minmax_pack / caar_neighbor_minmax_unpack: 1 per call
+   (none when nothing is selected, and none for a pack of a part that shares no point), caar_euler_step, caar_norms,
+   ...) */
 long long caar_launch_count(caar_handle h);
 /* CUDA-event stopwatch on the stream the kernels are launched on: start records an event, stop records a
    second one, waits for it and returns the device time between the two in milliseconds. */
@@ -387,8 +389,8 @@ int caar_limit_tracers(caar_handle h, int nets, int nete, int qtl, int qsize, in
    nothing else changes. tl, qtl and qsize are checked whatever the mask.
    Departure from HOMME: edgeVunpack adds an element's neighbours to that element's own value, so HOMME's copies of one
    point may differ in the last bit; here every copy receives the identical value.
-   Partitioned handles: only the copies this handle holds are summed. Exchanging the sums of shared points with other
-   handles (HOMME's bndry_exchangeV between ranks) is not provided.
+   Partitioned handles: only the copies this handle holds are summed; caar_dss_pack / caar_dss_unpack below assemble
+   the copies other handles hold too.
 
    caar_neighbor_minmax: HOMME's neighbor_minmax on the handle's limiter bounds (caar_tracer_bounds). N(e) is the set of
    elements other than e that share at least one gid with e (on a cubed sphere the edge and vertex neighbours). For every
@@ -411,6 +413,64 @@ int caar_neighbor_minmax(caar_handle h, int qsize);
    Returns CAAR_ERR_STATE before caar_set_params or caar_set_connectivity, CAAR_ERR_INVALID for an element range other than
    [0, nelem) (the DSS spans the handle), and every error of caar_run_rk5, leaving *ctl unchanged. */
 int caar_run_rk5_dss(caar_handle h, caar_control* ctl, double dt, int nsteps, int mode);
+
+/* ---- the DSS and neighbor_minmax across partitioned handles: HOMME's edgeVpack / bndry_exchangeV / edgeVunpack ----
+   A mesh of nelem_global elements is cut into nparts contiguous blocks, one per handle (one per GPU or rank). The
+   library packs what other parts need into a device send buffer; the caller moves opaque segments with its own
+   transport (NCCL, CUDA-aware MPI, device copies between handles of one process); the library unpacks from a device
+   receive buffer and finishes the sum. Over any block partition the assembled values of every handle are, bit for bit,
+   those caar_dss / caar_neighbor_minmax give on one handle that holds the whole mesh: the copies of a point are ordered
+   by (global e, p), and every operation is rounded separately as there.
+
+   caar_set_partition: gid[nelem_global][4][4] is the global-id map of the whole mesh, in CAAR_LAYOUT_CXX or
+   CAAR_LAYOUT_F90 order as in caar_set_connectivity. part_start[nparts + 1] ascends strictly from 0 to nelem_global;
+   this handle holds global elements [part_start[part], part_start[part + 1]), local element e being global
+   part_start[part] + e. Callers whose parts are not contiguous (HOMME's space-filling-curve partitions give each rank a
+   set) renumber their elements first, so that each rank's local order defines its block. Synchronous; builds every
+   table on the host once (a sort of the 16 nelem_global copies); replaces any earlier connectivity or partition, and a
+   later caar_set_connectivity replaces it; works before caar_set_params. From then on caar_dss and
+   caar_neighbor_minmax keep their local-only meaning, as if caar_set_connectivity had been given the handle's slice of
+   gid; so does caar_run_rk5_dss, which therefore assembles HOMME's step only on a handle that holds the whole mesh.
+   Allocates the two exchange buffers, sized for the largest selection (all four fields with qsize_d tracers, and the
+   bounds of qsize_d tracers), until caar_destroy or the next map. CAAR_ERR_INVALID for a null handle, gid or
+   part_start, nparts < 1, part outside [0, nparts), part_start not ascending from 0 to nelem_global, a block size other
+   than the handle's nelem, or a bad layout; CAAR_ERR_UNSUPPORTED for nelem_global >= 2^27.
+
+   caar_dss_pack / caar_dss_unpack take caar_dss's arguments, with its checks and selection rules. pack writes the send
+   buffer: segment q (for every other part q) holds, for each local copy of a point that part q also holds a copy of,
+   the copy's spheremp and its selected values at every level. unpack reads the receive buffer and performs the whole DSS
+   of this handle in place, interior points included: the copies of every point, those held by other parts taken from
+   the received segments, are ordered by (global e, p), and m, r = 1/m and S follow caar_dss's formulas in that order;
+   every local copy gets S*r. The remote spheremp values come from the records, so a re-uploaded spheremp is used there
+   too. The record layout and the order inside a segment are the library's, derived by both sides from the same global
+   map; the caller moves segment p->q of part p's send buffer to segment p of part q's receive buffer, byte for byte.
+   pack and unpack of one exchange must use the same field_mask, tl, qtl and qsize: mixing them is a caller error that
+   is not detected. With nparts == 1 unpack equals caar_dss bit for bit.
+
+   caar_neighbor_minmax_pack / caar_neighbor_minmax_unpack: the same on the limiter bounds. Segment q holds the
+   [qsize][L][2] bounds of every local element that has a neighbour in part q. unpack is caar_neighbor_minmax's rule over
+   N(e) of the whole mesh: e's own value first, then every neighbour, local or remote, in ascending global element order
+   (which also fixes which of -0.0 and +0.0 survives). It writes the second array as caar_neighbor_minmax does.
+
+   caar_halo_segments: for op CAAR_HALO_DSS with (field_mask, qsize), or CAAR_HALO_MINMAX with qsize (the mask is then
+   only checked), returns the device send and receive buffers and the offsets, in doubles, of every segment: segment q
+   is [send_off[q], send_off[q+1]) of *send and [recv_off[q], recv_off[q+1]) of *recv. send_off of p->q on part p has
+   the size of recv_off of q<-p on part q; the segments to and from this part itself are empty. Synchronous, launches
+   nothing; CAAR_ERR_INVALID for null outputs or a bad op, mask or qsize.
+
+   pack and unpack are asynchronous on the handle's stream. The caller's transport must be ordered after pack and
+   unpack after the transport (with caar_set_stream on the transport's stream this is free). Before
+   caar_set_partition every call here but caar_set_partition returns CAAR_ERR_STATE; a rejected call launches nothing
+   and changes nothing. */
+enum { CAAR_HALO_DSS = 0, CAAR_HALO_MINMAX = 1 };
+int caar_set_partition(caar_handle h, const long long* gid, int nelem_global, const int* part_start, int nparts,
+                       int part, int layout);
+int caar_dss_pack(caar_handle h, unsigned field_mask, int tl, int qtl, int qsize, int weighting);
+int caar_dss_unpack(caar_handle h, unsigned field_mask, int tl, int qtl, int qsize, int weighting);
+int caar_neighbor_minmax_pack(caar_handle h, int qsize);
+int caar_neighbor_minmax_unpack(caar_handle h, int qsize);
+int caar_halo_segments(caar_handle h, int op, unsigned field_mask, int qsize, double** send, double** recv,
+                       size_t* send_off, size_t* recv_off);
 
 /* ---- the weak-form operators behind hyperviscosity (SURVEY §8f rank 4) ----
    Level-local like the tracer step, on the same kernel skeleton, in the pointers_only index conventions

@@ -17,6 +17,7 @@ from .capi import (  # noqa: F401
     field_shape, compute_and_apply_rhs, saxpby_host, EXPORTED_SYMBOLS, HOST_ZERO_COPY, host_register,
     host_unregister, CHECKSUM_FIELDS, X_VSTAR, X_QTENS, X_TENSORVISC, X_SCALAR_IN, X_SCALAR_OUT, OP_DIVERGENCE_WK,
     OP_LAPLACE_SIMPLE, OP_LAPLACE_TENSOR, OP_LAPLACE_TENSOR_REPLACE, DSS_ASSEMBLE, DSS_PROJECT, DSS_FIELDS,
+    HALO_DSS, HALO_MINMAX,
 )
 
 __all__ = [

@@ -31,6 +31,7 @@ X_VSTAR, X_QTENS, X_TENSORVISC, X_SCALAR_IN, X_SCALAR_OUT = 0, 1, 2, 3, 4
 OP_DIVERGENCE_WK, OP_LAPLACE_SIMPLE, OP_LAPLACE_TENSOR, OP_LAPLACE_TENSOR_REPLACE = 0, 1, 2, 3
 DSS_ASSEMBLE, DSS_PROJECT = 0, 1
 DSS_FIELDS = ("elem_state_dp3d", "elem_state_v", "elem_state_T", "elem_state_Qdp")   # what caar_dss can select
+HALO_DSS, HALO_MINMAX = 0, 1
 
 # every symbol include/caar_b200.h declares (tests check the library exports all of them)
 EXPORTED_SYMBOLS = (
@@ -44,7 +45,8 @@ EXPORTED_SYMBOLS = (
     "caar_saxpby_host", "caar_checksums", "caar_upload_range", "caar_download_range", "caar_describe",
     "caar_sphere_wk", "caar_run_rk5", "caar_advect_tracers", "caar_bounds_upload", "caar_bounds_download",
     "caar_tracer_bounds", "caar_limit_tracers", "caar_set_connectivity", "caar_dss", "caar_neighbor_minmax",
-    "caar_run_rk5_dss",
+    "caar_run_rk5_dss", "caar_set_partition", "caar_dss_pack", "caar_dss_unpack", "caar_neighbor_minmax_pack",
+    "caar_neighbor_minmax_unpack", "caar_halo_segments",
 )
 CHECKSUM_FIELDS = ("elem_state_dp3d", "elem_state_v", "elem_state_T", "elem_derived_eta_dot_dpdn",
                    "elem_derived_omega_p", "elem_derived_phi", "elem_derived_vn0")
@@ -149,6 +151,14 @@ def load_library():
     lib.caar_dss.argtypes = [C.c_void_p, C.c_uint, C.c_int, C.c_int, C.c_int, C.c_int]
     lib.caar_neighbor_minmax.argtypes = [C.c_void_p, C.c_int]
     lib.caar_run_rk5_dss.argtypes = [C.c_void_p, C.POINTER(Control), C.c_double, C.c_int, C.c_int]
+    lib.caar_set_partition.argtypes = [C.c_void_p, C.POINTER(C.c_longlong), C.c_int, C.POINTER(C.c_int), C.c_int,
+                                       C.c_int, C.c_int]
+    lib.caar_dss_pack.argtypes = lib.caar_dss.argtypes
+    lib.caar_dss_unpack.argtypes = lib.caar_dss.argtypes
+    lib.caar_neighbor_minmax_pack.argtypes = [C.c_void_p, C.c_int]
+    lib.caar_neighbor_minmax_unpack.argtypes = [C.c_void_p, C.c_int]
+    lib.caar_halo_segments.argtypes = [C.c_void_p, C.c_int, C.c_uint, C.c_int, C.POINTER(C.c_void_p),
+                                       C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]
     lib.caar_upload_layout.argtypes = [C.c_void_p, C.POINTER(Arrays), C.c_uint, C.c_int]
     lib.caar_download_layout.argtypes = [C.c_void_p, C.POINTER(Arrays), C.c_uint, C.c_int]
     lib.caar_set_params_f90.argtypes = [C.c_void_p, C.POINTER(Constants), C.POINTER(C.c_double), C.c_double,
@@ -213,6 +223,7 @@ class Caar:
         self.h = C.c_void_p()
         _check(self.lib, self.lib.caar_create(C.byref(self.h), C.byref(self.dims), device), "caar_create")
         self.control = Control(0, nelem, 0, 1, 2, 0, 1.0)
+        self.device = device
 
     def close(self):
         if getattr(self, "h", None) is not None and self.h:
@@ -461,6 +472,60 @@ class Caar:
         if sync:
             self.sync()
 
+    # -- the DSS and neighbor_minmax across partitioned handles --------------------------------------------------------
+    def set_partition(self, gid, part_start, part, layout=LAYOUT_CXX):
+        """caar_set_partition: gid [nelem_global][4][4] int64 of the whole mesh; this handle holds the elements
+        [part_start[part], part_start[part + 1])."""
+        gid = np.ascontiguousarray(gid, dtype=np.int64)
+        ps = np.ascontiguousarray(part_start, dtype=np.int32)
+        if gid.size % 16:
+            raise CaarError(f"gid: need 16 ids per element, got {gid.size}")
+        _check(self.lib, self.lib.caar_set_partition(self.h, gid.ctypes.data_as(C.POINTER(C.c_longlong)), gid.size // 16,
+                                                     ps.ctypes.data_as(C.POINTER(C.c_int)), len(ps) - 1, int(part),
+                                                     int(layout)), "caar_set_partition")
+        self.nparts = len(ps) - 1
+
+    def _dss_call(self, fn, what, names, tl, qtl, qsize, weighting, sync):
+        tl = self.control.np1 if tl is None else tl
+        for n in names:
+            if n not in DSS_FIELDS:
+                raise CaarError(f"{n}: {what} selects only {DSS_FIELDS}")
+        _check(self.lib, fn(self.h, _mask(names) if names else 0, int(tl), int(qtl), int(qsize), int(weighting)), what)
+        if sync:
+            self.sync()
+
+    def dss_pack(self, names, tl=None, qtl=0, qsize=0, weighting=DSS_ASSEMBLE, sync=True):
+        """caar_dss_pack: the records of the named fields for every other part into the send buffer."""
+        self._dss_call(self.lib.caar_dss_pack, "caar_dss_pack", names, tl, qtl, qsize, weighting, sync)
+
+    def dss_unpack(self, names, tl=None, qtl=0, qsize=0, weighting=DSS_ASSEMBLE, sync=True):
+        """caar_dss_unpack: the whole DSS of the handle in place, remote copies from the receive buffer."""
+        self._dss_call(self.lib.caar_dss_unpack, "caar_dss_unpack", names, tl, qtl, qsize, weighting, sync)
+
+    def neighbor_minmax_pack(self, qsize, sync=True):
+        _check(self.lib, self.lib.caar_neighbor_minmax_pack(self.h, int(qsize)), "caar_neighbor_minmax_pack")
+        if sync:
+            self.sync()
+
+    def neighbor_minmax_unpack(self, qsize, sync=True):
+        _check(self.lib, self.lib.caar_neighbor_minmax_unpack(self.h, int(qsize)), "caar_neighbor_minmax_unpack")
+        if sync:
+            self.sync()
+
+    def halo_segments(self, op, names=(), qsize=0):
+        """caar_halo_segments -> (send, recv, send_off, recv_off): torch float64 CUDA tensors viewing the handle's
+        two exchange buffers (valid until the handle is closed or its map replaced) and the segment offsets in doubles,
+        numpy int64 [nparts + 1] each; segment q is send[send_off[q]:send_off[q + 1]]."""
+        import torch
+        n = self.nparts + 1
+        sp, rp = C.c_void_p(), C.c_void_p()
+        so, ro = (C.c_size_t * n)(), (C.c_size_t * n)()
+        _check(self.lib, self.lib.caar_halo_segments(self.h, int(op), _mask(names) if names else 0, int(qsize),
+                                                     C.byref(sp), C.byref(rp), so, ro), "caar_halo_segments")
+        so, ro = np.array(so[:], dtype=np.int64), np.array(ro[:], dtype=np.int64)
+        dev = torch.device("cuda", self.device)
+        return _device_view(sp.value, int(so[-1]), dev), _device_view(rp.value, int(ro[-1]), dev), so, ro
+
     def download_qtens(self, qtens=None):
         E, L, Q, _ = self.shape_args
         if qtens is None:
@@ -534,6 +599,21 @@ class Caar:
 
     def norms(self, tl=None):
         return np.sqrt(self.sumsq(tl))
+
+
+class _CudaArray:
+    """__cuda_array_interface__ of n float64 at a device pointer, for torch.as_tensor"""
+
+    def __init__(self, ptr, n):
+        self.__cuda_array_interface__ = {"shape": (n,), "typestr": "<f8", "data": (ptr, False), "version": 3,
+                                         "strides": None}
+
+
+def _device_view(ptr, n, device):
+    import torch
+    if n == 0:
+        return torch.empty(0, dtype=torch.float64, device=device)
+    return torch.as_tensor(_CudaArray(ptr, n), device=device)
 
 
 def compute_and_apply_rhs(state, mode=MODE_FAST, device=0):

@@ -1,5 +1,6 @@
 // caar_capi.cu — the C-ABI of include/caar_b200.h over the CUDA kernels. No CPU fallback: every
 // compute entry point needs a CUDA device and fails with CAAR_ERR_CUDA otherwise.
+#include <algorithm>
 #include <cstdarg>
 #include <cstddef>
 #include <cstdio>
@@ -76,6 +77,7 @@ struct caar_handle_s {
   double* bounds;  // [nelem][qsize_d][nlev][2] tracer limiter bounds (allocated and zeroed on first use)
   double* bounds_next;  // the same shape: caar_neighbor_minmax writes it, then it and `bounds` swap
   caar::DssTables dss;  // connectivity of caar_set_connectivity (dss.start == nullptr before it)
+  caar::HaloTables halo;  // exchange tables and buffers of caar_set_partition (halo.start == nullptr before it)
   double* stage;  // device staging buffer of the Fortran-layout copies (allocated on first use)
   // device [2]: the tile scheduler of the thread-per-level laplacians (next chunk, warps done), zero between launches.
   // One pair per handle: all launches of a handle are ordered on its stream, so no two of them share it.
@@ -145,9 +147,59 @@ int check_connected(const caar_handle_s* h, const char* who) {
   return CAAR_OK;
 }
 
+// caar_set_partition was called
+int check_partitioned(const caar_handle_s* h, const char* who) {
+  if (!h) return fail(CAAR_ERR_INVALID, "%s: null handle", who);
+  if (!h->halo.start) return fail(CAAR_ERR_STATE, "caar_set_partition must be called before %s", who);
+  return CAAR_OK;
+}
+// the selection of caar_dss, caar_dss_pack and caar_dss_unpack
+int check_dss_args(const caar_handle_s* h, unsigned field_mask, int tl, int qtl, int qsize, int weighting) {
+  const unsigned fields = CAAR_F_DP3D | CAAR_F_V | CAAR_F_T | CAAR_F_QDP;
+  if (field_mask & ~fields) return fail(CAAR_ERR_INVALID, "field_mask=0x%x: only dp3d, v, T and Qdp", field_mask);
+  if (int rc = check_time_level(h, tl)) return rc;
+  if (int rc = check_qtl(qtl)) return rc;
+  if (int rc = check_qsize(h, qsize)) return rc;
+  if (weighting != CAAR_DSS_ASSEMBLE && weighting != CAAR_DSS_PROJECT) return fail(CAAR_ERR_INVALID, "weighting=%d", weighting);
+  return CAAR_OK;
+}
+
 void free_dss_tables(const caar::DssTables& t) {
   for (int* p : {t.start, t.copy, t.nb_start, t.nb})
     if (p) cudaFree(p);
+}
+void free_halo_tables(const caar::HaloTables& t) {
+  for (int* p : {t.start, t.copy, t.nb_start, t.nb, t.send_copy, t.send_el})
+    if (p) cudaFree(p);
+  for (int2* p : {t.send_seg, t.recv_seg})
+    if (p) cudaFree(p);
+  for (double* p : {t.send, t.recv})
+    if (p) cudaFree(p);
+  delete[] t.rec;
+}
+
+// a device copy of v (at least one element allocated); the copy is queued on s
+template <typename T>
+cudaError_t upload_vector(T** dst, const std::vector<T>& v, cudaStream_t s) {
+  cudaError_t e = cudaMalloc(dst, (v.empty() ? 1 : v.size()) * sizeof(T));
+  if (e == cudaSuccess && !v.empty()) e = cudaMemcpyAsync(*dst, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice, s);
+  return e;
+}
+
+cudaError_t upload_dss_tables(const caar::DssHostTables& t, caar::DssTables* d, cudaStream_t s) {
+  cudaError_t e = cudaSuccess;
+  int** dst[4] = {&d->start, &d->copy, &d->nb_start, &d->nb};
+  const std::vector<int>* src[4] = {&t.start, &t.copy, &t.nb_start, &t.nb};
+  for (int i = 0; i < 4 && e == cudaSuccess; ++i) e = upload_vector(dst[i], *src[i], s);
+  return e;
+}
+
+// per DSS record {first record of its segment, records in that segment}, from the segments' record offsets
+std::vector<int2> record_segments(const std::vector<int>& rec) {
+  std::vector<int2> out;
+  for (size_t q = 0; q + 1 < rec.size(); ++q)
+    for (int r = rec[q]; r < rec[q + 1]; ++r) out.push_back(make_int2(rec[q], rec[q + 1] - rec[q]));
+  return out;
 }
 
 int validate_control(const caar_handle_s* h, const caar_control* ctl) {
@@ -292,6 +344,7 @@ int caar_destroy(caar_handle h) {
   if (h->bounds) cudaFree(h->bounds);
   if (h->bounds_next) cudaFree(h->bounds_next);
   free_dss_tables(h->dss);
+  free_halo_tables(h->halo);
   for (int x = 0; x < CAAR_NUM_EXTRA; ++x)
     if (h->extra[x]) cudaFree(h->extra[x]);
   if (h->hybi_dev) cudaFree(h->hybi_dev);
@@ -981,34 +1034,23 @@ int caar_set_connectivity(caar_handle h, const long long* gid, int layout) {
   std::memset(&d, 0, sizeof d);
   d.ngroups = caar::build_dss_tables(cxx.data(), E, &t);
   DeviceGuard guard(h->device);
-  cudaError_t e = cudaSuccess;
-  int** dst[4] = {&d.start, &d.copy, &d.nb_start, &d.nb};
-  const std::vector<int>* src[4] = {&t.start, &t.copy, &t.nb_start, &t.nb};
-  for (int i = 0; i < 4 && e == cudaSuccess; ++i) {
-    const size_t bytes = (src[i]->empty() ? 1 : src[i]->size()) * sizeof(int);
-    e = cudaMalloc(dst[i], bytes);
-    if (e == cudaSuccess && !src[i]->empty())
-      e = cudaMemcpyAsync(*dst[i], src[i]->data(), src[i]->size() * sizeof(int), cudaMemcpyHostToDevice, h->stream);
-  }
+  cudaError_t e = upload_dss_tables(t, &d, h->stream);
   if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
   if (e != cudaSuccess) {  // the earlier map stays
     free_dss_tables(d);
     return fail(e == cudaErrorMemoryAllocation ? CAAR_ERR_NOMEM : CAAR_ERR_CUDA, "caar_set_connectivity: %s",
                 cudaGetErrorString(e));
   }
-  free_dss_tables(h->dss);  // the stream is idle: no launch still reads the earlier map
+  free_dss_tables(h->dss);  // the stream is idle: no launch still reads the earlier map or partition
+  free_halo_tables(h->halo);
+  std::memset(&h->halo, 0, sizeof h->halo);
   h->dss = d;
   return CAAR_OK;
 }
 
 int caar_dss(caar_handle h, unsigned field_mask, int tl, int qtl, int qsize, int weighting) {
   if (int rc = check_connected(h, "caar_dss")) return rc;
-  const unsigned fields = CAAR_F_DP3D | CAAR_F_V | CAAR_F_T | CAAR_F_QDP;
-  if (field_mask & ~fields) return fail(CAAR_ERR_INVALID, "field_mask=0x%x: only dp3d, v, T and Qdp", field_mask);
-  if (int rc = check_time_level(h, tl)) return rc;
-  if (int rc = check_qtl(qtl)) return rc;
-  if (int rc = check_qsize(h, qsize)) return rc;
-  if (weighting != CAAR_DSS_ASSEMBLE && weighting != CAAR_DSS_PROJECT) return fail(CAAR_ERR_INVALID, "weighting=%d", weighting);
+  if (int rc = check_dss_args(h, field_mask, tl, qtl, qsize, weighting)) return rc;
   if (!(field_mask & (CAAR_F_DP3D | CAAR_F_V | CAAR_F_T)) && !((field_mask & CAAR_F_QDP) && qsize > 0)) return CAAR_OK;
   DeviceGuard guard(h->device);
   CU_TRY(caar::launch_dss(make_args(h, nullptr), h->dss, field_mask, tl, qtl, qsize, weighting, h->stream));
@@ -1029,6 +1071,144 @@ int caar_neighbor_minmax(caar_handle h, int qsize) {
   ++h->launches;
   h->bounds = h->bounds_next;
   h->bounds_next = bounds;
+  return CAAR_OK;
+}
+
+// ---- the exchange of shared points between partitioned handles ---------------------------------------------------
+int caar_set_partition(caar_handle h, const long long* gid, int nelem_global, const int* part_start, int nparts,
+                       int part, int layout) {
+  if (!h || !gid || !part_start) return fail(CAAR_ERR_INVALID, "null argument");
+  if (nparts < 1 || part < 0 || part >= nparts) return fail(CAAR_ERR_INVALID, "part=%d of nparts=%d", part, nparts);
+  if (layout != CAAR_LAYOUT_CXX && layout != CAAR_LAYOUT_F90) return fail(CAAR_ERR_INVALID, "layout=%d", layout);
+  if (nelem_global >= (1 << 27))
+    return fail(CAAR_ERR_UNSUPPORTED, "nelem_global=%d: copies are packed as e*16 + p in 32 bits", nelem_global);
+  if (part_start[0] != 0 || part_start[nparts] != nelem_global)
+    return fail(CAAR_ERR_INVALID, "part_start must run from 0 to nelem_global=%d", nelem_global);
+  for (int q = 0; q < nparts; ++q)
+    if (part_start[q + 1] <= part_start[q]) return fail(CAAR_ERR_INVALID, "part_start is not ascending at %d", q);
+  const int E = h->dims.nelem, e0 = part_start[part];
+  if (part_start[part + 1] - e0 != E)
+    return fail(CAAR_ERR_INVALID, "block %d has %d elements, the handle %d", part, part_start[part + 1] - e0, E);
+  std::vector<long long> cxx(gid, gid + (size_t)nelem_global * 16);
+  if (layout == CAAR_LAYOUT_F90)  // as in caar_set_connectivity
+    for (size_t e = 0; e < (size_t)nelem_global; ++e)
+      for (int i = 0; i < 4; ++i)
+        for (int j = 0; j < 4; ++j) cxx[e * 16 + 4 * i + j] = gid[e * 16 + 4 * j + i];
+  caar::DssHostTables lt;
+  caar::HaloHostTables ht;
+  caar::DssTables d;
+  caar::HaloTables x;
+  std::memset(&d, 0, sizeof d);
+  std::memset(&x, 0, sizeof x);
+  d.ngroups = caar::build_dss_tables(cxx.data() + (size_t)e0 * 16, E, &lt);
+  caar::build_halo_tables(cxx.data(), nelem_global, part_start, nparts, part, &ht);
+  x.nparts = nparts;
+  x.ngroups = (int)ht.start.size() - 1;
+  x.nsend = ht.rec[0][nparts];
+  x.nrecv = ht.rec[1][nparts];
+  x.nsend_el = ht.rec[2][nparts];
+  x.nrecv_el = ht.rec[3][nparts];
+  x.rec = new (std::nothrow) int[4 * ((size_t)nparts + 1)];
+  if (!x.rec) return fail(CAAR_ERR_NOMEM, "host allocation failed");
+  for (int k = 0; k < 4; ++k) std::copy(ht.rec[k].begin(), ht.rec[k].end(), x.rec + k * ((size_t)nparts + 1));
+  // the buffers hold the largest selection: every DSS field with qsize_d tracers, or the bounds of qsize_d tracers
+  const size_t nv = caar::dss_record_doubles(CAAR_F_DP3D | CAAR_F_V | CAAR_F_T | CAAR_F_QDP, h->dims.qsize_d,
+                                             h->dims.nlev);
+  const size_t row = (size_t)h->dims.qsize_d * h->dims.nlev * 2;
+  const size_t send_n = std::max((size_t)x.nsend * nv, (size_t)x.nsend_el * row);
+  const size_t recv_n = std::max((size_t)x.nrecv * nv, (size_t)x.nrecv_el * row);
+  DeviceGuard guard(h->device);
+  cudaError_t e = upload_dss_tables(lt, &d, h->stream);
+  int** dst[6] = {&x.start, &x.copy, &x.nb_start, &x.nb, &x.send_copy, &x.send_el};
+  const std::vector<int>* src[6] = {&ht.start, &ht.copy, &ht.nb_start, &ht.nb, &ht.send_copy, &ht.send_el};
+  for (int i = 0; i < 6 && e == cudaSuccess; ++i) e = upload_vector(dst[i], *src[i], h->stream);
+  const std::vector<int2> send_seg = record_segments(ht.rec[0]), recv_seg = record_segments(ht.rec[1]);
+  if (e == cudaSuccess) e = upload_vector(&x.send_seg, send_seg, h->stream);
+  if (e == cudaSuccess) e = upload_vector(&x.recv_seg, recv_seg, h->stream);
+  if (e == cudaSuccess) e = cudaMalloc(&x.send, std::max(send_n, (size_t)1) * sizeof(double));
+  if (e == cudaSuccess) e = cudaMalloc(&x.recv, std::max(recv_n, (size_t)1) * sizeof(double));
+  if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+  if (e != cudaSuccess) {  // the earlier map or partition stays
+    free_dss_tables(d);
+    free_halo_tables(x);
+    return fail(e == cudaErrorMemoryAllocation ? CAAR_ERR_NOMEM : CAAR_ERR_CUDA, "caar_set_partition: %s",
+                cudaGetErrorString(e));
+  }
+  free_dss_tables(h->dss);  // the stream is idle: no launch still reads the earlier tables
+  free_halo_tables(h->halo);
+  h->dss = d;
+  h->halo = x;
+  return CAAR_OK;
+}
+
+int caar_dss_pack(caar_handle h, unsigned field_mask, int tl, int qtl, int qsize, int weighting) {
+  if (int rc = check_partitioned(h, "caar_dss_pack")) return rc;
+  if (int rc = check_dss_args(h, field_mask, tl, qtl, qsize, weighting)) return rc;
+  if (caar::dss_record_doubles(field_mask, qsize, h->dims.nlev) == 0 || h->halo.nsend == 0) return CAAR_OK;
+  DeviceGuard guard(h->device);
+  CU_TRY(caar::launch_dss_pack(make_args(h, nullptr), h->halo, field_mask, tl, qtl, qsize, h->stream));
+  ++h->launches;
+  return CAAR_OK;
+}
+
+int caar_dss_unpack(caar_handle h, unsigned field_mask, int tl, int qtl, int qsize, int weighting) {
+  if (int rc = check_partitioned(h, "caar_dss_unpack")) return rc;
+  if (int rc = check_dss_args(h, field_mask, tl, qtl, qsize, weighting)) return rc;
+  if (caar::dss_record_doubles(field_mask, qsize, h->dims.nlev) == 0) return CAAR_OK;
+  DeviceGuard guard(h->device);
+  CU_TRY(caar::launch_dss_unpack(make_args(h, nullptr), h->halo, field_mask, tl, qtl, qsize, weighting, h->stream));
+  ++h->launches;
+  return CAAR_OK;
+}
+
+int caar_neighbor_minmax_pack(caar_handle h, int qsize) {
+  if (int rc = check_partitioned(h, "caar_neighbor_minmax_pack")) return rc;
+  if (int rc = check_qsize(h, qsize)) return rc;
+  if (qsize == 0 || h->halo.nsend_el == 0) return CAAR_OK;
+  DeviceGuard guard(h->device);
+  double* bounds = nullptr;
+  if (int rc = bounds_buffer(h, &bounds)) return rc;
+  CU_TRY(caar::launch_neighbor_minmax_pack(h->halo, h->dims.qsize_d, h->dims.nlev, qsize, bounds, h->stream));
+  ++h->launches;
+  return CAAR_OK;
+}
+
+int caar_neighbor_minmax_unpack(caar_handle h, int qsize) {
+  if (int rc = check_partitioned(h, "caar_neighbor_minmax_unpack")) return rc;
+  if (int rc = check_qsize(h, qsize)) return rc;
+  if (qsize == 0) return CAAR_OK;
+  DeviceGuard guard(h->device);
+  double* bounds = nullptr;
+  if (int rc = bounds_buffer(h, &bounds)) return rc;
+  if (!h->bounds_next) CU_TRY(cudaMalloc(&h->bounds_next, bounds_count(h->dims) * sizeof(double)));
+  CU_TRY(caar::launch_neighbor_minmax_unpack(h->halo, h->dims.nelem, h->dims.qsize_d, h->dims.nlev, qsize, bounds,
+                                             h->bounds_next, h->stream));
+  ++h->launches;
+  h->bounds = h->bounds_next;
+  h->bounds_next = bounds;
+  return CAAR_OK;
+}
+
+int caar_halo_segments(caar_handle h, int op, unsigned field_mask, int qsize, double** send, double** recv,
+                       size_t* send_off, size_t* recv_off) {
+  if (int rc = check_partitioned(h, "caar_halo_segments")) return rc;
+  if (!send || !recv || !send_off || !recv_off) return fail(CAAR_ERR_INVALID, "null argument");
+  if (op != CAAR_HALO_DSS && op != CAAR_HALO_MINMAX) return fail(CAAR_ERR_INVALID, "op=%d", op);
+  if (field_mask & ~(CAAR_F_DP3D | CAAR_F_V | CAAR_F_T | CAAR_F_QDP))
+    return fail(CAAR_ERR_INVALID, "field_mask=0x%x: only dp3d, v, T and Qdp", field_mask);
+  if (int rc = check_qsize(h, qsize)) return rc;
+  const caar::HaloTables& x = h->halo;
+  const size_t n = (size_t)x.nparts + 1;
+  const size_t nv = op == CAAR_HALO_DSS ? caar::dss_record_doubles(field_mask, qsize, h->dims.nlev)
+                                        : (size_t)qsize * h->dims.nlev * 2;
+  const int* srec = x.rec + (op == CAAR_HALO_DSS ? 0 : 2) * n;
+  const int* rrec = srec + n;
+  for (size_t q = 0; q < n; ++q) {
+    send_off[q] = (size_t)srec[q] * nv;
+    recv_off[q] = (size_t)rrec[q] * nv;
+  }
+  *send = x.send;
+  *recv = x.recv;
   return CAAR_OK;
 }
 

@@ -162,6 +162,42 @@ cudaError_t launch_dss(const KernelArgs& a, const DssTables& t, unsigned mask, i
 // none for qsize == 0
 cudaError_t launch_neighbor_minmax(const DssTables& t, int nelem, int qsize_d, int L, int qsize, const double* in,
                                    double* out, cudaStream_t s);
+// The exchange of shared points between partitioned handles (caar_set_partition). A record is what one part sends
+// another for one of its copies (DSS) or one of its elements (neighbour bounds); segment q of a buffer holds the
+// records for or from part q, in the order of the global sort by (gid, global e, p) (DSS) or of ascending global
+// element (bounds), so that sender and receiver derive the same order from the same map.
+//   DSS:    every local group, its copies in global (e, p) order; a local copy is e*16 + p, a remote one -1 - R with R
+//           its record in the receive buffer. Segment q is [nv][n_q] (value v of record r at v*n_q + r, v = 0 the
+//           copy's spheremp, then the selected slices level by level), starting at double rec_start_q * nv.
+//   bounds: nb[nb_start[e] .. nb_start[e+1]) is N(e) in ascending global order, a local element e or nelem + R for row
+//           R of the receive buffer; row R is the [qsize][L][2] bounds of one element at double R * qsize * L * 2.
+struct HaloHostTables {
+  std::vector<int> start, copy, nb_start, nb;
+  std::vector<int> send_copy, send_el;  // the local copy of every DSS send record, the local element of every row
+  // record offsets of the segments, [nparts + 1] each: DSS send, DSS receive, bounds send, bounds receive
+  std::vector<int> rec[4];
+};
+struct HaloTables {  // on the device, but for the record offsets
+  int nparts, ngroups, nsend, nrecv, nsend_el, nrecv_el;
+  int *start, *copy, *nb_start, *nb, *send_copy, *send_el;
+  int2 *send_seg, *recv_seg;  // per DSS record: {first record of its segment, records in that segment}
+  int* rec;                   // host [4][nparts + 1]: HaloHostTables::rec
+  double *send, *recv;        // the exchange buffers
+};
+// gid [nelem_global][16] in the C order; part_start as caar_set_partition checks it
+void build_halo_tables(const long long* gid, int nelem_global, const int* part_start, int nparts, int part,
+                       HaloHostTables* t);
+// doubles of one DSS record for a selection (spheremp + every selected value of a copy); 0 when nothing is selected
+size_t dss_record_doubles(unsigned mask, int qsize, int L);
+// one launch each; the pack none when nothing is selected or there is no record to send
+cudaError_t launch_dss_pack(const KernelArgs& a, const HaloTables& t, unsigned mask, int tl, int qtl, int qsize,
+                            cudaStream_t s);
+cudaError_t launch_dss_unpack(const KernelArgs& a, const HaloTables& t, unsigned mask, int tl, int qtl, int qsize,
+                              int weighting, cudaStream_t s);
+cudaError_t launch_neighbor_minmax_pack(const HaloTables& t, int qsize_d, int L, int qsize, const double* bounds,
+                                        cudaStream_t s);
+cudaError_t launch_neighbor_minmax_unpack(const HaloTables& t, int nelem, int qsize_d, int L, int qsize,
+                                          const double* in, double* out, cudaStream_t s);
 // checksums of the seven mutated arrays + energy norms (caar_aux.cu); partial [nelem][8][2], bits [nelem][7]
 cudaError_t launch_checksums(const KernelArgs& a, int tl, int nets, int nete, double cp, double* partial,
                              unsigned long long* bits, double* out16, unsigned long long* out7, cudaStream_t s);

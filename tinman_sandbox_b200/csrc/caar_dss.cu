@@ -21,6 +21,11 @@
 // neighbor_minmax_kernel: one thread per (e, iq, k) bound pair of the whole array, k fastest, so that a warp reads one
 // contiguous row of each neighbour. It reads the old bounds and writes a second array (the caller swaps the two), so
 // the result does not depend on the order in which threads run; tracers iq >= qsize are copied.
+//
+// Across partitioned handles (caar_set_partition; tables and buffer layout at HaloHostTables in caar_device.cuh):
+// dss_pack_kernel writes one record per boundary copy for the other parts; dss_unpack_kernel is dss_kernel's walk in
+// which groups with remote copies read those copies from the received records; neighbor_minmax_pack_kernel and
+// neighbor_minmax_unpack_kernel do the same with the bound rows of boundary elements.
 #include <algorithm>
 #include <cstring>
 #include <vector>
@@ -136,6 +141,28 @@ __device__ __forceinline__ void dss_slice(double* base, size_t estride, const Ds
   }
 }
 
+// One group: the spheremp of its copies, m, r, then every selected slice; g.c0, g.n and g.cp (the first FAST_COPIES
+// copies, the first one repeated beyond g.n) are set, and every copy is local
+template <bool PROJECT>
+__device__ __forceinline__ void dss_group(const DssArgs& A, Group& g) {
+#pragma unroll
+  for (int c = 0; c < FAST_COPIES; ++c) g.s[c] = A.spheremp[g.cp[c]];
+  double m = g.s[0];
+#pragma unroll
+  for (int c = 1; c < FAST_COPIES; ++c)
+    if (c < g.n) m = __dadd_rn(m, g.s[c]);
+  for (int c = FAST_COPIES; c < g.n; ++c) m = __dadd_rn(m, A.spheremp[A.copy[g.c0 + c]]);
+  g.r = __ddiv_rn(1.0, m);
+#pragma unroll 1
+  for (int run = 0; run < A.nruns; ++run)
+#pragma unroll 1
+    for (int j = 0; j < A.count[run]; ++j) {
+      double* base = A.base[run] + j * A.step[run];
+      if (A.w[run] == 2) dss_slice<2, PROJECT>(base, A.estride[run], A, g);
+      else dss_slice<1, PROJECT>(base, A.estride[run], A, g);
+    }
+}
+
 template <bool PROJECT>
 __global__ void __launch_bounds__(DSS_THREADS, DSS_CTAS_PER_SM) dss_kernel(const DssArgs A) {
   for (size_t i = (size_t)blockIdx.x * DSS_THREADS + threadIdx.x; i < (size_t)A.ngroups;
@@ -144,25 +171,156 @@ __global__ void __launch_bounds__(DSS_THREADS, DSS_CTAS_PER_SM) dss_kernel(const
     g.c0 = A.start[i];
     g.n = A.start[i + 1] - g.c0;
 #pragma unroll
+    for (int c = 0; c < FAST_COPIES; ++c) g.cp[c] = A.copy[g.c0 + (c < g.n ? c : 0)];
+    dss_group<PROJECT>(A, g);
+  }
+}
+
+// ---- the exchange between partitioned handles ----
+// A DSS buffer (HaloTables): record R, in the segment seg[R] = {first record, records}, holds value v at
+// buf[first * nv + v * records + R - first]
+struct HaloArgs {
+  double* buf;      // the send buffer (pack) or the receive buffer (unpack)
+  const int2* seg;  // [records]
+  const int* copy;  // pack: the local copy e*16 + p of every record
+  int nrec, nv;
+};
+
+__device__ __forceinline__ double* record(const HaloArgs& H, int R, size_t* stride) {
+  const int2 sg = H.seg[R];
+  *stride = (size_t)sg.y;
+  return H.buf + (size_t)sg.x * H.nv + (R - sg.x);
+}
+
+// One thread per send record: spheremp, then the selected slices level by level, each batch of values loaded before
+// it is stored. Consecutive records are consecutive doubles of every value row, so the stores of a warp coalesce.
+__global__ void __launch_bounds__(DSS_THREADS) dss_pack_kernel(const DssArgs A, const HaloArgs H) {
+  constexpr int LV = 8;
+  for (int R = blockIdx.x * DSS_THREADS + threadIdx.x; R < H.nrec; R += gridDim.x * DSS_THREADS) {
+    const int cp = H.copy[R];
+    size_t st;
+    double* o = record(H, R, &st);
+    o[0] = A.spheremp[cp];
+    o += st;
+#pragma unroll 1
+    for (int run = 0; run < A.nruns; ++run)
+#pragma unroll 1
+      for (int j = 0; j < A.count[run]; ++j) {
+        const int W = A.w[run];
+        const double* p = A.base[run] + j * A.step[run] + (size_t)(cp >> 4) * A.estride[run] + (cp & 15) * W;
+        const int n = A.L * W;  // value v = k*W + w of the slice is p[k * 16 W + w]
+#pragma unroll 1
+        for (int v0 = 0; v0 < n; v0 += LV) {
+          double f[LV];
+#pragma unroll
+          for (int i = 0; i < LV; ++i)
+            if (v0 + i < n) f[i] = p[(size_t)((v0 + i) / W) * 16 * W + (v0 + i) % W];
+#pragma unroll
+          for (int i = 0; i < LV; ++i)
+            if (v0 + i < n) o[(size_t)(v0 + i) * st] = f[i];
+        }
+        o += (size_t)n * st;
+      }
+  }
+}
+
+// One slice of a group with remote copies: dss_slice's general loop, with a remote copy's value v0 + k*W + w and its
+// spheremp read from its record; only the local copies are written
+template <int W, bool PROJECT>
+__device__ __forceinline__ void dss_slice_halo(double* base, size_t estride, const DssArgs& A, const HaloArgs& H,
+                                               const Group& g, int v0) {
+#pragma unroll 1
+  for (int k = 0; k < A.L; ++k) {
+    double S[W];
+#pragma unroll 1
+    for (int c = 0; c < g.n; ++c) {
+      const int cp = A.copy[g.c0 + c];
+      double f[W], s;
+      if (cp >= 0) {
+        load<W>(base + (size_t)(cp >> 4) * estride + (size_t)k * 16 * W + (cp & 15) * W, f);
+        s = PROJECT ? A.spheremp[cp] : 0.0;
+      } else {
+        size_t st;
+        const double* o = record(H, -1 - cp, &st);
+#pragma unroll
+        for (int w = 0; w < W; ++w) f[w] = o[(size_t)(v0 + k * W + w) * st];
+        s = PROJECT ? o[0] : 0.0;
+      }
+#pragma unroll
+      for (int w = 0; w < W; ++w) {
+        const double t = PROJECT ? __dmul_rn(s, f[w]) : f[w];
+        S[w] = c == 0 ? t : __dadd_rn(S[w], t);
+      }
+    }
+#pragma unroll
+    for (int w = 0; w < W; ++w) S[w] = __dmul_rn(S[w], g.r);
+#pragma unroll 1
+    for (int c = 0; c < g.n; ++c) {
+      const int cp = A.copy[g.c0 + c];
+      if (cp >= 0) store<W>(base + (size_t)(cp >> 4) * estride + (size_t)k * 16 * W + (cp & 15) * W, S);
+    }
+  }
+}
+
+// dss_kernel's walk over the groups of HaloTables. A group whose copies are all local takes dss_kernel's path, so that
+// without remote copies the result is caar_dss's bit for bit; a group with remote copies takes the general loop. In
+// place as dss_kernel: a local value is read and written by the thread of its group only, and the receive buffer is
+// only read.
+template <bool PROJECT>
+__global__ void __launch_bounds__(DSS_THREADS, DSS_CTAS_PER_SM) dss_unpack_kernel(const DssArgs A, const HaloArgs H) {
+  for (size_t i = (size_t)blockIdx.x * DSS_THREADS + threadIdx.x; i < (size_t)A.ngroups;
+       i += (size_t)gridDim.x * DSS_THREADS) {
+    Group g;
+    g.c0 = A.start[i];
+    g.n = A.start[i + 1] - g.c0;
+    bool local = true;
+#pragma unroll
     for (int c = 0; c < FAST_COPIES; ++c) {
       g.cp[c] = A.copy[g.c0 + (c < g.n ? c : 0)];
-      g.s[c] = A.spheremp[g.cp[c]];
+      local = local && g.cp[c] >= 0;
     }
-    double m = g.s[0];
-#pragma unroll
-    for (int c = 1; c < FAST_COPIES; ++c)
-      if (c < g.n) m = __dadd_rn(m, g.s[c]);
-    for (int c = FAST_COPIES; c < g.n; ++c) m = __dadd_rn(m, A.spheremp[A.copy[g.c0 + c]]);
+    for (int c = FAST_COPIES; c < g.n; ++c) local = local && A.copy[g.c0 + c] >= 0;
+    if (local) {
+      dss_group<PROJECT>(A, g);
+      continue;
+    }
+    double m = 0.0;
+#pragma unroll 1
+    for (int c = 0; c < g.n; ++c) {
+      const int cp = A.copy[g.c0 + c];
+      size_t st;
+      const double s = cp >= 0 ? A.spheremp[cp] : record(H, -1 - cp, &st)[0];
+      m = c == 0 ? s : __dadd_rn(m, s);
+    }
     g.r = __ddiv_rn(1.0, m);
+    int v0 = 1;
 #pragma unroll 1
     for (int run = 0; run < A.nruns; ++run)
 #pragma unroll 1
       for (int j = 0; j < A.count[run]; ++j) {
         double* base = A.base[run] + j * A.step[run];
-        if (A.w[run] == 2) dss_slice<2, PROJECT>(base, A.estride[run], A, g);
-        else dss_slice<1, PROJECT>(base, A.estride[run], A, g);
+        if (A.w[run] == 2) dss_slice_halo<2, PROJECT>(base, A.estride[run], A, H, g, v0);
+        else dss_slice_halo<1, PROJECT>(base, A.estride[run], A, H, g, v0);
+        v0 += A.L * A.w[run];
       }
   }
+}
+
+// neighbor_minmax of bound pair i; with HALO a neighbour q >= nelem is row q - nelem of rin, rrow pairs apart
+template <bool HALO>
+__device__ __forceinline__ double2 minmax_pair(const double2* __restrict__ in, const int* __restrict__ nb_start,
+                                               const int* __restrict__ nb, size_t i, int row, int L, int qsize,
+                                               const double2* __restrict__ rin, int nelem, int rrow) {
+  const int e = (int)(i / row), o = (int)(i - (size_t)e * row);
+  double2 b = in[i];
+  if (o / L < qsize)
+    for (int j = nb_start[e]; j < nb_start[e + 1]; ++j) {
+      const int q = nb[j];
+      const double2 t = (!HALO || q < nelem) ? in[(size_t)q * row + o] : rin[(size_t)(q - nelem) * rrow + o];
+      if (t.x < b.x) b.x = t.x;
+      if (t.y > b.y) b.y = t.y;
+    }
+  return b;
 }
 
 __global__ void __launch_bounds__(DSS_THREADS) neighbor_minmax_kernel(const double2* __restrict__ in,
@@ -171,16 +329,26 @@ __global__ void __launch_bounds__(DSS_THREADS) neighbor_minmax_kernel(const doub
                                                                       const int* __restrict__ nb, size_t n, int row,
                                                                       int L, int qsize) {
   // row = qsize_d * L bound pairs per element
+  for (size_t i = (size_t)blockIdx.x * DSS_THREADS + threadIdx.x; i < n; i += (size_t)gridDim.x * DSS_THREADS)
+    out[i] = minmax_pair<false>(in, nb_start, nb, i, row, L, qsize, nullptr, 0, 0);
+}
+
+// neighbor_minmax_kernel with received rows of qsize * L pairs
+__global__ void __launch_bounds__(DSS_THREADS) neighbor_minmax_unpack_kernel(
+    const double2* __restrict__ in, double2* __restrict__ out, const int* __restrict__ nb_start,
+    const int* __restrict__ nb, size_t n, int row, int L, int qsize, const double2* __restrict__ rin, int nelem) {
+  for (size_t i = (size_t)blockIdx.x * DSS_THREADS + threadIdx.x; i < n; i += (size_t)gridDim.x * DSS_THREADS)
+    out[i] = minmax_pair<true>(in, nb_start, nb, i, row, L, qsize, rin, nelem, qsize * L);
+}
+
+// one thread per (send row, pair): row R is the first rrow pairs of element el[R]
+__global__ void __launch_bounds__(DSS_THREADS) neighbor_minmax_pack_kernel(const double2* __restrict__ in,
+                                                                           double2* __restrict__ out,
+                                                                           const int* __restrict__ el, size_t n,
+                                                                           int row, int rrow) {
   for (size_t i = (size_t)blockIdx.x * DSS_THREADS + threadIdx.x; i < n; i += (size_t)gridDim.x * DSS_THREADS) {
-    const int e = (int)(i / row), o = (int)(i - (size_t)e * row);
-    double2 b = in[i];
-    if (o / L < qsize)
-      for (int j = nb_start[e]; j < nb_start[e + 1]; ++j) {
-        const double2 t = in[(size_t)nb[j] * row + o];
-        if (t.x < b.x) b.x = t.x;
-        if (t.y > b.y) b.y = t.y;
-      }
-    out[i] = b;
+    const size_t R = i / rrow;
+    out[i] = in[(size_t)el[R] * row + (i - R * rrow)];
   }
 }
 
@@ -192,6 +360,36 @@ unsigned grid_for(Kernel* k, size_t items, int max_per_sm, LaunchCache& cache, c
   size_t blocks = (items + DSS_THREADS - 1) / DSS_THREADS;
   const size_t wave = (size_t)std::min(per_sm, max_per_sm) * sm_count();
   return (unsigned)std::min(blocks, wave);
+}
+
+bool selected(unsigned mask, int qsize) {
+  return (mask & (CAAR_F_DP3D | CAAR_F_V | CAAR_F_T)) || ((mask & CAAR_F_QDP) && qsize > 0);
+}
+
+// the selected slices of caar_dss as runs, over the groups start / copy
+DssArgs dss_args(const KernelArgs& a, unsigned mask, int tl, int qtl, int qsize, const int* start, const int* copy,
+                 int ngroups) {
+  DssArgs A;
+  std::memset(&A, 0, sizeof A);
+  const size_t lf = (size_t)a.nlev * 16;
+  auto add = [&](double* base, size_t estride, int w, int count, size_t step) {
+    A.base[A.nruns] = base;
+    A.estride[A.nruns] = estride;
+    A.w[A.nruns] = w;
+    A.count[A.nruns] = count;
+    A.step[A.nruns++] = step;
+  };
+  if (mask & CAAR_F_DP3D) add(a.dp3d + tl * lf, a.ntl * lf, 1, 1, 0);
+  if (mask & CAAR_F_V) add(a.v + 2 * tl * lf, 2 * a.ntl * lf, 2, 1, 0);
+  if (mask & CAAR_F_T) add(a.T + tl * lf, a.ntl * lf, 1, 1, 0);
+  if ((mask & CAAR_F_QDP) && qsize > 0)  // Qdp is const in KernelArgs for the kernels that read it; this is the mirror
+    add(const_cast<double*>(a.Qdp) + qtl * lf, 2 * a.qsize_d * lf, 1, qsize, 2 * lf);
+  A.spheremp = a.spheremp;
+  A.start = start;
+  A.copy = copy;
+  A.ngroups = ngroups;
+  A.L = a.nlev;
+  return A;
 }
 
 }  // namespace
@@ -242,29 +440,120 @@ int build_dss_tables(const long long* gid, int nelem, DssHostTables* t) {
   return (int)G;
 }
 
+void build_halo_tables(const long long* gid, int nelem_global, const int* part_start, int nparts, int part,
+                       HaloHostTables* t) {
+  const int e0 = part_start[part], nl = part_start[part + 1] - e0;
+  const size_t ncopy = (size_t)nelem_global * 16;
+  struct Copy {
+    long long gid;
+    int cp;  // global e*16 + p
+  };
+  std::vector<Copy> c(ncopy);
+  for (size_t i = 0; i < ncopy; ++i) c[i] = Copy{gid[i], (int)i};
+  std::sort(c.begin(), c.end(), [](const Copy& a, const Copy& b) { return a.gid != b.gid ? a.gid < b.gid : a.cp < b.cp; });
+  auto part_of = [&](int ge) { return (int)(std::upper_bound(part_start, part_start + nparts + 1, ge) - part_start) - 1; };
+  auto is_local = [&](int ge) { return ge >= e0 && ge < e0 + nl; };
+  // the runs of one gid that hold a local copy; the remote copies of each (received, in global sort order per sender)
+  // and the local copies for every other part that holds the point (sent, in the same order)
+  std::vector<std::pair<size_t, size_t>> runs;
+  std::vector<std::vector<size_t>> recv(nparts);
+  std::vector<std::vector<int>> send(nparts);
+  std::vector<long long> pairs;  // el * nelem_global + ge for local el and every other element ge that shares a point
+  std::vector<int> parts;
+  for (size_t a = 0, b; a < ncopy; a = b) {
+    bool local = false;
+    for (b = a; b < ncopy && c[b].gid == c[a].gid; ++b) local = local || is_local(c[b].cp >> 4);
+    if (!local) continue;
+    runs.emplace_back(a, b);
+    parts.clear();
+    for (size_t i = a; i < b; ++i) {
+      const int gi = c[i].cp >> 4;
+      if (!is_local(gi)) {
+        const int q = part_of(gi);
+        recv[q].push_back(i);
+        if (std::find(parts.begin(), parts.end(), q) == parts.end()) parts.push_back(q);
+        continue;
+      }
+      for (size_t j = a; j < b; ++j) {
+        const int gj = c[j].cp >> 4;
+        if (gj != gi) pairs.push_back((long long)(gi - e0) * nelem_global + gj);
+      }
+    }
+    std::sort(parts.begin(), parts.end());
+    for (int q : parts)
+      for (size_t i = a; i < b; ++i)
+        if (is_local(c[i].cp >> 4)) send[q].push_back(c[i].cp - e0 * 16);
+  }
+  for (auto& r : t->rec) r.assign((size_t)nparts + 1, 0);
+  std::vector<int> rid(ncopy, -1);  // record of every received copy, by its place in c
+  for (int q = 0; q < nparts; ++q) {
+    t->rec[0][q + 1] = t->rec[0][q] + (int)send[q].size();
+    t->rec[1][q + 1] = t->rec[1][q] + (int)recv[q].size();
+    for (size_t k = 0; k < recv[q].size(); ++k) rid[recv[q][k]] = t->rec[1][q] + (int)k;
+    t->send_copy.insert(t->send_copy.end(), send[q].begin(), send[q].end());
+  }
+  // the local groups in the order of their owners, every copy in global (e, p) order
+  std::sort(runs.begin(), runs.end(), [&](const std::pair<size_t, size_t>& x, const std::pair<size_t, size_t>& y) {
+    auto owner = [&](const std::pair<size_t, size_t>& r) {
+      size_t i = r.first;
+      while (!is_local(c[i].cp >> 4)) ++i;
+      return c[i].cp;
+    };
+    return owner(x) < owner(y);
+  });
+  t->start.assign(1, 0);
+  t->copy.clear();
+  for (const auto& r : runs) {
+    for (size_t i = r.first; i < r.second; ++i)
+      t->copy.push_back(is_local(c[i].cp >> 4) ? c[i].cp - e0 * 16 : -1 - rid[i]);
+    t->start.push_back((int)t->copy.size());
+  }
+  // neighbours: N(el) ascending by global element; a remote one is the row of its element among those received from
+  // its part, which are the elements of that part with a neighbour here, ascending
+  std::sort(pairs.begin(), pairs.end());
+  pairs.erase(std::unique(pairs.begin(), pairs.end()), pairs.end());
+  std::vector<std::vector<int>> send_el(nparts), recv_el(nparts);
+  for (long long pr : pairs) {
+    const int el = (int)(pr / nelem_global), gj = (int)(pr % nelem_global);
+    if (is_local(gj)) continue;
+    const int q = part_of(gj);
+    recv_el[q].push_back(gj);
+    if (send_el[q].empty() || send_el[q].back() != el) send_el[q].push_back(el);  // pairs ascend in el
+  }
+  for (int q = 0; q < nparts; ++q) {
+    std::sort(recv_el[q].begin(), recv_el[q].end());
+    recv_el[q].erase(std::unique(recv_el[q].begin(), recv_el[q].end()), recv_el[q].end());
+    t->rec[2][q + 1] = t->rec[2][q] + (int)send_el[q].size();
+    t->rec[3][q + 1] = t->rec[3][q] + (int)recv_el[q].size();
+    t->send_el.insert(t->send_el.end(), send_el[q].begin(), send_el[q].end());
+  }
+  t->nb_start.assign((size_t)nl + 1, 0);
+  t->nb.resize(pairs.size());
+  for (size_t i = 0; i < pairs.size(); ++i) {
+    const int el = (int)(pairs[i] / nelem_global), gj = (int)(pairs[i] % nelem_global);
+    if (is_local(gj)) {
+      t->nb[i] = gj - e0;
+    } else {
+      const int q = part_of(gj);
+      const auto& r = recv_el[q];
+      t->nb[i] = nl + t->rec[3][q] + (int)(std::lower_bound(r.begin(), r.end(), gj) - r.begin());
+    }
+    ++t->nb_start[el + 1];
+  }
+  for (int e = 0; e < nl; ++e) t->nb_start[e + 1] += t->nb_start[e];
+}
+
+size_t dss_record_doubles(unsigned mask, int qsize, int L) {
+  if (!selected(mask, qsize)) return 0;
+  const int per_level = !!(mask & CAAR_F_DP3D) + 2 * !!(mask & CAAR_F_V) + !!(mask & CAAR_F_T) +
+                        ((mask & CAAR_F_QDP) ? qsize : 0);
+  return 1 + (size_t)per_level * L;
+}
+
 cudaError_t launch_dss(const KernelArgs& a, const DssTables& t, unsigned mask, int tl, int qtl, int qsize,
                        int weighting, cudaStream_t s) {
-  if (!(mask & (CAAR_F_DP3D | CAAR_F_V | CAAR_F_T)) && !((mask & CAAR_F_QDP) && qsize > 0)) return cudaSuccess;
-  DssArgs A;
-  std::memset(&A, 0, sizeof A);
-  const size_t lf = (size_t)a.nlev * 16;
-  auto add = [&](double* base, size_t estride, int w, int count, size_t step) {
-    A.base[A.nruns] = base;
-    A.estride[A.nruns] = estride;
-    A.w[A.nruns] = w;
-    A.count[A.nruns] = count;
-    A.step[A.nruns++] = step;
-  };
-  if (mask & CAAR_F_DP3D) add(a.dp3d + tl * lf, a.ntl * lf, 1, 1, 0);
-  if (mask & CAAR_F_V) add(a.v + 2 * tl * lf, 2 * a.ntl * lf, 2, 1, 0);
-  if (mask & CAAR_F_T) add(a.T + tl * lf, a.ntl * lf, 1, 1, 0);
-  if ((mask & CAAR_F_QDP) && qsize > 0)  // Qdp is const in KernelArgs for the kernels that read it; this is the mirror
-    add(const_cast<double*>(a.Qdp) + qtl * lf, 2 * a.qsize_d * lf, 1, qsize, 2 * lf);
-  A.spheremp = a.spheremp;
-  A.start = t.start;
-  A.copy = t.copy;
-  A.ngroups = t.ngroups;
-  A.L = a.nlev;
+  if (!selected(mask, qsize)) return cudaSuccess;
+  const DssArgs A = dss_args(a, mask, tl, qtl, qsize, t.start, t.copy, t.ngroups);
   static LaunchCache cache[2];
   cudaError_t e = cudaSuccess;
   if (weighting == CAAR_DSS_PROJECT) {
@@ -290,6 +579,66 @@ cudaError_t launch_neighbor_minmax(const DssTables& t, int nelem, int qsize_d, i
   neighbor_minmax_kernel<<<grid, DSS_THREADS, 0, s>>>(reinterpret_cast<const double2*>(in),
                                                       reinterpret_cast<double2*>(out), t.nb_start, t.nb, n,
                                                       qsize_d * L, L, qsize);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_dss_pack(const KernelArgs& a, const HaloTables& t, unsigned mask, int tl, int qtl, int qsize,
+                            cudaStream_t s) {
+  if (!selected(mask, qsize) || t.nsend == 0) return cudaSuccess;
+  const DssArgs A = dss_args(a, mask, tl, qtl, qsize, nullptr, nullptr, 0);
+  const HaloArgs H{t.send, t.send_seg, t.send_copy, t.nsend, (int)dss_record_doubles(mask, qsize, a.nlev)};
+  static LaunchCache cache;
+  cudaError_t e = cudaSuccess;
+  const unsigned grid = grid_for(dss_pack_kernel, (size_t)t.nsend, 2048 / DSS_THREADS, cache, &e);
+  if (e != cudaSuccess) return e;
+  dss_pack_kernel<<<grid, DSS_THREADS, 0, s>>>(A, H);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_dss_unpack(const KernelArgs& a, const HaloTables& t, unsigned mask, int tl, int qtl, int qsize,
+                              int weighting, cudaStream_t s) {
+  if (!selected(mask, qsize)) return cudaSuccess;
+  const DssArgs A = dss_args(a, mask, tl, qtl, qsize, t.start, t.copy, t.ngroups);
+  const HaloArgs H{t.recv, t.recv_seg, nullptr, t.nrecv, (int)dss_record_doubles(mask, qsize, a.nlev)};
+  static LaunchCache cache[2];
+  cudaError_t e = cudaSuccess;
+  if (weighting == CAAR_DSS_PROJECT) {
+    const unsigned grid = grid_for(dss_unpack_kernel<true>, (size_t)t.ngroups, DSS_CTAS_PER_SM, cache[1], &e);
+    if (e != cudaSuccess) return e;
+    dss_unpack_kernel<true><<<grid, DSS_THREADS, 0, s>>>(A, H);
+  } else {
+    const unsigned grid = grid_for(dss_unpack_kernel<false>, (size_t)t.ngroups, DSS_CTAS_PER_SM, cache[0], &e);
+    if (e != cudaSuccess) return e;
+    dss_unpack_kernel<false><<<grid, DSS_THREADS, 0, s>>>(A, H);
+  }
+  return cudaGetLastError();
+}
+
+cudaError_t launch_neighbor_minmax_pack(const HaloTables& t, int qsize_d, int L, int qsize, const double* bounds,
+                                        cudaStream_t s) {
+  const size_t n = (size_t)t.nsend_el * qsize * L;
+  if (n == 0) return cudaSuccess;
+  static LaunchCache cache;
+  cudaError_t e = cudaSuccess;
+  const unsigned grid = grid_for(neighbor_minmax_pack_kernel, n, 2048 / DSS_THREADS, cache, &e);
+  if (e != cudaSuccess) return e;
+  neighbor_minmax_pack_kernel<<<grid, DSS_THREADS, 0, s>>>(reinterpret_cast<const double2*>(bounds),
+                                                           reinterpret_cast<double2*>(t.send), t.send_el, n,
+                                                           qsize_d * L, qsize * L);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_neighbor_minmax_unpack(const HaloTables& t, int nelem, int qsize_d, int L, int qsize,
+                                          const double* in, double* out, cudaStream_t s) {
+  if (qsize <= 0) return cudaSuccess;
+  static LaunchCache cache;
+  const size_t n = (size_t)nelem * qsize_d * L;
+  cudaError_t e = cudaSuccess;
+  const unsigned grid = grid_for(neighbor_minmax_unpack_kernel, n, 2048 / DSS_THREADS, cache, &e);
+  if (e != cudaSuccess) return e;
+  neighbor_minmax_unpack_kernel<<<grid, DSS_THREADS, 0, s>>>(
+      reinterpret_cast<const double2*>(in), reinterpret_cast<double2*>(out), t.nb_start, t.nb, n, qsize_d * L, L,
+      qsize, reinterpret_cast<const double2*>(t.recv), nelem);
   return cudaGetLastError();
 }
 

@@ -1,7 +1,8 @@
 #!/usr/bin/env python
 """Times caar_dss, caar_neighbor_minmax and caar_run_rk5_dss on resident data over cubed-sphere connectivity.
-    python tools/dss_bench.py [--reps 10]
-Prints one JSON line per case:
+    python tools/dss_bench.py [--reps 10] [--parts N]
+With --parts N it times only the exchange across partitioned handles (parts_case below). Otherwise it prints one JSON
+line per case:
   state DSS (v, T, dp3d; ASSEMBLE) at 86400 x 72 (ne = 120) and 48600 x 128 (ne = 90)
   Qdp DSS (PROJECT) at 86400 x 72 with qsize 4 and 21600 x 72 (ne = 60) with qsize 35
   caar_neighbor_minmax at the two Qdp sizes
@@ -17,6 +18,7 @@ import argparse
 import json
 import os
 import sys
+import time
 
 import numpy as np
 
@@ -122,12 +124,81 @@ def rk5_case(reps, peak, info):
         report(f"step_{k}", "panel", E, L, nbytes, min(ms[k]), float(np.median(ms[k])), None, peak, info)
 
 
+def parts_case(nparts, reps, peak, info):
+    """N handles on one GPU hold the blocks of the ne = 120 mesh (86400 x 72, panel order; blocks as
+    partition.element_range cuts them) and assemble dp3d, v and T (ASSEMBLE). Timed with CUDA events on one stream,
+    alternating rep by rep, on one non-default stream: caar_dss_pack on every part, the segment copies (one torch copy_ per non-empty segment,
+    cudaMemcpyAsync), caar_dss_unpack on every part, and caar_dss on one handle that holds the whole mesh. Bytes:
+    pack reads and writes every record, the copies read and write every segment, unpack and the whole-mesh DSS read and
+    write every value once (unpack also reads the records). Also reported: the host time of caar_set_partition per
+    part and the largest number of boundary copies a part sends."""
+    import torch
+    from tinman_sandbox_b200.partition import element_range
+    ne, L = 120, 72
+    E = 6 * ne * ne
+    gid = mesh(ne, "panel")
+    ps = [element_range(p, nparts, E)[0] for p in range(nparts)] + [E]
+    stream = torch.cuda.Stream()      # not the default stream: caar_set_stream(h, 0) means the handle's own
+    whole = tb.Caar(E, L, 1, 1)
+    whole.upload({"elem_spheremp": np.ones((E, 4, 4))}, names=("elem_spheremp",))
+    whole.set_connectivity(gid)
+    whole.set_stream(stream.cuda_stream)
+    hs, build_ms = [], []
+    for p in range(nparts):
+        h = tb.Caar(ps[p + 1] - ps[p], L, 1, 1)
+        h.upload({"elem_spheremp": np.ones((ps[p + 1] - ps[p], 4, 4))}, names=("elem_spheremp",))
+        t0 = time.perf_counter()
+        h.set_partition(gid, ps, p)
+        build_ms.append((time.perf_counter() - t0) * 1e3)
+        h.set_stream(stream.cuda_stream)
+        hs.append(h)
+    segs = [h.halo_segments(tb.HALO_DSS, STATE, 0) for h in hs]
+    moves = [(segs[q][1][segs[q][3][p]:segs[q][3][p + 1]], segs[p][0][segs[p][2][q]:segs[p][2][q + 1]])
+             for q in range(nparts) for p in range(nparts) if segs[q][3][p + 1] > segs[q][3][p]]
+
+    def copies():
+        with torch.cuda.stream(stream):
+            for dst, src in moves:
+                dst.copy_(src)
+    runs = {"pack": lambda: [h.dss_pack(STATE, tl=0, sync=False) for h in hs], "copies": copies,
+            "unpack": lambda: [h.dss_unpack(STATE, tl=0, sync=False) for h in hs],
+            "whole_dss": lambda: whole.dss(STATE, tl=0, sync=False)}
+    nv = 1 + 4 * L
+    sent = sum(int(s[2][-1]) for s in segs) * 8
+    value_bytes = 2 * 4 * E * L * 16 * 8
+    nbytes = {"pack": 2 * sent, "copies": 2 * sent, "unpack": value_bytes + sent, "whole_dss": value_bytes}
+    for fn in runs.values():
+        fn()
+    torch.cuda.synchronize()
+    ms = {k: [] for k in runs}
+    for _ in range(reps):
+        for k, fn in runs.items():
+            a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            a.record(stream)
+            fn()
+            b.record(stream)
+            b.synchronize()
+            ms[k].append(a.elapsed_time(b))
+    for k in runs:
+        report(f"parts{nparts}_{k}", "panel", E, L, nbytes[k], min(ms[k]), float(np.median(ms[k])), None, peak, info)
+    records = max(int(s[2][-1]) for s in segs) // nv
+    print(json.dumps(dict(case=f"parts{nparts}_set_partition", E=E, host_ms_max=round(max(build_ms), 1),
+                          host_ms_mean=round(float(np.mean(build_ms)), 1), max_send_records=records,
+                          max_send_fraction=round(records / (16 * max(np.diff(ps))), 4), **info)), flush=True)
+    for h in hs + [whole]:
+        h.close()
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reps", type=int, default=10)
+    ap.add_argument("--parts", type=int, default=0, help="time the exchange over this many handles of the ne = 120 mesh")
     args = ap.parse_args()
     info = gpu_info()
     peak = copy_peak_gbps()
+    if args.parts:
+        parts_case(args.parts, args.reps, peak, info)
+        return
     dss_cases(args.reps, peak, info)
     rk5_case(max(3, args.reps // 2), peak, info)
 
