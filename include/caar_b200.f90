@@ -72,7 +72,7 @@ module caar_b200
             caar_bounds_upload, caar_bounds_download, caar_sphere_wk, caar_extra_upload, caar_extra_download, caar_last_error, &
             caar_host_register, caar_host_unregister, caar_describe, caar_set_connectivity, caar_dss, caar_neighbor_minmax, &
             caar_run_rk5_dss, caar_set_partition, caar_dss_pack, caar_dss_unpack, caar_neighbor_minmax_pack, &
-            caar_neighbor_minmax_unpack, caar_halo_segments
+            caar_neighbor_minmax_unpack, caar_halo_segments, caar_rk5_stage, caar_dss_interior, caar_dss_boundary
 
   interface
     ! int caar_create(caar_handle* out, const caar_dims* dims, int device);
@@ -141,6 +141,17 @@ module caar_b200
       type(caar_control), intent(inout) :: ctl
       real(c_double), value :: dt
       integer(c_int), value :: nsteps, mode
+      integer(c_int) :: rc
+    end function
+    ! int caar_rk5_stage(caar_handle h, const caar_control* ctl, double dt, int stage, int mode, int* tl);
+    ! stage 0..4 of caar_run_rk5's step (the compute_and_apply_rhs calls of prim_advance_exp); tl = the level it wrote
+    function caar_rk5_stage(handle, ctl, dt, stage, mode, tl) bind(C, name="caar_rk5_stage") result(rc)
+      import :: c_ptr, c_int, c_double, caar_control
+      type(c_ptr), value :: handle
+      type(caar_control), intent(in) :: ctl
+      real(c_double), value :: dt
+      integer(c_int), value :: stage, mode
+      integer(c_int), intent(out) :: tl
       integer(c_int) :: rc
     end function
     subroutine caar_update_time_levels(ctl) bind(C, name="caar_update_time_levels")
@@ -262,6 +273,19 @@ module caar_b200
       integer(c_int) :: rc
     end function
     function caar_dss_unpack(handle, field_mask, tl, qtl, qsize, weighting) bind(C, name="caar_dss_unpack") result(rc)
+      import :: c_ptr, c_int
+      type(c_ptr), value :: handle
+      integer(c_int), value :: field_mask, tl, qtl, qsize, weighting
+      integer(c_int) :: rc
+    end function
+    ! caar_dss_unpack in two: the points with every copy on this rank (may overlap bndry_exchangeV), then the others
+    function caar_dss_interior(handle, field_mask, tl, qtl, qsize, weighting) bind(C, name="caar_dss_interior") result(rc)
+      import :: c_ptr, c_int
+      type(c_ptr), value :: handle
+      integer(c_int), value :: field_mask, tl, qtl, qsize, weighting
+      integer(c_int) :: rc
+    end function
+    function caar_dss_boundary(handle, field_mask, tl, qtl, qsize, weighting) bind(C, name="caar_dss_boundary") result(rc)
       import :: c_ptr, c_int
       type(c_ptr), value :: handle
       integer(c_int), value :: field_mask, tl, qtl, qsize, weighting

@@ -249,12 +249,28 @@ void caar_update_time_levels(caar_control* ctl);
    CAAR_ERR_STATE before caar_set_params and CAAR_ERR_INVALID for a null control, nsteps < 0, a bad mode or
    levels that are not pairwise distinct, leaving *ctl unchanged. No DSS runs between stages; caar_run_rk5_dss runs one. */
 int caar_run_rk5(caar_handle h, caar_control* ctl, double dt, int nsteps, int mode);
+/* One stage of caar_run_rk5's step: row `stage` in [0, 5) of the table above (rows 1..5 are stages 0..4), with
+   *ctl holding the levels on entry to the step. Stage 4 first launches the combination c, as caar_run_rk5 does. *tl
+   receives the level the stage wrote: nm1 for stage 0, np1 for the others; that is the level a DSS after the stage
+   assembles. *ctl is not rotated: the caller calls caar_update_time_levels after stage 4. Exactly:
+     stages 0..4, then caar_update_time_levels(ctl)                          is caar_run_rk5(h, ctl, dt, 1, mode)
+     the same with caar_dss(h, CAAR_F_V | CAAR_F_T | CAAR_F_DP3D, *tl, 0, 0, CAAR_DSS_ASSEMBLE) after every stage
+                                                                             is caar_run_rk5_dss(h, ctl, dt, 1, mode)
+   bit for bit: both run these stages' launches in this order. On partitioned handles (caar_set_partition) the DSS
+   after every stage is caar_dss_pack, the caller's transport, caar_dss_interior and caar_dss_boundary (below); over a
+   block partition the parts then hold, bit for bit, the slices of caar_run_rk5_dss on one handle that holds the whole
+   mesh. Asynchronous on the handle's stream; 1 launch (2 for stage 4), none for an empty element range. Returns every
+   error of caar_run_rk5 (pairwise-distinct levels included) and CAAR_ERR_INVALID for a stage outside [0, 5) or a null
+   tl; a rejected call launches nothing and changes nothing, *tl included. */
+int caar_rk5_stage(caar_handle h, const caar_control* ctl, double dt, int stage, int mode, int* tl);
 int caar_sync(caar_handle h);
 /* number of kernel launches issued through this handle since creation (caar_run, caar_run_rk5: 6 per step,
-   caar_run_rk5_dss: 11 per step, caar_advect_tracers: 4 per step, caar_tracer_bounds and caar_limit_tracers: 1 per call
+   caar_run_rk5_dss: 11 per step, caar_rk5_stage: 1 (2 for stage 4), caar_advect_tracers: 4 per step, caar_tracer_bounds and caar_limit_tracers: 1 per call
    (none for an empty range or qsize == 0), caar_dss and caar_neighbor_minmax: 1 per call (none when nothing is
    selected), caar_dss_pack / caar_dss_unpack and caar_neighbor_minmax_pack / caar_neighbor_minmax_unpack: 1 per call
-   (none when nothing is selected, and none for a pack of a part that shares no point), caar_euler_step, caar_norms,
+   (none when nothing is selected, and none for a pack of a part that shares no point), caar_dss_interior /
+   caar_dss_boundary: at most 1 per call (none when nothing is selected or the part has no interior / boundary group),
+   caar_euler_step, caar_norms,
    ...) */
 long long caar_launch_count(caar_handle h);
 /* CUDA-event stopwatch on the stream the kernels are launched on: start records an event, stop records a
@@ -430,7 +446,8 @@ int caar_run_rk5_dss(caar_handle h, caar_control* ctl, double dt, int nsteps, in
    table on the host once (a sort of the 16 nelem_global copies); replaces any earlier connectivity or partition, and a
    later caar_set_connectivity replaces it; works before caar_set_params. From then on caar_dss and
    caar_neighbor_minmax keep their local-only meaning, as if caar_set_connectivity had been given the handle's slice of
-   gid; so does caar_run_rk5_dss, which therefore assembles HOMME's step only on a handle that holds the whole mesh.
+   gid; so does caar_run_rk5_dss. On a part, HOMME's step is caar_rk5_stage with caar_dss_pack, the transport,
+   caar_dss_interior and caar_dss_boundary after every stage (at caar_rk5_stage).
    Allocates the two exchange buffers, sized for the largest selection (all four fields with qsize_d tracers, and the
    bounds of qsize_d tracers), until caar_destroy or the next map. CAAR_ERR_INVALID for a null handle, gid or
    part_start, nparts < 1, part outside [0, nparts), part_start not ascending from 0 to nelem_global, a block size other
@@ -447,6 +464,16 @@ int caar_run_rk5_dss(caar_handle h, caar_control* ctl, double dt, int nsteps, in
    pack and unpack of one exchange must use the same field_mask, tl, qtl and qsize: mixing them is a caller error that
    is not detected. With nparts == 1 unpack equals caar_dss bit for bit.
 
+   caar_dss_interior / caar_dss_boundary split caar_dss_unpack in two, with its arguments, checks and selection rules.
+   The local groups (the points with a copy on this handle) are interior when every copy is on this handle and boundary
+   when at least one copy is on another part. interior assembles the interior groups; it reads neither buffer and
+   writes no copy that caar_dss_pack reads (a copy pack sends belongs to a point another part holds), so it may be
+   queued before or after pack and may run while the segments are in flight. boundary assembles the boundary groups
+   and reads the receive buffer, so it follows the transport. The two, in either order, give caar_dss_unpack's result
+   bit for bit (the same operations in the same order per point), and so, over a block partition, the whole-mesh
+   caar_dss. Each is at most one launch: none when nothing is selected, interior none when every local group has a
+   remote copy, boundary none when there is no remote copy (nparts == 1, or a part that shares no point).
+
    caar_neighbor_minmax_pack / caar_neighbor_minmax_unpack: the same on the limiter bounds. Segment q holds the
    [qsize][L][2] bounds of every local element that has a neighbour in part q. unpack is caar_neighbor_minmax's rule over
    N(e) of the whole mesh: e's own value first, then every neighbour, local or remote, in ascending global element order
@@ -458,8 +485,8 @@ int caar_run_rk5_dss(caar_handle h, caar_control* ctl, double dt, int nsteps, in
    the size of recv_off of q<-p on part q; the segments to and from this part itself are empty. Synchronous, launches
    nothing; CAAR_ERR_INVALID for null outputs or a bad op, mask or qsize.
 
-   pack and unpack are asynchronous on the handle's stream. The caller's transport must be ordered after pack and
-   unpack after the transport (with caar_set_stream on the transport's stream this is free). Before
+   pack, unpack, interior and boundary are asynchronous on the handle's stream. The caller's transport must be ordered
+   after pack, and unpack or boundary after the transport (with caar_set_stream on the transport's stream this is free). Before
    caar_set_partition every call here but caar_set_partition returns CAAR_ERR_STATE; a rejected call launches nothing
    and changes nothing. */
 enum { CAAR_HALO_DSS = 0, CAAR_HALO_MINMAX = 1 };
@@ -467,6 +494,8 @@ int caar_set_partition(caar_handle h, const long long* gid, int nelem_global, co
                        int part, int layout);
 int caar_dss_pack(caar_handle h, unsigned field_mask, int tl, int qtl, int qsize, int weighting);
 int caar_dss_unpack(caar_handle h, unsigned field_mask, int tl, int qtl, int qsize, int weighting);
+int caar_dss_interior(caar_handle h, unsigned field_mask, int tl, int qtl, int qsize, int weighting);
+int caar_dss_boundary(caar_handle h, unsigned field_mask, int tl, int qtl, int qsize, int weighting);
 int caar_neighbor_minmax_pack(caar_handle h, int qsize);
 int caar_neighbor_minmax_unpack(caar_handle h, int qsize);
 int caar_halo_segments(caar_handle h, int op, unsigned field_mask, int qsize, double** send, double** recv,

@@ -46,7 +46,7 @@ EXPORTED_SYMBOLS = (
     "caar_sphere_wk", "caar_run_rk5", "caar_advect_tracers", "caar_bounds_upload", "caar_bounds_download",
     "caar_tracer_bounds", "caar_limit_tracers", "caar_set_connectivity", "caar_dss", "caar_neighbor_minmax",
     "caar_run_rk5_dss", "caar_set_partition", "caar_dss_pack", "caar_dss_unpack", "caar_neighbor_minmax_pack",
-    "caar_neighbor_minmax_unpack", "caar_halo_segments",
+    "caar_neighbor_minmax_unpack", "caar_halo_segments", "caar_rk5_stage", "caar_dss_interior", "caar_dss_boundary",
 )
 CHECKSUM_FIELDS = ("elem_state_dp3d", "elem_state_v", "elem_state_T", "elem_derived_eta_dot_dpdn",
                    "elem_derived_omega_p", "elem_derived_phi", "elem_derived_vn0")
@@ -133,6 +133,7 @@ def load_library():
     lib.caar_set_vertical_coordinate.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_double)]
     lib.caar_run_stepping.argtypes = [C.c_void_p, C.POINTER(Control), C.c_int, C.c_int]
     lib.caar_run_rk5.argtypes = [C.c_void_p, C.POINTER(Control), C.c_double, C.c_int, C.c_int]
+    lib.caar_rk5_stage.argtypes = [C.c_void_p, C.POINTER(Control), C.c_double, C.c_int, C.c_int, C.POINTER(C.c_int)]
     lib.caar_update_time_levels.argtypes = [C.POINTER(Control)]
     lib.caar_update_time_levels.restype = None
     lib.caar_extra_count.restype = C.c_size_t
@@ -155,6 +156,8 @@ def load_library():
                                        C.c_int, C.c_int]
     lib.caar_dss_pack.argtypes = lib.caar_dss.argtypes
     lib.caar_dss_unpack.argtypes = lib.caar_dss.argtypes
+    lib.caar_dss_interior.argtypes = lib.caar_dss.argtypes
+    lib.caar_dss_boundary.argtypes = lib.caar_dss.argtypes
     lib.caar_neighbor_minmax_pack.argtypes = [C.c_void_p, C.c_int]
     lib.caar_neighbor_minmax_unpack.argtypes = [C.c_void_p, C.c_int]
     lib.caar_halo_segments.argtypes = [C.c_void_p, C.c_int, C.c_uint, C.c_int, C.POINTER(C.c_void_p),
@@ -372,6 +375,20 @@ class Caar:
         if sync:
             self.sync()
 
+    def rk5_stage(self, stage, dt, mode=MODE_FAST, sync=True):
+        """Stage `stage` (0..4) of run_rk5's step on self.control's levels (caar_rk5_stage) -> the level it wrote, which
+        a DSS after the stage assembles; self.control is not rotated (update_time_levels after stage 4)."""
+        tl = C.c_int(-1)
+        _check(self.lib, self.lib.caar_rk5_stage(self.h, C.byref(self.control), float(dt), int(stage), mode,
+                                                 C.byref(tl)), "caar_rk5_stage")
+        if sync:
+            self.sync()
+        return tl.value
+
+    def update_time_levels(self):
+        """caar_update_time_levels on self.control."""
+        self.lib.caar_update_time_levels(C.byref(self.control))
+
     # -- the step after CAAR: tracer advection RHS (LV/EulerStepFunctor.hpp:33-66) ------------------------
     def upload_vstar(self, vstar):
         E, L, Q, _ = self.shape_args
@@ -501,6 +518,14 @@ class Caar:
     def dss_unpack(self, names, tl=None, qtl=0, qsize=0, weighting=DSS_ASSEMBLE, sync=True):
         """caar_dss_unpack: the whole DSS of the handle in place, remote copies from the receive buffer."""
         self._dss_call(self.lib.caar_dss_unpack, "caar_dss_unpack", names, tl, qtl, qsize, weighting, sync)
+
+    def dss_interior(self, names, tl=None, qtl=0, qsize=0, weighting=DSS_ASSEMBLE, sync=True):
+        """caar_dss_interior: the points whose copies are all on this handle; reads neither exchange buffer."""
+        self._dss_call(self.lib.caar_dss_interior, "caar_dss_interior", names, tl, qtl, qsize, weighting, sync)
+
+    def dss_boundary(self, names, tl=None, qtl=0, qsize=0, weighting=DSS_ASSEMBLE, sync=True):
+        """caar_dss_boundary: the points with a copy on another part, remote copies from the receive buffer."""
+        self._dss_call(self.lib.caar_dss_boundary, "caar_dss_boundary", names, tl, qtl, qsize, weighting, sync)
 
     def neighbor_minmax_pack(self, qsize, sync=True):
         _check(self.lib, self.lib.caar_neighbor_minmax_pack(self.h, int(qsize)), "caar_neighbor_minmax_pack")

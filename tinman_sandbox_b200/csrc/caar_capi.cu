@@ -169,7 +169,7 @@ void free_dss_tables(const caar::DssTables& t) {
     if (p) cudaFree(p);
 }
 void free_halo_tables(const caar::HaloTables& t) {
-  for (int* p : {t.start, t.copy, t.nb_start, t.nb, t.send_copy, t.send_el})
+  for (int* p : {t.start, t.copy, t.nb_start, t.nb, t.send_copy, t.send_el, t.istart, t.icopy, t.bstart, t.bcopy})
     if (p) cudaFree(p);
   for (int2* p : {t.send_seg, t.recv_seg})
     if (p) cudaFree(p);
@@ -585,14 +585,49 @@ int caar_run(caar_handle h, const caar_control* ctl, int nsteps, int mode) {
 
 namespace {
 
-// The checks and the step loop of caar_run_rk5 and caar_run_rk5_dss; with `dss`, caar_dss of v, T and dp3d at the
-// stage's np1 follows every stage
-int run_rk5(caar_handle h, caar_control* ctl, double dt, int nsteps, int mode, bool dss, const char* who) {
-  bool fast = false;
-  if (int rc = check_run(h, ctl, nsteps, mode, who, &fast)) return rc;
+// The checks of caar_run_rk5, caar_run_rk5_dss and caar_rk5_stage
+int check_rk5(caar_handle h, const caar_control* ctl, int nsteps, int mode, const char* who, bool* fast) {
+  if (int rc = check_run(h, ctl, nsteps, mode, who, fast)) return rc;
   if (ctl->n0 == ctl->np1 || ctl->n0 == ctl->nm1 || ctl->np1 == ctl->nm1)  // stage 1 would overwrite u0
     return fail(CAAR_ERR_INVALID, "%s needs pairwise distinct time levels (n0=%d np1=%d nm1=%d)", who, ctl->n0,
                 ctl->np1, ctl->nm1);
+  return CAAR_OK;
+}
+
+// Stage k of one RK5 step on the levels of *ctl (not rotated), the combination first for k == 4; with `dss`, caar_dss
+// of v, T and dp3d at the stage's np1 follows. *tl = that np1. The caller holds the device.
+int rk5_stage(caar_handle h, const caar_control* ctl, double dt, int k, bool fast, bool dss, int* tl) {
+  const int n0 = ctl->n0, np1 = ctl->np1, nm1 = ctl->nm1;
+  const double w = h->c.eta_ave_w;
+  // prim_advance_exp, tstep_type == 5: {n0, np1, nm1, dt2, eta_ave_w} of the five compute_and_apply_rhs calls
+  const struct { int n0, np1, nm1; double dt2, eta_ave_w; } stage[5] = {
+      {n0, nm1, n0, dt / 5, w / 4},          {nm1, np1, n0, dt / 5, 0.0},          {np1, np1, n0, dt / 3, 0.0},
+      {np1, np1, n0, (2 * dt) / 3, 0.0},     {np1, np1, nm1, (3 * dt) / 4, (3 * w) / 4}};
+  *tl = stage[k].np1;
+  if (ctl->nete == ctl->nets) return CAAR_OK;
+  if (k == 4) {  // u(nm1) = (5 u1 - u0)/4
+    CU_TRY(caar::launch_rk5_combine(make_args(h, ctl), ctl->nets, ctl->nete, nm1, n0, h->stream));
+    ++h->launches;
+  }
+  caar::KernelArgs a = make_args(h, ctl);
+  a.n0 = stage[k].n0;
+  a.np1 = stage[k].np1;
+  a.nm1 = stage[k].nm1;
+  a.dt2 = stage[k].dt2;
+  a.eta_ave_w = stage[k].eta_ave_w;
+  if (int rc = launch_rhs(h, a, 1, fast)) return rc;
+  if (dss) {
+    CU_TRY(caar::launch_dss(a, h->dss, CAAR_F_V | CAAR_F_T | CAAR_F_DP3D, stage[k].np1, 0, 0, CAAR_DSS_ASSEMBLE,
+                            h->stream));
+    ++h->launches;
+  }
+  return CAAR_OK;
+}
+
+// The checks and the step loop of caar_run_rk5 and caar_run_rk5_dss
+int run_rk5(caar_handle h, caar_control* ctl, double dt, int nsteps, int mode, bool dss, const char* who) {
+  bool fast = false;
+  if (int rc = check_rk5(h, ctl, nsteps, mode, who, &fast)) return rc;
   if (dss) {
     if (int rc = check_connected(h, who)) return rc;
     if (ctl->nets != 0 || ctl->nete != h->dims.nelem)
@@ -600,31 +635,10 @@ int run_rk5(caar_handle h, caar_control* ctl, double dt, int nsteps, int mode, b
                   ctl->nete, h->dims.nelem);
   }
   DeviceGuard guard(h->device);
-  const double w = h->c.eta_ave_w;
   for (int s = 0; s < nsteps; ++s) {
-    const int n0 = ctl->n0, np1 = ctl->np1, nm1 = ctl->nm1;
-    // prim_advance_exp, tstep_type == 5: {n0, np1, nm1, dt2, eta_ave_w} of the five compute_and_apply_rhs calls
-    const struct { int n0, np1, nm1; double dt2, eta_ave_w; } stage[5] = {
-        {n0, nm1, n0, dt / 5, w / 4},          {nm1, np1, n0, dt / 5, 0.0},          {np1, np1, n0, dt / 3, 0.0},
-        {np1, np1, n0, (2 * dt) / 3, 0.0},     {np1, np1, nm1, (3 * dt) / 4, (3 * w) / 4}};
-    for (int k = 0; k < 5 && ctl->nete > ctl->nets; ++k) {
-      if (k == 4) {  // u(nm1) = (5 u1 - u0)/4
-        CU_TRY(caar::launch_rk5_combine(make_args(h, ctl), ctl->nets, ctl->nete, nm1, n0, h->stream));
-        ++h->launches;
-      }
-      caar::KernelArgs a = make_args(h, ctl);
-      a.n0 = stage[k].n0;
-      a.np1 = stage[k].np1;
-      a.nm1 = stage[k].nm1;
-      a.dt2 = stage[k].dt2;
-      a.eta_ave_w = stage[k].eta_ave_w;
-      if (int rc = launch_rhs(h, a, 1, fast)) return rc;
-      if (dss) {
-        CU_TRY(caar::launch_dss(a, h->dss, CAAR_F_V | CAAR_F_T | CAAR_F_DP3D, stage[k].np1, 0, 0, CAAR_DSS_ASSEMBLE,
-                                h->stream));
-        ++h->launches;
-      }
-    }
+    int tl = 0;
+    for (int k = 0; k < 5; ++k)
+      if (int rc = rk5_stage(h, ctl, dt, k, fast, dss, &tl)) return rc;
     caar_update_time_levels(ctl);
   }
   return CAAR_OK;
@@ -638,6 +652,18 @@ int caar_run_rk5(caar_handle h, caar_control* ctl, double dt, int nsteps, int mo
 
 int caar_run_rk5_dss(caar_handle h, caar_control* ctl, double dt, int nsteps, int mode) {
   return run_rk5(h, ctl, dt, nsteps, mode, true, "caar_run_rk5_dss");
+}
+
+int caar_rk5_stage(caar_handle h, const caar_control* ctl, double dt, int stage, int mode, int* tl) {
+  bool fast = false;
+  if (int rc = check_rk5(h, ctl, 1, mode, "caar_rk5_stage", &fast)) return rc;
+  if (stage < 0 || stage >= 5) return fail(CAAR_ERR_INVALID, "stage=%d outside [0,5)", stage);
+  if (!tl) return fail(CAAR_ERR_INVALID, "caar_rk5_stage: null tl");
+  DeviceGuard guard(h->device);
+  int out = 0;
+  if (int rc = rk5_stage(h, ctl, dt, stage, fast, false, &out)) return rc;
+  *tl = out;
+  return CAAR_OK;
 }
 
 // ---- caar_run_host: one RHS evaluation on HOST arrays, pipelined over element chunks --------------------
@@ -1108,6 +1134,8 @@ int caar_set_partition(caar_handle h, const long long* gid, int nelem_global, co
   x.nrecv = ht.rec[1][nparts];
   x.nsend_el = ht.rec[2][nparts];
   x.nrecv_el = ht.rec[3][nparts];
+  x.ninterior = (int)ht.istart.size() - 1;
+  x.nboundary = (int)ht.bstart.size() - 1;
   x.rec = new (std::nothrow) int[4 * ((size_t)nparts + 1)];
   if (!x.rec) return fail(CAAR_ERR_NOMEM, "host allocation failed");
   for (int k = 0; k < 4; ++k) std::copy(ht.rec[k].begin(), ht.rec[k].end(), x.rec + k * ((size_t)nparts + 1));
@@ -1119,9 +1147,10 @@ int caar_set_partition(caar_handle h, const long long* gid, int nelem_global, co
   const size_t recv_n = std::max((size_t)x.nrecv * nv, (size_t)x.nrecv_el * row);
   DeviceGuard guard(h->device);
   cudaError_t e = upload_dss_tables(lt, &d, h->stream);
-  int** dst[6] = {&x.start, &x.copy, &x.nb_start, &x.nb, &x.send_copy, &x.send_el};
-  const std::vector<int>* src[6] = {&ht.start, &ht.copy, &ht.nb_start, &ht.nb, &ht.send_copy, &ht.send_el};
-  for (int i = 0; i < 6 && e == cudaSuccess; ++i) e = upload_vector(dst[i], *src[i], h->stream);
+  int** dst[10] = {&x.start, &x.copy, &x.nb_start, &x.nb, &x.send_copy, &x.send_el, &x.istart, &x.icopy, &x.bstart, &x.bcopy};
+  const std::vector<int>* src[10] = {&ht.start, &ht.copy, &ht.nb_start, &ht.nb, &ht.send_copy, &ht.send_el,
+                                     &ht.istart, &ht.icopy, &ht.bstart, &ht.bcopy};
+  for (int i = 0; i < 10 && e == cudaSuccess; ++i) e = upload_vector(dst[i], *src[i], h->stream);
   const std::vector<int2> send_seg = record_segments(ht.rec[0]), recv_seg = record_segments(ht.rec[1]);
   if (e == cudaSuccess) e = upload_vector(&x.send_seg, send_seg, h->stream);
   if (e == cudaSuccess) e = upload_vector(&x.recv_seg, recv_seg, h->stream);
@@ -1157,6 +1186,26 @@ int caar_dss_unpack(caar_handle h, unsigned field_mask, int tl, int qtl, int qsi
   if (caar::dss_record_doubles(field_mask, qsize, h->dims.nlev) == 0) return CAAR_OK;
   DeviceGuard guard(h->device);
   CU_TRY(caar::launch_dss_unpack(make_args(h, nullptr), h->halo, field_mask, tl, qtl, qsize, weighting, h->stream));
+  ++h->launches;
+  return CAAR_OK;
+}
+
+int caar_dss_interior(caar_handle h, unsigned field_mask, int tl, int qtl, int qsize, int weighting) {
+  if (int rc = check_partitioned(h, "caar_dss_interior")) return rc;
+  if (int rc = check_dss_args(h, field_mask, tl, qtl, qsize, weighting)) return rc;
+  if (caar::dss_record_doubles(field_mask, qsize, h->dims.nlev) == 0 || h->halo.ninterior == 0) return CAAR_OK;
+  DeviceGuard guard(h->device);
+  CU_TRY(caar::launch_dss_interior(make_args(h, nullptr), h->halo, field_mask, tl, qtl, qsize, weighting, h->stream));
+  ++h->launches;
+  return CAAR_OK;
+}
+
+int caar_dss_boundary(caar_handle h, unsigned field_mask, int tl, int qtl, int qsize, int weighting) {
+  if (int rc = check_partitioned(h, "caar_dss_boundary")) return rc;
+  if (int rc = check_dss_args(h, field_mask, tl, qtl, qsize, weighting)) return rc;
+  if (caar::dss_record_doubles(field_mask, qsize, h->dims.nlev) == 0 || h->halo.nboundary == 0) return CAAR_OK;
+  DeviceGuard guard(h->device);
+  CU_TRY(caar::launch_dss_boundary(make_args(h, nullptr), h->halo, field_mask, tl, qtl, qsize, weighting, h->stream));
   ++h->launches;
   return CAAR_OK;
 }

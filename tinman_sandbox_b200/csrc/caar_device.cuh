@@ -171,15 +171,19 @@ cudaError_t launch_neighbor_minmax(const DssTables& t, int nelem, int qsize_d, i
 //           copy's spheremp, then the selected slices level by level), starting at double rec_start_q * nv.
 //   bounds: nb[nb_start[e] .. nb_start[e+1]) is N(e) in ascending global order, a local element e or nelem + R for row
 //           R of the receive buffer; row R is the [qsize][L][2] bounds of one element at double R * qsize * L * 2.
+//   The local groups split in two CSRs of the same form, each in owner order: interior (istart / icopy: every copy
+//   local) and boundary (bstart / bcopy: at least one remote copy, encoded as in copy). Every copy dss_pack reads is a
+//   boundary copy, so the interior launch may run while the segments are in flight.
 struct HaloHostTables {
   std::vector<int> start, copy, nb_start, nb;
+  std::vector<int> istart, icopy, bstart, bcopy;
   std::vector<int> send_copy, send_el;  // the local copy of every DSS send record, the local element of every row
   // record offsets of the segments, [nparts + 1] each: DSS send, DSS receive, bounds send, bounds receive
   std::vector<int> rec[4];
 };
 struct HaloTables {  // on the device, but for the record offsets
-  int nparts, ngroups, nsend, nrecv, nsend_el, nrecv_el;
-  int *start, *copy, *nb_start, *nb, *send_copy, *send_el;
+  int nparts, ngroups, nsend, nrecv, nsend_el, nrecv_el, ninterior, nboundary;
+  int *start, *copy, *nb_start, *nb, *send_copy, *send_el, *istart, *icopy, *bstart, *bcopy;
   int2 *send_seg, *recv_seg;  // per DSS record: {first record of its segment, records in that segment}
   int* rec;                   // host [4][nparts + 1]: HaloHostTables::rec
   double *send, *recv;        // the exchange buffers
@@ -194,6 +198,12 @@ cudaError_t launch_dss_pack(const KernelArgs& a, const HaloTables& t, unsigned m
                             cudaStream_t s);
 cudaError_t launch_dss_unpack(const KernelArgs& a, const HaloTables& t, unsigned mask, int tl, int qtl, int qsize,
                               int weighting, cudaStream_t s);
+// unpack split in two: the interior groups (dss_kernel on istart / icopy), none when there is none, and the boundary
+// groups (dss_boundary_kernel on bstart / bcopy, reading the receive buffer), none when there is none
+cudaError_t launch_dss_interior(const KernelArgs& a, const HaloTables& t, unsigned mask, int tl, int qtl, int qsize,
+                                int weighting, cudaStream_t s);
+cudaError_t launch_dss_boundary(const KernelArgs& a, const HaloTables& t, unsigned mask, int tl, int qtl, int qsize,
+                                int weighting, cudaStream_t s);
 cudaError_t launch_neighbor_minmax_pack(const HaloTables& t, int qsize_d, int L, int qsize, const double* bounds,
                                         cudaStream_t s);
 cudaError_t launch_neighbor_minmax_unpack(const HaloTables& t, int nelem, int qsize_d, int L, int qsize,

@@ -25,7 +25,9 @@
 // Across partitioned handles (caar_set_partition; tables and buffer layout at HaloHostTables in caar_device.cuh):
 // dss_pack_kernel writes one record per boundary copy for the other parts; dss_unpack_kernel is dss_kernel's walk in
 // which groups with remote copies read those copies from the received records; neighbor_minmax_pack_kernel and
-// neighbor_minmax_unpack_kernel do the same with the bound rows of boundary elements.
+// neighbor_minmax_unpack_kernel do the same with the bound rows of boundary elements. caar_dss_interior runs dss_kernel on
+// the local groups without remote copies; caar_dss_boundary runs dss_boundary_kernel, one thread per (group with a
+// remote copy, slice, batch of levels), on the others.
 #include <algorithm>
 #include <cstring>
 #include <vector>
@@ -306,6 +308,147 @@ __global__ void __launch_bounds__(DSS_THREADS, DSS_CTAS_PER_SM) dss_unpack_kerne
   }
 }
 
+// ---- the boundary groups alone (caar_dss_boundary) ----
+constexpr int BATCH = 4;  // levels per thread of dss_boundary_kernel: 18 batches at nlev 72
+
+// Levels k0 .. k0+BATCH (clipped to L) of one slice of the boundary group copy[c0 .. c0+n): m and r in copy order,
+// then, per level, every copy (local from the field, remote from its record, value v0 + k*W + w) summed in copy order;
+// only the local copies are written. The operations and their order are dss_unpack_kernel's for a group with remote
+// copies, so the bits are too. Groups of up to FAST_COPIES copies load the whole batch before any store.
+template <int W, bool PROJECT>
+__device__ __forceinline__ void boundary_batch(double* base, size_t estride, const DssArgs& A, const HaloArgs& H,
+                                               int c0, int n, int v0, int k0) {
+  const int nk = min(BATCH, A.L - k0);
+  if (n <= FAST_COPIES) {
+    double* p[FAST_COPIES];  // level k0 of the copy
+    int ws[FAST_COPIES];     // doubles between components: 1 for a local copy, its segment's records for a remote one
+    double s[FAST_COPIES];
+    bool loc[FAST_COPIES];
+#pragma unroll
+    for (int c = 0; c < FAST_COPIES; ++c) {
+      const int cp = A.copy[c0 + (c < n ? c : 0)];
+      loc[c] = cp >= 0;
+      if (loc[c]) {
+        p[c] = base + (size_t)(cp >> 4) * estride + (size_t)k0 * 16 * W + (cp & 15) * W;
+        ws[c] = 1;
+        s[c] = A.spheremp[cp];
+      } else {
+        size_t st;
+        double* o = record(H, -1 - cp, &st);
+        p[c] = o + (size_t)(v0 + k0 * W) * st;
+        ws[c] = (int)st;
+        s[c] = o[0];
+      }
+    }
+    double m = s[0];
+#pragma unroll
+    for (int c = 1; c < FAST_COPIES; ++c)
+      if (c < n) m = __dadd_rn(m, s[c]);
+    const double r = __ddiv_rn(1.0, m);
+    constexpr int LV = BATCH / W;  // levels in flight: 4 values of every copy, as in dss_slice
+#pragma unroll 1
+    for (int j0 = 0; j0 < nk; j0 += LV) {
+      double f[LV][FAST_COPIES][W];
+#pragma unroll
+      for (int j = 0; j < LV; ++j)
+#pragma unroll
+        for (int c = 0; c < FAST_COPIES; ++c)
+          if (j0 + j < nk && c < n) {
+            const double* q = p[c] + (size_t)(j0 + j) * (loc[c] ? 16 * W : W * ws[c]);
+            if (loc[c]) {
+              load<W>(q, f[j][c]);
+            } else {
+#pragma unroll
+              for (int w = 0; w < W; ++w) f[j][c][w] = q[(size_t)w * ws[c]];
+            }
+          }
+#pragma unroll
+      for (int j = 0; j < LV; ++j) {
+        if (j0 + j >= nk) break;
+        double out[W];
+#pragma unroll
+        for (int w = 0; w < W; ++w) {
+          double S = PROJECT ? __dmul_rn(s[0], f[j][0][w]) : f[j][0][w];
+#pragma unroll
+          for (int c = 1; c < FAST_COPIES; ++c)
+            if (c < n) S = __dadd_rn(S, PROJECT ? __dmul_rn(s[c], f[j][c][w]) : f[j][c][w]);
+          out[w] = __dmul_rn(S, r);
+        }
+#pragma unroll
+        for (int c = 0; c < FAST_COPIES; ++c)
+          if (c < n && loc[c]) store<W>(p[c] + (size_t)(j0 + j) * 16 * W, out);
+      }
+    }
+    return;
+  }
+  double m = 0.0;
+#pragma unroll 1
+  for (int c = 0; c < n; ++c) {
+    const int cp = A.copy[c0 + c];
+    size_t st;
+    const double s = cp >= 0 ? A.spheremp[cp] : record(H, -1 - cp, &st)[0];
+    m = c == 0 ? s : __dadd_rn(m, s);
+  }
+  const double r = __ddiv_rn(1.0, m);
+#pragma unroll 1
+  for (int k = k0; k < k0 + nk; ++k) {  // dss_slice_halo's level loop over this batch
+    double S[W];
+#pragma unroll 1
+    for (int c = 0; c < n; ++c) {
+      const int cp = A.copy[c0 + c];
+      double f[W], s;
+      if (cp >= 0) {
+        load<W>(base + (size_t)(cp >> 4) * estride + (size_t)k * 16 * W + (cp & 15) * W, f);
+        s = PROJECT ? A.spheremp[cp] : 0.0;
+      } else {
+        size_t st;
+        const double* o = record(H, -1 - cp, &st);
+#pragma unroll
+        for (int w = 0; w < W; ++w) f[w] = o[(size_t)(v0 + k * W + w) * st];
+        s = PROJECT ? o[0] : 0.0;
+      }
+#pragma unroll
+      for (int w = 0; w < W; ++w) {
+        const double t = PROJECT ? __dmul_rn(s, f[w]) : f[w];
+        S[w] = c == 0 ? t : __dadd_rn(S[w], t);
+      }
+    }
+#pragma unroll
+    for (int w = 0; w < W; ++w) S[w] = __dmul_rn(S[w], r);
+#pragma unroll 1
+    for (int c = 0; c < n; ++c) {
+      const int cp = A.copy[c0 + c];
+      if (cp >= 0) store<W>(base + (size_t)(cp >> 4) * estride + (size_t)k * 16 * W + (cp & 15) * W, S);
+    }
+  }
+}
+
+// One thread per (boundary group, selected slice, batch of BATCH levels), the group fastest, so that a warp walks
+// neighbouring points of one element and consecutive records. In place without atomics: every (local copy, slice,
+// level) is read and written by one thread, and the receive buffer is only read.
+template <bool PROJECT>
+__global__ void __launch_bounds__(DSS_THREADS, DSS_CTAS_PER_SM) dss_boundary_kernel(const DssArgs A, const HaloArgs H,
+                                                                                     int nslices) {
+  const int nbatch = (A.L + BATCH - 1) / BATCH;
+  const size_t total = (size_t)A.ngroups * nslices * nbatch;
+  for (size_t i = (size_t)blockIdx.x * DSS_THREADS + threadIdx.x; i < total; i += (size_t)gridDim.x * DSS_THREADS) {
+    const int g = (int)(i % A.ngroups);
+    const size_t rest = i / A.ngroups;
+    const int k0 = (int)(rest % nbatch) * BATCH;
+    int j = (int)(rest / nbatch), run = 0, v0 = 1;  // slice j -> run, slice within the run, first value of its record
+    while (j >= A.count[run]) {
+      v0 += A.count[run] * A.L * A.w[run];
+      j -= A.count[run];
+      ++run;
+    }
+    v0 += j * A.L * A.w[run];
+    double* base = A.base[run] + j * A.step[run];
+    const int c0 = A.start[g], n = A.start[g + 1] - c0;
+    if (A.w[run] == 2) boundary_batch<2, PROJECT>(base, A.estride[run], A, H, c0, n, v0, k0);
+    else boundary_batch<1, PROJECT>(base, A.estride[run], A, H, c0, n, v0, k0);
+  }
+}
+
 // neighbor_minmax of bound pair i; with HALO a neighbour q >= nelem is row q - nelem of rin, rrow pairs apart
 template <bool HALO>
 __device__ __forceinline__ double2 minmax_pair(const double2* __restrict__ in, const int* __restrict__ nb_start,
@@ -503,10 +646,20 @@ void build_halo_tables(const long long* gid, int nelem_global, const int* part_s
   });
   t->start.assign(1, 0);
   t->copy.clear();
+  t->istart.assign(1, 0);
+  t->icopy.clear();
+  t->bstart.assign(1, 0);
+  t->bcopy.clear();
   for (const auto& r : runs) {
+    const size_t g0 = t->copy.size();
     for (size_t i = r.first; i < r.second; ++i)
       t->copy.push_back(is_local(c[i].cp >> 4) ? c[i].cp - e0 * 16 : -1 - rid[i]);
     t->start.push_back((int)t->copy.size());
+    const bool interior = std::all_of(t->copy.begin() + g0, t->copy.end(), [](int cp) { return cp >= 0; });
+    std::vector<int>& st = interior ? t->istart : t->bstart;
+    std::vector<int>& cp = interior ? t->icopy : t->bcopy;
+    cp.insert(cp.end(), t->copy.begin() + g0, t->copy.end());
+    st.push_back((int)cp.size());
   }
   // neighbours: N(el) ascending by global element; a remote one is the row of its element among those received from
   // its part, which are the elements of that part with a neighbour here, ascending
@@ -550,20 +703,58 @@ size_t dss_record_doubles(unsigned mask, int qsize, int L) {
   return 1 + (size_t)per_level * L;
 }
 
-cudaError_t launch_dss(const KernelArgs& a, const DssTables& t, unsigned mask, int tl, int qtl, int qsize,
-                       int weighting, cudaStream_t s) {
+namespace {
+
+// dss_kernel over the groups start / copy: caar_dss, and the interior groups of a partitioned handle
+cudaError_t launch_dss_groups(const KernelArgs& a, const int* start, const int* copy, int ngroups, unsigned mask,
+                              int tl, int qtl, int qsize, int weighting, cudaStream_t s) {
   if (!selected(mask, qsize)) return cudaSuccess;
-  const DssArgs A = dss_args(a, mask, tl, qtl, qsize, t.start, t.copy, t.ngroups);
+  const DssArgs A = dss_args(a, mask, tl, qtl, qsize, start, copy, ngroups);
   static LaunchCache cache[2];
   cudaError_t e = cudaSuccess;
   if (weighting == CAAR_DSS_PROJECT) {
-    const unsigned grid = grid_for(dss_kernel<true>, (size_t)t.ngroups, DSS_CTAS_PER_SM, cache[1], &e);
+    const unsigned grid = grid_for(dss_kernel<true>, (size_t)ngroups, DSS_CTAS_PER_SM, cache[1], &e);
     if (e != cudaSuccess) return e;
     dss_kernel<true><<<grid, DSS_THREADS, 0, s>>>(A);
   } else {
-    const unsigned grid = grid_for(dss_kernel<false>, (size_t)t.ngroups, DSS_CTAS_PER_SM, cache[0], &e);
+    const unsigned grid = grid_for(dss_kernel<false>, (size_t)ngroups, DSS_CTAS_PER_SM, cache[0], &e);
     if (e != cudaSuccess) return e;
     dss_kernel<false><<<grid, DSS_THREADS, 0, s>>>(A);
+  }
+  return cudaGetLastError();
+}
+
+}  // namespace
+
+cudaError_t launch_dss(const KernelArgs& a, const DssTables& t, unsigned mask, int tl, int qtl, int qsize,
+                       int weighting, cudaStream_t s) {
+  return launch_dss_groups(a, t.start, t.copy, t.ngroups, mask, tl, qtl, qsize, weighting, s);
+}
+
+cudaError_t launch_dss_interior(const KernelArgs& a, const HaloTables& t, unsigned mask, int tl, int qtl, int qsize,
+                                int weighting, cudaStream_t s) {
+  if (t.ninterior == 0) return cudaSuccess;
+  return launch_dss_groups(a, t.istart, t.icopy, t.ninterior, mask, tl, qtl, qsize, weighting, s);
+}
+
+cudaError_t launch_dss_boundary(const KernelArgs& a, const HaloTables& t, unsigned mask, int tl, int qtl, int qsize,
+                                int weighting, cudaStream_t s) {
+  if (!selected(mask, qsize) || t.nboundary == 0) return cudaSuccess;
+  const DssArgs A = dss_args(a, mask, tl, qtl, qsize, t.bstart, t.bcopy, t.nboundary);
+  const HaloArgs H{t.recv, t.recv_seg, nullptr, t.nrecv, (int)dss_record_doubles(mask, qsize, a.nlev)};
+  int nslices = 0;
+  for (int r = 0; r < A.nruns; ++r) nslices += A.count[r];
+  const size_t items = (size_t)t.nboundary * nslices * ((a.nlev + BATCH - 1) / BATCH);
+  static LaunchCache cache[2];
+  cudaError_t e = cudaSuccess;
+  if (weighting == CAAR_DSS_PROJECT) {
+    const unsigned grid = grid_for(dss_boundary_kernel<true>, items, 2048 / DSS_THREADS, cache[1], &e);
+    if (e != cudaSuccess) return e;
+    dss_boundary_kernel<true><<<grid, DSS_THREADS, 0, s>>>(A, H, nslices);
+  } else {
+    const unsigned grid = grid_for(dss_boundary_kernel<false>, items, 2048 / DSS_THREADS, cache[0], &e);
+    if (e != cudaSuccess) return e;
+    dss_boundary_kernel<false><<<grid, DSS_THREADS, 0, s>>>(A, H, nslices);
   }
   return cudaGetLastError();
 }

@@ -1,7 +1,8 @@
 #!/usr/bin/env python
 """Times caar_dss, caar_neighbor_minmax and caar_run_rk5_dss on resident data over cubed-sphere connectivity.
     python tools/dss_bench.py [--reps 10] [--parts N]
-With --parts N it times only the exchange across partitioned handles (parts_case below). Otherwise it prints one JSON
+With --parts N it times only the exchange across partitioned handles (parts_case below: pack, copies, unpack,
+interior and boundary alone and summed) and HOMME's RK5 step on N handles of one GPU (parts_rk5_case). Otherwise it prints one JSON
 line per case:
   state DSS (v, T, dp3d; ASSEMBLE) at 86400 x 72 (ne = 120) and 48600 x 128 (ne = 90)
   Qdp DSS (PROJECT) at 86400 x 72 with qsize 4 and 21600 x 72 (ne = 60) with qsize 35
@@ -160,13 +161,21 @@ def parts_case(nparts, reps, peak, info):
         with torch.cuda.stream(stream):
             for dst, src in moves:
                 dst.copy_(src)
+    def split():
+        for h in hs:
+            h.dss_interior(STATE, tl=0, sync=False)
+            h.dss_boundary(STATE, tl=0, sync=False)
     runs = {"pack": lambda: [h.dss_pack(STATE, tl=0, sync=False) for h in hs], "copies": copies,
             "unpack": lambda: [h.dss_unpack(STATE, tl=0, sync=False) for h in hs],
+            "interior": lambda: [h.dss_interior(STATE, tl=0, sync=False) for h in hs],
+            "boundary": lambda: [h.dss_boundary(STATE, tl=0, sync=False) for h in hs],
+            "interior_boundary": split,
             "whole_dss": lambda: whole.dss(STATE, tl=0, sync=False)}
     nv = 1 + 4 * L
     sent = sum(int(s[2][-1]) for s in segs) * 8
     value_bytes = 2 * 4 * E * L * 16 * 8
-    nbytes = {"pack": 2 * sent, "copies": 2 * sent, "unpack": value_bytes + sent, "whole_dss": value_bytes}
+    nbytes = {"pack": 2 * sent, "copies": 2 * sent, "unpack": value_bytes + sent, "interior": value_bytes - 2 * sent,
+              "boundary": 3 * sent, "interior_boundary": value_bytes + sent, "whole_dss": value_bytes}
     for fn in runs.values():
         fn()
     torch.cuda.synchronize()
@@ -189,6 +198,76 @@ def parts_case(nparts, reps, peak, info):
         h.close()
 
 
+def parts_rk5_case(nparts, reps, peak, info):
+    """HOMME's RK5 step on N handles of one GPU holding the blocks of the ne = 120 mesh (86400 x 72, fast mode), per
+    stage: caar_rk5_stage on every part, caar_dss_pack on every part, the segment copies, caar_dss_interior and
+    caar_dss_boundary on every part (partition.run_rk5_dss's sequence with device copies for the transport), against
+    caar_run_rk5_dss on one handle that holds the whole mesh, alternating step by step on one stream. The bytes are
+    rk5_case's step_rk5_dss model."""
+    import torch
+    from tinman_sandbox_b200.partition import element_range
+    ne, L, P = 120, 72, 257
+    E = 6 * ne * ne
+    gid = mesh(ne, "panel")
+    ps = [element_range(p, nparts, E)[0] for p in range(nparts)] + [E]
+    pool = harness.PortOracle().init(P, L)
+    pool.arrays["elem_spheremp"][...] = 1.0
+    stream = torch.cuda.Stream()
+
+    def handle(e0, e1):
+        h = tb.Caar(e1 - e0, L)
+        h.set_params(pool.consts, pool.dvv, pool.ps0, pool.hyai)
+        h.set_control(0, e1 - e0, 0, 1, 2, int(pool.ctl[5]), dt2=pool.dt2)
+        for a0 in range(0, e1 - e0, P):
+            a1 = min(e1 - e0, a0 + P)
+            h.upload_range({n: np.ascontiguousarray(a[:a1 - a0]) for n, a in pool.arrays.items()}, a0, a1)
+        h.set_stream(stream.cuda_stream)
+        return h
+    whole = handle(0, E)
+    whole.set_connectivity(gid)
+    hs = []
+    for p in range(nparts):
+        h = handle(ps[p], ps[p + 1])
+        h.set_partition(gid, ps, p)
+        hs.append(h)
+    segs = [h.halo_segments(tb.HALO_DSS, STATE, 0) for h in hs]
+    moves = [(segs[q][1][segs[q][3][p]:segs[q][3][p + 1]], segs[p][0][segs[p][2][q]:segs[p][2][q + 1]])
+             for q in range(nparts) for p in range(nparts) if segs[q][3][p + 1] > segs[q][3][p]]
+
+    def step():
+        for k in range(5):
+            tls = [h.rk5_stage(k, 1.0, tb.MODE_FAST, sync=False) for h in hs]
+            for h, tl in zip(hs, tls):
+                h.dss_pack(STATE, tl=tl, sync=False)
+            with torch.cuda.stream(stream):
+                for dst, src in moves:
+                    dst.copy_(src)
+            for h, tl in zip(hs, tls):
+                h.dss_interior(STATE, tl=tl, sync=False)
+            for h, tl in zip(hs, tls):
+                h.dss_boundary(STATE, tl=tl, sync=False)
+        for h in hs:
+            h.update_time_levels()
+    runs = {"parts": step, "whole": lambda: whole.run_rk5_dss(1, 1.0, tb.MODE_FAST, sync=False)}
+    for fn in runs.values():
+        fn()
+    torch.cuda.synchronize()
+    ms = {k: [] for k in runs}
+    for _ in range(reps):
+        for k, fn in runs.items():
+            a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            a.record(stream)
+            fn()
+            b.record(stream)
+            b.synchronize()
+            ms[k].append(a.elapsed_time(b))
+    for k in runs:
+        report(f"parts{nparts}_step_rk5_dss_{k}", "panel", E, L, 122.5e9, min(ms[k]), float(np.median(ms[k])), None,
+               peak, info)
+    for h in hs + [whole]:
+        h.close()
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reps", type=int, default=10)
@@ -198,6 +277,7 @@ def main():
     peak = copy_peak_gbps()
     if args.parts:
         parts_case(args.parts, args.reps, peak, info)
+        parts_rk5_case(args.parts, max(3, args.reps // 2), peak, info)
         return
     dss_cases(args.reps, peak, info)
     rk5_case(max(3, args.reps // 2), peak, info)
