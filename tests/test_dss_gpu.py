@@ -1,6 +1,7 @@
 """caar_set_connectivity, caar_dss, caar_neighbor_minmax and caar_run_rk5_dss on the GPU, bit for bit against
 tests/dss_oracle.py: cubed spheres (permuted, with rotated element blocks) and random meshes with up to 8 copies per
-point, at nlev 72, 30 and 128, every field alone and all together, both weightings, every tl, both qtl, qsize < qsize_d,
+point, at nlev 72, 30 and 128 and at 2, 3, 5, 7, 26, 80, 127 and 131 (every residue of the level batches' tails), every
+field alone and all together, both weightings, every tl, both qtl, qsize < qsize_d,
 with every value outside the selection compared by bits; a size where the walk over the groups wraps; the full ne = 120
 mesh; the five-call limited tracer step; the RK5 step with a DSS after every stage; argument errors, launch counts,
 connectivity input and run-to-run bits."""
@@ -61,7 +62,11 @@ MESHES = {
     "cube5": lambda rng: do.cubed_sphere_gid(5, rng),
     "random8": lambda rng: do.random_gid(40, rng, 8),
 }
-CASES = [("cube2", 72), ("cube3", 30), ("cube5", 128), ("random8", 72), ("random8", 30), ("cube3", 72)]
+# nlev 72, 30, 128, then the tails of dss_slice's level batches (2 levels of v, 4 of a scalar): L % 4 = 0, 1, 2, 3 and a
+# single partial batch, on groups of up to 4 copies (cube*) and of up to 8 (random8)
+CASES = [("cube2", 72), ("cube3", 30), ("cube5", 128), ("random8", 72), ("random8", 30), ("cube3", 72),
+         ("cube2", 2), ("random8", 3), ("cube3", 5), ("random8", 7), ("cube2", 26), ("cube3", 80), ("random8", 80),
+         ("cube5", 127), ("random8", 131), ("cube2", 131)]
 SELECTIONS = [(n,) for n in ALL4] + [ALL4]
 
 
@@ -166,13 +171,17 @@ def test_full_size_ne120():
 
 # ---- neighbor_minmax ------------------------------------------------------------------------------------------------
 
-@pytest.mark.parametrize("mesh", ["cube3", "random8"])
-def test_neighbor_minmax_equals_oracle(mesh):
-    """Random bounds [E][4][30][2], qsize 3: bit for bit with the numpy transcription, tracer 3 untouched; a second call
+MINMAX_CASES = [("cube3", 30), ("random8", 30), ("cube3", 3), ("random8", 5), ("cube2", 80), ("random8", 127),
+                ("cube3", 131)]
+
+
+@pytest.mark.parametrize("mesh,L", MINMAX_CASES, ids=[m if L == 30 else f"{m}-L{L}" for m, L in MINMAX_CASES])
+def test_neighbor_minmax_equals_oracle(mesh, L):
+    """Random bounds [E][4][L][2], qsize 3: bit for bit with the numpy transcription, tracer 3 untouched; a second call
     widens again from the first call's output."""
     rng = np.random.default_rng(7)
     gid = MESHES[mesh](rng)
-    E, L, Qd = gid.shape[0], 30, 4
+    E, Qd = gid.shape[0], 4
     conn = do.Connectivity(gid)
     b = np.ascontiguousarray(np.sort(rng.standard_normal((E, Qd, L, 2)), -1))
     h = tb.Caar(E, L, Qd)
@@ -256,12 +265,16 @@ def rk5_state(L, seed):
     return s, gid
 
 
-@pytest.mark.parametrize("eulerian", [False, True], ids=["lagrangian", "eulerian"])
-def test_rk5_dss_strict_bit_identical(eulerian):
-    """Strict mode, 2 steps on a permuted ne = 3 sphere: every array equal to rk5_dss_step in every bit, 11 launches per
-    step, levels rotated twice."""
-    s, gid = rk5_state(72, 31 + eulerian)
-    hybi = np.linspace(0.0, 1.0, 73) ** 1.5 if eulerian else None
+RK5_DSS_CASES = [(False, 72), (True, 72), (False, 5), (True, 5), (False, 127), (True, 127)]
+
+
+@pytest.mark.parametrize("eulerian,L", RK5_DSS_CASES,
+                         ids=[("eulerian" if e else "lagrangian") + ("" if L == 72 else f"-L{L}") for e, L in RK5_DSS_CASES])
+def test_rk5_dss_strict_bit_identical(eulerian, L):
+    """Strict mode, 2 steps on a permuted ne = 3 sphere at nlev 72, 5 and 127: every array equal to rk5_dss_step in every
+    bit, 11 launches per step, levels rotated twice."""
+    s, gid = rk5_state(L, 31 + eulerian + (L != 72) * L)
+    hybi = np.linspace(0.0, 1.0, L + 1) ** 1.5 if eulerian else None
     want = s.copy()
     conn = do.Connectivity(gid)
     for _ in range(2):

@@ -1,7 +1,9 @@
 """caar_set_partition, caar_dss_pack / caar_dss_unpack, caar_neighbor_minmax_pack / caar_neighbor_minmax_unpack and
 caar_halo_segments on the GPU: N handles on one device hold the blocks of a mesh, and torch copies move the segments
 between them. The assembled fields of every handle equal, bit for bit, one whole-mesh handle's caar_dss and the oracle,
-with every value outside the selection unchanged and the receive buffers NaN outside the moved segments; ne = 60 in 4
+at nlev 72, 30, 128 and at 2, 3, 5, 7, 26, 80, 127 and 131, with every value outside the selection unchanged and both
+exchange buffers NaN wherever the current call does not write them (the whole send buffer before every pack, the whole
+receive buffer outside the moved segments); ne = 60 in 4
 parts and ne = 120 in 8 parts; neighbor_minmax with -0.0 / +0.0; the limited tracer step run partitioned; nparts == 1;
 argument errors, launch counts and pairwise segment sizes."""
 import ctypes as C
@@ -61,13 +63,30 @@ def download_parts(hs, ps, E, L, Qd, ntl, names):
     return out
 
 
+def whole_buffers(h):
+    """(send, recv): views of the whole of a handle's two exchange buffers, which are sized for the largest selection of
+    either exchange"""
+    Qd = h.shape_args[2]
+    segs = [h.halo_segments(op, names, Qd) for op, names in ((tb.HALO_DSS, ALL4), (tb.HALO_MINMAX, ()))]
+    return tuple(max((s[i] for s in segs), key=lambda t: t.numel()) for i in (0, 1))
+
+
+def nan_fill(hs, which):
+    """a NaN bit pattern over the whole send (0) or receive (1) buffer of every handle: a record a pack leaves
+    unwritten, or a read outside the current selection's segments, is then a NaN in a compared value, not a stale
+    record of an earlier call"""
+    import torch
+    for h in hs:
+        whole_buffers(h)[which].view(torch.int64).fill_(0x7FF8DEADBEEF0001)
+    torch.cuda.synchronize()       # the handles run on streams of their own
+
+
 def move_segments(hs, op, names, qsize):
-    """segment p->q of part p's send buffer to segment p of part q's receive buffer, each receive buffer NaN first;
-    checks that the segment sizes agree pairwise"""
+    """segment p->q of part p's send buffer to segment p of part q's receive buffer, each whole receive buffer NaN
+    first; checks that the segment sizes agree pairwise"""
     import torch
     segs = [h.halo_segments(op, names, qsize) for h in hs]
-    for _, recv, _, _ in segs:
-        recv.fill_(float("nan"))
+    nan_fill(hs, 1)
     for q, (_, recv, _, ro) in enumerate(segs):
         for p, (send, _, so_, _) in enumerate(segs):
             assert so_[q + 1] - so_[q] == ro[p + 1] - ro[p], (p, q)
@@ -79,6 +98,7 @@ def move_segments(hs, op, names, qsize):
 
 
 def exchange_dss(hs, names, tl=0, qtl=0, qsize=0, weighting=tb.DSS_ASSEMBLE):
+    nan_fill(hs, 0)
     for h in hs:
         h.dss_pack(names, tl=tl, qtl=qtl, qsize=qsize, weighting=weighting)
     move_segments(hs, tb.HALO_DSS, names, qsize)
@@ -87,6 +107,7 @@ def exchange_dss(hs, names, tl=0, qtl=0, qsize=0, weighting=tb.DSS_ASSEMBLE):
 
 
 def exchange_minmax(hs, qsize):
+    nan_fill(hs, 0)
     for h in hs:
         h.neighbor_minmax_pack(qsize)
     move_segments(hs, tb.HALO_MINMAX, (), qsize)
@@ -106,9 +127,14 @@ MESHES = {
     "cube5": lambda rng: do.cubed_sphere_gid(5, rng),
     "random8": isolated_random,
 }
-# mesh, nlev, partition: a number of random blocks (the first of one element), or part_start itself
+# mesh, nlev, partition: a number of random blocks (the first of one element), or part_start itself. After nlev 72, 30
+# and 128, the tails of the level batches: L % 4 = 0, 1, 2, 3 and L < 4 (dss_slice, dss_pack_kernel and
+# dss_boundary_kernel's last batch), on groups of up to 4 copies (cube*) and more (random8), with one-element parts
 CASES = [("cube2", 72, 3), ("cube2", 30, [0, 1, 8, 9, 16, 17, 24]), ("cube3", 30, 7), ("cube5", 128, 2),
-         ("random8", 72, [0, 1, 39, 40]), ("random8", 30, 3), ("cube3", 72, 1)]
+         ("random8", 72, [0, 1, 39, 40]), ("random8", 30, 3), ("cube3", 72, 1),
+         ("cube2", 2, 3), ("random8", 3, [0, 1, 39, 40]), ("cube3", 5, 7), ("cube2", 7, [0, 1, 8, 9, 16, 17, 24]),
+         ("random8", 7, 3), ("random8", 26, 4), ("cube3", 80, 4), ("cube5", 127, 3), ("random8", 131, [0, 1, 39, 40]),
+         ("cube2", 131, 2)]
 SELECTIONS = [(n,) for n in ALL4] + [ALL4]
 
 
@@ -180,13 +206,19 @@ def test_large_meshes(ne, nparts):
         h.close()
 
 
-@pytest.mark.parametrize("mesh,parts", [("cube3", 7), ("random8", [0, 1, 39, 40]), ("cube2", 1)])
-def test_partitioned_neighbor_minmax(mesh, parts):
+MINMAX_CASES = [("cube3", 7, 30), ("random8", [0, 1, 39, 40], 30), ("cube2", 1, 30), ("cube3", 7, 3),
+                ("random8", [0, 1, 39, 40], 5), ("cube2", 3, 80), ("random8", 3, 127), ("cube5", 4, 131)]
+
+
+@pytest.mark.parametrize("mesh,parts,L", MINMAX_CASES,
+                         ids=[f"{m}-{p if isinstance(p, int) else 'parts1'}" + ("" if L == 30 else f"-L{L}")
+                              for m, p, L in MINMAX_CASES])
+def test_partitioned_neighbor_minmax(mesh, parts, L):
     """Random bounds with -0.0 and +0.0 side by side, qsize 3 of 4 then 1: the parts equal the whole-mesh
     caar_neighbor_minmax and the oracle bit for bit; tracer 3 untouched."""
     rng = np.random.default_rng(21)
     gid = MESHES[mesh](rng)
-    E, L, Qd = gid.shape[0], 30, 4
+    E, Qd = gid.shape[0], 4
     ps = np.array(parts, dtype=np.int32) if not isinstance(parts, int) else dpo.block_partition(E, parts, rng)
     conn = do.Connectivity(gid)
     b = np.sort(rng.standard_normal((E, Qd, L, 2)), -1)
@@ -314,31 +346,38 @@ def test_one_part_and_local_meaning_kept():
 
 def test_segments_are_the_selection():
     """Segment sizes: DSS records of 1 + (fields' values per level) * L doubles, bounds rows of qsize * L * 2; equal
-    pairwise across parts; the receive segments of a part sum to the records it reads."""
+    pairwise across parts; the receive segments of a part sum to the records it reads. At nlev 16 with qsize_d 3, and at
+    nlev 127 with qsize_d 35, where the record of every field and tracer (1 + 39 * 127 doubles) is odd and the largest
+    the buffers are sized for."""
     rng = np.random.default_rng(41)
     gid = do.cubed_sphere_gid(2, rng)
-    E, L, Qd = 24, 16, 3
     ps = np.array([0, 5, 11, 24], dtype=np.int32)
-    hs = []
-    for p in range(3):
-        h = tb.Caar(int(ps[p + 1] - ps[p]), L, Qd, 2)
-        h.set_partition(gid, ps, p)
-        hs.append(h)
     parts = [dpo.Part(gid, ps, p) for p in range(3)]
-    for names, qs, per in ((("elem_state_T",), 0, 1), (("elem_state_v",), 0, 2), (ALL4, 2, 6), (ALL4, 3, 7),
-                           (("elem_state_Qdp",), 0, 0)):
-        for h, pt in zip(hs, parts):
-            _, _, so_, ro = h.halo_segments(tb.HALO_DSS, names, qs)
-            nv = 1 + per * L if per else 0
-            assert list(np.diff(so_)) == [len(x) * nv for x in pt.send]
-            assert list(np.diff(ro)) == [len(x) * nv for x in pt.recv]
-    for qs in (1, 3):
-        for h, pt in zip(hs, parts):
-            _, _, so_, ro = h.halo_segments(tb.HALO_MINMAX, (), qs)
-            assert list(np.diff(so_)) == [len(x) * qs * L * 2 for x in pt.send_el]
-            assert list(np.diff(ro)) == [len(x) * qs * L * 2 for x in pt.recv_el]
-    for h in hs:
-        h.close()
+    for L, Qd in ((16, 3), (127, 35)):
+        hs = []
+        for p in range(3):
+            h = tb.Caar(int(ps[p + 1] - ps[p]), L, Qd, 2)
+            h.set_partition(gid, ps, p)
+            hs.append(h)
+        for names, qs, per in ((("elem_state_T",), 0, 1), (("elem_state_v",), 0, 2), (ALL4, 2, 6), (ALL4, 3, 7),
+                               (("elem_state_Qdp",), 0, 0), (ALL4, Qd, 4 + Qd)):
+            for h, pt in zip(hs, parts):
+                _, _, so_, ro = h.halo_segments(tb.HALO_DSS, names, qs)
+                nv = 1 + per * L if per else 0
+                assert list(np.diff(so_)) == [len(x) * nv for x in pt.send], (L, names, qs)
+                assert list(np.diff(ro)) == [len(x) * nv for x in pt.recv], (L, names, qs)
+        for qs in (1, 3, Qd):
+            for h, pt in zip(hs, parts):
+                _, _, so_, ro = h.halo_segments(tb.HALO_MINMAX, (), qs)
+                assert list(np.diff(so_)) == [len(x) * qs * L * 2 for x in pt.send_el], (L, qs)
+                assert list(np.diff(ro)) == [len(x) * qs * L * 2 for x in pt.recv_el], (L, qs)
+        for h, pt in zip(hs, parts):      # what nan_fill covers: the largest selection of either exchange
+            nv, row = 1 + (4 + Qd) * L, Qd * L * 2
+            send, recv = whole_buffers(h)
+            assert send.numel() == max(sum(map(len, pt.send)) * nv, sum(map(len, pt.send_el)) * row), L
+            assert recv.numel() == max(sum(map(len, pt.recv)) * nv, sum(map(len, pt.recv_el)) * row), L
+        for h in hs:
+            h.close()
 
 
 # ---- argument errors and launch counts ------------------------------------------------------------------------------

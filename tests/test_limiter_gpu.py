@@ -1,5 +1,6 @@
 """caar_tracer_bounds and caar_limit_tracers (HOMME's quasi-monotone limiter, limiter_option 8) on the GPU, bit for bit
-against the numpy transcription of tests/limiter_oracle.py: at nlev 72, 30 and 128, qsize < qsize_d, sub-ranges, both
+against the numpy transcription of tests/limiter_oracle.py: at nlev 72, 30, 128, 5, 80 and 127, qsize < qsize_d and
+qsize = qsize_d = 35, sub-ranges, both
 qtl, dp_tl != qtl and a size where every warp walks many tiles, with sentinels wherever the calls must not write;
 after a strict and a fast caar_advect_tracers step; at 86400 x 72 on a sample of elements, with the whole output
 bounded and conserving mass; plus argument checks, launch counts and run-to-run bits."""
@@ -99,6 +100,10 @@ CASES = [
     dict(E=24, L=72, Qd=2, qsize=1, range=(4, 6), qtl=1, dp_tl=1, seed=4),
     # 2990 x 4 x 72 problems: 26910 tiles of 32, about 11 per warp of one resident wave
     dict(E=3000, L=72, Qd=5, qsize=4, range=(5, 2995), qtl=1, dp_tl=0, seed=5),
+    # odd and E3SM v3 level counts; 35 of 35 tracers: no tracer outside the selection and the longest bounds rows
+    dict(E=35, L=5, Qd=3, qsize=2, range=(2, 34), qtl=1, dp_tl=2, seed=6),
+    dict(E=36, L=80, Qd=4, qsize=3, range=(1, 35), qtl=0, dp_tl=1, seed=7),
+    dict(E=9, L=127, Qd=35, qsize=35, range=(0, 9), qtl=1, dp_tl=0, seed=8),
 ]
 
 

@@ -1,8 +1,9 @@
 """caar_rk5_stage, caar_dss_interior and caar_dss_boundary on the GPU, bit for bit: the five public stages compose to
-caar_run_rk5 and, with caar_dss after each, to caar_run_rk5_dss (strict and fast, Lagrangian and Eulerian, nlev 72 and
-30, 2 steps); interior + boundary in either order, and interior queued before pack, equal caar_dss_unpack and the
-whole-mesh caar_dss for every selection; several handles on one GPU step HOMME's RK5 step with the split DSS and equal
-one whole-mesh caar_run_rk5_dss; ne = 120 in 8 parts; rejected calls; and two ranks over NCCL
+caar_run_rk5 and, with caar_dss after each, to caar_run_rk5_dss (strict and fast, Lagrangian and Eulerian, nlev 72, 30,
+5, 80 and 127, 2 steps); interior + boundary in either order, and interior queued before pack, equal caar_dss_unpack and
+the whole-mesh caar_dss for every selection, at the level counts of tests/test_dss_partition_gpu.py's CASES; several
+handles on one GPU step HOMME's RK5 step with the split DSS and equal one whole-mesh caar_run_rk5_dss (nlev 72, 80, 127
+and 5); ne = 120 in 8 parts; rejected calls; and two ranks over NCCL
 (partition.run_rk5_dss)."""
 import ctypes as C
 import os
@@ -19,7 +20,7 @@ import dss_partition_oracle as dpo
 import rk5_partition_oracle as rpo
 from oracle import harness
 from test_dss_partition_gpu import (ALL4, CASES, MESHES, SEL_NAMES, SELECTIONS, download_parts, move_segments,
-                                    part_handles, random_fields, upload_parts)
+                                    nan_fill, part_handles, random_fields, upload_parts)
 
 pytestmark = pytest.mark.gpu
 INVALID, STATE_ERR = 1, 5
@@ -62,7 +63,7 @@ def download_all(h, s, E):
 
 @pytest.mark.parametrize("mode", [tb.MODE_STRICT, tb.MODE_FAST], ids=["strict", "fast"])
 @pytest.mark.parametrize("eulerian", [False, True], ids=["lagrangian", "eulerian"])
-@pytest.mark.parametrize("L", [72, 30])
+@pytest.mark.parametrize("L", [72, 30, 5, 80, 127])
 def test_stages_compose_to_run_rk5_and_run_rk5_dss(mode, eulerian, L):
     """2 steps: stages 0..4 + update_time_levels equal caar_run_rk5, and with caar_dss(V|T|DP3D, *tl) after every
     stage equal caar_run_rk5_dss, in every bit of every array; 1, 1, 1, 1, 2 launches; *tl = nm1, np1, np1, np1, np1."""
@@ -97,6 +98,7 @@ def split_dss(hs, names, tl, qtl, qs, w, order):
     if order == "interior_before_pack":
         for h in hs:
             h.dss_interior(names, tl=tl, qtl=qtl, qsize=qs, weighting=w)
+    nan_fill(hs, 0)
     for h in hs:
         h.dss_pack(names, tl=tl, qtl=qtl, qsize=qs, weighting=w)
     move_segments(hs, tb.HALO_DSS, names, qs)
@@ -136,6 +138,7 @@ def test_interior_and_boundary_equal_unpack(mesh, L, parts):
             ref = {n: np.empty(tb.field_shape(n, E, L, Qd, ntl)) for n in ALL4}
             whole.download(ref, names=ALL4)
             upload_parts(us, ps, inp, ALL4)
+            nan_fill(us, 0)
             for h in us:
                 h.dss_pack(names, tl=tl, qtl=qtl, qsize=qs, weighting=w)
             move_segments(us, tb.HALO_DSS, names, qs)
@@ -172,6 +175,7 @@ def step_parts(hs, nsteps, dt, mode):
     for _ in range(nsteps):
         for k in range(5):
             tls = [h.rk5_stage(k, dt, mode, sync=False) for h in hs]
+            nan_fill(hs, 0)
             for h, tl in zip(hs, tls):
                 h.dss_pack(STATE, tl=tl)
             move_segments(hs, tb.HALO_DSS, STATE, 0)
@@ -182,12 +186,18 @@ def step_parts(hs, nsteps, dt, mode):
             h.update_time_levels()
 
 
-@pytest.mark.parametrize("ne,nparts,mode", [(4, 3, tb.MODE_STRICT), (4, 3, tb.MODE_FAST), (30, 4, tb.MODE_FAST)],
-                         ids=["ne4-3-strict", "ne4-3-fast", "ne30-4-fast"])
-def test_partitioned_rk5_step_equals_whole_mesh(ne, nparts, mode):
+STEP_CASES = [(4, 3, tb.MODE_STRICT, 72), (4, 3, tb.MODE_FAST, 72), (30, 4, tb.MODE_FAST, 72),
+              (4, 3, tb.MODE_FAST, 80), (4, 3, tb.MODE_STRICT, 127), (4, 3, tb.MODE_STRICT, 5)]
+
+
+@pytest.mark.parametrize("ne,nparts,mode,L", STEP_CASES,
+                         ids=[f"ne{ne}-{n}-{'strict' if m == tb.MODE_STRICT else 'fast'}" + ("" if L == 72 else f"-L{L}")
+                              for ne, n, m, L in STEP_CASES])
+def test_partitioned_rk5_step_equals_whole_mesh(ne, nparts, mode, L):
     """2 RK5 steps with the split DSS after every stage on nparts handles of one GPU equal one whole-mesh
-    caar_run_rk5_dss in every bit of every array (ne = 4 permuted with a one-element block; ne = 30 in even blocks)."""
-    s, gid = rk5_state(ne, 72, 70 + ne)
+    caar_run_rk5_dss in every bit of every array (ne = 4 permuted with a one-element block; ne = 30 in even blocks), at
+    nlev 72, 80, 127 and 5."""
+    s, gid = rk5_state(ne, L, 70 + ne + (L != 72) * L)
     E = s.nelem
     rng = np.random.default_rng(ne)
     ps = dpo.block_partition(E, nparts, rng) if ne == 4 else \
