@@ -72,7 +72,8 @@ module caar_b200
             caar_bounds_upload, caar_bounds_download, caar_sphere_wk, caar_extra_upload, caar_extra_download, caar_last_error, &
             caar_host_register, caar_host_unregister, caar_describe, caar_set_connectivity, caar_dss, caar_neighbor_minmax, &
             caar_run_rk5_dss, caar_set_partition, caar_dss_pack, caar_dss_unpack, caar_neighbor_minmax_pack, &
-            caar_neighbor_minmax_unpack, caar_halo_segments, caar_rk5_stage, caar_dss_interior, caar_dss_boundary
+            caar_neighbor_minmax_unpack, caar_halo_segments, caar_rk5_stage, caar_dss_interior, caar_dss_boundary, &
+            caar_vertical_remap
 
   interface
     ! int caar_create(caar_handle* out, const caar_dims* dims, int device);
@@ -211,6 +212,14 @@ module caar_b200
       import :: c_ptr, c_int
       type(c_ptr), value :: handle
       integer(c_int), value :: nets, nete, qtl, qsize, dp_tl
+      integer(c_int) :: rc
+    end function
+    ! HOMME's vertical_remap for rsplit > 0 (remap_Q_ppm, vert_remap_q_alg = 1) of T, v at tl and Qdp(qtl) of tracers
+    ! iq < qsize from dp3d(tl) to the hybrid reference levels, then dp3d(tl) = dp; tl and qtl are zero-based
+    function caar_vertical_remap(handle, nets, nete, tl, qtl, qsize) bind(C, name="caar_vertical_remap") result(rc)
+      import :: c_ptr, c_int
+      type(c_ptr), value :: handle
+      integer(c_int), value :: nets, nete, tl, qtl, qsize
       integer(c_int) :: rc
     end function
     function caar_bounds_upload(handle, host) bind(C, name="caar_bounds_upload") result(rc)

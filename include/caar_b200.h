@@ -153,7 +153,8 @@ int caar_device_count(void);
 int caar_create(caar_handle* out, const caar_dims* dims, int device);
 int caar_destroy(caar_handle h);
 
-/* Constants + Derivative + HVCoord of TestData (PO/data_structures.cpp:117-163). hyai has nlev+1 entries. */
+/* Constants + Derivative + HVCoord of TestData (PO/data_structures.cpp:117-163). hyai has nlev+1 entries. caar_run*
+   read only hyai[0]; the whole hyai is kept on the device for caar_vertical_remap. Synchronous. */
 int caar_set_params(caar_handle h, const caar_constants* c, const double dvv[16], double ps0,
                     const double* hyai);
 
@@ -163,7 +164,9 @@ int caar_set_params(caar_handle h, const caar_constants* c, const double dvv[16]
    running sum of div(v dp) and hybi, vertical advection of T and v (preq_vertadv), the dp3d update with the
    vertical flux difference, and derived_eta_dot_dpdn accumulates the real flux:
    F/routine_extracted.F90:227-262,270-277,325-334,515-517; LV/CaarFunctor.hpp:504-547. hybi has nlev+1 entries
-   (F hvcoord%hybi; ignored when rsplit > 0). The reference holds no runnable implementation of this branch:
+   (F hvcoord%hybi). A given hybi is kept on the device whatever rsplit is (a NULL hybi with rsplit > 0 keeps the one
+   given before): caar_vertical_remap reads it, while caar_run* read hybi only when rsplit == 0, so with rsplit > 0 their
+   results do not depend on it. The reference holds no runnable implementation of the Eulerian branch:
    parity is against the tests' own CPU restatement of these formulas only ("parity unpinned", DESIGN.md §3). */
 int caar_set_vertical_coordinate(caar_handle h, int rsplit, const double* hybi);
 
@@ -270,7 +273,7 @@ int caar_sync(caar_handle h);
    selected), caar_dss_pack / caar_dss_unpack and caar_neighbor_minmax_pack / caar_neighbor_minmax_unpack: 1 per call
    (none when nothing is selected, and none for a pack of a part that shares no point), caar_dss_interior /
    caar_dss_boundary: at most 1 per call (none when nothing is selected or the part has no interior / boundary group),
-   caar_euler_step, caar_norms,
+   caar_vertical_remap: 2 per call (none for an empty range), caar_euler_step, caar_norms,
    ...) */
 long long caar_launch_count(caar_handle h);
 /* CUDA-event stopwatch on the stream the kernels are launched on: start records an event, stop records a
@@ -374,6 +377,63 @@ int caar_bounds_upload(caar_handle h, const double* host);
 int caar_bounds_download(caar_handle h, double* host);
 int caar_tracer_bounds(caar_handle h, int nets, int nete, int qtl, int qsize, int dp_tl);
 int caar_limit_tracers(caar_handle h, int nets, int nete, int qtl, int qsize, int dp_tl);
+
+/* ---- the vertical remap: HOMME's vertical_remap for rsplit > 0 ----
+   On the vertically Lagrangian coordinate (rsplit > 0) every step moves mass between the layers of dp3d; HOMME brings
+   the columns back to the hybrid reference levels every rsplit steps, after prim_step. caar_vertical_remap is that call
+   with remap1 = remap_Q_ppm and vert_remap_q_alg = 1 (PPM with mirrored ghost cells), on the columns (e, p) of the
+   elements [nets, nete), asynchronously on the handle's stream. Per column:
+     dp_star = dp3d(tl);  ps = hyai[0]*ps0 + S, S the sequential sum of dp_star over k
+     dp[k] = (hyai[k+1]-hyai[k])*ps0 + (hybi[k+1]-hybi[k])*ps         (hyai of caar_set_params, hybi of
+                                                                       caar_set_vertical_coordinate)
+     T(tl) is remapped as T*dp_star and divided by dp; so is each component of v(tl); Qdp(qtl) of the tracers
+     iq < qsize is remapped as mass; finally dp3d(tl) = dp.
+   Nothing else changes: the other time levels, the other Qdp level, the tracers iq >= qsize, the elements outside the
+   range and every derived field. There is no mode: every operation is rounded separately (no FMA contraction, IEEE
+   divisions, sums sequential in k), so the results are bit-reproducible and equal tests/remap_oracle.py bit for bit.
+
+   The restatement, in HOMME's 1-based indices (C level k-1 is Fortran level k). Ghost cells gs = 2 are mirrored:
+   x(1-i) = x(i) and x(nlev+i) = x(nlev+1-i) for i = 1, 2. Integer powers are products: x**2 = x*x, x**3 = (x*x)*x.
+   Expressions evaluate left to right as written. Per column:
+     pio(1)=0; pin(1)=0; for k=1..nlev: pio(k+1)=pio(k)+dpo(k); pin(k+1)=pin(k)+dpn(k)     (dpo=dp_star, dpn=dp)
+     pio(nlev+2)=pio(nlev+1)+1;  pin(nlev+1)=pio(nlev+1);  mirror dpo into -1..nlev+2
+     for k=1..nlev: kk=k; while pio(kk) <= pin(k+1) { kk=kk+1; if kk==nlev+2 break }; kk=kk-1; if kk==nlev+1 kk=nlev
+                    kid(k)=kk;  z2(k) = (pin(k+1) - (pio(kk)+pio(kk+1))*0.5) / dpo(kk)          (z1 = -0.5)
+     grid, with dx = dpo:
+       j=0..nlev+1: r1=dx(j)/((dx(j-1)+dx(j))+dx(j+1));  r2=(2*dx(j-1)+dx(j))/(dx(j+1)+dx(j));
+                    r3=(dx(j)+2*dx(j+1))/(dx(j-1)+dx(j))
+       j=0..nlev:   r4=dx(j)/(dx(j)+dx(j+1));  r5=1/(((dx(j-1)+dx(j))+dx(j+1))+dx(j+2));
+                    r6=((2*dx(j+1))*dx(j))/(dx(j)+dx(j+1));  r7=(dx(j-1)+dx(j))/(2*dx(j)+dx(j+1));
+                    r8=(dx(j+2)+dx(j+1))/(2*dx(j+1)+dx(j));  r9=(dx(j)*(dx(j-1)+dx(j)))/(2*dx(j)+dx(j+1));
+                    r10=(dx(j+1)*(dx(j+1)+dx(j+2)))/(dx(j)+2*dx(j+1))
+     per field f (the values to remap: T*dp_star, v_c*dp_star, or Qdp):
+       masso(1)=0; k=1..nlev: masso(k+1)=masso(k)+f(k); a(k)=f(k)/dpo(k);   mirror a into -1..nlev+2
+       j=0..nlev+1: da = r1*(r2*(a(j+1)-a(j)) + r3*(a(j)-a(j-1)))
+                    dma(j) = min(|da|, 2*|a(j)-a(j-1)|, 2*|a(j+1)-a(j)|) * copysign(1, da)
+                    if ((a(j+1)-a(j))*(a(j)-a(j-1)) <= 0) dma(j) = 0
+       j=0..nlev:   ai(j) = (a(j) + r4*(a(j+1)-a(j))) + r5*(((r6*(r7-r8))*(a(j+1)-a(j)) - r9*dma(j+1)) + r10*dma(j))
+       j=1..nlev:   al=ai(j-1); ar=ai(j)
+                    if ((ar-a(j))*(a(j)-al) <= 0) { al=a(j); ar=a(j) }
+                    if ((ar-al)*(a(j)-(al+ar)/2) >  (ar-al)**2/6) al = 3*a(j) - 2*ar
+                    if ((ar-al)*(a(j)-(al+ar)/2) < -(ar-al)**2/6) ar = 3*a(j) - 2*al
+                    c0(j) = 1.5*a(j) - (al+ar)/4;  c1(j) = ar-al;  c2(j) = -6*a(j) + 3*(al+ar)
+       massn1=0; k=1..nlev: kk=kid(k); x2=z2(k); x1=-0.5
+                    massn2 = masso(kk) + ((c0*(x2-x1) + (c1*(x2**2-x1**2))/2) + (c2*(x2**3-x1**3))/3)(kk) * dpo(kk)
+                    f(k) = massn2 - massn1;  massn1 = massn2
+   The result is T = f/dp, v_c = f/dp and Qdp = f. The search never returns a cell above k-1, so a new interface more
+   than one cell above its old position falls into HOMME's extrapolated parabola of cell k-1; the result still
+   conserves mass. The contract covers dp_star > 0 and dp > 0 (HOMME aborts on a negative thickness); outside it the
+   call only keeps every index in bounds, with kid clamped to [1, nlev].
+
+   Errors: CAAR_ERR_STATE before caar_set_params or when no hybi was ever given; CAAR_ERR_UNSUPPORTED on a handle with
+   rsplit == 0; CAAR_ERR_INVALID for a null handle, a bad element range, tl outside [0, ntl), qtl not 0 or 1 or qsize
+   outside [0, qsize_d]. A rejected call launches nothing and changes nothing. 2 launches, none for an empty range.
+
+   One remap interval of HOMME's rsplit > 0 time loop, on a handle that holds the whole mesh (E elements):
+     rsplit times: caar_run_rk5_dss(h, &ctl, dt, 1, mode), then the limited tracer step above (with the new qn0)
+     caar_vertical_remap(h, 0, E, ctl.n0, qn0, qsize)     ctl.n0: after the rotation, the level the last step wrote
+   The remap is column-local (no connectivity, no DSS, no exchange), so partitioned handles run it unchanged. */
+int caar_vertical_remap(caar_handle h, int nets, int nete, int tl, int qtl, int qsize);
 
 /* ---- the direct stiffness summation (DSS) over shared element-boundary points ----
    HOMME's compute_and_apply_rhs stores spheremp*(state + dt*rhs) and then assembles the values at the GLL points that two

@@ -47,6 +47,7 @@ EXPORTED_SYMBOLS = (
     "caar_tracer_bounds", "caar_limit_tracers", "caar_set_connectivity", "caar_dss", "caar_neighbor_minmax",
     "caar_run_rk5_dss", "caar_set_partition", "caar_dss_pack", "caar_dss_unpack", "caar_neighbor_minmax_pack",
     "caar_neighbor_minmax_unpack", "caar_halo_segments", "caar_rk5_stage", "caar_dss_interior", "caar_dss_boundary",
+    "caar_vertical_remap",
 )
 CHECKSUM_FIELDS = ("elem_state_dp3d", "elem_state_v", "elem_state_T", "elem_derived_eta_dot_dpdn",
                    "elem_derived_omega_p", "elem_derived_phi", "elem_derived_vn0")
@@ -148,6 +149,7 @@ def load_library():
     lib.caar_bounds_download.argtypes = [C.c_void_p, C.POINTER(C.c_double)]
     lib.caar_tracer_bounds.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]
     lib.caar_limit_tracers.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]
+    lib.caar_vertical_remap.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]
     lib.caar_set_connectivity.argtypes = [C.c_void_p, C.POINTER(C.c_longlong), C.c_int]
     lib.caar_dss.argtypes = [C.c_void_p, C.c_uint, C.c_int, C.c_int, C.c_int, C.c_int]
     lib.caar_neighbor_minmax.argtypes = [C.c_void_p, C.c_int]
@@ -449,6 +451,19 @@ class Caar:
         nete = self.control.nete if nete is None else nete
         _check(self.lib, self.lib.caar_limit_tracers(self.h, nets, nete, int(qtl), int(qsize), int(dp_tl)),
                "caar_limit_tracers")
+        if sync:
+            self.sync()
+
+    # -- the vertical remap (rsplit > 0) -----------------------------------------------------------------------------
+    def vertical_remap(self, tl=None, qtl=0, qsize=0, nets=None, nete=None, sync=True):
+        """caar_vertical_remap: HOMME's PPM remap of T, v at time level tl (default control.np1) and Qdp(qtl) of tracers
+        iq < qsize from dp3d(tl) to the reference levels of hyai (set_params) and hybi (set_vertical_coordinate), then
+        dp3d(tl) = dp."""
+        tl = self.control.np1 if tl is None else tl
+        nets = self.control.nets if nets is None else nets
+        nete = self.control.nete if nete is None else nete
+        _check(self.lib, self.lib.caar_vertical_remap(self.h, int(nets), int(nete), int(tl), int(qtl), int(qsize)),
+               "caar_vertical_remap")
         if sync:
             self.sync()
 

@@ -58,7 +58,8 @@ struct caar_handle_s {
   bool params_set;
   caar_constants c;
   double dvv[16], ps0, hyai0;
-  double* partial;    // [nelem][16] device: norms use [nelem][3], checksums [nelem][8][2]
+  double* hyai_dev;  // [nlev+1], the whole hyai of caar_set_params (caar_vertical_remap)
+  double* partial;    // [nelem][16] device: norms use [nelem][3], checksums [nelem][8][2], caar_vertical_remap ps [nelem][16]
   unsigned long long* bits;  // [nelem][7] device (checksums)
   double* out3;       // [16 doubles + 7 u64] device: results of the norm / checksum reductions
   double* out3_host;  // the same, pinned
@@ -72,7 +73,7 @@ struct caar_handle_s {
   cudaEvent_t ev_fence;
   // caar_run_host zero-copy path: TMA descriptors over the caller's mapped host arrays, rebuilt when they move
   int rsplit;        // > 0 vertically Lagrangian (default 1), 0 Eulerian
-  double* hybi_dev;  // [nlev+1], Eulerian branch only
+  double* hybi_dev;  // [nlev+1]: the Eulerian branch of caar_run* and caar_vertical_remap
   double* extra[5];  // arrays beyond struct Arrays: vstar, qtens, tensorVisc, scalar in / out (allocated on first use)
   double* bounds;  // [nelem][qsize_d][nlev][2] tracer limiter bounds (allocated and zeroed on first use)
   double* bounds_next;  // the same shape: caar_neighbor_minmax writes it, then it and `bounds` swap
@@ -348,6 +349,7 @@ int caar_destroy(caar_handle h) {
   for (int x = 0; x < CAAR_NUM_EXTRA; ++x)
     if (h->extra[x]) cudaFree(h->extra[x]);
   if (h->hybi_dev) cudaFree(h->hybi_dev);
+  if (h->hyai_dev) cudaFree(h->hyai_dev);
   if (h->out3_host) cudaFreeHost(h->out3_host);
   if (h->lapflat_sched) cudaFree(h->lapflat_sched);
   if (h->ev0) cudaEventDestroy(h->ev0);
@@ -366,6 +368,13 @@ int caar_destroy(caar_handle h) {
 
 int caar_set_params(caar_handle h, const caar_constants* c, const double dvv[16], double ps0, const double* hyai) {
   if (!h || !c || !dvv || !hyai) return fail(CAAR_ERR_INVALID, "null argument");
+  {
+    DeviceGuard guard(h->device);
+    const size_t bytes = (size_t)(h->dims.nlev + 1) * sizeof(double);
+    if (!h->hyai_dev) CU_TRY(cudaMalloc(&h->hyai_dev, bytes));
+    CU_TRY(cudaMemcpyAsync(h->hyai_dev, hyai, bytes, cudaMemcpyHostToDevice, h->stream));
+    CU_TRY(cudaStreamSynchronize(h->stream));
+  }
   h->c = *c;
   std::memcpy(h->dvv, dvv, sizeof h->dvv);
   h->ps0 = ps0;
@@ -377,8 +386,8 @@ int caar_set_params(caar_handle h, const caar_constants* c, const double dvv[16]
 int caar_set_vertical_coordinate(caar_handle h, int rsplit, const double* hybi) {
   if (!h) return fail(CAAR_ERR_INVALID, "null handle");
   if (rsplit < 0) return fail(CAAR_ERR_INVALID, "rsplit=%d", rsplit);
-  if (rsplit == 0) {
-    if (!hybi) return fail(CAAR_ERR_INVALID, "rsplit=0 (Eulerian) needs hybi[nlev+1]");
+  if (rsplit == 0 && !hybi) return fail(CAAR_ERR_INVALID, "rsplit=0 (Eulerian) needs hybi[nlev+1]");
+  if (hybi) {  // kept for any rsplit: caar_vertical_remap reads it; caar_run* read it only when rsplit == 0
     DeviceGuard guard(h->device);
     const size_t bytes = (size_t)(h->dims.nlev + 1) * sizeof(double);
     if (!h->hybi_dev) CU_TRY(cudaMalloc(&h->hybi_dev, bytes));
@@ -1308,6 +1317,22 @@ int caar_sync(caar_handle h) {
   if (!h) return fail(CAAR_ERR_INVALID, "null handle");
   DeviceGuard guard(h->device);
   CU_TRY(cudaStreamSynchronize(h->stream));
+  return CAAR_OK;
+}
+
+int caar_vertical_remap(caar_handle h, int nets, int nete, int tl, int qtl, int qsize) {
+  if (int rc = check_handle(h, "caar_vertical_remap")) return rc;
+  if (!h->hybi_dev) return fail(CAAR_ERR_STATE, "caar_vertical_remap needs hybi (caar_set_vertical_coordinate)");
+  if (h->rsplit == 0) return fail(CAAR_ERR_UNSUPPORTED, "caar_vertical_remap: rsplit=0 (Eulerian) has no remap");
+  if (int rc = check_range(h, nets, nete)) return rc;
+  if (int rc = check_time_level(h, tl)) return rc;
+  if (int rc = check_qtl(qtl)) return rc;
+  if (int rc = check_qsize(h, qsize)) return rc;
+  if (nete == nets) return CAAR_OK;
+  DeviceGuard guard(h->device);
+  CU_TRY(caar::launch_vertical_remap(make_args(h, nullptr), h->hyai_dev, h->partial, nets, nete, tl, qtl, qsize,
+                                     h->stream));
+  h->launches += 2;
   return CAAR_OK;
 }
 

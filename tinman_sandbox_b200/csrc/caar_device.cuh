@@ -141,6 +141,11 @@ cudaError_t launch_tracer_bounds(const KernelArgs& a, int nets, int nete, int qt
                                  cudaStream_t s);
 cudaError_t launch_limit_tracers(const KernelArgs& a, int nets, int nete, int qtl, int qsize, int dp_tl, double* bounds,
                                  cudaStream_t s);
+// vertical remap (caar_remap.cu) of T, v at time level tl and Qdp(qtl) of tracers < qsize on [nets,nete) from dp3d(tl)
+// to the reference levels of hyai [nlev+1] (device) and a.hybi, then dp3d(tl) = dp; ps [nelem][16] is scratch. Two
+// launches, none for an empty range.
+cudaError_t launch_vertical_remap(const KernelArgs& a, const double* hyai, double* ps, int nets, int nete, int tl,
+                                  int qtl, int qsize, cudaStream_t s);
 // DSS and neighbour bounds (caar_dss.cu) over the connectivity of caar_set_connectivity. The groups of copies of one
 // global id, in the order of their owners (first copies in (e, p) order): group g is copy[start[g] .. start[g+1]), each
 // copy e*16 + p in (e, p) order. nb[nb_start[e] .. nb_start[e+1]) are the other elements that share a point with e,
